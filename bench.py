@@ -4,7 +4,7 @@
 Metric (BASELINE.json): env steps/s (movegen + step + terminal/reward, random policy) -- and DQN TD
 updates/s as the `dqn` object -- at 1/2/4/8 B200, next to the reference CPU path on the host cores.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--plies P]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--plies P] [--dump-outputs DIR]
   torchrun ... bench.py --gpus N ...          (one rank per GPU, env shards, no data-path collective)
   python bench.py --impl reference ...        (the reference's own ChessBoard path on the host cores)
 
@@ -13,6 +13,8 @@ this GPU (default 4096 = BASELINE configs[1]).  Scaling is weak: E envs per GPU.
 Timing: W warm-up steps, then exactly K steps, each bracketed by CUDA events on the launching stream
 (the library is pointed at torch's current stream), L2 flushed between steps outside the timed
 intervals; barrier + synchronize on both sides; max over ranks.
+--dump-outputs DIR writes what the timed steps hand their caller (see dump_outputs) as .npy files, so that two
+builds can be compared output for output: the seeds are fixed, so the same arguments give the same inputs.
 """
 import argparse
 import json
@@ -26,6 +28,24 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 ALGO_BYTES_PER_STEP = 136   # read 64 B record + write 64 B record + 8 B outputs (SURVEY 8d, DESIGN.md)
+DUMP_MAX_ENVS = 65536       # 416 B of dumped arrays per env: at most 27 MB
+
+
+def dump_outputs(out_dir, boards, stats):
+    """The boards after the last timed step (the 90 square codes and every other field of the record; a fixed, seeded sample of
+    DUMP_MAX_ENVS envs when there are more, their indices in env_index) and the statistics of the timed steps, as float arrays."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.arange(len(boards))
+    if len(idx) > DUMP_MAX_ENVS:
+        idx = np.sort(np.random.default_rng(0).choice(len(idx), DUMP_MAX_ENVS, replace=False))
+    b = boards[idx]
+    s = np.arange(90)
+    out = {"env_index": idx.astype(np.float64), "board_squares": ((b["sq"][:, s >> 3] >> (4 * (s & 7))) & 15).astype(np.float32)}
+    out.update({"board_" + f: b[f].astype(np.float64) for f in boards.dtype.names if f != "sq"})
+    out.update({"stats_" + f: np.array([stats[f]], np.float64) for f in stats.dtype.names})
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -211,7 +231,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-aux", action="store_true")
     ap.add_argument("--no-dqn", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the boards and statistics of the timed steps to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     # stdout carries exactly ONE JSON line: libraries that write to fd 1 on their own (NCCL prints "NCCL version ..." there) are sent to
     # stderr for the whole run, and the line goes to the saved descriptor at the end
     global _REAL_STDOUT
@@ -273,6 +296,8 @@ def main():
     ms = sum(a.elapsed_time(b) for a, b in evs)
     st = env.stats(reset=True)
     assert int(st["steps"]) == E * P * args.steps, "stats mismatch: kernel did not apply every ply"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env.get_boards(), st)
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -2,8 +2,8 @@
 
 * ``oracle()``  -> oracle/_build/libxq_oracle.so, the plain-C restatement (oracle/xq_oracle.c)
 * ``ref()``     -> oracle/_ref/libxq_ref.so, the reference's own sources compiled unmodified
-                   (None when it has not been built; it cannot be rebuilt on the GPU box because
-                   /root/reference does not exist there, the prebuilt file travels instead)
+                   (None when it has not been built and XQ_REFERENCE_SRC names no checkout of the
+                   reference project to build it from; the tests that need it skip then)
 """
 import ctypes as C
 import os
@@ -12,7 +12,7 @@ import subprocess
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_SRC = "/root/reference"
+REF_SRC = os.environ.get("XQ_REFERENCE_SRC", "")
 
 ENV_DTYPE = np.dtype([("sq", "<u4", (12,)), ("move_count", "<u2"), ("player", "u1"), ("flags", "u1"),
                       ("red_score", "<i4"), ("black_score", "<i4"), ("ctr", "<u4")])
@@ -23,16 +23,16 @@ assert ENV_DTYPE.itemsize == 64 and TRACE_DTYPE.itemsize == 8 and STATS_DTYPE.it
 
 
 def build(force=False):
-    """Compile the C restatement, and the verbatim reference when /root/reference is present."""
+    """Compile the C restatement, and the verbatim reference when XQ_REFERENCE_SRC names a checkout of it."""
     targets = ["oracle"]
     if os.path.isdir(REF_SRC):
-        targets.append("ref")
+        targets += ["ref", "REF=" + os.path.abspath(REF_SRC)]
     args = ["make", "-C", HERE] + (["-B"] if force else []) + targets
     subprocess.run(args, check=True, stdout=subprocess.DEVNULL)
     if os.path.isdir(REF_SRC) and os.path.exists("/usr/local/cuda/bin/nvcc"):
-        # the reference's own CUDA network (src/dqn.cu unmodified, sm_100a): golden generation on a GPU box and bench.py's reference_train leg;
+        # the reference's own CUDA network (src/dqn.cu unmodified, sm_100a): golden generation on a B200 and bench.py's reference_train leg;
         # optional -- without it that leg times the CPU definition of the network
-        subprocess.run(["make", "-C", HERE] + (["-B"] if force else []) + ["refcuda"], check=False, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        subprocess.run(["make", "-C", HERE] + (["-B"] if force else []) + ["refcuda", "REF=" + os.path.abspath(REF_SRC)], check=False, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
 
 
 _P = C.c_void_p

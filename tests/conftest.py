@@ -29,13 +29,28 @@ def oracle_lib(O):
 def ref_lib(O):
     R = O.ref()
     if R is None:
-        pytest.skip("oracle/_ref/libxq_ref.so not built (no /root/reference here)")
+        pytest.skip("oracle/_ref/libxq_ref.so not built (set XQ_REFERENCE_SRC to a checkout of the reference project)")
     return R
 
 
 @pytest.fixture(scope="session")
 def golden():
     return np.load(os.path.join(ROOT, "tests", "golden", "rules_ref.npz"))
+
+
+@pytest.fixture(scope="session")
+def make_golden():
+    """tests/golden/make_golden.py as a module: the inputs, loops and checks the stored reference answers were made with"""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("make_golden", os.path.join(ROOT, "tests", "golden", "make_golden.py"))
+    mg = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mg)
+    return mg
+
+
+@pytest.fixture(scope="session")
+def answers():
+    return np.load(os.path.join(ROOT, "tests", "golden", "reference_answers.npz"))
 
 
 @pytest.fixture(scope="session")

@@ -48,17 +48,13 @@ def test_cpp_adapter_transcript(tmp_path, O):
 
 
 @pytest.mark.parametrize("mode", ["trainparity", "selfplayparity"])
-def test_cpp_chessai_train_equals_the_reference_chessai_train(tmp_path, O, mode):
+def test_cpp_chessai_train_equals_the_reference_chessai_train(tmp_path, O, make_golden, answers, mode):
     """The drop-in claim end to end: `ChessAI::train(2)` / `ChessAI::startSelfPlay(2)` (src/chessai.cpp:191-266) of the C++ adapter (every device operation through the C ABI: legal lists, selectAction,
-    movePiece, state, FP64 forward / TD step as written, target sync) against the reference's OWN `ChessAI::train(2)` (oracle/_ref, unmodified
-    sources) started from the same model file and fed the same rand() stream: same gameCompleted events, final weights equal to 1e-10."""
-    R = O.ref()
-    if R is None:
-        pytest.skip("oracle/_ref/libxq_ref.so not built")
+    movePiece, state, FP64 forward / TD step as written, target sync) against the reference's OWN `ChessAI::train(2)` (unmodified
+    sources) started from the same model file and fed the same rand() stream: same gameCompleted events, final weights equal to 1e-10.
+    The reference's result is stored in tests/golden/reference_answers.npz; with oracle/_ref built it is also run live."""
     import cn_chess_ai_b200 as xq
-    rng = np.random.default_rng(77)
-    w = rng.uniform(-0.05, 0.05, 1260 * 128 + 128 * 8100)
-    b = rng.uniform(-0.05, 0.05, 128 + 8100)
+    w, b, stream = make_golden.adapter_inputs()
     net = xq.DQN([1260, 128, 8100])
     net.set_params(w, b)
     net.save_model(tmp_path / "in.bin")
@@ -70,16 +66,14 @@ def test_cpp_chessai_train_equals_the_reference_chessai_train(tmp_path, O, mode)
     net.load_model(tmp_path / "out.bin")
     w_gpu, b_gpu = net.get_params()
     net.close()
-    # the adapter's DQN::selectAction draws (coin31, idx31) from xq_rng(0xD09A, 0, call); the reference consumes rand() once, and once more when exploring
-    n = 600
-    x = O.rng_np(0xD09A, np.zeros(n, np.uint64), np.arange(n, dtype=np.uint32))
-    stream = []
-    for v in x:
-        coin, idx = int(v) & 0x7FFFFFFF, int(v) >> 33
-        stream.append(coin)
-        if coin / 2147483647.0 < 0.1:
-            stream.append(idx)
-    stream = np.array(stream, np.int32)
+    key = "adapter_train" if mode == "trainparity" else "adapter_selfplay"
+    assert ev_gpu == list(answers[key + "_events"]) and len(ev_gpu) == 6
+    assert int(answers[key + "_consumed"]) <= len(stream)
+    make_golden.check_loop(answers, key, w, b, stream, w_gpu, b_gpu, 1e-10)
+    assert np.abs(w_gpu - w).max() > 1e-6
+    R = O.ref()
+    if R is None:
+        return
     h = C.c_void_p(R.ref_env_new())
     R.ref_rand_load(stream, len(stream))
     w_ref, b_ref = np.zeros_like(w), np.zeros_like(b)
@@ -97,4 +91,3 @@ def test_cpp_chessai_train_equals_the_reference_chessai_train(tmp_path, O, mode)
     R.ref_env_free(h)
     assert ev_gpu == list(ev_ref) and len(ev_gpu) == 6
     assert np.abs(w_gpu - w_ref).max() < 1e-10 and np.abs(b_gpu - b_ref).max() < 1e-10
-    assert np.abs(w_gpu - w).max() > 1e-6

@@ -2,6 +2,8 @@
 
 * against tests/golden/rules_ref.npz, generated from the reference's own sources compiled
   unmodified (tests/golden/make_golden.py) -- runs anywhere, also on the GPU box;
+* against tests/golden/reference_answers.npz, the reference's answers where it was once compared live (see
+  make_golden.answers);
 * live, in lock step, against oracle/_ref/libxq_ref.so when that library is present.
 """
 import ctypes as C
@@ -109,8 +111,16 @@ def test_eps_threshold(oracle_lib):
                 assert ((c / 2147483647.0) < eps) == (c < t)
 
 
-def test_lockstep_vs_reference(O, oracle_lib, ref_lib):
-    """oracle and the unmodified reference classes play the same random games move by move"""
+def test_lockstep_vs_reference(O, oracle_lib, make_golden, answers):
+    """oracle and the unmodified reference classes play the same random games move by move: against the reference's answers
+    stored in tests/golden/reference_answers.npz, and live against oracle/_ref when it is built"""
+    got = make_golden.lockstep_answers(oracle_lib)
+    for k, v in got.items():
+        assert np.array_equal(v, answers["lockstep_" + k]), k
+    assert int(got["over"].sum()) >= 20
+    ref_lib = O.ref()
+    if ref_lib is None:
+        return
     h = C.c_void_p(ref_lib.ref_env_new())
     rng = np.random.default_rng(0)
     e = O.new_envs(1)
@@ -153,8 +163,15 @@ def test_lockstep_vs_reference(O, oracle_lib, ref_lib):
     assert games >= 20
 
 
-def test_arbitrary_boards_vs_reference(O, oracle_lib, ref_lib):
-    """unreachable positions: generator lists and the stand-alone predicate (SURVEY A.3 caveat)"""
+def test_arbitrary_boards_vs_reference(O, oracle_lib, make_golden, answers):
+    """unreachable positions: generator lists and the stand-alone predicate (SURVEY A.3 caveat); against the reference's answers
+    stored in tests/golden/reference_answers.npz, and live against oracle/_ref when it is built"""
+    got = make_golden.arbitrary_answers(oracle_lib)
+    for k, v in got.items():
+        assert np.array_equal(v, answers["arbitrary_" + k]), k
+    ref_lib = O.ref()
+    if ref_lib is None:
+        return
     h = C.c_void_p(ref_lib.ref_env_new())
     rng = np.random.default_rng(9)
     buf = np.zeros(512, np.int32)
@@ -180,8 +197,15 @@ def test_arbitrary_boards_vs_reference(O, oracle_lib, ref_lib):
     ref_lib.ref_env_free(h)
 
 
-def test_rollout_vs_reference_driver(O, oracle_lib, ref_lib):
-    """whole trajectories: same draws => identical traces for 1500 plies (auto-reset included)"""
+def test_rollout_vs_reference_driver(O, oracle_lib, make_golden, answers):
+    """whole trajectories: same draws => identical traces for 1500 plies (auto-reset included); against the reference's trace
+    stored in tests/golden/reference_answers.npz, and live against oracle/_ref when it is built"""
+    got = make_golden.rollout_answers(oracle_lib)
+    for k, v in got.items():
+        assert np.array_equal(v, answers["rollout_" + k]), k
+    ref_lib = O.ref()
+    if ref_lib is None:
+        return
     seed, env_id, plies = 99, 5, 1500
     draws = (O.rng_draws(seed, env_id, 0, plies) >> np.uint64(33)).astype(np.uint32)
     h = C.c_void_p(ref_lib.ref_env_new())
@@ -200,17 +224,22 @@ def test_rollout_vs_reference_driver(O, oracle_lib, ref_lib):
 
 
 @pytest.mark.parametrize("self_play", [False, True])
-def test_train_loop_vs_reference(O, oracle_lib, ref_lib, self_play, tmp_path, monkeypatch):
+def test_train_loop_vs_reference(O, oracle_lib, make_golden, answers, self_play, tmp_path, monkeypatch):
     """SURVEY 8(a) rows a12-a18 end to end: the reference's OWN ChessAI::train / startSelfPlay (src/chessai.cpp:85-170, :191-266: selectAction with its rand()
     stream injected, movePiece, evaluateBoard, done one ply early, TD target from the ONLINE network over all 8100 outputs,
-    backpropagate as written, gameCompleted) against the same loop composed from the oracle's restatements.  Same events, same games,
-    final weights equal to rounding (the reference network here is oracle/nn_cpu.cpp's CPU definition of NeuralNetwork)."""
-    LA = np.array([1260, 128, 8100], np.int32)
-    rng = np.random.default_rng(5)
-    w = rng.uniform(-0.05, 0.05, 1260 * 128 + 128 * 8100)
-    b = rng.uniform(-0.05, 0.05, 128 + 8100)
-    draws = rng.integers(0, 2 ** 31 - 1, 2000, dtype=np.int64).astype(np.int32)
+    backpropagate as written, gameCompleted) against the same loop composed from the oracle's restatements (make_golden.oracle_train_loop).
+    Same events, same draws consumed, final weights equal to rounding: against the reference's result stored in
+    tests/golden/reference_answers.npz, and live against oracle/_ref when it is built (its network is oracle/nn_cpu.cpp's CPU definition)."""
+    w, b, draws = make_golden.train_loop_inputs()
     episodes = 2
+    events, pos, plies, w2, b2 = make_golden.oracle_train_loop(oracle_lib, w, b, draws, episodes, self_play)
+    key = "selfplay" if self_play else "train"
+    assert plies > 20 and events == list(answers[key + "_events"]) and pos == int(answers[key + "_consumed"])
+    make_golden.check_loop(answers, key, w, b, draws, w2, b2, 1e-12)
+    assert np.abs(w2 - w).max() > 1e-6                                        # the weights did move
+    ref_lib = O.ref()
+    if ref_lib is None:
+        return
     h = C.c_void_p(ref_lib.ref_env_new())
     ref_lib.ref_rand_load(draws, len(draws))
     w_ref, b_ref = np.zeros_like(w), np.zeros_like(b)
@@ -222,47 +251,9 @@ def test_train_loop_vs_reference(O, oracle_lib, ref_lib, self_play, tmp_path, mo
     ref_lib.ref_events_get(ev_ref)
     consumed = ref_lib.ref_rand_consumed()
     ref_lib.ref_env_free(h)
-
-    w2, b2 = w.copy(), b.copy()
-    pos, events, plies = 0, [], 0
-    acts = np.zeros(128, np.uint16)
-    state, nxt, q, qs, qn, tgt = np.zeros(1260), np.zeros(1260), np.zeros(8100), np.zeros(8100), np.zeros(8100), np.zeros(8100)
-    for ep in range(episodes):
-        e = O.new_envs(1)
-        player, move_count = 0, 0                                             # chessai.cpp:90-94
-        oracle_lib.xqo_state(e.ctypes.data, state)
-        while not oracle_lib.xqo_game_over(e.ctypes.data) and (self_play or move_count < 200):
-            if self_play:
-                player = int(e[0]["player"])                                  # :198 board->getCurrentPlayer()
-            n = oracle_lib.xqo_all_actions(e.ctypes.data, player, acts)
-            if n == 0:
-                break
-            coin = int(draws[pos]); pos += 1
-            idx = 0
-            if coin / 2147483647.0 < 0.1:                                     # dqn.cpp:30-33: the second rand() only when exploring
-                idx = int(draws[pos]); pos += 1
-            else:
-                oracle_lib.xqo_nn_forward(LA, 3, w2, b2, state, q)
-            a = int(acts[oracle_lib.xqo_select_action(q, acts, n, coin, idx, 0.1)])
-            f, t = a >> 7, a & 127
-            oracle_lib.xqo_move(e.ctypes.data, f // 9, f % 9, t // 9, t % 9)
-            move_count = int(e[0]["move_count"])
-            reward = oracle_lib.xqo_evaluate(e.ctypes.data, player, move_count)
-            oracle_lib.xqo_state(e.ctypes.data, nxt)
-            done = bool(oracle_lib.xqo_game_over(e.ctypes.data)) or (not self_play and move_count + 1 >= 200)      # :119 vs :227
-            oracle_lib.xqo_nn_forward(LA, 3, w2, b2, state, qs)
-            if not done:
-                oracle_lib.xqo_nn_forward(LA, 3, w2, b2, nxt, qn)
-            oracle_lib.xqo_td_target(qs, qn, 8100, t, float(reward), int(done), 0.99, tgt)
-            oracle_lib.xqo_nn_backprop(LA, 3, w2, b2, state, tgt, 0.001, 0)
-            state[:] = nxt
-            player ^= 1
-            plies += 1
-        events += [ep + 1, int(e[0]["red_score"]), int(e[0]["black_score"])]
-    assert pos == consumed and plies > 20
+    assert pos == consumed
     assert list(ev_ref) == events
     assert np.abs(w2 - w_ref).max() < 1e-12 and np.abs(b2 - b_ref).max() < 1e-12
-    assert np.abs(w2 - w).max() > 1e-6                                        # the weights did move
 
 
 def test_reference_train_bench_leg(ref_lib):

@@ -56,10 +56,17 @@ def test_known_answers(O, oracle_lib):
     assert _oracle(oracle_lib, rec)[0][0] == 44
 
 
-def test_oracle_equals_reference_composition(O, oracle_lib, ref_lib):
-    """the pin: xqo_all_actions_strict == the reference's own getAllValidActions / movePiece / getPieceAt composed the same way"""
-    recs = np.concatenate([harvest_positions(O, 40, 5, 31, seed=2), random_boards(O, 150, seed=5, max_pieces=24)])
+def test_oracle_equals_reference_composition(O, oracle_lib, make_golden, answers):
+    """the pin: xqo_all_actions_strict == the reference's own getAllValidActions / movePiece / getPieceAt composed the same way:
+    its lists stored in tests/golden/reference_answers.npz, and live against oracle/_ref when it is built"""
+    recs = make_golden.strict_positions()
     c1, a1 = _oracle(oracle_lib, recs)
+    c0, _ = _oracle(oracle_lib, recs, strict=False)
+    assert (c1 == answers["strict_counts"]).all() and (a1 == answers["strict_lists"]).all()
+    assert int(c0.sum()) - int(c1.sum()) == int(answers["strict_rejected"]) > 50          # the filter is exercised
+    ref_lib = O.ref()
+    if ref_lib is None:
+        return
     h = ref_lib.ref_env_new()
     buf = np.zeros(256, np.int32)
     rejected = 0
