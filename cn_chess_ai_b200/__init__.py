@@ -9,3 +9,11 @@ from .dqn import AS_WRITTEN, CORRECTED, DQN  # noqa: F401
 from .replay import ReplayBuffer, act, collect, td_update_replay, td_update_replay_n  # noqa: F401
 from .trainer import GAME_EVENT_DTYPE, drain_game_events, enable_game_events, train  # noqa: F401
 from .benchmarks import bench_dqn  # noqa: F401
+
+
+def __getattr__(name):
+    """TorchEnv (torch_env.py) is loaded on first use: importing the package does not import torch"""
+    if name == "TorchEnv":
+        from .torch_env import TorchEnv
+        return TorchEnv
+    raise AttributeError(f"module {__name__!r} has no attribute {name!r}")

@@ -20,6 +20,11 @@ TRANSITION_DTYPE = np.dtype([("s", "<u4", (12,)), ("s2", "<u4", (12,)), ("action
 assert TRANSITION_DTYPE.itemsize == 128
 MAX_ACTIONS = 128
 STATE_SIZE = 1260
+POLICY_ACTIONS = 8100     # policy index = from * 90 + to (include/xq.h: XQ_POLICY_ACTIONS)
+MASK_WORDS = 254          # uint32 words of a packed legal-action mask
+DTYPE_F32, DTYPE_BF16, DTYPE_U8 = 0, 1, 2
+VIEW_ABSOLUTE, VIEW_SIDE_TO_MOVE = 0, 1
+PICK_GREEDY, PICK_SAMPLE, PICK_GIVEN = 0, 1, 2
 
 
 class XQError(RuntimeError):
@@ -73,6 +78,9 @@ def lib():
     L.xq_env_step_device.argtypes = [_P, _P, C.c_int] + [C.POINTER(_P)] * 5
     L.xq_env_get_stats.argtypes = [_P, _P, C.c_int]
     L.xq_env_state_onehot.argtypes = [_P, _P]
+    L.xq_env_observe_device.argtypes = [_P, _P, C.c_int, C.c_int, _P]
+    L.xq_env_legal_mask_device.argtypes = [_P, _P, C.c_int, C.c_int]
+    L.xq_env_policy_step_device.argtypes = [_P, _P, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int] + [_P] * 7
     _lib = L
     return L
 

@@ -131,6 +131,21 @@ class BatchedEnv:
         check(self._L.xq_env_get_stats(self._h, ptr(stats), 1 if reset else 0))
         return stats[0]
 
+    # ---- device-resident interface for external policies: raw device pointers (ints), asynchronous on the handle's stream ----
+    def observe_device(self, planes_ptr, dtype, view, aux_ptr):
+        """xq_env_observe_device: planes [n][14][10][9] (dtype DTYPE_*), aux int32 [n][4]; either pointer may be None"""
+        check(self._L.xq_env_observe_device(self._h, planes_ptr, dtype, view, aux_ptr))
+
+    def legal_mask_device(self, mask_ptr, packed, view):
+        """xq_env_legal_mask_device: uint32 [n][254] (packed) or uint8 [n][8100]"""
+        check(self._L.xq_env_legal_mask_device(self._h, mask_ptr, 1 if packed else 0, view))
+
+    def policy_step_device(self, scores_ptr, scores_dtype, pick, temperature, view, auto_reset, actions_ptr, logp_ptr=None, reward_ptr=None,
+                           done_ptr=None, winner_ptr=None, captured_ptr=None, valid_ptr=None):
+        """xq_env_policy_step_device: one ply from a policy's scores (PICK_GREEDY / PICK_SAMPLE) or given policy indices (PICK_GIVEN)"""
+        check(self._L.xq_env_policy_step_device(self._h, scores_ptr, scores_dtype, pick, float(temperature), view, 1 if auto_reset else 0,
+                                                actions_ptr, logp_ptr, reward_ptr, done_ptr, winner_ptr, captured_ptr, valid_ptr))
+
     def state_onehot(self):
         out = np.empty((self.n, STATE_SIZE), dtype=np.float64)
         check(self._L.xq_env_state_onehot(self._h, ptr(out)))

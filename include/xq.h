@@ -161,6 +161,51 @@ int xq_env_get_stats(xq_env_t h, xq_env_stats* stats_host, int reset);
 /* ChessAI::getStateRepresentation, src/chessai.cpp:268-289: out_host[n][1260] doubles */
 int xq_env_state_onehot(xq_env_t h, double* out_host);
 
+/* ---- device-resident interface for a policy that is not the library's DQN (a CNN, an actor-critic, ...) ----
+ * All three calls are asynchronous on the handle's stream and write into CALLER-PROVIDED device buffers (a torch tensor's data_ptr()
+ * can be passed straight in); the handle keeps no outputs.  Any optional pointer may be NULL.  Same rules as every other entry point
+ * (the reference's, not standard Xiangqi).
+ *
+ * View.  XQ_VIEW_ABSOLUTE is the reference's frame.  XQ_VIEW_SIDE_TO_MOVE shows an env with Black to move rotated by 180 degrees:
+ * square s <-> 89 - s = (9-r)*9 + (8-c), and colours swapped (channels 0..6 the mover's pieces, 7..13 the opponent's).  The same
+ * mapping applies to observation planes, mask indices, score indices and given / returned actions.  Envs with Red to move (and envs
+ * whose player byte is not 0 or 1) are not transformed.
+ * Policy index.  from*90 + to in the frame of the view: XQ_POLICY_ACTIONS = 8,100 entries, the output width of the reference network. */
+enum { XQ_DTYPE_F32 = 0, XQ_DTYPE_BF16 = 1, XQ_DTYPE_U8 = 2 };
+enum { XQ_VIEW_ABSOLUTE = 0, XQ_VIEW_SIDE_TO_MOVE = 1 };
+enum { XQ_PICK_GREEDY = 0, XQ_PICK_SAMPLE = 1, XQ_PICK_GIVEN = 2 };
+#define XQ_POLICY_ACTIONS 8100            /* policy index = from*90 + to, in the frame of `view` */
+#define XQ_MASK_WORDS 254                 /* packed mask: ceil(8100/32) uint32 per env, bits >= 8100 zero */
+
+/* Observation: planes_dev[n][14][10][9] of 0/1 in f32, bf16 or u8 (dtype).  Absolute view: channel code-1 holds the reference's
+ * one-hot, planes[e][ch][s] == getStateRepresentation[s*14 + ch] (src/chessai.cpp:268-289).  aux_dev[n][4] int32 = player, move_count,
+ * red_score, black_score, always in absolute terms.  planes_dev must be 16-byte aligned. */
+int xq_env_observe_device(xq_env_t h, void* planes_dev, int dtype, int view, int32_t* aux_dev);
+/* Legal-action mask: the set of ChessAI::getAllValidActions(currentPlayer) (src/chessai.cpp:347-368) as policy indices.
+ * packed != 0: uint32 [n][XQ_MASK_WORDS], index i is bit i%32 of word i/32 (for rollout buffers, 1 KB per env).
+ * packed == 0: uint8 [n][8100] of 0/1 (usable as a torch.bool for masked_fill, 8 KB per env).  mask_dev must be 16-byte aligned. */
+int xq_env_legal_mask_device(xq_env_t h, void* mask_dev, int packed, int view);
+/* One ply for every env from a policy's output, one call: move generation, the choice, ChessBoard::movePiece, reward, terminal, winner
+ * and the optional reset; the outputs after the choice are exactly those of xq_env_step_device with the chosen action.
+ * scores_dev: [n][8100] f32 or bf16 (scores_dtype), contiguous, in the view's frame; only the entries of legal actions are read.
+ * Cleaned scores: NaN counts as -inf, +inf as FLT_MAX.
+ *  XQ_PICK_GREEDY: the FIRST legal action in reference list order with the largest score (strict >, as DQN::selectAction).
+ *  XQ_PICK_SAMPLE: a draw from softmax(score / temperature) over the legal actions.  x = xq_rng(seed, env_id0 + e, rec.ctr),
+ *    u = (float)(x >> 40) * 2^-24; m = max, S = sum of exp((l_k - m) / T) in reference list order; the action is the first k whose
+ *    running sum exceeds u*S (the last legal action if rounding leaves none).  The draw uses the env's ply counter: results do not
+ *    depend on how envs are sharded over handles or GPUs.
+ *  XQ_PICK_GIVEN: actions_dev (int64 policy indices, -1 = none) is read, not written.  An index outside [0, 8100) or not legal is
+ *    rejected like an xq_env_step action: valid = 0, the board is unchanged.  With scores_dev non-NULL, logp is the given action's
+ *    log-probability (PPO's re-evaluation of stored actions).
+ * If every legal score is -inf (or NaN) the first action in reference order is played, and logp is NaN.  An empty list (also any env
+ * whose player byte is not 0 or 1) behaves like xq_env_step_device with XQ_ACTION_NONE.
+ * Outputs: actions_dev (GREEDY / SAMPLE) int64 [n] = the chosen policy index, -1 for an empty list; logp_dev f32 [n] = (l_k - m)/T - log S
+ * of the played action (NaN when not defined: empty list, rejected or scoreless GIVEN); reward i32 [n]; done, winner, captured, valid u8 [n].
+ * temperature must be finite and > 0 for SAMPLE and whenever logp is computed; otherwise the call returns XQ_ERR_INVALID. */
+int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dtype, int pick, float temperature, int view,
+                              int auto_reset, int64_t* actions_dev, float* logp_dev, int32_t* reward_dev, uint8_t* done_dev,
+                              uint8_t* winner_dev, uint8_t* captured_dev, uint8_t* valid_dev);
+
 /* ---- DQN: replaces DQN (include/dqn.h:97-116, src/dqn.cpp) + NeuralNetwork (include/dqn.h:43-95, src/dqn.cu) ----
  * Parameters use the reference layout (src/dqn.cu:112-140): weights = layer after layer, each [out][in]
  * row-major; biases = layer after layer.
