@@ -4,7 +4,7 @@ Host-side mirror of the C ABI in include/xq.h; the hot path lives in csrc/ as ha
 """
 from ._lib import (ENV_DTYPE, MAX_ACTIONS, STATE_SIZE, STATS_DTYPE, TRACE_DTYPE, TRANSITION_DTYPE, XQError,  # noqa: F401
                    lib)
-from .env import BatchedEnv, action  # noqa: F401
+from .env import BatchedEnv, BatchedSearch, action, search_bytes_per_tree  # noqa: F401
 from .dqn import AS_WRITTEN, CORRECTED, DQN  # noqa: F401
 from .replay import ReplayBuffer, act, collect, td_update_replay, td_update_replay_n  # noqa: F401
 from .trainer import GAME_EVENT_DTYPE, drain_game_events, enable_game_events, train  # noqa: F401
@@ -12,8 +12,11 @@ from .benchmarks import bench_dqn  # noqa: F401
 
 
 def __getattr__(name):
-    """TorchEnv (torch_env.py) is loaded on first use: importing the package does not import torch"""
+    """TorchEnv (torch_env.py) and TorchSearch (torch_search.py) are loaded on first use: importing the package does not import torch"""
     if name == "TorchEnv":
         from .torch_env import TorchEnv
         return TorchEnv
+    if name == "TorchSearch":
+        from .torch_search import TorchSearch
+        return TorchSearch
     raise AttributeError(f"module {__name__!r} has no attribute {name!r}")

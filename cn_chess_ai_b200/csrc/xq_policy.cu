@@ -266,6 +266,17 @@ __global__ void __launch_bounds__(kThreads) policy_step_generic_kernel(PolicyArg
     policy_apply(b, mt, a.envs, env, c.k >= 0, from, to, a.auto_reset, a.reward, a.done, a.winner, a.captured, a.valid);
 }
 
+// observe_kernel on any array of records (xq_search.cu observes the leaves of its trees); planes 16-byte aligned, dtype checked by the caller
+cudaError_t launch_observe(const xq_env_rec* recs, int64_t n, void* planes, int dtype, int view, int32_t* aux, cudaStream_t stream) {
+    uint8_t* p = static_cast<uint8_t*>(planes);
+    const unsigned grid = (unsigned)((n + kObsBoards - 1) / kObsBoards);
+    if (dtype == XQ_DTYPE_F32) observe_kernel<XQ_DTYPE_F32><<<grid, kObsThreads, 0, stream>>>(recs, n, p, view, aux);
+    else if (dtype == XQ_DTYPE_BF16) observe_kernel<XQ_DTYPE_BF16><<<grid, kObsThreads, 0, stream>>>(recs, n, p, view, aux);
+    else observe_kernel<XQ_DTYPE_U8><<<grid, kObsThreads, 0, stream>>>(recs, n, p, view, aux);
+    ++g_launches;
+    return cudaGetLastError();
+}
+
 }  // namespace xq
 
 // ==========================================================================================

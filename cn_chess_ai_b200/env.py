@@ -8,7 +8,8 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import ENV_DTYPE, MAX_ACTIONS, STATE_SIZE, STATS_DTYPE, TRACE_DTYPE, check, lib, ptr
+from ._lib import (ENV_DTYPE, MAX_ACTIONS, SEARCH_EDGE_DTYPE, SEARCH_MAX_EDGES, SEARCH_NODE_DTYPE, STATE_SIZE, STATS_DTYPE, TRACE_DTYPE,
+                   check, lib, ptr)
 
 
 def action(from_sq, to_sq):
@@ -150,3 +151,65 @@ class BatchedEnv:
         out = np.empty((self.n, STATE_SIZE), dtype=np.float64)
         check(self._L.xq_env_state_onehot(self._h, ptr(out)))
         return out
+
+
+def search_bytes_per_tree(max_simulations):
+    """device memory one tree of a BatchedSearch with this capacity takes"""
+    b = C.c_int64()
+    check(lib().xq_search_bytes_per_tree(max_simulations, C.byref(b)))
+    return b.value
+
+
+class BatchedSearch:
+    """xq_search_*: one PUCT tree per env of `env` (a BatchedEnv), capacity max_simulations simulations per reset.  Raw device pointers
+    (ints), asynchronous on the env's stream; close() before the env is closed."""
+
+    def __init__(self, env, max_simulations):
+        self._L = lib()
+        self._h = C.c_void_p()
+        check(self._L.xq_search_create(env.handle, max_simulations, C.byref(self._h)))
+        self.env = env
+        self.n = env.n
+        self.max_simulations = int(max_simulations)
+
+    def close(self):
+        if self._h:
+            self._L.xq_search_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def reset(self):
+        check(self._L.xq_search_reset(self._h))
+
+    def select_device(self, c_puct, fpu, status_ptr=None, winner_ptr=None, reward_ptr=None, depth_ptr=None):
+        check(self._L.xq_search_select_device(self._h, float(c_puct), float(fpu), status_ptr, winner_ptr, reward_ptr, depth_ptr))
+
+    def leaves_device(self):
+        """device address of the [n] leaf records of the last selection"""
+        p = C.c_void_p()
+        check(self._L.xq_search_leaves_device(self._h, C.byref(p)))
+        return p.value
+
+    def observe_leaves_device(self, planes_ptr, dtype, view, aux_ptr):
+        check(self._L.xq_search_observe_leaves_device(self._h, planes_ptr, dtype, view, aux_ptr))
+
+    def expand_backup_device(self, scores_ptr, scores_dtype, temperature, view, values_ptr, noise_ptr=None, noise_eps=0.0):
+        check(self._L.xq_search_expand_backup_device(self._h, scores_ptr, scores_dtype, float(temperature), view, values_ptr, noise_ptr,
+                                                     float(noise_eps)))
+
+    def root_device(self, view, visits_ptr, q_ptr, best_ptr):
+        check(self._L.xq_search_root_device(self._h, view, visits_ptr, q_ptr, best_ptr))
+
+    def get_tree(self, tree):
+        """synchronous read-back of one tree: (nodes SEARCH_NODE_DTYPE [n_nodes], edges SEARCH_EDGE_DTYPE [n_nodes][128])"""
+        cap = self.max_simulations + 1
+        nodes = np.zeros(cap, SEARCH_NODE_DTYPE)
+        edges = np.zeros((cap, SEARCH_MAX_EDGES), SEARCH_EDGE_DTYPE)
+        cnt = C.c_int32()
+        check(self._L.xq_search_get_tree(self._h, int(tree), ptr(nodes), ptr(edges), C.byref(cnt)))
+        return nodes[:cnt.value].copy(), edges[:cnt.value].copy()

@@ -1,0 +1,116 @@
+"""TorchSearch: batched PUCT tree search (one tree per env) for a policy/value network written in PyTorch, on the device
+(include/xq.h: xq_search_*).
+
+Each simulation selects one leaf per tree, observes all leaves at once, calls the network once on them and hands its scores and values
+back; selection, child creation, expansion and backup run in the library's kernels on torch's current stream.  Actions and visit counts
+use the policy indices from * 90 + to of TorchEnv, in the frame of `view`.
+"""
+from collections import namedtuple
+
+import torch
+
+from ._lib import POLICY_ACTIONS
+from .env import BatchedSearch
+from .torch_env import _OBS_DTYPES, _SCORE_DTYPES, _view
+
+SelectResult = namedtuple("SelectResult", "status winner reward depth")
+RootResult = namedtuple("RootResult", "visits q best")
+
+# leaf status (xq_search_select_device)
+NEEDS_EVALUATION, GENERAL_CAPTURED, MOVE_CAP, NO_LEGAL_ACTION = 0, 1, 2, 3
+
+
+class TorchSearch:
+    """max_simulations simulations per reset on the envs of `tenv` (a TorchEnv); the roots are the envs' boards at reset()"""
+
+    def __init__(self, tenv, max_simulations):
+        self.tenv = tenv
+        self.n = tenv.n
+        self.device = tenv.device
+        self.search = BatchedSearch(tenv.env, max_simulations)
+        self.max_simulations = self.search.max_simulations
+
+    def close(self):
+        self.search.close()
+
+    def reset(self):
+        self.tenv._enter()
+        self.search.reset()
+
+    def select(self, c_puct=1.5, fpu=0.0):
+        """one leaf per tree: SelectResult of tensors [n]: status / winner uint8, reward / depth int32"""
+        self.tenv._enter()
+        status, winner = (torch.empty(self.n, dtype=torch.uint8, device=self.device) for _ in range(2))
+        reward, depth = (torch.empty(self.n, dtype=torch.int32, device=self.device) for _ in range(2))
+        self.search.select_device(c_puct, fpu, status.data_ptr(), winner.data_ptr(), reward.data_ptr(), depth.data_ptr())
+        return SelectResult(status, winner, reward, depth)
+
+    def leaves(self):
+        """the leaf records of the last selection as a uint8 [n, 64] tensor aliasing the library's buffer (xq_env_rec each; valid until
+        the next select: clone() to keep them)"""
+        ptr = self.search.leaves_device()
+        n = self.n
+
+        class _Leaves:
+            __cuda_array_interface__ = {"shape": (n, 64), "typestr": "|u1", "data": (ptr, False), "version": 3, "strides": None}
+
+        return torch.as_tensor(_Leaves(), device=self.device)
+
+    def observe(self, dtype=torch.bfloat16, view="side"):
+        """the leaves as TorchEnv.observe shows envs: (planes [n, 14, 10, 9], aux int32 [n, 4])"""
+        if dtype not in _OBS_DTYPES:
+            raise ValueError(f"dtype must be one of {list(_OBS_DTYPES)}")
+        v = _view(view)
+        self.tenv._enter()
+        planes = torch.empty((self.n, 14, 10, 9), dtype=dtype, device=self.device)
+        aux = torch.empty((self.n, 4), dtype=torch.int32, device=self.device)
+        self.search.observe_leaves_device(planes.data_ptr(), _OBS_DTYPES[dtype], v, aux.data_ptr())
+        return planes, aux
+
+    def expand_backup(self, scores, values, temperature=1.0, root_noise=None, noise_eps=0.25, view="side"):
+        """scores [n, 8100] (f32 / bf16, frame of `view`) expand the leaves that need evaluation; values f32 [n] (from each leaf's side
+        to move) are backed up for every leaf.  root_noise f32 [n, 8100]: mixed into the root's priors when the root is expanded."""
+        v = _view(view)
+        self.tenv._check(scores, "scores", list(_SCORE_DTYPES), (self.n, POLICY_ACTIONS))
+        self.tenv._check(values, "values", [torch.float32], (self.n,))
+        if root_noise is not None:
+            self.tenv._check(root_noise, "root_noise", [torch.float32], (self.n, POLICY_ACTIONS))
+        self.tenv._enter()
+        self.search.expand_backup_device(scores.data_ptr(), _SCORE_DTYPES[scores.dtype], temperature, v, values.data_ptr(),
+                                         None if root_noise is None else root_noise.data_ptr(), noise_eps)
+
+    def root(self, view="side"):
+        """RootResult: visits int32 [n, 8100] (frame of `view`), q f32 [n] (NaN without a visited edge), best int64 [n] (the most-visited
+        root action, -1 without a visited edge: the input of TorchEnv.step(actions=best, pick="given"))"""
+        v = _view(view)
+        self.tenv._enter()
+        visits = torch.empty((self.n, POLICY_ACTIONS), dtype=torch.int32, device=self.device)
+        q = torch.empty(self.n, dtype=torch.float32, device=self.device)
+        best = torch.empty(self.n, dtype=torch.int64, device=self.device)
+        self.search.root_device(v, visits.data_ptr(), q.data_ptr(), best.data_ptr())
+        return RootResult(visits, q, best)
+
+    @staticmethod
+    def outcome_values(status, winner, aux, cap_value=0.0):
+        """a default value of terminal leaves, from the leaf's side to move (aux[:, 0], absolute colour): +1 / -1 when a General was
+        captured and the side to move is / is not the winner, cap_value at the move cap, -1 without a legal action, 0 elsewhere"""
+        player = aux[:, 0].to(torch.int32)
+        won = torch.where(winner.to(torch.int32) == player, 1.0, -1.0)
+        v = torch.zeros(status.shape, dtype=torch.float32, device=status.device)
+        v = torch.where(status == GENERAL_CAPTURED, won, v)
+        v = torch.where(status == MOVE_CAP, torch.full_like(v, float(cap_value)), v)
+        return torch.where(status == NO_LEGAL_ACTION, torch.full_like(v, -1.0), v)
+
+    def run(self, evaluate, n_simulations, c_puct=1.5, fpu=0.0, temperature=1.0, root_noise=None, noise_eps=0.25, view="side",
+            obs_dtype=torch.bfloat16, cap_value=0.0):
+        """reset + n_simulations simulations: evaluate(planes) -> (scores [n, 8100], values [n]) is called once per simulation on the
+        leaves; at terminal leaves outcome_values replaces the network's value.  Returns root(view)."""
+        self.reset()
+        for _ in range(n_simulations):
+            sel = self.select(c_puct, fpu)
+            planes, aux = self.observe(obs_dtype, view)
+            scores, values = evaluate(planes)
+            values = values.reshape(self.n).to(torch.float32).contiguous()
+            values = torch.where(sel.status != NEEDS_EVALUATION, self.outcome_values(sel.status, sel.winner, aux, cap_value), values)
+            self.expand_backup(scores.contiguous(), values, temperature, root_noise, noise_eps, view)
+        return self.root(view)

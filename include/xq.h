@@ -206,6 +206,83 @@ int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dty
                               int auto_reset, int64_t* actions_dev, float* logp_dev, int32_t* reward_dev, uint8_t* done_dev,
                               uint8_t* winner_dev, uint8_t* captured_dev, uint8_t* valid_dev);
 
+/* ---- device-resident batched tree search (PUCT / MCTS) for an external policy/value network ----
+ * One tree per env of an env handle; each simulation selects one leaf per tree, the caller evaluates all leaves with ONE network call
+ * and hands back scores and values; everything in between stays on the device.  Every call is asynchronous on the env handle's stream
+ * and device; destroy the search before the env.  Same rules as every other entry point (the reference's).
+ *
+ * Tree.  The root is the env's record at xq_search_reset.  A node holds its board as an xq_env_rec; a child's record equals, bit for bit,
+ * what xq_env_step_device (auto_reset = 0) makes of the parent's record and the edge's action (move_count, player, scores, ctr included).
+ * Edges are a node's legal actions in reference list order (xq_env_legal_moves; the first 128), each with the prior P, the visit count N,
+ * the value sum W (from the side to move at the parent) and the child.  N_node = simulations whose path contained the node, leaf included.
+ * Selection (one leaf per tree per simulation, no virtual loss), from the root: a node not yet expanded, or terminal, is the leaf;
+ * otherwise the edge with the largest Q + U, ties to the smaller list index, in f32 with no contraction, in this order:
+ *   Q = N > 0 ? W / N : fpu,   U = ((c_puct * P) * sqrt(N_node)) / (1 + N).
+ * If that edge has no child yet, the child is made and is the leaf: a simulation adds at most one node per tree.
+ * Leaf status (u8): 0 needs evaluation, 1 a General was captured, 2 move cap (move_count >= 200), 3 no legal action (known once the node
+ * was expanded to zero edges: the first simulation that reaches such a node reports 0, later ones 3).  A General captured on the 200th
+ * ply is status 1.  Also per tree: winner (as xq_env_step: getWinner), the reward of the move that made the leaf (0 at the root), the
+ * depth (plies below the root).
+ * Expansion (status 0 only): scores [n][8100] (f32 / bf16, in the frame of `view`, cleaned as in xq_env_policy_step_device; only legal
+ * entries are read) give P_k = exp((l_k - m) / T) / S, S summed in list order, uniform 1 / count if every legal score is -inf.  At the root
+ * only, with root_noise_dev [n][8100] f32 (finite; e.g. Dirichlet noise the caller draws over the legal mask):
+ * P <- (1 - eps) * P + eps * noise[index].  The library draws no random numbers.
+ * Backup (every status): the caller's value of the leaf, from the leaf's side to move, NaN -> 0, clamped to [-1, 1]; going up,
+ * v <- -v, the edge gets N += 1 and W += v, every node on the path N_node += 1.  The library has no value convention for terminal leaves.
+ *
+ * Call order: xq_search_reset, then per simulation select -> (leaves / observe_leaves, any number of times) -> expand_backup; anything
+ * else is XQ_ERR_STATE, as is a select past max_simulations since the reset.  root_device and get_tree work at any time after a reset.
+ * Memory: (max_simulations + 1) x 2,389 + 73 bytes per tree (xq_search_bytes_per_tree): per node a record, 21 bytes of node state and
+ * 128 edge slots of 18 bytes (P, N, W, child, action); per tree the leaf record and 9 bytes. */
+typedef struct xq_search_s* xq_search_t;
+#define XQ_SEARCH_MAX_EDGES 128
+typedef struct {
+    xq_env_rec rec;       /* the node's board */
+    int32_t parent;       /* node index in the tree, -1 at the root (node 0) */
+    int32_t visits;       /* N_node */
+    int32_t reward;       /* reward of the move that made the node (0 at the root) */
+    int32_t depth;        /* plies below the root */
+    uint8_t parent_edge;  /* list index of the edge from the parent */
+    uint8_t n_edges;      /* edges after expansion */
+    uint8_t expanded;
+    uint8_t status;       /* 0 not terminal, 1 General captured, 2 move cap, 3 expanded without a legal action */
+    uint8_t winner;       /* getWinner of the node's board */
+    uint8_t reserved[3];
+} xq_search_node;         /* 88 B */
+typedef struct {
+    int32_t action;       /* absolute policy index from * 90 + to, -1 past n_edges */
+    float prior;
+    int32_t visits;       /* N */
+    float value_sum;      /* W, from the side to move at the parent */
+    int32_t child;        /* node index, -1 none */
+} xq_search_edge;         /* 20 B */
+
+/* capacity max_simulations + 1 nodes per tree; XQ_ERR_NOMEM when the device memory cannot be had.  The trees are empty until a reset. */
+int xq_search_create(xq_env_t env, int max_simulations, xq_search_t* out);
+int xq_search_destroy(xq_search_t s);
+int xq_search_bytes_per_tree(int max_simulations, int64_t* bytes);
+/* roots = the env's current records (read in stream order), every tree empty, simulation count 0 */
+int xq_search_reset(xq_search_t s);
+/* one leaf per tree; c_puct finite and >= 0, fpu finite.  Outputs [n] (any may be NULL): status u8, winner u8, reward i32, depth i32 */
+int xq_search_select_device(xq_search_t s, float c_puct, float fpu, uint8_t* status_dev, uint8_t* winner_dev, int32_t* reward_dev,
+                            int32_t* depth_dev);
+/* device address of the [n] leaf records of the last selection (valid until the next select) */
+int xq_search_leaves_device(xq_search_t s, void** leaf_recs_dev);
+/* xq_env_observe_device on the leaf records: same planes / aux contract */
+int xq_search_observe_leaves_device(xq_search_t s, void* planes_dev, int dtype, int view, int32_t* aux_dev);
+/* expansion of the status-0 leaves and backup of every leaf: scores_dev [n][8100] (scores_dtype f32 / bf16), temperature finite > 0,
+ * values_dev f32 [n] (required), root_noise_dev f32 [n][8100] or NULL, noise_eps in [0, 1] */
+int xq_search_expand_backup_device(xq_search_t s, const void* scores_dev, int scores_dtype, float temperature, int view,
+                                   const float* values_dev, const float* root_noise_dev, float noise_eps);
+/* per root (any output may be NULL): visits_dev int32 [n][8100] (16-byte aligned) = the root edges' N at their policy indices in the frame
+ * of `view`, 0 elsewhere; q_dev f32 [n] = sum W / sum N over the root's edges (sums in list order; NaN when no edge was visited); best_dev
+ * int64 [n] = policy index (frame of `view`) of the most-visited root edge, first in list order on ties, -1 when no edge was visited --
+ * the input of xq_env_policy_step_device with XQ_PICK_GIVEN. */
+int xq_search_root_device(xq_search_t s, int view, int32_t* visits_dev, float* q_dev, int64_t* best_dev);
+/* synchronous read-back of one tree: nodes_host[max_simulations + 1], edges_host [max_simulations + 1][128] (may be NULL; edges past a
+ * node's n_edges have action -1 and child -1), *n_nodes = nodes in the tree */
+int xq_search_get_tree(xq_search_t s, int64_t tree, xq_search_node* nodes_host, xq_search_edge* edges_host, int32_t* n_nodes);
+
 /* ---- DQN: replaces DQN (include/dqn.h:97-116, src/dqn.cpp) + NeuralNetwork (include/dqn.h:43-95, src/dqn.cu) ----
  * Parameters use the reference layout (src/dqn.cu:112-140): weights = layer after layer, each [out][in]
  * row-major; biases = layer after layer.
