@@ -115,8 +115,7 @@ def bench_dqn(stream, peaks, world=1, local=0, dist=None, envs=65536, replay_cap
            "us_per_update_median": us_sorted[len(us_sorted) // 2], "us_per_update_min": us_sorted[0], "us_per_update_calls": [1e3 * x / updates for x in per_call],
            "timed": "%d calls x %d sequential updates (%d kernel launches); mean over all, median / min over the calls, max over ranks" % (calls, updates, calls * updates * 4),
            "batch_per_gpu": batch, "replay_transitions_per_gpu": replay_cap,
-           "grad_allreduce": (("inside the gradient contraction kernel over peer memory: reduce-scatter of the 16-row blocks to owner ranks + all-gather, flag-in-data lines"
-                               if os.environ.get("XQ_DIST_FUSED_MODE", "owner") != "allgather" else "inside the gradient contraction kernel: every block to every rank + flags")
+           "grad_allreduce": ("inside the gradient contraction kernel over peer memory: reduce-scatter of the 16-row blocks to owner ranks + all-gather, flag-in-data lines"
                               if fused else "nccl all_reduce + apply kernel") if world > 1 else False,
            "replicas_identical": replicas_identical if world > 1 else None,
            "selfplay_eps_greedy_steps_per_s": envs * plies * world / (collect_ms * 1e-3), "selfplay_envs_per_gpu": envs,

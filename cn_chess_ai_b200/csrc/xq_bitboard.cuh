@@ -1,7 +1,7 @@
 // xq_bitboard.cuh -- per-piece move COUNT (+ a 32-bit descriptor) and k-th-move DECODE (from the descriptor) on 90-bit occupancy bitboards.
 //
-// Used by the slot-parallel rollout kernel (xq_rollout.cu): one thread owns one piece, warps are
-// piece-type uniform, so every function here runs without divergence across a warp.  Sliders are
+// Used by the team kernels (xq_rollout_team.cuh): the pieces a thread owns are piece-type uniform
+// across a warp, so every function here runs without divergence across a warp.  Sliders are
 // O(1): the rank / file occupancy is pulled out of the row-major / column-major bitboards with a
 // funnel shift and the first and second blocker on each ray come from ffs/clz -- no per-square
 // loops.  Emission order is the reference's (SURVEY Appendix A.3): direction order as written in

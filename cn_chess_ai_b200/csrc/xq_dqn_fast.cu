@@ -93,8 +93,8 @@ struct Fast {
     float* zpart_b = nullptr;
     CUtensorMap tmH2_b;
     cudaStream_t aux = nullptr, main_hi = nullptr;
-    cudaEvent_t ev_join = nullptr, ev_tdb[2] = {nullptr, nullptr};
-    cudaEvent_t ev_fork = nullptr, ev_aux[2] = {nullptr, nullptr}, ev_free[2] = {nullptr, nullptr}, ev_td[2] = {nullptr, nullptr};
+    cudaEvent_t ev_join = nullptr;
+    cudaEvent_t ev_fork = nullptr, ev_aux[2] = {nullptr, nullptr}, ev_td[2] = {nullptr, nullptr};
     // multi-GPU gradient exchange over peer memory (xq_dqn_dist_*): when connected, the compact gradient of an update is written
     // into slot `parity` of this rank's exchange buffer, which every peer maps through CUDA IPC
     uint8_t* exch = nullptr;                           // [2][kGradPad] FP32 gradient slots | flags[kMaxRanks] u32 | status u32
@@ -104,7 +104,6 @@ struct Fast {
     bool connected = false;
     uint32_t *status_host = nullptr, *status_dev = nullptr;   // mapped pinned word: epoch of the first exchange that timed out (sticky; read without a sync)
     long long timeout_ticks = 0;                       // clock64 ticks (XQ_DIST_TIMEOUT_MS, default 20 s)
-    int fused_mode = 2;                                // DW_FUSED_OWNER, or DW_FUSED_ALLGATHER with XQ_DIST_FUSED_MODE=allgather
     uint8_t* hg_stage = nullptr;                       // device staging of xq_dqn_dist_allgather
     uint8_t* hg_pin = nullptr;                         // pinned host staging: [send kHgCap | recv kMaxRanks x kHgCap]
     uint32_t hg_seq = 0;
@@ -121,8 +120,8 @@ struct Fast {
     uint64_t w_version = 1, actq_version = 0, actz_version = 0;   // online W0 / b0 version; version W0Q / actZ were built from
     int act_slot = 0;
     int64_t act_carried_n = -1;
-    CUtensorMap tmActHiS[4], tmActLoS[4];              // the parts of the collector's env range (multi-stream plies)
-    int64_t act_sub_n = -1; int act_sub_parts = 0;
+    CUtensorMap tmActHiS[2], tmActLoS[2];              // the halves of the collector's env range (two-stream plies)
+    int64_t act_sub_n = -1;
     CUtensorMap tmActHi, tmActLo, tmW1q, tmW1loq;
     int64_t tm_rows = 0;
 };
@@ -408,7 +407,7 @@ __device__ __forceinline__ uint32_t sw128_offset(int row, int col) {   // byte o
 
 template <int MODE>
 __global__ void __launch_bounds__(kGemmThreads, 1) l1_gemm_kernel(const __grid_constant__ CUtensorMap tmH, const __grid_constant__ CUtensorMap tmW1,
-                                                                 const float* __restrict__ b1, int M, int m_first, int m_tiles, int n_splits,
+                                                                 const float* __restrict__ b1, int M, int m_tiles, int n_splits,
                                                                  float* __restrict__ zpart, int64_t zstride, float* __restrict__ Q) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);   // SW128 tiles need 1024-B alignment
@@ -428,7 +427,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) l1_gemm_kernel(const __grid_c
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int n_tile = blockIdx.x, split = blockIdx.y;
     const int n0 = n_tile * BN;
-    // rows of this CTA: m-tiles m_first + split, + n_splits, ... of the launch's range [m_first, m_first + m_tiles)
+    // rows of this CTA: m-tiles split, split + n_splits, ... of [0, m_tiles)
     const int my_tiles = (m_tiles - split + n_splits - 1) / n_splits;
     if (threadIdx.x == 0) XQ_TL(0, 0);
 
@@ -445,7 +444,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) l1_gemm_kernel(const __grid_c
         tc::pdl_wait();             // W1 / b1 were final before the producer of H started; H itself is the predecessor's output
         for (int i = 0; i < kAStages && i < my_tiles; ++i) {
             tc::mbar_expect_tx(a_full + i, kABytes);
-            const int row0 = (m_first + split + i * n_splits) * BM;
+            const int row0 = (split + i * n_splits) * BM;
             for (int kb = 0; kb < kKBlocks; ++kb) tc::tma_load_2d(sA + i * kABytes + kb * (BM * BK * 2), &tmH, kb * BK, row0, a_full + i);
         }
     }
@@ -497,7 +496,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) l1_gemm_kernel(const __grid_c
                 const int st = i % kAStages;
                 tc::mbar_wait(a_empty + st, ((i / kAStages) & 1) ^ 1);
                 tc::mbar_expect_tx(a_full + st, kABytes);
-                const int row0 = (m_first + split + i * n_splits) * BM;
+                const int row0 = (split + i * n_splits) * BM;
                 for (int kb = 0; kb < kKBlocks; ++kb) tc::tma_load_2d(sA + st * kABytes + kb * (BM * BK * 2), &tmH, kb * BK, row0, a_full + st);
             }
         }
@@ -539,7 +538,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) l1_gemm_kernel(const __grid_c
         constexpr int kHalfCols = BN / 2;                                   // 112 = 3 x 32 + 16 columns
         for (int i = 0; i < my_tiles; ++i) {
             const int acc = i & 1;
-            const int row = (m_first + split + i * n_splits) * BM + quarter * 32 + lane;
+            const int row = (split + i * n_splits) * BM + quarter * 32 + lane;
             tc::mbar_wait(acc_full + acc, (i >> 1) & 1);
             if (warp == 4 && lane == 0 && i < 8) XQ_TL(0, 20 + i);
             tc::tc_fence_after();
@@ -816,10 +815,8 @@ __global__ void __launch_bounds__(256) td_delta_kernel(uint32_t* __restrict__ cb
 constexpr int kMaxRanks = 16;
 constexpr int kGradPad = (kGradSize + 3) / 4 * 4;
 constexpr size_t kExchFlagsOff = sizeof(float) * 2 * (size_t)kMaxRanks * kGradPad;                 // 16-byte aligned
-constexpr int kExchBlocks = 96;                                                                      // >= 11 row tiles x 8 splits of the gradient contraction
-constexpr size_t kExchBlockFlagsOff = kExchFlagsOff + sizeof(uint32_t) * (kMaxRanks + 4);           // [kMaxRanks source ranks][kExchBlocks] u32: epoch of the last landed row block
-constexpr size_t kExchOldBytes = kExchBlockFlagsOff + sizeof(uint32_t) * kMaxRanks * kExchBlocks;
-// Owner mode (the default fused exchange): reduce-scatter + all-gather of the 16-row blocks with the flag carried INSIDE the data
+constexpr size_t kExchFlagsEnd = kExchFlagsOff + sizeof(uint32_t) * (kMaxRanks + 4);                   // flags, status word, completion counter, 2 spare
+// The fused exchange: reduce-scatter + all-gather of the 16-row blocks with the flag carried INSIDE the data
 // (the idea of the "LL" / "LL128" protocols of collective libraries): a 16-byte line holds three FP32 values x, y, z and the word
 // epoch ^ x ^ y ^ z, written by one 16-byte vector store and read by one 16-byte vector load -- the receiver polls the data itself, no
 // fence, no separate flag.  A line is accepted when x ^ y ^ z ^ w equals the epoch it waits for, so a line caught half-written (old and
@@ -832,7 +829,7 @@ constexpr int kLLBlocks = 88;                                                   
 constexpr int kLLLinesPerThread = 3;
 constexpr int kLLLinesPerBlock = kLLLinesPerThread * 256;
 constexpr size_t kLLBlockBytes = (size_t)kLLLinesPerBlock * 16;                                      // 12 KB for 8.4 KB of payload
-constexpr size_t kExchLL1Off = (kExchOldBytes + 255) / 256 * 256;
+constexpr size_t kExchLL1Off = (kExchFlagsEnd + 255) / 256 * 256;
 constexpr size_t kExchLL1Bytes = 2 * (size_t)kMaxRanks * kLLBlocks * kLLBlockBytes;                  // 33 MB
 constexpr size_t kExchLL2Off = kExchLL1Off + kExchLL1Bytes;
 constexpr size_t kExchLL2Bytes = 2 * (size_t)kLLBlocks * kLLBlockBytes;                              // 2 MB
@@ -866,12 +863,11 @@ struct DwPush {               // world == 0: the gradient stays local (grad)
     PeerPtrs peers;
     int rank = 0, world = 0, parity = 0;
     uint32_t epoch = 0;
-    int fused = 0;            // the contraction itself exchanges its row blocks, sums them and applies the SGD step (no exchange kernel):
-                              // 2 = owner mode (reduce-scatter + all-gather of the blocks, flag-in-data lines), 1 = every block to every rank + flags
+    bool fused = false;       // the contraction itself exchanges its row blocks (reduce-scatter + all-gather of the blocks, flag-in-data lines),
+                              // sums them and applies the SGD step (no exchange kernel)
     long long timeout = 0;    // clock64 ticks a wait for a peer may last; then the update is NOT applied and *status is raised (sticky)
     uint32_t* status = nullptr;   // host-mapped word: epoch of the first exchange that timed out (0 = none)
 };
-enum { DW_FUSED_ALLGATHER = 1, DW_FUSED_OWNER = 2 };
 
 // ---------------------------------------------------------------------------------------------
 // dW0^T = X^T . delta0 on tcgen05: C[feature 0..1279][hidden 0..127] = sum_b onehot_b[feature] * delta0_b[hidden].
@@ -1130,7 +1126,7 @@ __global__ void __launch_bounds__(kDwThreads, 1) dw_gemm_kernel(const __grid_con
 #pragma unroll
         for (int p = 0; p < kDwSplits; ++p) db1 += __ldcg(dbpart + p * BM + threadIdx.x);      // the 8 per-CTA sums in fixed order
     }
-    if (push.fused == DW_FUSED_OWNER) {
+    if (push.fused) {
         // ===== multi-GPU, ONE kernel: contraction -> reduce-scatter -> all-gather -> SGD, row block by row block, over peer memory =====
         // Block blk (the 16 rows this CTA reduced) is OWNED by rank blk % world.  The same CTA (mt, ks) of every rank handles the same block and
         // the same thread the same elements, so the exchange is thread to thread:
@@ -1229,59 +1225,6 @@ __global__ void __launch_bounds__(kDwThreads, 1) dw_gemm_kernel(const __grid_con
         if (!exch_ok) { *push.status = flag; __threadfence_system(); }
         acc[0] = make_float4(g[0], g[1], g[2], g[3]); acc[1] = make_float4(g[4], g[5], g[6], g[7]);
         if (owns_db1 && exch_ok) b1[threadIdx.x] -= lr * g[8];
-    } else if (push.fused) {
-        // ===== A/B alternative (XQ_DIST_FUSED_MODE=allgather): every block to every rank, then a flag per (rank, block) =====
-        // 1. push this CTA's 16 reduced rows (and db1, for the CTA that owns it) into slot (parity, my rank) of every rank's buffer
-        const size_t slot = exch_slot_floats(push.parity, push.rank);
-#pragma unroll
-        for (int u = 0; u < 2; ++u)
-            if (e[u] >= 0)
-                for (int r = 0; r < push.world; ++r) *reinterpret_cast<float4*>(push.peers.p[r] + sizeof(float) * (slot + (size_t)e[u])) = acc[u];
-        if (owns_db1)
-            for (int r = 0; r < push.world; ++r) *reinterpret_cast<float*>(push.peers.p[r] + sizeof(float) * (slot + (size_t)(kGradB1 + threadIdx.x))) = db1;
-        // 2. "row block b of gradient `epoch` of this rank has landed": CTA barrier, then one release store at system scope per peer (the release is
-        //    cumulative over everything the barrier ordered before it -- the pattern of a semaphore release)
-        const int blk = mt * kDwSplits + ks;
-        __shared__ int s_timed_out;
-        if (threadIdx.x == 0) s_timed_out = 0;
-        __syncthreads();
-        if ((int)threadIdx.x < push.world) {
-            uint32_t* f = reinterpret_cast<uint32_t*>(push.peers.p[threadIdx.x] + kExchBlockFlagsOff) + push.rank * kExchBlocks + blk;
-            asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(f), "r"(push.epoch) : "memory");
-            // 3. the same row block of every rank has landed HERE (the spin is on local memory; every rank pushes before it waits, and
-            //    all 88 CTAs of a contraction are resident, so nobody waits for a CTA that cannot run)
-            const uint32_t* mine = reinterpret_cast<const uint32_t*>(push.peers.p[push.rank] + kExchBlockFlagsOff) + threadIdx.x * kExchBlocks + blk;
-            const long long t0 = clock64();
-            uint32_t v;
-            do {
-                asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(mine) : "memory");
-                if ((int32_t)(v - push.epoch) >= 0) break;
-                if (clock64() - t0 > push.timeout) { s_timed_out = 1; *push.status = push.epoch; __threadfence_system(); break; }   // sticky: the update is not applied
-            } while (true);
-        }
-        __syncthreads();
-        if (s_timed_out) exch_ok = false;
-        // 4. sum the `world` copies in rank order (the same order on every rank: bit-identical replicas) and apply W -= lr * g
-        const float* base = reinterpret_cast<const float*>(push.peers.p[push.rank]);
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-            if (e[u] < 0) continue;
-            float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-            for (int r = 0; r < push.world; ++r) {               // this rank's own rows are still in registers (same values as its slot)
-                const float4 v = r == push.rank ? acc[u] : ld_peer_f4(base + exch_slot_floats(push.parity, r) + (size_t)e[u]);
-                g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
-            }
-            acc[u] = g;
-        }
-        if (owns_db1) {
-            float g = 0.0f;
-            for (int r = 0; r < push.world; ++r) {
-                float v = db1;
-                if (r != push.rank) asm volatile("ld.volatile.global.f32 %0, [%1];" : "=f"(v) : "l"(base + exch_slot_floats(push.parity, r) + (size_t)(kGradB1 + threadIdx.x)) : "memory");
-                g += v;
-            }
-            if (exch_ok) b1[threadIdx.x] -= lr * g;
-        }
     }
 #pragma unroll
     for (int u = 0; u < 2; ++u) {
@@ -1518,21 +1461,14 @@ static int make_tmap_cb(CUtensorMap* m, const void* base, int64_t n, int64_t ld)
 }
 
 // launch with programmatic stream serialization (PDL), optionally as thread-block clusters along y
-// g_launched_event (set by the caller for ONE launch, then cleared here): an event recorded once every CTA of the grid has begun execution
-// (cudaLaunchAttributeLaunchCompletionEvent) -- "this kernel holds its SMs now"
-static thread_local cudaEvent_t g_launched_event = nullptr;
 template <typename... KArgs, typename... Args>
 static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, int cluster_y, Args&&... args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute at[3];
+    cudaLaunchAttribute at[2];
     int na = 0;
     at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[na].val.programmaticStreamSerializationAllowed = 1; ++na;
     if (cluster_y > 1) { at[na].id = cudaLaunchAttributeClusterDimension; at[na].val.clusterDim.x = 1; at[na].val.clusterDim.y = cluster_y; at[na].val.clusterDim.z = 1; ++na; }
-    if (g_launched_event) {
-        at[na].id = cudaLaunchAttributeLaunchCompletionEvent; at[na].val.launchCompletionEvent.event = g_launched_event; at[na].val.launchCompletionEvent.flags = 0; ++na;
-        g_launched_event = nullptr;
-    }
     cfg.attrs = at; cfg.numAttrs = na;
     ++g_launches;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
@@ -1546,7 +1482,7 @@ static inline DwPush dw_push(Fast* f, bool apply, bool fused = false) {
     DwPush p;
     if (!apply && f->connected) {
         for (int r = 0; r < kMaxRanks; ++r) p.peers.p[r] = f->peer[r];
-        p.rank = f->rank; p.world = f->world; p.parity = f->parity; p.epoch = f->epoch + 1; p.fused = fused ? f->fused_mode : 0;
+        p.rank = f->rank; p.world = f->world; p.parity = f->parity; p.epoch = f->epoch + 1; p.fused = fused;
         p.timeout = f->timeout_ticks; p.status = f->status_dev;
     } else {
         for (int r = 0; r < kMaxRanks; ++r) p.peers.p[r] = nullptr;
@@ -1567,9 +1503,8 @@ void dqn_fast_destroy(xq_dqn_s* h) {
     if (f->aux) cudaStreamDestroy(f->aux);
     if (f->main_hi) cudaStreamDestroy(f->main_hi);
     if (f->ev_join) cudaEventDestroy(f->ev_join);
-    for (int i = 0; i < 2; ++i) if (f->ev_tdb[i]) cudaEventDestroy(f->ev_tdb[i]);
     if (f->ev_fork) cudaEventDestroy(f->ev_fork);
-    for (int i = 0; i < 2; ++i) { if (f->ev_aux[i]) cudaEventDestroy(f->ev_aux[i]); if (f->ev_free[i]) cudaEventDestroy(f->ev_free[i]); if (f->ev_td[i]) cudaEventDestroy(f->ev_td[i]); }
+    for (int i = 0; i < 2; ++i) { if (f->ev_aux[i]) cudaEventDestroy(f->ev_aux[i]); if (f->ev_td[i]) cudaEventDestroy(f->ev_td[i]); }
     cudaFree(f->W0T); cudaFree(f->b0); cudaFree(f->W1); cudaFree(f->b1); cudaFree(f->W1bf); cudaFree(f->W1lo); cudaFree(f->actHhi); cudaFree(f->actHlo);
     cudaFree(f->W0Q); cudaFree(f->b0Q); cudaFree(f->zOpen); cudaFree(f->actMax); cudaFree(f->actZ); cudaFree(f->actPrev);
     cudaFree(f->tW0T); cudaFree(f->tb0); cudaFree(f->tW1); cudaFree(f->tb1); cudaFree(f->tW1bf);
@@ -1685,24 +1620,22 @@ int dqn_fast_weights(xq_dqn_s* h, FastWeights* out) {
 }
 void dqn_target_changed(xq_dqn_s* h) { if (h->fast) h->fast->target_current = false; }
 
-// rows [128 tile_first, 128 (tile_first + tile_count)) of the batch (tile_count <= 0: all of them), cut into row_splits CTAs per column tile
+// the n rows of the batch, cut into row_splits CTAs per column tile
 static int launch_gemm(xq_dqn_s* h, int mode, const CUtensorMap& tmA, const CUtensorMap& tmB, const float* b1, int64_t n, float* q,
-                       cudaStream_t stream = nullptr, float* zpart = nullptr, int row_splits = 0, int tile_first = 0, int tile_count = 0) {
+                       cudaStream_t stream = nullptr, float* zpart = nullptr, int row_splits = 0) {
     Fast* f = h->fast;
     if (!stream) stream = h->stream;
     if (!zpart) zpart = f->zpart;
-    const int all_tiles = (int)((n + BM - 1) / BM);
-    const int m_tiles = tile_count > 0 ? std::min(tile_count, all_tiles - tile_first) : all_tiles - tile_first;
-    if (m_tiles <= 0) return XQ_OK;
+    const int m_tiles = (int)((n + BM - 1) / BM);
     int n_splits = row_splits > 0 ? row_splits : 148 / kNTiles;      // default: 4 row splits x 37 column tiles = 148 CTAs
     if (n_splits > m_tiles) n_splits = m_tiles;
     const dim3 grid(kNTiles, n_splits);
     const int64_t zstride = (f->cap + BM - 1) / BM * BM;
     if (mode == EPI_ROWMAX)
-        XQ_CUDA(launch_pdl(l1_gemm_kernel<EPI_ROWMAX>, grid, dim3(kGemmThreads), kGemmSmem, stream, 1, tmA, tmB, b1, (int)n, tile_first, m_tiles, n_splits,
+        XQ_CUDA(launch_pdl(l1_gemm_kernel<EPI_ROWMAX>, grid, dim3(kGemmThreads), kGemmSmem, stream, 1, tmA, tmB, b1, (int)n, m_tiles, n_splits,
                            zpart, zstride, (float*)nullptr));
     else
-        XQ_CUDA(launch_pdl(l1_gemm_kernel<EPI_STORE_TANH>, grid, dim3(kGemmThreads), kGemmSmem, stream, 1, tmA, tmB, b1, (int)n, tile_first, m_tiles, n_splits,
+        XQ_CUDA(launch_pdl(l1_gemm_kernel<EPI_STORE_TANH>, grid, dim3(kGemmThreads), kGemmSmem, stream, 1, tmA, tmB, b1, (int)n, m_tiles, n_splits,
                            (float*)nullptr, zstride, q));
     return XQ_OK;
 }
@@ -1741,8 +1674,7 @@ int dqn_q90_device(xq_dqn_s* h, const xq_env_rec* envs_dev, int64_t n, float* q9
         f->act_slot ^= 1;
         f->actq_version = f->w_version;
     }
-    static const bool incremental = [] { const char* e = getenv("XQ_ACT_INCREMENTAL"); return !(e && atoi(e) == 0); }();     // 0: gather every ply (A/B runs; same results)
-    const int fresh_all = (!incremental || f->actz_version != f->w_version) ? 1 : 0;
+    const int fresh_all = f->actz_version != f->w_version ? 1 : 0;
     // `carried`: the caller's act_team_kernel has already brought the sums, the remembered boards and h(s) of these n envs up to date
     // (tail of the previous ply of the same xq_selfplay_collect call); only valid while nothing else could have touched them
     if (!(carried && !fresh_all && n == f->act_carried_n)) {
@@ -1754,7 +1686,7 @@ int dqn_q90_device(xq_dqn_s* h, const xq_env_rec* envs_dev, int64_t n, float* q9
     f->act_carried_n = n;
     if (carry) {
         carry->W0Q = f->W0Q; carry->zOpen = f->zOpen; carry->inv_scale = reinterpret_cast<const float*>(f->actMax + 2);
-        carry->Z = incremental ? f->actZ : nullptr; carry->Prev = f->actPrev; carry->Hhi = f->actHhi; carry->Hlo = f->actHlo;
+        carry->Z = f->actZ; carry->Prev = f->actPrev; carry->Hhi = f->actHhi; carry->Hlo = f->actHlo;
     }
     const int m_tiles = (int)((n + BM - 1) / BM);
     XQ_CUDA(launch_pdl(q90_gemm_kernel, dim3(m_tiles < 148 ? m_tiles : 148), dim3(kGemmThreads), kQSmem, stream, 1, f->tmActHi, f->tmActLo, f->tmW1q,
@@ -1762,30 +1694,30 @@ int dqn_q90_device(xq_dqn_s* h, const xq_env_rec* envs_dev, int64_t n, float* q9
     return XQ_OK;
 }
 
-// Part `part` of `n_parts` of the n envs of a collector call whose layer-0 sums are carried by the act kernel (dqn_q90_device has run for the
-// whole range in this call): only the contraction, on `stream`, with tensor maps over the part's rows of h(s).  Parts are equal multiples of
-// the 128-env tile (the last one takes the rest); *off / *m return the part's env range.
-int dqn_q90_part(xq_dqn_s* h, int64_t n, int n_parts, int part, float* q90_dev, cudaStream_t stream, ActCarry* carry, int64_t* off_out, int64_t* m_out) {
+// Half `half` (0 or 1) of the n envs of a collector call whose layer-0 sums are carried by the act kernel (dqn_q90_device has run for the
+// whole range in this call): only the contraction, on `stream`, with tensor maps over the half's rows of h(s).  The first half is a multiple
+// of the 128-env tile, the second takes the rest; *off / *m return the half's env range.
+int dqn_q90_half(xq_dqn_s* h, int64_t n, int half, float* q90_dev, cudaStream_t stream, ActCarry* carry, int64_t* off_out, int64_t* m_out) {
     Fast* f = h->fast;
-    if (!f || n != f->act_rows || n != f->act_carried_n) return fail(XQ_ERR_STATE, "dqn_q90_part: the whole range has not been prepared");
-    if (n_parts < 1 || n_parts > 4 || part < 0 || part >= n_parts) return fail(XQ_ERR_INVALID, "dqn_q90_part: bad part");
-    const int64_t size = ((n + n_parts - 1) / n_parts + BM - 1) / BM * BM;
-    if (size * (n_parts - 1) >= n) return fail(XQ_ERR_INVALID, "dqn_q90_part: too few envs for %d parts", n_parts);
-    if (f->act_sub_n != n || f->act_sub_parts != n_parts) {
-        for (int k = 0; k < n_parts; ++k) {
+    if (!f || n != f->act_rows || n != f->act_carried_n) return fail(XQ_ERR_STATE, "dqn_q90_half: the whole range has not been prepared");
+    if (half < 0 || half > 1) return fail(XQ_ERR_INVALID, "dqn_q90_half: bad half");
+    const int64_t size = ((n + 1) / 2 + BM - 1) / BM * BM;
+    if (size >= n) return fail(XQ_ERR_INVALID, "dqn_q90_half: too few envs for two halves");
+    if (f->act_sub_n != n) {
+        for (int k = 0; k < 2; ++k) {
             const int64_t o = k * size, m = std::min<int64_t>(size, n - o);
             if (int rc = make_tmap(&f->tmActHiS[k], f->actHhi + o * kHid, m, BM)) return rc;
             if (int rc = make_tmap(&f->tmActLoS[k], f->actHlo + o * kHid, m, BM)) return rc;
         }
-        f->act_sub_n = n; f->act_sub_parts = n_parts;
+        f->act_sub_n = n;
     }
-    const int64_t off = part * size, m = std::min<int64_t>(size, n - off);
+    const int64_t off = half * size, m = std::min<int64_t>(size, n - off);
     if (carry) {
         carry->W0Q = f->W0Q; carry->zOpen = f->zOpen; carry->inv_scale = reinterpret_cast<const float*>(f->actMax + 2);
         carry->Z = f->actZ + off * kHid; carry->Prev = f->actPrev + off * 12; carry->Hhi = f->actHhi + off * kHid; carry->Hlo = f->actHlo + off * kHid;
     }
     const int m_tiles = (int)((m + BM - 1) / BM);
-    XQ_CUDA(launch_pdl(q90_gemm_kernel, dim3(m_tiles < 148 ? m_tiles : 148), dim3(kGemmThreads), kQSmem, stream, 1, f->tmActHiS[part], f->tmActLoS[part], f->tmW1q,
+    XQ_CUDA(launch_pdl(q90_gemm_kernel, dim3(m_tiles < 148 ? m_tiles : 148), dim3(kGemmThreads), kQSmem, stream, 1, f->tmActHiS[half], f->tmActLoS[half], f->tmW1q,
                        f->tmW1loq, (const float*)f->b1, (int)m, m_tiles, q90_dev + off * QN));
     *off_out = off; *m_out = m;
     return XQ_OK;
@@ -1871,7 +1803,7 @@ int dqn_exchange_apply(xq_dqn_s* h, double lr);
 // n_updates sequential TD updates on replay draws (counters counter0, counter0 + 1, ...), bit-identical to n_updates calls of
 // dqn_td_update_sampled(..., use_target_net = 1, apply = 1), but software-pipelined over two streams: between two target syncs the
 // bootstrap branch of an update -- h(s') with the TARGET net and the [B x 128] x [128 x 8100] row-max GEMM -- does not depend on the
-// online weights, so for update i+1 (and i+2) it runs on an auxiliary stream underneath update i's online branch
+// online weights, so for update i+1 it runs on an auxiliary stream underneath update i's online branch
 // [h(s) -> TD error -> gradient contraction + SGD], which alone stays on the critical path.  Two slots of (h(s'), row-max partials).
 int dqn_td_update_pipelined(xq_dqn_s* h, const void* ring, int64_t size, uint64_t seed, uint32_t counter0, int64_t n, int n_updates, double lr) {
     if (int rc = ensure_fast(h)) return rc;
@@ -1887,29 +1819,28 @@ int dqn_td_update_pipelined(xq_dqn_s* h, const void* ring, int64_t size, uint64_
                                                                                           // when both branches have EQUAL priority (29.0 us per update; 34.4 with the
                                                                                           // online branch on a higher-priority stream, 41 with the bootstrap branch higher)
         XQ_CUDA(cudaEventCreateWithFlags(&f->ev_fork, cudaEventDisableTiming));
-        for (int i = 0; i < 2; ++i) { XQ_CUDA(cudaEventCreateWithFlags(&f->ev_aux[i], cudaEventDisableTiming)); XQ_CUDA(cudaEventCreateWithFlags(&f->ev_free[i], cudaEventDisableTiming)); XQ_CUDA(cudaEventCreateWithFlags(&f->ev_td[i], cudaEventDisableTiming)); }
+        for (int i = 0; i < 2; ++i) { XQ_CUDA(cudaEventCreateWithFlags(&f->ev_aux[i], cudaEventDisableTiming)); XQ_CUDA(cudaEventCreateWithFlags(&f->ev_td[i], cudaEventDisableTiming)); }
     }
     const int64_t ld = (f->cap + BM - 1) / BM * BM;
     // The online branch (the critical path) can run on a stream of the library with a HIGHER priority than the bootstrap branch.  Measured per
     // update (batch 4096 per GPU, us; equal priorities / online branch higher):  1 GPU 33.5 (29.6 .. 35.5 from call to call) / 34.6;  2 GPUs 36.3 / 38.9;
     // 8 GPUs 47.1 (43.9 .. 48.5) / 42.5 (+- 0.1).  With equal priorities the row-max GEMM of update i+1 and the 88 whole-SM CTAs of the contraction of
     // update i race for SMs; once the contraction also waits for its peers' row blocks (it then holds its SMs for ~17 us instead of ~10) losing that
-    // race costs more than the GEMM's loss of the SMs under the h(s) gather, so the default is: higher priority from 4 ranks on.  XQ_TD_MAIN_PRIO=0|1 forces.
-    static const int main_prio_env = [] { const char* e = getenv("XQ_TD_MAIN_PRIO"); return e ? atoi(e) : -1; }();
-    const int main_prio = main_prio_env >= 0 ? main_prio_env : (f->connected && f->world >= 4 ? 1 : 0);
+    // race costs more than the GEMM's loss of the SMs under the h(s) gather, so the rule is: higher priority from 4 ranks on.
+    const bool main_prio = f->connected && f->world >= 4;
     if (main_prio && !f->main_hi) {
         int lo = 0, hi = 0;
         XQ_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
         XQ_CUDA(cudaStreamCreateWithPriority(&f->main_hi, cudaStreamNonBlocking, hi));
     }
-    if (!f->ev_join) { XQ_CUDA(cudaEventCreateWithFlags(&f->ev_join, cudaEventDisableTiming)); for (int i = 0; i < 2; ++i) XQ_CUDA(cudaEventCreateWithFlags(&f->ev_tdb[i], cudaEventDisableTiming)); }
+    if (!f->ev_join) XQ_CUDA(cudaEventCreateWithFlags(&f->ev_join, cudaEventDisableTiming));
     cudaStream_t main = main_prio ? f->main_hi : h->stream, aux = f->aux;
     XQ_CUDA(cudaEventRecord(f->ev_fork, h->stream));             // the target net and the ring are final for the other streams
     XQ_CUDA(cudaStreamWaitEvent(aux, f->ev_fork, 0));
     if (main != h->stream) XQ_CUDA(cudaStreamWaitEvent(main, f->ev_fork, 0));
     // bootstrap branch of update i into slot i & 1, in two parts.  h(s') (small CTAs) is enqueued early and runs under the online branch of
-    // update i-1; the row-max GEMM needs a whole SM's shared memory per CTA, exactly like the gradient contraction of the online branch, so it
-    // is released only when update i-1 is complete and then runs next to update i's h(s) gather (which leaves the shared memory free).
+    // update i-1; the row-max GEMM needs a whole SM's shared memory per CTA, exactly like the gradient contraction of the online branch, so
+    // when it is released decides whether it sits on the critical path (below).
     auto aux_l0 = [&](int i) -> int {
         const int slot = i & 1;
         const BatchRef ref{reinterpret_cast<const uint8_t*>(ring), size, seed, counter0 + (uint32_t)i, 1};
@@ -1917,89 +1848,37 @@ int dqn_td_update_pipelined(xq_dqn_s* h, const void* ring, int64_t size, uint64_
                            slot ? f->H2bf_b : f->H2bf, f->cb, ld, f->info_slots, 0, 2));
         return XQ_OK;
     };
-    // When the row-max GEMM of update i+1 is released (XQ_TD_EARLY_GEMM, default 2) and into how many row splits it is cut (XQ_TD_GEMM_SPLITS,
-    // default 5 = 185 CTAs instead of 4 = 148) decides whether it sits on the critical path of update i+1:
-    //   0  when update i is complete: it then runs next to update i+1's h(s) gather, 12 us against 7 us -- the TD-error kernel waits for it
-    //   1  when the TD-error kernel of update i has run: the gradient contraction's 88 CTAs are resident by then (programmatic dependent
-    //      launch) and leave 60 SMs idle, on which a good part of the GEMM is done before the contraction ends
-    //   2  when the row-max partials of update i are in, i.e. BEFORE the TD-error kernel of update i: the GEMM's CTAs start under the
-    //      TD-error kernel (small CTAs, they co-reside), the contraction's 88 CTAs take their SMs as they become free, and
-    //      the GEMM is (nearly) done when the contraction ends.  Slot reuse: the partials slot of update i+1 was last read by the TD-error
-    //      kernel of update i-1, which precedes the event in stream order.
-    // Measured per update at batch 4096: mode 0 / 4 splits 36.4 us; mode 1: 36.4 / 34.0 / 34.8 / 36.2 us with 4 / 5 / 6 / 7 splits;
-    // mode 2: 29.6 / 29.0 / 29.0 / 31.1 us with 4 / 5 / 6 / 8 splits; enqueued a whole update ahead (no event): 33.4 us.  Same results bit for bit.
-    static const int early = [] { const char* e = getenv("XQ_TD_EARLY_GEMM"); return e ? atoi(e) : 2; }();
-    static const int splits = [] { const char* e = getenv("XQ_TD_GEMM_SPLITS"); return e ? atoi(e) : 0; }();
-    static const bool fuse_exchange = [] { const char* e = getenv("XQ_DIST_FUSED_GEMM"); return !(e && atoi(e) == 0); }();   // 0: exchange in a kernel of its own (A/B runs)
-    //   3  TWO updates ahead, when update i is complete: the GEMM of update i+2 then runs under the h(s) gather and the TD-error kernel of update
-    //      i+1 -- small CTAs it co-resides with on all 148 SMs -- and is out of the way when the contraction of update i+1 wants 88 whole SMs (11
-    //      clusters of 8 in one GPC each): nothing races for SMs any more.  Slot reuse: the partials slot of update i+2 was last read by the
-    //      TD-error kernel of update i, h(s') of update i+2 is written after the GEMM of update i in stream order.
-    //   4  in TWO parts sized for the two windows of update i that tolerate it: part A (XQ_TD_GEMM_A_TILES of the 32 row tiles, default 20, one short
-    //      CTA per SM: 37 column tiles x 4 row splits) is released before the TD-error kernel of update i, co-resides with its small CTAs and is gone
-    //      when the contraction's 88 whole-SM CTAs want their SMs; part B (the other row tiles, 37 x 2 CTAs) is released when the TD-error kernel has
-    //      COMPLETED -- the contraction's CTAs are resident by then (programmatic dependent launch) -- and runs on the 60 SMs they leave free.  Nothing
-    //      of the GEMM is left when the h(s) gather of update i+1 (which cannot share an SM with a GEMM CTA: registers) starts: no race for SMs.
-    //   5  when every CTA of the gradient contraction of update i has BEGUN execution (cudaLaunchAttributeLaunchCompletionEvent on that launch):
-    //      with programmatic dependent launch the contraction's 88 CTAs become resident while the TD-error kernel still runs, so the GEMM is
-    //      released a few microseconds after mode 2 would release it -- but never before the contraction holds its SMs: the order the "fast"
-    //      calls of mode 2 happen to get, made the only order.
-    static const int a_tiles = [] { const char* e = getenv("XQ_TD_GEMM_A_TILES"); return e ? atoi(e) : 20; }();
+    // The row-max GEMM of update i+1 is released when the row-max partials of update i are in, i.e. BEFORE the TD-error kernel of update i:
+    // the GEMM's CTAs start under the TD-error kernel (small CTAs, they co-reside), the contraction's 88 CTAs take their SMs as they become
+    // free, and the GEMM is (nearly) done when the contraction ends.  It is cut into 5 row splits (185 CTAs instead of 4 x 37 = 148).  Slot
+    // reuse: the partials slot of update i+1 was last read by the TD-error kernel of update i-1, which precedes the event in stream order.
+    // Measured per update at batch 4096: 29.0 us; 29.6 / 29.0 / 31.1 us with 4 / 6 / 8 splits; released when update i is complete 36.4 us,
+    // after its TD-error kernel 34.0 us; enqueued a whole update ahead (no event) 33.4 us.  Same results bit for bit (DESIGN.md section 4).
     auto aux_gemm = [&](int i, cudaEvent_t gate) -> int {
         const int slot = i & 1;
         if (gate) XQ_CUDA(cudaStreamWaitEvent(aux, gate, 0));
-        if (int rc = launch_gemm(h, EPI_ROWMAX, slot ? f->tmH2_b : f->tmH2, f->tmTW1, f->tb1, n, nullptr, aux, slot ? f->zpart_b : f->zpart,
-                                 splits > 0 ? splits : (early ? 5 : 0))) return rc;
+        if (int rc = launch_gemm(h, EPI_ROWMAX, slot ? f->tmH2_b : f->tmH2, f->tmTW1, f->tb1, n, nullptr, aux, slot ? f->zpart_b : f->zpart, 5)) return rc;
         XQ_CUDA(cudaEventRecord(f->ev_aux[slot], aux));
         return XQ_OK;
     };
-    auto aux_gemm_part = [&](int i, cudaEvent_t gate, bool part_b) -> int {
-        const int slot = i & 1;
-        if (gate) XQ_CUDA(cudaStreamWaitEvent(aux, gate, 0));
-        if (int rc = launch_gemm(h, EPI_ROWMAX, slot ? f->tmH2_b : f->tmH2, f->tmTW1, f->tb1, n, nullptr, aux, slot ? f->zpart_b : f->zpart,
-                                 part_b ? 2 : 4, part_b ? a_tiles : 0, part_b ? 0 : a_tiles)) return rc;
-        if (part_b) XQ_CUDA(cudaEventRecord(f->ev_aux[slot], aux));
-        return XQ_OK;
-    };
-    // the update before update i has consumed the slot of update i in modes 0-2: gate on its TD-error kernel (modes 1, 2) or its completion (mode 0)
-    auto gate_of = [&](int i) -> cudaEvent_t { return i >= 1 ? (early ? f->ev_td[(i - 1) & 1] : f->ev_free[(i - 1) & 1]) : nullptr; };
     if (int rc = aux_l0(0)) return rc;
-    if (early == 4) { if (int rc = aux_gemm_part(0, nullptr, false)) return rc; if (int rc = aux_gemm_part(0, nullptr, true)) return rc; }
-    else if (int rc = aux_gemm(0, nullptr)) return rc;
-    if (early == 3 && n_updates > 1) {      // fill: the first two bootstrap branches start at once
-        if (int rc = aux_l0(1)) return rc;
-        if (int rc = aux_gemm(1, nullptr)) return rc;
-    }
+    if (int rc = aux_gemm(0, nullptr)) return rc;
     for (int i = 0; i < n_updates; ++i) {
         const int slot = i & 1;
         const BatchRef ref{reinterpret_cast<const uint8_t*>(ring), size, seed, counter0 + (uint32_t)i, 1};
-        if (early == 3) { if (i + 2 < n_updates) if (int rc = aux_l0(i + 2)) return rc; }
-        else if (i + 1 < n_updates) if (int rc = aux_l0(i + 1)) return rc;
+        if (i + 1 < n_updates) if (int rc = aux_l0(i + 1)) return rc;
         XQ_CUDA(launch_pdl(l0_pair_kernel, dim3(blocks(n, kL0Warps)), dim3(kL0Warps * 32), 0, main, 1, ref, n, f->W0T, f->b0, f->tW0T, f->tb0, f->Hf,
                            f->H2bf, f->cb, ld, f->info_slots, kInfoSlots * 4, 1));
         XQ_CUDA(cudaStreamWaitEvent(main, f->ev_aux[slot], 0));  // the row-max partials of this update
-        // XQ_TD_FIRST_LATE=k (probe): the first k updates of a call release the next GEMM AFTER their TD-error kernel (mode 1) -- the contraction of
-        // update 0 then certainly gets its SMs first; does the pipeline stay in that order for the rest of the call?
-        static const int first_late = [] { const char* e = getenv("XQ_TD_FIRST_LATE"); return e ? atoi(e) : 0; }();
-        const bool late = early == 2 && i < first_late;
-        if (early == 2 && !late) { XQ_CUDA(cudaEventRecord(f->ev_td[slot], main)); if (i + 1 < n_updates) if (int rc = aux_gemm(i + 1, gate_of(i + 1))) return rc; }
-        if (early == 4) { XQ_CUDA(cudaEventRecord(f->ev_td[slot], main)); if (i + 1 < n_updates) if (int rc = aux_gemm_part(i + 1, f->ev_td[slot], false)) return rc; }
+        XQ_CUDA(cudaEventRecord(f->ev_td[slot], main));
+        if (i + 1 < n_updates) if (int rc = aux_gemm(i + 1, f->ev_td[slot])) return rc;
         XQ_CUDA(launch_pdl(td_delta_kernel, dim3(blocks(n * 32, 256)), dim3(256), 0, main, 1, f->cb, n, f->Hf, f->W1, f->b1, slot ? f->zpart_b : f->zpart,
                            ld, kParts, (float)h->gamma, h->mode, f->d0hi, f->d0lo, f->ghi, f->glo, ld, f->info_slots));
-        if (early == 1 || late) { XQ_CUDA(cudaEventRecord(f->ev_td[slot], main)); if (i + 1 < n_updates) if (int rc = aux_gemm(i + 1, gate_of(i + 1))) return rc; }
-        if (early == 4) { XQ_CUDA(cudaEventRecord(f->ev_tdb[slot], main)); if (i + 1 < n_updates) if (int rc = aux_gemm_part(i + 1, f->ev_tdb[slot], true)) return rc; }
-        if (early == 5 && i + 1 < n_updates) g_launched_event = f->ev_tdb[slot];
+        // multi-GPU: the contraction exchanges the gradient and applies the SGD step itself
         XQ_CUDA(launch_pdl(dw_gemm_kernel, dim3(kDwMTiles, kDwSplits), dim3(kDwThreads), kDwSmem, main, kDwSplits, f->tmD0hi, f->tmD0lo, f->tmGhi,
                            f->tmGlo, f->tmCb, (int)n, f->part, f->dbpart, f->info_slots, f->info, cur_grad(f), f->W0T, f->b0, f->W1, f->b1, f->W1bf,
-                           f->W1lo, (float)lr, f->connected ? 0 : 1, dw_push(f, !f->connected, fuse_exchange)));
-        if (early == 5 && i + 1 < n_updates) if (int rc = aux_gemm(i + 1, f->ev_tdb[slot])) return rc;
-        if (f->connected) {      // multi-GPU
-            if (fuse_exchange) { ++f->epoch; f->parity ^= 1; }                  // the contraction exchanged the gradient and applied the SGD step itself
-            else if (int rc = dqn_exchange_apply(h, lr)) return rc;              // two kernels: push + [wait, sum, SGD]
-        }
-        XQ_CUDA(cudaEventRecord(f->ev_free[slot], main));
-        if (!early && i + 1 < n_updates) if (int rc = aux_gemm(i + 1, gate_of(i + 1))) return rc;
-        if (early == 3 && i + 2 < n_updates) if (int rc = aux_gemm(i + 2, f->ev_free[slot])) return rc;
+                           f->W1lo, (float)lr, f->connected ? 0 : 1, dw_push(f, !f->connected, true)));
+        if (f->connected) { ++f->epoch; f->parity ^= 1; }
     }
     if (main != h->stream) {                // the online branch ran on the library's own high-priority stream: join
         XQ_CUDA(cudaEventRecord(f->ev_join, main));
@@ -2097,8 +1976,6 @@ int xq_dqn_dist_connect(xq_dqn_t h, int rank, int world, const void* handles) {
         int khz = 0;
         XQ_CUDA(cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, h->device));
         f->timeout_ticks = (long long)(ms * (double)(khz > 0 ? khz : 2000000));
-        const char* m = getenv("XQ_DIST_FUSED_MODE");
-        f->fused_mode = (m && !strcmp(m, "allgather")) ? DW_FUSED_ALLGATHER : DW_FUSED_OWNER;
     }
     return XQ_OK;
 }

@@ -63,7 +63,7 @@ int dqn_fast_weights(xq_dqn_s* h, FastWeights* out);
 // `carried`: skip the layer-0 kernel because the caller's act_team_kernel kept the per-env sums and h(s) current; `carry` receives what it needs to do so
 int dqn_q90_device(xq_dqn_s* h, const xq_env_rec* envs_dev, int64_t n, float* q90_dev, cudaStream_t stream, bool carried = false, ActCarry* carry = nullptr);
 // the contraction for part `part` of `n_parts` of a prepared, carried env range (multi-stream collector plies)
-int dqn_q90_part(xq_dqn_s* h, int64_t n, int n_parts, int part, float* q90_dev, cudaStream_t stream, xq::ActCarry* carry, int64_t* off_out, int64_t* m_out);
+int dqn_q90_half(xq_dqn_s* h, int64_t n, int half, float* q90_dev, cudaStream_t stream, xq::ActCarry* carry, int64_t* off_out, int64_t* m_out);
 // TD update on n uniform draws from a replay ring, resolved in place (no gather pass)
 int dqn_td_update_sampled(xq_dqn_s* h, const void* ring, int64_t size, uint64_t seed, uint32_t counter, int64_t n, int use_target_net,
                           double lr, int apply);   // brings the FP32 copies up to date and returns them   // the FP64 target parameters were rewritten

@@ -300,7 +300,7 @@ struct xq_env_s {
     uint32_t* d_lists = nullptr;      // n*64 words, allocated on first use
     xq_trace_rec* d_trace = nullptr; int64_t trace_cap = 0;
     double* d_state = nullptr;
-    uint8_t* d_nonstd = nullptr;      // n flags written by the slot kernel
+    uint8_t* d_nonstd = nullptr;      // n flags written by the fused rollout and list kernels
     bool maybe_nonstd = false;        // set once boards were injected (xq_env_set_boards)
     // finished-game events of the self-play collector (xq_env_enable_game_events)
     xq_game_event* d_events = nullptr; unsigned long long* d_event_count = nullptr; int64_t event_cap = 0; uint32_t event_ply = 0;
@@ -316,9 +316,7 @@ struct xq_env_s {
 static inline unsigned grid_for(int64_t n, int per_block) { return (unsigned)((n + per_block - 1) / per_block); }
 
 namespace xq {
-cudaError_t launch_rollout_slots(xq_env_rec* envs, int64_t n, uint64_t env_id0, uint64_t seed, int n_plies, xq_trace_rec* trace,
-                                 xq_env_stats* stats, uint8_t* nonstd, cudaStream_t stream);
-cudaError_t launch_rollout_team(int team, xq_env_rec* envs, int64_t n, uint64_t env_id0, uint64_t seed, int n_plies, xq_trace_rec* trace,
+cudaError_t launch_rollout_team(xq_env_rec* envs, int64_t n, uint64_t env_id0, uint64_t seed, int n_plies, xq_trace_rec* trace,
                                 xq_env_stats* stats, uint8_t* nonstd, cudaStream_t stream, const xq_env_rec* src, xq_env_rec* mirror);
 cudaError_t launch_legal_moves_team(const xq_env_rec* envs, int64_t n, uint8_t* counts, uint32_t* actions, uint8_t* nonstd, cudaStream_t stream);
 cudaError_t launch_rollout_lane(xq_env_rec* envs, int64_t n, uint64_t env_id0, uint64_t seed, int n_plies, xq_trace_rec* trace, xq_env_stats* stats,
@@ -329,30 +327,26 @@ cudaError_t launch_pick_random(const xq_env_rec* envs, int64_t n, uint64_t env_i
 }
 // ordered action lists of every env into h->d_u8[0] (counts) and h->d_lists ([n][128] u16): the register-resident kernel (xq_rollout_lane.cu)
 // for every board with a standard piece set, then the generic thread-per-board kernel for the boards it flagged (only possible after
-// xq_env_set_boards injected exotic positions).  XQ_LEGAL_LANE=0 runs the generic kernel on every env (A/B runs); same results.
+// xq_env_set_boards injected exotic positions).
 static int launch_legal_moves(xq_env_s* h) {
-    static const bool lane = [] { const char* e = getenv("XQ_LEGAL_LANE"); return !(e && atoi(e) == 0); }();
     h->async_dirty = true;
     if (!h->d_lists) XQ_CUDA(cudaMalloc(&h->d_lists, sizeof(uint32_t) * 64 * h->n));
     // few envs: the team kernel (4 threads per board, a quarter of the per-thread chain); many: one thread per board.  XQ_LEGAL_TEAM=0|1 forces.
     // (read per call: the tests switch kernels inside one process)
     const char* te = getenv("XQ_LEGAL_TEAM");
-    const char* tm = getenv("XQ_LEGAL_TEAM_MAX");
     const int team_env = te ? atoi(te) : -1;
-    const int64_t team_max = tm ? (int64_t)atoll(tm) : (int64_t)18944;      // 592 schedulers x 32: measured 12.3 against 14.4 us at 16,384 envs, 16.4 both at 24,576
-    const bool team = team_env >= 0 ? team_env != 0 : h->n <= team_max;
-    if (lane && team) XQ_CUDA(launch_legal_moves_team(h->d_envs, h->n, h->d_u8[0], h->d_lists, h->d_nonstd, h->stream));
-    else if (lane) XQ_CUDA(launch_legal_moves_lane(h->d_envs, h->n, h->d_u8[0], h->d_lists, h->d_nonstd, h->stream));
-    if (!lane || h->maybe_nonstd) {
-        legal_moves_kernel<<<grid_for(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->d_u8[0], h->d_lists, lane ? h->d_nonstd : nullptr);
+    const bool team = team_env >= 0 ? team_env != 0 : h->n <= 18944;      // 592 schedulers x 32: measured 12.3 against 14.4 us at 16,384 envs, 16.4 both at 24,576
+    if (team) XQ_CUDA(launch_legal_moves_team(h->d_envs, h->n, h->d_u8[0], h->d_lists, h->d_nonstd, h->stream));
+    else XQ_CUDA(launch_legal_moves_lane(h->d_envs, h->n, h->d_u8[0], h->d_lists, h->d_nonstd, h->stream));
+    if (h->maybe_nonstd) {
+        legal_moves_kernel<<<grid_for(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->d_u8[0], h->d_lists, h->d_nonstd);
         XQ_LAUNCH_CHECK();
     }
     return XQ_OK;
 }
 // threads per board of the fused rollout kernel: 1 = rollout_lane_kernel (xq_rollout_lane.cu: the whole board in one thread's registers,
-// no barrier, nothing replicated), the default above 9,472 envs (148 SMs x 64); 4 = rollout_team_kernel<4> (xq_rollout_team.cu), the default below;
-// 8 = rollout_team_kernel<8> and 16 = rollout_slots_kernel (xq_rollout.cu) are kept for A/B runs: XQ_ROLLOUT_TEAM=1|4|8|16 forces one.
-// All four are bit-identical.
+// no barrier, nothing replicated), the default above 9,472 envs (148 SMs x 64); 4 = rollout_team_kernel (xq_rollout_team.cu), the default below.
+// XQ_ROLLOUT_TEAM=1|4 forces one (scripts/rollout_sweep.py re-measures the crossover).  Both are bit-identical.
 // Measured on one B200 (steps/s, 200 / 200 / 100 / 32 plies per launch):   envs      4096     8192     16,384    65,536    1M
 //   board per thread (1)                                                             2.98e9   5.94e9   1.17e10   1.61e10   1.83e10
 //   team of 4 (4)                                                                    3.90e9   6.45e9   8.6e9     1.04e10   1.01e10
@@ -361,10 +355,10 @@ static int launch_legal_moves(xq_env_s* h) {
 // fewer instructions per env step (56 against 87 warp-instructions) wins.
 static int rollout_team(int64_t n) {
     static const int forced = [] { const char* e = getenv("XQ_ROLLOUT_TEAM"); return e ? atoi(e) : 0; }();
-    if (forced == 1 || forced == 4 || forced == 8 || forced == 16) return forced;
+    if (forced == 1 || forced == 4) return forced;
     return n <= 148 * 64 ? 4 : 1;      // up to two team CTAs (32 boards each) per SM; measured (env steps/s, team / lane): 4096 3.9e9 / 3.0e9, 8192 6.4e9 / 5.9e9, 10,240 6.6e9 / 7.4e9
 }
-// Fused rollout = team kernel (xq_rollout_team.cu; or the 16-thread slot kernel, xq_rollout.cu) for every board with a standard piece set, then the generic
+// Fused rollout = lane or team kernel (xq_rollout_lane.cu, xq_rollout_team.cu) for every board with a standard piece set, then the generic
 // thread-per-board kernel for the boards it flagged (only possible after xq_env_set_boards injected exotic positions).
 // src / mirror (optional, xq_env_rollout_random_io with pinned host buffers): the kernels read the boards straight from MAPPED host memory and
 // write the final boards to mapped host memory as well as to the device array -- no copy launches on the stream.  A board the first kernel leaves
@@ -372,10 +366,8 @@ static int rollout_team(int64_t n) {
 static int launch_rollout(xq_env_s* h, int n_plies, xq_trace_rec* d_trace, const xq_env_rec* src = nullptr, xq_env_rec* mirror = nullptr) {
     if (n_plies >= (1 << 24)) return fail(XQ_ERR_INVALID, "rollout: n_plies must be < 2^24 per launch");
     h->async_dirty = true;
-    const int team = rollout_team(h->n);
-    if (team == 1) XQ_CUDA(launch_rollout_lane(h->d_envs, h->n, h->env_id0, h->seed, n_plies, d_trace, h->d_stats, h->d_nonstd, h->stream, src, mirror));
-    else if (team == 16) XQ_CUDA(launch_rollout_slots(h->d_envs, h->n, h->env_id0, h->seed, n_plies, d_trace, h->d_stats, h->d_nonstd, h->stream));
-    else XQ_CUDA(launch_rollout_team(team, h->d_envs, h->n, h->env_id0, h->seed, n_plies, d_trace, h->d_stats, h->d_nonstd, h->stream, src, mirror));
+    if (rollout_team(h->n) == 1) XQ_CUDA(launch_rollout_lane(h->d_envs, h->n, h->env_id0, h->seed, n_plies, d_trace, h->d_stats, h->d_nonstd, h->stream, src, mirror));
+    else XQ_CUDA(launch_rollout_team(h->d_envs, h->n, h->env_id0, h->seed, n_plies, d_trace, h->d_stats, h->d_nonstd, h->stream, src, mirror));
     if (h->maybe_nonstd) {
         rollout_random_kernel<<<grid_for(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->env_id0, h->seed, n_plies, d_trace,
                                                                                     h->d_stats, h->d_nonstd, mirror);
@@ -385,8 +377,7 @@ static int launch_rollout(xq_env_s* h, int n_plies, xq_trace_rec* d_trace, const
 }
 // device alias of a pinned, mapped, 16-byte aligned host buffer (cudaHostAlloc / cudaHostRegister under unified addressing), or null
 static void* mapped_alias(const void* host) {
-    static const bool on = [] { const char* e = getenv("XQ_IO_ZEROCOPY"); return !(e && atoi(e) == 0); }();
-    if (!on || !host || (reinterpret_cast<uintptr_t>(host) & 15u)) return nullptr;
+    if (!host || (reinterpret_cast<uintptr_t>(host) & 15u)) return nullptr;
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, host) != cudaSuccess) { cudaGetLastError(); return nullptr; }
     return a.type == cudaMemoryTypeHost ? a.devicePointer : nullptr;
@@ -698,8 +689,7 @@ static int rollout_io_enqueue(xq_env_s* h, const xq_env_rec* boards_in_host, int
     if (!h->ev_io) XQ_CUDA(cudaEventCreateWithFlags(&h->ev_io, cudaEventDisableTiming));
     const int64_t need = (int64_t)n_plies * h->n;
     if (trace_host) if (int rc = reserve_trace(h, need)) return rc;
-    static const bool side_on = [] { const char* e = getenv("XQ_IO_SIDE_STREAMS"); return !(e && atoi(e) == 0); }();
-    if (side_streams && side_on) {
+    if (side_streams) {
         if (!h->io_in) {
             XQ_CUDA(cudaStreamCreateWithFlags(&h->io_in, cudaStreamNonBlocking)); XQ_CUDA(cudaStreamCreateWithFlags(&h->io_out, cudaStreamNonBlocking));
             XQ_CUDA(cudaEventCreateWithFlags(&h->ev_in, cudaEventDisableTiming)); XQ_CUDA(cudaEventCreateWithFlags(&h->ev_run, cudaEventDisableTiming));
@@ -726,10 +716,9 @@ static int rollout_io_enqueue(xq_env_s* h, const xq_env_rec* boards_in_host, int
         h->io_pending = true;      // nothing else may be called on the handle until _wait: the copies out are not ordered against the compute stream
         return XQ_OK;
     }
-    // pinned (mapped) host buffers are read / written by the rollout kernel itself: two copy launches less on the stream (XQ_IO_ZEROCOPY=0: always copy)
-    const bool direct = rollout_team(h->n) != 16;
-    const xq_env_rec* src = direct ? static_cast<const xq_env_rec*>(mapped_alias(boards_in_host)) : nullptr;
-    xq_env_rec* mirror = direct ? static_cast<xq_env_rec*>(mapped_alias(boards_out_host)) : nullptr;
+    // pinned (mapped) host buffers are read / written by the rollout kernel itself: two copy launches less on the stream
+    const xq_env_rec* src = static_cast<const xq_env_rec*>(mapped_alias(boards_in_host));
+    xq_env_rec* mirror = static_cast<xq_env_rec*>(mapped_alias(boards_out_host));
     if (boards_in_host) {
         if (!src) XQ_CUDA(cudaMemcpyAsync(h->d_envs, boards_in_host, sizeof(xq_env_rec) * h->n, cudaMemcpyHostToDevice, h->stream));
         h->maybe_nonstd = true;

@@ -6,7 +6,7 @@
 // instead of 16 times.  The ply itself lives in xq_rollout_team.cuh (host-compilable, diffed against the oracle by
 // tests/hostsim); this file is the load / store conversion, the barriers and the launch.
 //
-// Replaces the loop body of ChessAI::train without the network (src/chessai.cpp:96-119), like rollout_slots_kernel.
+// Replaces the loop body of ChessAI::train without the network (src/chessai.cpp:96-119).
 #include "xq_common.cuh"
 #include "xq_rollout_team.cuh"
 
@@ -179,14 +179,13 @@ __global__ void __launch_bounds__(kTB * T) rollout_team_kernel(xq_env_rec* __res
     }
 }
 
-cudaError_t launch_rollout_team(int team, xq_env_rec* envs, int64_t n, uint64_t env_id0, uint64_t seed, int n_plies, xq_trace_rec* trace,
+cudaError_t launch_rollout_team(xq_env_rec* envs, int64_t n, uint64_t env_id0, uint64_t seed, int n_plies, xq_trace_rec* trace,
                                 xq_env_stats* stats, uint8_t* nonstd, cudaStream_t stream, const xq_env_rec* src, xq_env_rec* mirror) {
     const unsigned grid = (unsigned)((n + kTB - 1) / kTB);
     const char* ve = getenv("XQ_TEAM_VIEW");      // A/B and tests (read per call): 0 registers, 1 shared-memory view
     const int view_env = ve ? atoi(ve) : -1;
     const bool mem = view_env >= 0 ? view_env != 0 : n > 148 * kTB;      // more than one CTA per SM: issue-bound enough for the view to pay (4.84e9 against 4.66e9 at 6144 envs)
-    if (team == 8) rollout_team_kernel<8, false><<<grid, kTB * 8, 0, stream>>>(envs, n, env_id0, seed, n_plies, trace, stats, nonstd, src, mirror);
-    else if (mem) rollout_team_kernel<4, true><<<grid, kTB * 4, 0, stream>>>(envs, n, env_id0, seed, n_plies, trace, stats, nonstd, src, mirror);
+    if (mem) rollout_team_kernel<4, true><<<grid, kTB * 4, 0, stream>>>(envs, n, env_id0, seed, n_plies, trace, stats, nonstd, src, mirror);
     else rollout_team_kernel<4, false><<<grid, kTB * 4, 0, stream>>>(envs, n, env_id0, seed, n_plies, trace, stats, nonstd, src, mirror);
     ++g_launches;
     return cudaGetLastError();

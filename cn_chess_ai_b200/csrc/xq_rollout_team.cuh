@@ -3,7 +3,7 @@
 // after the other, phase by phase, and diffs the whole trace against the oracle before any GPU time); the kernel in
 // xq_rollout_team.cu is these phases with two __syncthreads per ply between them.
 //
-// Why teams: in the 16-threads-per-board kernel (rollout_slots_kernel) every thread keeps a replica of the board and repeats the
+// Why teams: in a 16-threads-per-board kernel (one thread per piece slot; DESIGN.md section 4) every thread keeps a replica of the board and repeats the
 // selection and the apply step -- ncu attributes 136 of its 407 warp-instructions per ply to move generation and 235 to the
 // replicated part.  With 4 slots per thread the replicated part is paid 4 times per board instead of 16 times, and warps stay
 // piece-type uniform: role = warp, lane = board, and position i of every lane of a warp holds the same piece type.
@@ -149,7 +149,7 @@ struct TeamPly {                   // scratch of one ply, phase A -> B -> C
     uint32_t cntw;
     uint32_t total;
 };
-// scores / material / reward / statistics / trace: role 0 alone, one barrier late (see rollout_slots_kernel)
+// scores / material / reward / statistics / trace: role 0 alone, one barrier late
 struct TeamBook {
     int red, black, mat_red, mat_black;
     uint32_t pend, pend_tr0;
@@ -183,7 +183,9 @@ XQ_HD void team_rng_chunk(const TeamRole& R, TeamShared<KB>& sh, int lane, int c
 }
 
 XQ_HD uint32_t team_mod_magic(uint32_t d) { return (0xFFFFFFFFu / d) + 1u; }
-XQ_HD uint32_t team_mod(uint32_t n, uint32_t d, uint32_t magic) {     // n % d, n < 2^31, 1 <= d <= 128 (see mod_small in xq_rollout.cu)
+// n % d for n < 2^31, 1 <= d <= 128 without a hardware divide: q = umulhi(n, ceil(2^32/d)) is floor(n/d) or one above
+// (error < n*d/2^32 < 1), so one conditional fix-up makes the remainder exact
+XQ_HD uint32_t team_mod(uint32_t n, uint32_t d, uint32_t magic) {
     const uint32_t q = umulhi_u(n, magic);
     const int32_t r = (int32_t)(n - q * d);
     return d == 1 ? 0u : (uint32_t)(r < 0 ? r + (int32_t)d : r);

@@ -36,12 +36,8 @@ cudaError_t launch_act_team(bool apply, xq_env_rec* envs, int64_t n, uint64_t en
                             uint16_t* actions_out, void* ring, int64_t ring_cap, int64_t ring_pos, xq_env_stats* stats, xq_game_event* events,
                             unsigned long long* event_count, int64_t event_cap, uint32_t event_ply, uint8_t* nonstd, const ActCarry* carry, uint32_t event_env0, cudaStream_t stream);
 
-cudaError_t launch_act_lane(bool apply, xq_env_rec* envs, int64_t n, uint64_t env_id0, uint64_t seed, const float* q90, uint32_t eps_thr, int train_done,
-                            uint16_t* actions_out, void* ring, int64_t ring_cap, int64_t ring_pos, xq_env_stats* stats, xq_game_event* events,
-                            unsigned long long* event_count, int64_t event_cap, uint32_t event_ply, uint8_t* nonstd, const ActCarry* carry, uint32_t event_env0, cudaStream_t stream);
-
 // Action selection (+ optional application), generic thread-per-board version (ordered list staged in shared memory): the fallback
-// of act_team_kernel (xq_act_team.cu) for boards with non-standard piece sets, or for every env with XQ_ACT_TEAM=0 (A/B runs).
+// of act_team_kernel (xq_act_team.cu) for boards with non-standard piece sets.
 template <bool APPLY>
 __global__ void __launch_bounds__(kThreads) act_kernel(xq_env_rec* __restrict__ envs, int64_t n, uint64_t env_id0, uint64_t seed,
                                                       const float* __restrict__ q90, uint32_t eps_thr, int train_done,
@@ -177,16 +173,17 @@ struct xq_replay_s {
 };
 
 // Scratch of the collector / xq_dqn_act, OWNED BY THE ENV HANDLE (two env handles on one device -- on different streams, or driven by two
-// host threads -- never share Q(s) rows, action buffers, auxiliary streams or fork / join events), released with it.
+// host threads -- never share Q(s) rows, action buffers, the auxiliary stream or fork / join events), released with it.
 struct SelfplayScratch {
     float* q90 = nullptr; int64_t cap = 0; uint16_t* actions = nullptr;
-    cudaStream_t aux[3] = {nullptr, nullptr, nullptr};
-    cudaEvent_t ev_fork = nullptr, ev_join[3] = {nullptr, nullptr, nullptr}, ev_order = nullptr;
+    cudaStream_t aux = nullptr;
+    cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_order = nullptr;
 };
 static void free_scratch(void* p) {
     SelfplayScratch* s = static_cast<SelfplayScratch*>(p);
     cudaFree(s->q90); cudaFree(s->actions);
-    for (int k = 0; k < 3; ++k) { if (s->aux[k]) cudaStreamDestroy(s->aux[k]); if (s->ev_join[k]) cudaEventDestroy(s->ev_join[k]); }
+    if (s->aux) cudaStreamDestroy(s->aux);
+    if (s->ev_join) cudaEventDestroy(s->ev_join);
     if (s->ev_fork) cudaEventDestroy(s->ev_fork);
     if (s->ev_order) cudaEventDestroy(s->ev_order);
     delete s;
@@ -220,25 +217,18 @@ static int order_after(cudaStream_t waiter, cudaStream_t producer, cudaEvent_t* 
 
 // One ply of selection (+ application) for every env: the team kernel (xq_act_team.cu) for boards with a standard piece set, then
 // the generic thread-per-board kernel for the boards it flagged (only possible after xq_env_set_boards injected exotic positions).
-// XQ_ACT_TEAM=0 runs the generic kernel on every env (A/B runs); both give the same results.
+// (A board-per-thread act kernel measured 74.7 us per ply against 60.5 at 65,536 envs: DESIGN.md section 4.)
 static int launch_act(bool apply, const EnvInfo& ei, const float* q90, uint32_t thr, int train_done, uint16_t* actions, Transition* ring, int64_t ring_cap,
                       int64_t ring_pos, xq_env_stats* stats, uint32_t event_ply, const ActCarry* carry = nullptr, uint32_t event_env0 = 0) {
-    static const bool team = [] { const char* e = getenv("XQ_ACT_TEAM"); return !(e && atoi(e) == 0); }();
-    // XQ_ACT_LANE=1: the board-per-thread kernel (xq_act_lane.cu) instead of the 4-threads-per-board kernel (xq_act_team.cu); same results.
-    // Measured at 65,536 envs: 74.7 us per ply against 60.5 -- see the header of xq_act_lane.cu -- so the team kernel stays the default.
-    static const bool lane = [] { const char* e = getenv("XQ_ACT_LANE"); return e && atoi(e) != 0; }();
-    if (team && lane) XQ_CUDA(launch_act_lane(apply, ei.d_envs, ei.n, ei.env_id0, ei.seed, q90, thr, train_done, actions, ring, ring_cap, ring_pos, stats,
-                                              ei.d_events, ei.d_event_count, ei.event_cap, event_ply, ei.d_nonstd, carry, event_env0, ei.stream));
-    else if (team) XQ_CUDA(launch_act_team(apply, ei.d_envs, ei.n, ei.env_id0, ei.seed, q90, thr, train_done, actions, ring, ring_cap, ring_pos, stats,
-                                      ei.d_events, ei.d_event_count, ei.event_cap, event_ply, ei.d_nonstd, carry, event_env0, ei.stream));
-    if (!team || ei.maybe_nonstd) {
-        const uint8_t* only = team ? ei.d_nonstd : nullptr;
+    XQ_CUDA(launch_act_team(apply, ei.d_envs, ei.n, ei.env_id0, ei.seed, q90, thr, train_done, actions, ring, ring_cap, ring_pos, stats,
+                            ei.d_events, ei.d_event_count, ei.event_cap, event_ply, ei.d_nonstd, carry, event_env0, ei.stream));
+    if (ei.maybe_nonstd) {
         if (apply)
             act_kernel<true><<<blocks(ei.n, kThreads), kThreads, 0, ei.stream>>>(ei.d_envs, ei.n, ei.env_id0, ei.seed, q90, thr, train_done, actions, ring, ring_cap,
-                                                                                ring_pos, stats, ei.d_events, ei.d_event_count, ei.event_cap, event_ply, only);
+                                                                                ring_pos, stats, ei.d_events, ei.d_event_count, ei.event_cap, event_ply, ei.d_nonstd);
         else
             act_kernel<false><<<blocks(ei.n, kThreads), kThreads, 0, ei.stream>>>(ei.d_envs, ei.n, ei.env_id0, ei.seed, q90, thr, train_done, actions, ring, ring_cap,
-                                                                                 ring_pos, stats, ei.d_events, ei.d_event_count, ei.event_cap, event_ply, only);
+                                                                                 ring_pos, stats, ei.d_events, ei.d_event_count, ei.event_cap, event_ply, ei.d_nonstd);
         XQ_LAUNCH_CHECK();
     }
     return XQ_OK;
@@ -366,16 +356,14 @@ int xq_selfplay_collect(xq_dqn_t h, xq_env_t env, xq_replay_t r, int n_plies, do
     const uint32_t thr = xq_eps_threshold(eps);
     // the team kernel carries the layer-0 sums and h(s) of its envs into the next ply (tail of act_team_kernel): from the second ply of
     // this call on, the layer-0 kernel is not launched.  Not when boards with non-standard piece sets may go through the generic kernel.
-    static const bool team = [] { const char* e = getenv("XQ_ACT_TEAM"); return !(e && atoi(e) == 0); }();
-    static const bool carry_on = [] { const char* e = getenv("XQ_ACT_CARRY"); return !(e && atoi(e) == 0); }();
-    const bool can_carry = team && carry_on && !ei.maybe_nonstd;
-    // Multi-stream plies (XQ_COLLECT_STREAMS, default 2): once the sums are carried, the env range is cut in equal parts that run their
-    // [contraction -> act] chains on streams of equal priority, out of step by themselves: the contraction of one part (tensor / HBM) and
-    // the tail of an act kernel (HBM) fill the SMs the other part's act kernel (instruction issue) leaves idle between its waves
-    static const int n_streams = [] { const char* e = getenv("XQ_COLLECT_STREAMS"); const int v = e ? atoi(e) : 2; return v < 1 ? 1 : (v > 4 ? 4 : v); }();
-    const bool multi = can_carry && n_streams > 1 && ei.n >= 4096 * n_streams;
+    const bool can_carry = !ei.maybe_nonstd;
+    // Two-stream plies from 8192 envs on: once the sums are carried, the env range is cut in two halves that run their
+    // [contraction -> act] chains on streams of equal priority, out of step by themselves: the contraction of one half (tensor / HBM) and
+    // the tail of an act kernel (HBM) fill the SMs the other half's act kernel (instruction issue) leaves idle between its waves
+    const bool multi = can_carry && ei.n >= 8192;
     if (multi && !sc->ev_fork) {
-        for (int k = 0; k < 3; ++k) { XQ_CUDA(cudaStreamCreateWithFlags(&sc->aux[k], cudaStreamNonBlocking)); XQ_CUDA(cudaEventCreateWithFlags(&sc->ev_join[k], cudaEventDisableTiming)); }
+        XQ_CUDA(cudaStreamCreateWithFlags(&sc->aux, cudaStreamNonBlocking));
+        XQ_CUDA(cudaEventCreateWithFlags(&sc->ev_join, cudaEventDisableTiming));
         XQ_CUDA(cudaEventCreateWithFlags(&sc->ev_fork, cudaEventDisableTiming));
     }
     bool carried = false, forked = false;
@@ -384,15 +372,15 @@ int xq_selfplay_collect(xq_dqn_t h, xq_env_t env, xq_replay_t r, int n_plies, do
         if (multi && carried) {
             if (!forked) {
                 XQ_CUDA(cudaEventRecord(sc->ev_fork, ei.stream));
-                for (int k = 1; k < n_streams; ++k) XQ_CUDA(cudaStreamWaitEvent(sc->aux[k - 1], sc->ev_fork, 0));
+                XQ_CUDA(cudaStreamWaitEvent(sc->aux, sc->ev_fork, 0));
                 forked = true;
             }
-            for (int part = n_streams - 1; part >= 0; --part) {
+            for (int half = 1; half >= 0; --half) {
                 EnvInfo eh = ei;
-                eh.stream = part ? sc->aux[part - 1] : ei.stream;
+                eh.stream = half ? sc->aux : ei.stream;
                 ActCarry cy;
                 int64_t o = 0, m = 0;
-                if (int rc = dqn_q90_part(h, ei.n, n_streams, part, sc->q90, eh.stream, &cy, &o, &m)) return rc;
+                if (int rc = dqn_q90_half(h, ei.n, half, sc->q90, eh.stream, &cy, &o, &m)) return rc;
                 eh.d_envs = ei.d_envs + o; eh.n = m; eh.env_id0 = ei.env_id0 + (uint64_t)o; eh.d_nonstd = ei.d_nonstd ? ei.d_nonstd + o : nullptr;
                 if (int rc = launch_act(true, eh, sc->q90 + o * kQPad, thr, train_done, nullptr, r ? r->d_ring : nullptr, r ? r->capacity : 1,
                                         r ? (ring_pos + o) % r->capacity : 0, d_stats, ei.event_ply + (uint32_t)p, &cy, (uint32_t)o)) return rc;
@@ -402,12 +390,11 @@ int xq_selfplay_collect(xq_dqn_t h, xq_env_t env, xq_replay_t r, int n_plies, do
             if (int rc = dqn_q90_device(h, ei.d_envs, ei.n, sc->q90, ei.stream, carried, &cy)) return rc;
             if (int rc = launch_act(true, ei, sc->q90, thr, train_done, nullptr, r ? r->d_ring : nullptr, r ? r->capacity : 1, ring_pos,
                                     d_stats, ei.event_ply + (uint32_t)p, can_carry ? &cy : nullptr)) return rc;
-            carried = can_carry && cy.Z != nullptr;
+            carried = can_carry;
         }
         if (r) r->total += ei.n;
     }
-    if (forked)
-        for (int k = 1; k < n_streams; ++k) { XQ_CUDA(cudaEventRecord(sc->ev_join[k - 1], sc->aux[k - 1])); XQ_CUDA(cudaStreamWaitEvent(ei.stream, sc->ev_join[k - 1], 0)); }
+    if (forked) { XQ_CUDA(cudaEventRecord(sc->ev_join, sc->aux)); XQ_CUDA(cudaStreamWaitEvent(ei.stream, sc->ev_join, 0)); }
     env_advance_event_ply(env, (uint32_t)n_plies);
     if (int rc = dqn_act_leave(h, ei.stream)) return rc;
     if (int rc = order_after(h->stream, ei.stream, &sc->ev_order)) return rc;    // later TD updates see the new transitions

@@ -365,8 +365,7 @@ int xq_dqn_apply_grads(xq_dqn_t h, double lr);
  * It replaces ncclAllReduce + xq_dqn_apply_grads.
  * EVERY applied update on a connected handle exchanges its gradient: xq_dqn_td_update / xq_dqn_td_update_device / _replay with apply = 1 and
  * xq_dqn_td_update_replay_n run the exchange INSIDE the gradient contraction kernel (contraction -> reduce-scatter of the 16-row blocks to
- * their owner ranks -> all-gather of the sums -> SGD, flag-in-data lines over peer memory; XQ_DIST_FUSED_MODE=allgather selects the older
- * every-block-to-every-rank variant for A/B runs).  Every rank must make the same sequence of update calls.
+ * their owner ranks -> all-gather of the sums -> SGD, flag-in-data lines over peer memory).  Every rank must make the same sequence of update calls.
  * A wait for a peer that lasts longer than XQ_DIST_TIMEOUT_MS (default 20000) does NOT apply the update and makes the handle fail
  * (XQ_ERR_STATE, sticky) on every later update / exchange call: the replicas may differ, recreate the handles.
  * xq_dqn_dist_status: timed_out = epoch of the first exchange that timed out (0 = none).

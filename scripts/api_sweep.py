@@ -1,4 +1,4 @@
-"""API-mode path on the device (lists -> pick -> step, three launches per ply): steps/s and per-kernel time; XQ_LEGAL_LANE=0 = the generic list kernel"""
+"""API-mode path on the device (lists -> pick -> step, three launches per ply): steps/s and per-kernel time; XQ_LEGAL_TEAM=0|1 forces the list kernel"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -35,5 +35,5 @@ for n, plies in sizes:
     b.record(s)
     torch.cuda.synchronize()
     ms_s = a.elapsed_time(b)
-    print(f"lane={os.environ.get('XQ_LEGAL_LANE','1')} team={os.environ.get('XQ_LEGAL_TEAM','auto')} envs={n}: api ply {1e3*ms/plies:.1f} us = {n*plies/(ms*1e-3):.3e} steps/s; list kernel {1e3*ms_l/plies:.1f} us ({321*n/(ms_l/plies*1e-3)/1e9:.0f} GB/s of 64+257 B/env); step kernel {1e3*ms_s/plies:.1f} us")
+    print(f"team={os.environ.get('XQ_LEGAL_TEAM','auto')} envs={n}: api ply {1e3*ms/plies:.1f} us = {n*plies/(ms*1e-3):.3e} steps/s; list kernel {1e3*ms_l/plies:.1f} us ({321*n/(ms_l/plies*1e-3)/1e9:.0f} GB/s of 64+257 B/env); step kernel {1e3*ms_s/plies:.1f} us")
     env.close()

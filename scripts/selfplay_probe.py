@@ -1,4 +1,4 @@
-"""eps-greedy self-play collector timing (65,536 envs): us per ply; XQ_ACT_LANE=0|1, XQ_COLLECT_STREAMS"""
+"""eps-greedy self-play collector timing (65,536 envs): us per ply"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -15,5 +15,5 @@ for n in (65536, 16384, 262144):
         a.record(s); xq.collect(net, env, rb, 32, 0.1); b.record(s)
         torch.cuda.synchronize()
         best = min(best, a.elapsed_time(b))
-    print(f"lane={os.environ.get('XQ_ACT_LANE','1')} streams={os.environ.get('XQ_COLLECT_STREAMS','2')} envs={n}: {1e3*best/32:.1f} us per ply = {n*32/(best*1e-3):.3e} steps/s")
+    print(f"envs={n}: {1e3*best/32:.1f} us per ply = {n*32/(best*1e-3):.3e} steps/s")
     env.close(); net.close(); rb.close()

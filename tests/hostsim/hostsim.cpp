@@ -271,7 +271,7 @@ int hs_team_all_actions(const xq_env_rec* recs, long n, uint8_t* counts, uint16_
     }
     return nonstd;
 }
-// DQN::selectAction through the board-per-thread functions (act_lane_kernel): same contract as hs_act_team
+// DQN::selectAction through the board-per-thread functions of xq_rollout_lane.cuh: same contract as hs_act_team
 int hs_act_lane(const xq_env_rec* recs, long n, uint64_t env_id0, uint64_t seed, const float* q90, uint32_t eps_thr, uint16_t* actions) {
     int nonstd = 0;
     uint32_t magic[XQ_MAX_ACTIONS + 1] = {0};
@@ -306,9 +306,10 @@ int hs_act_lane(const xq_env_rec* recs, long n, uint64_t env_id0, uint64_t seed,
 int hs_lane_rollout(xq_env_rec* recs, long n, uint64_t env_id0, uint64_t seed, int n_plies, xq_trace_rec* trace, xq_env_stats* stats) {
     return lane_rollout_host(recs, n, env_id0, seed, n_plies, trace, stats);
 }
-// whole fused rollout through the team kernel's phases; returns the number of boards it does not handle (non-standard piece sets)
+// whole fused rollout through the team kernel's phases; returns the number of boards it does not handle (non-standard piece sets),
+// or -1 for a team size other than 4, the only one the rollout kernel runs
 int hs_team_rollout(int team, xq_env_rec* recs, long n, uint64_t env_id0, uint64_t seed, int n_plies, xq_trace_rec* trace, xq_env_stats* stats) {
-    return team == 8 ? team_rollout_host<8>(recs, n, env_id0, seed, n_plies, trace, stats) : team_rollout_host<4>(recs, n, env_id0, seed, n_plies, trace, stats);
+    return team == 4 ? team_rollout_host<4>(recs, n, env_id0, seed, n_plies, trace, stats) : -1;
 }
 // opt-in strict legality (xq_rules.cuh: leaves_general_safe): the reference-ordered list filtered
 void hs_all_actions_strict(const xq_env_rec* recs, long n, uint8_t* counts, uint16_t* actions) {

@@ -108,18 +108,17 @@ def _team_vs_oracle(O, L, H, team, recs, seed, id0, plies):
 
 
 def test_team_rollout_phases(O, oracle_lib, hostsim):
-    """xq_rollout_team.cuh (rollout_team_kernel<4>, <8>): the three phases of a ply, run thread by thread on the host, reproduce the
+    """xq_rollout_team.cuh (rollout_team_kernel, teams of 4): the three phases of a ply, run thread by thread on the host, reproduce the
     oracle's fused rollout record for record -- from the opening over several games, resumed in the middle of games (Black to
     move, captured pieces, non-zero scores and counters) and from finished boards"""
     mid = harvest_positions(O, 600, 6, 37, seed=5)       # snapshots after 37, 74, ... plies: both colours to move
     fin = O.new_envs(8)
     fin["move_count"][:4] = 200
     fin["sq"][4:, 0] &= np.uint32(0xFFF0FFFF)           # Red general gone: never stepped, restarted (chessai.cpp:90,96)
-    for team in (4, 8):
-        _team_vs_oracle(O, oracle_lib, hostsim, team, O.new_envs(1500), 11, 5000, 450)
-        _team_vs_oracle(O, oracle_lib, hostsim, team, mid, 77, 0, 230)
-        _team_vs_oracle(O, oracle_lib, hostsim, team, mid, 78, 123456789012, 1)
-        _team_vs_oracle(O, oracle_lib, hostsim, team, fin, 3, 9, 40)
+    _team_vs_oracle(O, oracle_lib, hostsim, 4, O.new_envs(1500), 11, 5000, 450)
+    _team_vs_oracle(O, oracle_lib, hostsim, 4, mid, 77, 0, 230)
+    _team_vs_oracle(O, oracle_lib, hostsim, 4, mid, 78, 123456789012, 1)
+    _team_vs_oracle(O, oracle_lib, hostsim, 4, fin, 3, 9, 40)
 
 
 def test_lane_list_emission(O, oracle_lib, hostsim, golden):
@@ -210,7 +209,7 @@ def test_team_act_selection(O, oracle_lib, hostsim):
         for i in range(n):
             qi = np.zeros(8100); qi[:96] = q[i]
             want[i] = lists[i, oracle_lib.xqo_select_action(qi, lists[i], int(counts[i]), int(coin[i]), int(idx[i]), eps)]
-        for name, fn in (("team", hostsim.hs_act_team), ("lane", hostsim.hs_act_lane)):      # act_team_kernel's phases; act_lane_kernel's functions
+        for name, fn in (("team", hostsim.hs_act_team), ("lane", hostsim.hs_act_lane)):      # act_team_kernel's phases; the board-per-thread functions of xq_rollout_lane.cuh
             got = np.zeros(n, np.uint16)
             assert fn(recs.ctypes.data, n, 31, 77, q.ctypes.data, thr, got.ctypes.data) == 0
             bad = np.nonzero(got != want)[0]
