@@ -2,8 +2,8 @@
 
 Host-side mirror of the C ABI in include/xq.h; the hot path lives in csrc/ as hand-written CUDA.
 """
-from ._lib import (ENV_DTYPE, MAX_ACTIONS, STATE_SIZE, STATS_DTYPE, TRACE_DTYPE, TRANSITION_DTYPE, XQError,  # noqa: F401
-                   lib)
+from ._lib import (ENV_DTYPE, MAX_ACTIONS, SEARCH_ADVANCE_MAX_SIMULATIONS, STATE_SIZE, STATS_DTYPE, TRACE_DTYPE,  # noqa: F401
+                   TRANSITION_DTYPE, XQError, lib)
 from .env import BatchedEnv, BatchedSearch, action, search_bytes_per_tree  # noqa: F401
 from .dqn import AS_WRITTEN, CORRECTED, DQN  # noqa: F401
 from .replay import ReplayBuffer, act, collect, td_update_replay, td_update_replay_n  # noqa: F401

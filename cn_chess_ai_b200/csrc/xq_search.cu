@@ -12,6 +12,7 @@
 //   a [list index][thread] shared row, the priors are taken over that row in list order, the backup walks the parent pointers.
 //   Boards the generator refuses go to search_expand_generic_kernel (all_actions, thread per board).
 // search_root_kernel: one CTA per tree, the dense visit row built in shared memory and written with 16-byte stores.
+// search_advance_kernel: one warp per tree, re-roots the tree at the played child in place (membership bitmap in shared memory).
 #include <string.h>
 
 #include <new>
@@ -46,11 +47,10 @@ __device__ __forceinline__ void search_status(const WordSummary& s, int move_cou
     winner = (uint8_t)((s.gen_red == 127 && s.gen_black == 127) ? NOCOLOR : (s.gen_red < s.gen_black ? RED : BLACK));
 }
 
-__global__ void __launch_bounds__(256) search_reset_kernel(SearchDev d, const xq_env_rec* __restrict__ envs) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= d.n) return;
+// tree t emptied down to a root holding the env's record `env` (xq_search_reset; xq_search_advance for a tree it does not keep)
+__device__ __forceinline__ void search_reset_tree(const SearchDev& d, int64_t t, const xq_env_rec* env) {
     const int64_t g = t * d.cap;
-    const uint4* src = reinterpret_cast<const uint4*>(envs + t);
+    const uint4* src = reinterpret_cast<const uint4*>(env);
     uint4* dst = reinterpret_cast<uint4*>(d.rec + g);
     uint32_t wd[12];
 #pragma unroll
@@ -59,12 +59,171 @@ __global__ void __launch_bounds__(256) search_reset_kernel(SearchDev d, const xq
         dst[i] = v;
         if (i < 3) { wd[4 * i] = v.x; wd[4 * i + 1] = v.y; wd[4 * i + 2] = v.z; wd[4 * i + 3] = v.w; }
     }
-    Meta m; m.load(envs + t);
+    Meta m; m.load(env);
     uint8_t term, win;
     search_status(summarize_words(wd), m.move_count, term, win);
     d.parent[g] = -1; d.pedge[g] = 0; d.visits[g] = 0; d.reward[g] = 0; d.depth[g] = 0;
     d.nedges[g] = 0; d.expanded[g] = 0; d.term[g] = term; d.winner[g] = win;
     d.count[t] = 1;
+}
+
+__global__ void __launch_bounds__(256) search_reset_kernel(SearchDev d, const xq_env_rec* __restrict__ envs) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= d.n) return;
+    search_reset_tree(d, t, envs + t);
+}
+
+// Re-rooting at the env's record (xq_search_advance), one warp per tree:
+//   1. the match m: the root, else the root's child whose 64-byte record equals the env's (the lanes split the children);
+//   2. m > 0: the membership bitmap and per-word prefix counts in shared memory (search_kept / search_membership of xq_search.cuh), one
+//      32-node word per round, each word a ballot iterated to its fixed point;
+//   3. no match, or more than cap - min_free kept nodes: the tree is rebuilt as search_reset_kernel builds it;
+//   4. m > 0: the kept nodes move to their new slots kAdvBatch at a time in increasing old index, the whole batch read before any of it
+//      is written (new index <= old index, so only slots already read are overwritten); the lanes split a node's edge slots.  Parents and
+//      children are renumbered through the bitmap, depths lowered by m's; m becomes the root.  The root noise is mixed into a kept,
+//      expanded root's priors (in place when m == 0).
+constexpr int kAdvWarps = 4;       // trees per CTA of the advance kernel
+constexpr int kAdvBatch = 2;       // nodes a warp moves per round
+constexpr int kAdvSlots = kSearchEdges / 32;
+
+__global__ void __launch_bounds__(32 * kAdvWarps) search_advance_kernel(SearchDev d, const xq_env_rec* __restrict__ envs, int min_free,
+                                                                       const float* __restrict__ noise, float eps, int view,
+                                                                       int32_t* __restrict__ kept_out) {
+    extern __shared__ uint32_t s_adv[];          // per warp: bits[words], then prefix[words]
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t t = (int64_t)blockIdx.x * kAdvWarps + warp;
+    if (t >= d.n) return;
+    const int words = (d.cap + 31) >> 5;
+    uint32_t* bits = s_adv + (size_t)warp * 2 * words;
+    int32_t* prefix = reinterpret_cast<int32_t*>(bits + words);
+    const int64_t g0 = t * d.cap, eb0 = g0 * kSearchEdges;
+    const int count = d.count[t];
+    uint4 e[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) e[i] = reinterpret_cast<const uint4*>(envs + t)[i];
+    auto same = [&](int64_t g) {
+        const uint4* r = reinterpret_cast<const uint4*>(d.rec + g);
+        bool eq = true;
+#pragma unroll
+        for (int i = 0; i < 4; ++i) { const uint4 v = r[i]; eq = eq && v.x == e[i].x && v.y == e[i].y && v.z == e[i].z && v.w == e[i].w; }
+        return eq;
+    };
+    // 1. the match
+    int m = -1;
+    if (same(g0)) {
+        m = 0;
+    } else if (d.expanded[g0]) {
+        const int ne = d.nedges[g0];
+        unsigned cand = 0xFFFFFFFFu;
+        for (int k = lane; k < ne; k += 32) {
+            const int c = d.child[eb0 + k];
+            if (c >= 0 && (unsigned)c < cand && same(g0 + c)) cand = (unsigned)c;
+        }
+        cand = __reduce_min_sync(0xFFFFFFFFu, cand);
+        if (cand != 0xFFFFFFFFu) m = (int)cand;
+    }
+    // 2. the membership
+    int kept = count;
+    const int last = (count - 1) >> 5;
+    if (m > 0) {
+        kept = 0;
+        for (int w = m >> 5; w <= last; ++w) {
+            const int base = w << 5, j = base + lane;
+            const int p = j < count ? d.parent[g0 + j] : -1;
+            uint32_t word = 0;
+            for (;;) {
+                const uint32_t next = __ballot_sync(0xFFFFFFFFu, j < count && search_kept(j, m, p, base, bits, word));
+                if (next == word) break;
+                word = next;
+            }
+            if (lane == 0) { bits[w] = word; prefix[w] = kept; }
+            kept += popc32(word);
+            __syncwarp();
+        }
+    }
+    // 3. a tree that is not kept
+    if (m < 0 || kept > d.cap - min_free) {
+        if (lane == 0) {
+            search_reset_tree(d, t, envs + t);
+            if (kept_out) kept_out[t] = 0;
+        }
+        return;
+    }
+    // 4. the move, and the root noise
+    const float* nz = noise ? noise + t * XQ_POLICY_ACTIONS : nullptr;
+    const bool flip = policy_flip(d.rec[g0 + m].player, view);
+    auto mix = [&](float p, int a) { return search_mix(p, nz[flip ? XQ_POLICY_ACTIONS - 1 - a : a], eps); };
+    if (m == 0) {
+        if (nz && d.expanded[g0]) {
+            const int ne = d.nedges[g0];
+            for (int k = lane; k < ne; k += 32) d.P[eb0 + k] = mix(d.P[eb0 + k], d.act[eb0 + k]);
+        }
+    } else {
+        const int dm = d.depth[g0 + m];
+        int w = m >> 5;
+        uint32_t rest = bits[w];
+        for (;;) {
+            int js[kAdvBatch];
+#pragma unroll
+            for (int b = 0; b < kAdvBatch; ++b) {
+                while (rest == 0 && w < last) rest = bits[++w];
+                js[b] = rest ? (w << 5) + ffs32(rest) - 1 : -1;
+                rest &= rest - 1;
+            }
+            if (js[0] < 0) break;
+            // read the batch
+            int parent[kAdvBatch], visits[kAdvBatch], reward[kAdvBatch], depth[kAdvBatch], ne[kAdvBatch];
+            uint8_t pedge[kAdvBatch], nedges[kAdvBatch], expanded[kAdvBatch], term[kAdvBatch], winner[kAdvBatch];
+            uint4 rec[kAdvBatch];
+            float P[kAdvBatch][kAdvSlots], W[kAdvBatch][kAdvSlots];
+            int N[kAdvBatch][kAdvSlots], C[kAdvBatch][kAdvSlots];
+            int16_t A[kAdvBatch][kAdvSlots];
+#pragma unroll
+            for (int b = 0; b < kAdvBatch; ++b) {
+                if (js[b] < 0) continue;
+                const int64_t g = g0 + js[b], eb = g * kSearchEdges;
+                parent[b] = d.parent[g]; visits[b] = d.visits[g]; reward[b] = d.reward[g]; depth[b] = d.depth[g];
+                pedge[b] = d.pedge[g]; expanded[b] = d.expanded[g]; term[b] = d.term[g]; winner[b] = d.winner[g];
+                nedges[b] = d.nedges[g];
+                ne[b] = expanded[b] ? nedges[b] : 0;        // only the edge slots of an expanded node hold edges
+                if (lane < 4) rec[b] = reinterpret_cast<const uint4*>(d.rec + g)[lane];
+#pragma unroll
+                for (int i = 0; i < kAdvSlots; ++i) {
+                    const int k = lane + 32 * i;
+                    if (k < ne[b]) { P[b][i] = d.P[eb + k]; N[b][i] = d.N[eb + k]; W[b][i] = d.W[eb + k]; C[b][i] = d.child[eb + k]; A[b][i] = d.act[eb + k]; }
+                }
+            }
+            __syncwarp();
+            // write it to the new slots
+#pragma unroll
+            for (int b = 0; b < kAdvBatch; ++b) {
+                if (js[b] < 0) continue;
+                const bool root = js[b] == m;
+                const int64_t g = g0 + search_new_index(bits, prefix, js[b]), eb = g * kSearchEdges;
+                if (lane == 0) {
+                    d.parent[g] = root ? -1 : search_new_index(bits, prefix, parent[b]);
+                    d.pedge[g] = root ? 0 : pedge[b];
+                    d.visits[g] = visits[b]; d.reward[g] = root ? 0 : reward[b]; d.depth[g] = depth[b] - dm;
+                    d.nedges[g] = nedges[b]; d.expanded[g] = expanded[b]; d.term[g] = term[b]; d.winner[g] = winner[b];
+                }
+                if (lane < 4) reinterpret_cast<uint4*>(d.rec + g)[lane] = rec[b];
+#pragma unroll
+                for (int i = 0; i < kAdvSlots; ++i) {
+                    const int k = lane + 32 * i;
+                    if (k < ne[b]) {
+                        d.P[eb + k] = root && nz ? mix(P[b][i], A[b][i]) : P[b][i];
+                        d.N[eb + k] = N[b][i]; d.W[eb + k] = W[b][i]; d.act[eb + k] = A[b][i];
+                        d.child[eb + k] = C[b][i] >= 0 ? search_new_index(bits, prefix, C[b][i]) : -1;
+                    }
+                }
+            }
+        }
+    }
+    // 5. the kept count
+    if (lane == 0) {
+        d.count[t] = kept;
+        if (kept_out) kept_out[t] = kept;
+    }
 }
 
 __global__ void __launch_bounds__(32 * kSelWarps) search_select_kernel(SearchDev d, float c_puct, float fpu, uint8_t* __restrict__ status,
@@ -363,6 +522,28 @@ int xq_search_reset(xq_search_t s) {
     XQ_LAUNCH_CHECK();
     s->maybe_nonstd = E.maybe_nonstd;
     s->sims = 0;
+    s->phase = 1;
+    return XQ_OK;
+}
+
+int xq_search_advance(xq_search_t s, int min_free, const float* root_noise_dev, float noise_eps, int view, int32_t* kept_dev) {
+    EnvInfo E;
+    if (int rc = enter(s, &E, "xq_search_advance")) return rc;
+    if (s->max_sims > XQ_SEARCH_ADVANCE_MAX_SIMULATIONS)
+        return fail(XQ_ERR_INVALID, "xq_search_advance: max_simulations %d (at most %d)", s->max_sims, XQ_SEARCH_ADVANCE_MAX_SIMULATIONS);
+    if (min_free < 1 || min_free > s->max_sims) return fail(XQ_ERR_INVALID, "xq_search_advance: min_free %d (1 .. %d)", min_free, s->max_sims);
+    if (!(noise_eps >= 0.f && noise_eps <= 1.f)) return fail(XQ_ERR_INVALID, "xq_search_advance: noise_eps must be in [0, 1]");
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_search_advance: view %d", view);
+    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_advance: the search was never reset (xq_search_reset)");
+    if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_search_advance: the last selection was not expanded and backed up");
+    // per warp (tree) the membership bitmap and one prefix count per 32-node word: cap / 4 bytes
+    const size_t smem = (size_t)kAdvWarps * 2 * 4 * (size_t)((s->d.cap + 31) / 32);
+    if (smem > 48 * 1024) XQ_CUDA(cudaFuncSetAttribute(search_advance_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    search_advance_kernel<<<grid_of(s->d.n, kAdvWarps), 32 * kAdvWarps, smem, E.stream>>>(s->d, E.d_envs, min_free, root_noise_dev, noise_eps,
+                                                                                         view, kept_dev);
+    XQ_LAUNCH_CHECK();
+    s->maybe_nonstd = s->maybe_nonstd || E.maybe_nonstd;      // kept boards descend from the old roots
+    s->sims = s->max_sims - min_free;
     s->phase = 1;
     return XQ_OK;
 }

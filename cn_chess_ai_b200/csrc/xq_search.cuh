@@ -1,5 +1,6 @@
 // xq_search.cuh -- host-compilable helpers of the batched tree search (xq_search.cu; include/xq.h: xq_search_*): the PUCT score of an
-// edge and its arg-max order, the priors of a freshly expanded node, the root-noise mix, the value cleaning and the backup along a path.
+// edge and its arg-max order, the priors of a freshly expanded node, the root-noise mix, the value cleaning, the backup along a path, and
+// the membership and renumbering of a tree re-rooted after a move (xq_search_advance).
 //
 // The arithmetic is spelled with explicitly rounded operations (__fmul_rn and friends on the device; plain operators on the host, where
 // tests/hostsim/search_shim.cpp is compiled with -ffp-contract=off) so that no multiply-add is contracted and numpy can restate every
@@ -9,6 +10,7 @@
 #include <math.h>
 #include <stdint.h>
 
+#include "xq_bitboard.cuh"
 #include "xq_policy.cuh"
 
 namespace xq {
@@ -90,6 +92,53 @@ XQ_HD void search_backup(int leaf, float value, const int32_t* parent, const uin
         node_visits[p] += 1;
         j = p;
     }
+}
+
+// ---- advance: re-rooting a tree at node m (0, or a child of the root) in place ----
+// Membership: keep[j] = j == m || (j > m && keep[parent[j]]), decidable in increasing index order because parent[j] < j.  It is held as a
+// bitmap of 32-node words with a prefix count per word (prefix[w] = kept nodes in words < w); a kept node's new index is
+// prefix[j >> 5] + the kept nodes below it in its word, never larger than j, so moving the kept nodes in increasing old index (each batch
+// read completely before it is written) overwrites only slots already read.
+
+// node j of the word that starts at `base`, its parent p: the parent's bit from `bits` (an earlier word, complete) or from `word` (this
+// word as far as it is known; iterated to its fixed point by search_keep_word)
+XQ_HD bool search_kept(int j, int m, int p, int base, const uint32_t* bits, uint32_t word) {
+    if (j == m) return true;
+    if (j < m || p < m) return false;
+    const uint32_t w = p >= base ? word >> (p - base) : bits[p >> 5] >> (p & 31);
+    return (w & 1u) != 0;
+}
+
+// the kept bits of nodes base .. base + 31 (< count) as the advance kernel's warp finds them: every lane evaluates search_kept against
+// the word of the last round (a ballot) until the word stops changing.  keep only grows and parents come first, so this ends at the
+// membership itself after at most 33 rounds.  Host restatement of the lanes for the CPU suite.
+XQ_HD uint32_t search_keep_word(int base, int count, int m, const int32_t* parent, const uint32_t* bits) {
+    uint32_t word = 0;
+    for (;;) {
+        uint32_t next = 0;
+        for (int l = 0; l < 32; ++l) {
+            const int j = base + l;
+            if (j < count && search_kept(j, m, parent[j], base, bits, word)) next |= 1u << l;
+        }
+        if (next == word) return word;
+        word = next;
+    }
+}
+
+// bits and prefix of words (m >> 5) .. (count - 1) >> 5 (the words below hold no kept node and are not written); returns the kept count
+XQ_HD int search_membership(int count, int m, const int32_t* parent, uint32_t* bits, int32_t* prefix) {
+    int kept = 0;
+    for (int w = m >> 5; w <= (count - 1) >> 5; ++w) {
+        bits[w] = search_keep_word(w << 5, count, m, parent, bits);
+        prefix[w] = kept;
+        kept += popc32(bits[w]);
+    }
+    return kept;
+}
+
+// the new index of kept node j
+XQ_HD int search_new_index(const uint32_t* bits, const int32_t* prefix, int j) {
+    return prefix[j >> 5] + popc32(bits[j >> 5] & ((1u << (j & 31)) - 1u));
 }
 
 }  // namespace xq

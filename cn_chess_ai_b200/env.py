@@ -186,6 +186,11 @@ class BatchedSearch:
     def reset(self):
         check(self._L.xq_search_reset(self._h))
 
+    def advance_device(self, min_free, noise_ptr=None, noise_eps=0.0, view=1, kept_ptr=None):
+        """xq_search_advance: re-root every tree at its env's current board (keep the played child's subtree, else rebuild the tree);
+        min_free more simulations are allowed afterwards.  kept int32 [n]: nodes carried over, 0 for a rebuilt tree"""
+        check(self._L.xq_search_advance(self._h, int(min_free), noise_ptr, float(noise_eps), view, kept_ptr))
+
     def select_device(self, c_puct, fpu, status_ptr=None, winner_ptr=None, reward_ptr=None, depth_ptr=None):
         check(self._L.xq_search_select_device(self._h, float(c_puct), float(fpu), status_ptr, winner_ptr, reward_ptr, depth_ptr))
 

@@ -37,6 +37,20 @@ class TorchSearch:
         self.tenv._enter()
         self.search.reset()
 
+    def advance(self, min_free, root_noise=None, noise_eps=0.25, view="side"):
+        """instead of reset() after a move: every tree is re-rooted at its env's current board, keeping the subtree (and its statistics)
+        of the child that was played, or rebuilt as reset() builds it when nothing matches (a game that ended and was reset) or the
+        subtree has more than max_simulations + 1 - min_free nodes.  Exactly min_free simulations are allowed afterwards.  root_noise
+        f32 [n, 8100] (frame of `view`): mixed into the priors of every kept, expanded root.  Returns kept int32 [n]: nodes carried over,
+        0 for a rebuilt tree."""
+        v = _view(view)
+        if root_noise is not None:
+            self.tenv._check(root_noise, "root_noise", [torch.float32], (self.n, POLICY_ACTIONS))
+        self.tenv._enter()
+        kept = torch.empty(self.n, dtype=torch.int32, device=self.device)
+        self.search.advance_device(min_free, None if root_noise is None else root_noise.data_ptr(), noise_eps, v, kept.data_ptr())
+        return kept
+
     def select(self, c_puct=1.5, fpu=0.0):
         """one leaf per tree: SelectResult of tensors [n]: status / winner uint8, reward / depth int32"""
         self.tenv._enter()
@@ -102,10 +116,12 @@ class TorchSearch:
         return torch.where(status == NO_LEGAL_ACTION, torch.full_like(v, -1.0), v)
 
     def run(self, evaluate, n_simulations, c_puct=1.5, fpu=0.0, temperature=1.0, root_noise=None, noise_eps=0.25, view="side",
-            obs_dtype=torch.bfloat16, cap_value=0.0):
+            obs_dtype=torch.bfloat16, cap_value=0.0, reset=True):
         """reset + n_simulations simulations: evaluate(planes) -> (scores [n, 8100], values [n]) is called once per simulation on the
-        leaves; at terminal leaves outcome_values replaces the network's value.  Returns root(view)."""
-        self.reset()
+        leaves; at terminal leaves outcome_values replaces the network's value.  reset=False continues from the current trees (after
+        advance(), or to add simulations to this move's search).  Returns root(view)."""
+        if reset:
+            self.reset()
         for _ in range(n_simulations):
             sel = self.select(c_puct, fpu)
             planes, aux = self.observe(obs_dtype, view)

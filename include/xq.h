@@ -231,7 +231,8 @@ int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dty
  * v <- -v, the edge gets N += 1 and W += v, every node on the path N_node += 1.  The library has no value convention for terminal leaves.
  *
  * Call order: xq_search_reset, then per simulation select -> (leaves / observe_leaves, any number of times) -> expand_backup; anything
- * else is XQ_ERR_STATE, as is a select past max_simulations since the reset.  root_device and get_tree work at any time after a reset.
+ * else is XQ_ERR_STATE, as is a select past max_simulations since the reset (past min_free since an xq_search_advance, which may
+ * take the place of the reset).  root_device and get_tree work at any time after a reset.
  * Memory: (max_simulations + 1) x 2,389 + 73 bytes per tree (xq_search_bytes_per_tree): per node a record, 21 bytes of node state and
  * 128 edge slots of 18 bytes (P, N, W, child, action); per tree the leaf record and 9 bytes. */
 typedef struct xq_search_s* xq_search_t;
@@ -263,6 +264,23 @@ int xq_search_destroy(xq_search_t s);
 int xq_search_bytes_per_tree(int max_simulations, int64_t* bytes);
 /* roots = the env's current records (read in stream order), every tree empty, simulation count 0 */
 int xq_search_reset(xq_search_t s);
+/* Subtree reuse between moves.  Re-root every tree at the node whose record equals its env's current record (read in stream order): the
+ * root itself, or the root's child with that record (at most one can match: two legal actions of one board never give the same board).
+ * All 64 bytes are compared, ctr and scores included, so after xq_env_policy_step_device (XQ_PICK_GIVEN, the root's best) or
+ * xq_env_step_device the played child matches; a rejected move keeps the whole tree; a finished, auto-reset game, or a move whose child
+ * was never made, matches nothing.  The matched node's subtree is kept with every statistic (record, reward, status, winner, edges,
+ * N_node); every other node is dropped; the kept nodes are renumbered by increasing old index (the new root is node 0), their depths
+ * lowered by the matched node's, and the new root gets parent -1, parent_edge 0, reward 0.  A tree keeps its subtree only if it has at
+ * most max_simulations + 1 - min_free nodes; a tree with no match or too large a subtree is rebuilt from the env's record exactly as
+ * xq_search_reset builds it.  Afterwards exactly min_free selects are allowed (1 <= min_free <= max_simulations; a simulation adds at most
+ * one node per tree, so each kept tree has room for them).  root_noise_dev [n][8100] f32 (frame of `view`) or NULL: mixed into the
+ * priors of every kept, expanded root as at expansion, P <- (1 - eps) * P + eps * noise[index]; a rebuilt root gets its noise at its
+ * expansion as before.  kept_dev int32 [n] or NULL: nodes carried over, 0 for a rebuilt tree.  Allowed after a reset when no selection is
+ * pending (XQ_ERR_STATE otherwise); noise_eps in [0, 1].  The kernel works in place (no memory beyond xq_search_bytes_per_tree) with a
+ * cap / 4-byte bitmap per tree in shared memory, which bounds max_simulations: a search with more than
+ * XQ_SEARCH_ADVANCE_MAX_SIMULATIONS is refused with XQ_ERR_INVALID. */
+#define XQ_SEARCH_ADVANCE_MAX_SIMULATIONS 65536
+int xq_search_advance(xq_search_t s, int min_free, const float* root_noise_dev, float noise_eps, int view, int32_t* kept_dev);
 /* one leaf per tree; c_puct finite and >= 0, fpu finite.  Outputs [n] (any may be NULL): status u8, winner u8, reward i32, depth i32 */
 int xq_search_select_device(xq_search_t s, float c_puct, float fpu, uint8_t* status_dev, uint8_t* winner_dev, int32_t* reward_dev,
                             int32_t* depth_dev);
