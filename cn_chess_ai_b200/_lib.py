@@ -32,6 +32,10 @@ SEARCH_NODE_DTYPE = np.dtype([("rec", ENV_DTYPE), ("parent", "<i4"), ("visits", 
                               ("reserved", "u1", (3,))])
 SEARCH_EDGE_DTYPE = np.dtype([("action", "<i4"), ("prior", "<f4"), ("visits", "<i4"), ("value_sum", "<f4"), ("child", "<i4")])
 assert SEARCH_NODE_DTYPE.itemsize == 88 and SEARCH_EDGE_DTYPE.itemsize == 20
+EXAMPLE_DTYPE = np.dtype([("rec", ENV_DTYPE), ("env", "<u8"), ("game", "<u4"), ("ply", "<u2"), ("n_edges", "u1"), ("reserved0", "u1"),
+                          ("z", "<f4"), ("q", "<f4"), ("total_visits", "<u4"), ("reserved1", "<u4"), ("action", "<i2", (128,)),
+                          ("visits", "<u4", (128,))])
+assert EXAMPLE_DTYPE.itemsize == 864
 
 
 class XQError(RuntimeError):
@@ -99,6 +103,15 @@ def lib():
     L.xq_search_expand_backup_device.argtypes = [_P, _P, C.c_int, C.c_float, C.c_int, _P, _P, C.c_float]
     L.xq_search_root_device.argtypes = [_P, C.c_int, _P, _P, _P]
     L.xq_search_get_tree.argtypes = [_P, C.c_int64, _P, _P, C.POINTER(C.c_int32)]
+    L.xq_examples_create.argtypes = [_P, C.c_int64, C.c_int, C.POINTER(_P)]
+    L.xq_examples_destroy.argtypes = [_P]
+    L.xq_examples_bytes.argtypes = [C.c_int64, C.c_int64, C.c_int, C.POINTER(C.c_int64)]
+    L.xq_examples_record_device.argtypes = [_P, _P, _P]
+    L.xq_examples_end_games_device.argtypes = [_P, _P, _P]
+    L.xq_examples_discard_device.argtypes = [_P, _P]
+    L.xq_examples_sample_device.argtypes = [_P, C.c_int64, C.c_uint64, C.c_uint32, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]
+    L.xq_examples_info.argtypes = [_P] + [C.POINTER(C.c_int64)] * 6
+    L.xq_examples_get.argtypes = [_P, C.c_int64, C.c_int64, _P]
     _lib = L
     return L
 

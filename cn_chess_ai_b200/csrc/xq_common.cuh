@@ -40,6 +40,13 @@ struct EnvInfo {
 int env_info(xq_env_t h, EnvInfo* out);
 void env_advance_event_ply(xq_env_t h, uint32_t plies);   // the collector applied `plies` more plies
 void** env_scratch_slot(xq_env_t h, void (*free_fn)(void*));   // the env handle's slot for the collector's scratch; free_fn runs when the handle is destroyed
+// what the example buffer (xq_examples.cu) reads of a search (xq_search.cu): its env, call state and the root rows of its slab
+struct SearchRoots {
+    xq_env_t env; int phase;         // phase: 0 never reset, 1 ready, 2 a selection pending
+    int64_t n; int cap;              // node j of tree t at g = t * cap + j; edge k of node g at g * 128 + k
+    const xq_env_rec* rec; const uint8_t *nedges, *expanded; const int32_t* N; const float* W; const int16_t* act;
+};
+int search_roots(xq_search_t s, SearchRoots* out);
 
 // ---- device helpers ---------------------------------------------------------------------------
 #if defined(__CUDACC__)

@@ -461,6 +461,13 @@ int enter(xq_search_t s, EnvInfo* E, const char* fn) {
 bool valid_view(int v) { return v == XQ_VIEW_ABSOLUTE || v == XQ_VIEW_SIDE_TO_MOVE; }
 }  // namespace
 
+int xq::search_roots(xq_search_t s, SearchRoots* out) {
+    if (!s) return fail(XQ_ERR_INVALID, "null search handle");
+    const SearchDev& d = s->d;
+    *out = SearchRoots{s->env, s->phase, d.n, d.cap, d.rec, d.nedges, d.expanded, d.N, d.W, d.act};
+    return XQ_OK;
+}
+
 extern "C" {
 
 int xq_search_create(xq_env_t env, int max_simulations, xq_search_t* out) {

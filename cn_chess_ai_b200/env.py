@@ -8,7 +8,7 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import (ENV_DTYPE, MAX_ACTIONS, SEARCH_EDGE_DTYPE, SEARCH_MAX_EDGES, SEARCH_NODE_DTYPE, STATE_SIZE, STATS_DTYPE, TRACE_DTYPE,
+from ._lib import (ENV_DTYPE, EXAMPLE_DTYPE, MAX_ACTIONS, SEARCH_EDGE_DTYPE, SEARCH_MAX_EDGES, SEARCH_NODE_DTYPE, STATE_SIZE, STATS_DTYPE, TRACE_DTYPE,
                    check, lib, ptr)
 
 
@@ -218,3 +218,65 @@ class BatchedSearch:
         cnt = C.c_int32()
         check(self._L.xq_search_get_tree(self._h, int(tree), ptr(nodes), ptr(edges), C.byref(cnt)))
         return nodes[:cnt.value].copy(), edges[:cnt.value].copy()
+
+
+def examples_bytes(n_envs, capacity, max_game_examples):
+    """device memory a BatchedExamples of this size allocates (the sampling scratch aside)"""
+    b = C.c_int64()
+    check(lib().xq_examples_bytes(int(n_envs), int(capacity), int(max_game_examples), C.byref(b)))
+    return b.value
+
+
+class BatchedExamples:
+    """xq_examples_*: the self-play example buffer of `env` (a BatchedEnv): per env a staging area of max_game_examples examples for the
+    game in progress, a ring of `capacity` committed examples.  Raw device pointers (ints), asynchronous on the env's stream; close()
+    before the env is closed."""
+
+    def __init__(self, env, capacity, max_game_examples=256):
+        self._L = lib()
+        self._h = C.c_void_p()
+        check(self._L.xq_examples_create(env.handle, int(capacity), int(max_game_examples), C.byref(self._h)))
+        self.env = env
+        self.n = env.n
+        self.capacity = int(capacity)
+        self.max_game_examples = int(max_game_examples)
+
+    def close(self):
+        if self._h:
+            self._L.xq_examples_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def record_device(self, search, mask_ptr=None):
+        """xq_examples_record_device: one example of every root of `search` (a BatchedSearch on the same env), u8 [n] mask or None"""
+        check(self._L.xq_examples_record_device(self._h, search._h, mask_ptr))
+
+    def end_games_device(self, ended_ptr, result_ptr):
+        """xq_examples_end_games_device: ended u8 [n], result f32 [n] from Red's side"""
+        check(self._L.xq_examples_end_games_device(self._h, ended_ptr, result_ptr))
+
+    def discard_device(self, mask_ptr=None):
+        check(self._L.xq_examples_discard_device(self._h, mask_ptr))
+
+    def sample_device(self, batch, seed, counter, view, planes_ptr, dtype, policy_ptr, value_ptr=None, q_ptr=None, mask_ptr=None,
+                      index_ptr=None):
+        check(self._L.xq_examples_sample_device(self._h, int(batch), int(seed), int(counter), view, planes_ptr, dtype, policy_ptr, value_ptr,
+                                                q_ptr, mask_ptr, index_ptr))
+
+    def info(self):
+        """synchronous: dict of size, capacity, total_committed, pending, dropped, stale"""
+        v = [C.c_int64() for _ in range(6)]
+        check(self._L.xq_examples_info(self._h, *(C.byref(x) for x in v)))
+        return dict(zip(("size", "capacity", "total_committed", "pending", "dropped", "stale"), (x.value for x in v)))
+
+    def get(self, first=0, n=None):
+        """synchronous read-back of ring slots [first, first + n): EXAMPLE_DTYPE [n]"""
+        n = self.capacity - first if n is None else n
+        out = np.zeros(n, EXAMPLE_DTYPE)
+        check(self._L.xq_examples_get(self._h, int(first), int(n), ptr(out)))
+        return out

@@ -301,6 +301,74 @@ int xq_search_root_device(xq_search_t s, int view, int32_t* visits_dev, float* q
  * node's n_edges have action -1 and child -1), *n_nodes = nodes in the tree */
 int xq_search_get_tree(xq_search_t s, int64_t tree, xq_search_node* nodes_host, xq_search_edge* edges_host, int32_t* n_nodes);
 
+/* ---- device-resident self-play example buffer: the training data of an AlphaZero-style policy/value network ----
+ * Bound to one env handle (asynchronous on its stream and device, unless a call says otherwise; destroy it before the env).  Each move,
+ * xq_examples_record_device stores one example per tree of a search on that env: the root's record and its root edges' actions and visit
+ * counts, in sparse form (the dense [8100] row is only built when a batch is sampled).  The examples of a game in progress wait in the
+ * env's staging area; xq_examples_end_games_device commits them to a ring with the game's result, and xq_examples_sample_device draws a
+ * training batch -- observation planes, policy targets, value targets, q, legal masks -- without a host synchronisation.
+ *
+ * Staging is per env, max_game_examples examples each (256 covers the reference's 200-move games with room for rejected moves recorded
+ * twice); an example recorded into a full staging area is dropped and counted.  Commit order is deterministic: the ended envs in
+ * increasing index, each env's examples in ply order, written at the ring head; the ring wraps and overwrites its oldest examples.
+ * Results are the caller's (the library has no outcome convention, as for terminal leaves of the search): result_dev[e] from Red's side,
+ * NaN -> 0, clamped to [-1, 1]; an example's z = result if Red is to move in its record, -result otherwise.
+ * A game that ends because the side to move has no legal action never reports done from a step (the step rejects XQ_ACTION_NONE and the
+ * board stays): the caller ends such a game through xq_examples_end_games_device itself.  After xq_env_reset / xq_env_set_boards the
+ * staged examples of the replaced games are stale: discard them (xq_examples_discard_device).
+ * Memory (xq_examples_bytes): (capacity + n_envs x max_game_examples) x 864 bytes, plus 20 bytes per env of counters and commit scratch
+ * and under 1.6 KB of global counters and alignment; sampling adds a scratch of 64 bytes per batch row that grows with the largest batch. */
+typedef struct xq_examples_s* xq_examples_t;
+typedef struct {
+    xq_env_rec rec;          /* the searched position: the tree's root record when it was recorded */
+    uint64_t env;            /* global env id (env_id0 + index): results do not depend on sharding */
+    uint32_t game;           /* games this env had ended in this buffer before this one (an ended game with no example counts too) */
+    uint16_t ply;            /* index of the example within its game's recorded examples, 0-based */
+    uint8_t n_edges;         /* root edges (0 if the root was never expanded) */
+    uint8_t reserved0;
+    float z;                 /* game result from the side to move at rec (set when the game is committed) */
+    float q;                 /* root q at record time: bit for bit xq_search_root_device's q (sum W / sum N, list order; NaN unvisited) */
+    uint32_t total_visits;   /* sum of visits[0 .. n_edges) */
+    uint32_t reserved1;
+    int16_t action[128];     /* absolute policy index from * 90 + to of root edge k (reference list order), -1 past n_edges */
+    uint32_t visits[128];    /* root edge N, 0 past n_edges */
+} xq_example;                /* 864 B = 27 x 32 B */
+
+/* capacity >= 1 committed examples, max_game_examples 1 .. 65,535 staged examples per env; XQ_ERR_NOMEM when the device memory cannot
+ * be had.  The buffer starts empty. */
+int xq_examples_create(xq_env_t env, int64_t capacity, int max_game_examples, xq_examples_t* out);
+int xq_examples_destroy(xq_examples_t b);
+/* the device memory xq_examples_create allocates (the sampling scratch aside) */
+int xq_examples_bytes(int64_t n_envs, int64_t capacity, int max_game_examples, int64_t* bytes);
+/* One example of the root of every tree of `s` (a search on the buffer's env: XQ_ERR_INVALID otherwise), or of the trees with
+ * mask_dev[e] != 0 (u8 [n]; NULL = all; e.g. playout-cap randomisation leaves the moves searched with a small budget out), appended to
+ * the env's staging area.  The search must have been reset and have no selection pending (XQ_ERR_STATE otherwise, as xq_search_advance).
+ * A tree whose root record differs in any of its 64 bytes from its env's current record (the env moved since the search: record after the
+ * step, or a missing xq_search_advance) is not recorded and counts as stale.  Recording an env twice in one game (after a rejected move)
+ * stores two examples. */
+int xq_examples_record_device(xq_examples_t b, xq_search_t s, const uint8_t* mask_dev);
+/* envs with ended_dev[e] != 0 (u8 [n], required) commit their staged examples to the ring with z from result_dev[e] (f32 [n], required,
+ * Red's side) and their game number; their staging areas empty and their game counts advance */
+int xq_examples_end_games_device(xq_examples_t b, const uint8_t* ended_dev, const float* result_dev);
+/* empty the staging area of the envs with mask_dev[e] != 0 (NULL = all); game counts do not change */
+int xq_examples_discard_device(xq_examples_t b, const uint8_t* mask_dev);
+/* One training batch of `batch` rows (> 0) drawn uniformly with replacement from the committed examples:
+ * index_i = (xq_rng(seed, i, counter) >> 1) % size (the rule of xq_replay_sample), size read on the device where the call runs in stream
+ * order.  planes_dev (required): xq_env_observe_device of rec (same dtype / view / alignment contract, no aux).  policy_dev (required,
+ * f32 [batch][8100], 16-byte aligned): visits[k] / total_visits (an f32 division of the two values converted to f32) at action[k] in the
+ * frame of `view`, 0 elsewhere; an all-zero row when total_visits is 0.  value_dev f32 [batch] = z, q_dev f32 [batch] = q, mask_dev
+ * (u32 [batch][254], 8-byte aligned) = the packed mask of the stored actions (xq_env_legal_mask_device(packed, view) of rec whenever the
+ * root was expanded and the board has at most 128 legal actions: every board of the reference's play), index_dev int64 [batch] = the ring
+ * slots; these four may be NULL.  An empty ring gives index -1, zero planes, policy and mask, NaN value and q. */
+int xq_examples_sample_device(xq_examples_t b, int64_t batch, uint64_t seed, uint32_t counter, int view, void* planes_dev, int dtype,
+                              float* policy_dev, float* value_dev, float* q_dev, uint32_t* mask_dev, int64_t* index_dev);
+/* synchronous: size = committed examples held (<= capacity), total_committed since create, pending = staged examples, dropped / stale
+ * counted since create; any pointer may be NULL */
+int xq_examples_info(xq_examples_t b, int64_t* size, int64_t* capacity, int64_t* total_committed, int64_t* pending, int64_t* dropped,
+                     int64_t* stale);
+/* synchronous read-back of raw ring slots [first, first + n) (tests, checkpointing); slot = commit number % capacity */
+int xq_examples_get(xq_examples_t b, int64_t first, int64_t n, xq_example* out_host);
+
 /* ---- DQN: replaces DQN (include/dqn.h:97-116, src/dqn.cpp) + NeuralNetwork (include/dqn.h:43-95, src/dqn.cu) ----
  * Parameters use the reference layout (src/dqn.cu:112-140): weights = layer after layer, each [out][in]
  * row-major; biases = layer after layer.
