@@ -102,6 +102,8 @@ def lib():
     L.xq_search_observe_leaves_device.argtypes = [_P, _P, C.c_int, C.c_int, _P]
     L.xq_search_expand_backup_device.argtypes = [_P, _P, C.c_int, C.c_float, C.c_int, _P, _P, C.c_float]
     L.xq_search_root_device.argtypes = [_P, C.c_int, _P, _P, _P]
+    L.xq_search_play_device.argtypes = [_P, C.c_float, C.c_int, C.c_int, C.c_int] + [_P] * 6
+    L.xq_search_root_noise_device.argtypes = [_P, C.c_float, C.c_float, C.c_uint64, _P, _P]
     L.xq_search_get_tree.argtypes = [_P, C.c_int64, _P, _P, C.POINTER(C.c_int32)]
     L.xq_examples_create.argtypes = [_P, C.c_int64, C.c_int, C.POINTER(_P)]
     L.xq_examples_destroy.argtypes = [_P]

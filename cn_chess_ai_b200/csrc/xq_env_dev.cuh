@@ -1,6 +1,8 @@
-// xq_env_dev.cuh -- device helpers shared by the thread-per-board kernels (xq_env.cu, xq_selfplay.cu).
+// xq_env_dev.cuh -- device helpers shared by the thread-per-board kernels (xq_env.cu, xq_selfplay.cu) and the board steps of the policy
+// and search kernels (xq_policy.cu, xq_search.cu).
 #pragma once
 #include "xq_common.cuh"
+#include "xq_bitboard.cuh"
 
 namespace xq {
 
@@ -67,6 +69,29 @@ __device__ __forceinline__ int apply_move(SmemBoard& b, Meta& m, int from, int t
     m.move_count++;
     m.player ^= 1;
     return cap;
+}
+
+// step_kernel (xq_env.cu) after its validation: movePiece + evaluateBoard + checkGameOver + getWinner, the optional reset, the outputs
+// (the policy step of xq_policy.cu and the search's play of xq_search.cu)
+__device__ __forceinline__ void policy_apply(SmemBoard& b, Meta& m, xq_env_rec* __restrict__ envs, int64_t env, bool ok, int from, int to, int auto_reset,
+                                             int32_t* reward, uint8_t* done, uint8_t* winner, uint8_t* captured, uint8_t* valid) {
+    const int mover = m.player;
+    int cap = 0;
+    if (ok) { cap = apply_move(b, m, from, to); m.ctr++; }
+    uint32_t wd[12];
+#pragma unroll
+    for (int i = 0; i < 12; ++i) wd[i] = b.base[i * b.stride];
+    const WordSummary s = summarize_words(wd);
+    const int diff = mover == RED ? s.mat_red - s.mat_black : s.mat_black - s.mat_red;
+    const bool over = m.move_count >= XQ_MAX_MOVES || s.gen_red == 127 || s.gen_black == 127;
+    const int win = (s.gen_red == 127 && s.gen_black == 127) ? NOCOLOR : (s.gen_red < s.gen_black ? RED : BLACK);
+    if (reward) reward[env] = reward_from_material(diff, m.move_count);
+    if (done) done[env] = over ? 1 : 0;
+    if (winner) winner[env] = (uint8_t)win;
+    if (captured) captured[env] = (uint8_t)cap;
+    if (valid) valid[env] = ok ? 1 : 0;
+    if (over && auto_reset) { reset_board(b); m.reset(); }
+    if (ok || (over && auto_reset)) { b.store(envs + env); m.store(envs + env); }
 }
 
 

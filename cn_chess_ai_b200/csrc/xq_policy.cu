@@ -158,28 +158,6 @@ __device__ __forceinline__ float load_score(const void* p, int64_t i) {
     return SDT == XQ_DTYPE_BF16 ? bf16_bits_to_float(__ldg(static_cast<const unsigned short*>(p) + i)) : __ldg(static_cast<const float*>(p) + i);
 }
 
-// step_kernel (xq_env.cu) after its validation: movePiece + evaluateBoard + checkGameOver + getWinner, the optional reset, the outputs
-__device__ __forceinline__ void policy_apply(SmemBoard& b, Meta& m, xq_env_rec* __restrict__ envs, int64_t env, bool ok, int from, int to, int auto_reset,
-                                             int32_t* reward, uint8_t* done, uint8_t* winner, uint8_t* captured, uint8_t* valid) {
-    const int mover = m.player;
-    int cap = 0;
-    if (ok) { cap = apply_move(b, m, from, to); m.ctr++; }
-    uint32_t wd[12];
-#pragma unroll
-    for (int i = 0; i < 12; ++i) wd[i] = b.base[i * b.stride];
-    const WordSummary s = summarize_words(wd);
-    const int diff = mover == RED ? s.mat_red - s.mat_black : s.mat_black - s.mat_red;
-    const bool over = m.move_count >= XQ_MAX_MOVES || s.gen_red == 127 || s.gen_black == 127;
-    const int win = (s.gen_red == 127 && s.gen_black == 127) ? NOCOLOR : (s.gen_red < s.gen_black ? RED : BLACK);
-    if (reward) reward[env] = reward_from_material(diff, m.move_count);
-    if (done) done[env] = over ? 1 : 0;
-    if (winner) winner[env] = (uint8_t)win;
-    if (captured) captured[env] = (uint8_t)cap;
-    if (valid) valid[env] = ok ? 1 : 0;
-    if (over && auto_reset) { reset_board(b); m.reset(); }
-    if (ok || (over && auto_reset)) { b.store(envs + env); m.store(envs + env); }
-}
-
 struct PolicyArgs {
     xq_env_rec* envs; int64_t n; uint64_t env_id0, seed;
     const void* scores; int pick; float t; int view, auto_reset;

@@ -13,6 +13,8 @@
 //   Boards the generator refuses go to search_expand_generic_kernel (all_actions, thread per board).
 // search_root_kernel: one CTA per tree, the dense visit row built in shared memory and written with 16-byte stores.
 // search_advance_kernel: one warp per tree, re-roots the tree at the played child in place (membership bitmap in shared memory).
+// search_play_kernel: one warp per tree, the move from the root's visit counts and the env's step with it.
+// search_noise_kernel: one warp per tree, Dirichlet noise drawn over the root's edges and mixed into its priors.
 #include <string.h>
 
 #include <new>
@@ -426,6 +428,120 @@ __global__ void __launch_bounds__(kRootThreads) search_root_kernel(SearchDev d, 
     }
 }
 
+// The move of every tree from its root's visit counts (xq_search_play_device), one warp per tree: the lanes compare the root record with
+// the env's and read the root's N row coalesced (edge k = lane + 32 i); the maximum and the total come from warp reductions.  Greedy: the
+// first edge with the maximum (a min-reduction over the lanes' first hits).  Sampled: the lanes write the weights to shared memory and lane 0
+// walks them in list order (search_play_sample).  Lane 0 then steps the env with the edge's action exactly as xq_env_policy_step_device
+// (policy_apply on a 12-word shared-memory board); a stale or unvisited root steps with no action.
+constexpr int kPlayWarps = 4;      // trees per CTA of the play and noise kernels
+
+struct PlayArgs {
+    xq_env_rec* envs; uint64_t env_id0, seed;
+    float tau; int sample_plies, view, auto_reset;
+    int64_t* actions; int32_t* reward; uint8_t *done, *winner, *captured, *valid;
+};
+
+__global__ void __launch_bounds__(32 * kPlayWarps) search_play_kernel(SearchDev d, PlayArgs a) {
+    __shared__ uint32_t s_b[kPlayWarps][12];
+    __shared__ float s_w[kPlayWarps][kSearchEdges];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t t = (int64_t)blockIdx.x * kPlayWarps + warp;
+    if (t >= d.n) return;
+    const int64_t g0 = t * d.cap, eb0 = g0 * kSearchEdges;
+    bool diff = false;
+    if (lane < 4) {
+        const uint4 rv = reinterpret_cast<const uint4*>(d.rec + g0)[lane], ev = reinterpret_cast<const uint4*>(a.envs + t)[lane];
+        diff = rv.x != ev.x || rv.y != ev.y || rv.z != ev.z || rv.w != ev.w;
+    }
+    const bool stale = __any_sync(0xFFFFFFFFu, diff);
+    const int ne = !stale && d.expanded[g0] ? d.nedges[g0] : 0;
+    int nv[kSearchEdges / 32];
+    int nmax = 0;
+#pragma unroll
+    for (int i = 0; i < kSearchEdges / 32; ++i) {
+        const int k = lane + 32 * i;
+        nv[i] = k < ne ? d.N[eb0 + k] : 0;
+        nmax = max(nmax, nv[i]);
+    }
+    nmax = __reduce_max_sync(0xFFFFFFFFu, nmax);
+    int kp = -1;
+    if (nmax > 0) {
+        const xq_env_rec& root = d.rec[g0];
+        if (a.tau == 0.f || (int)root.move_count >= a.sample_plies) {
+            int first = kSearchEdges;
+#pragma unroll
+            for (int i = kSearchEdges / 32 - 1; i >= 0; --i) first = nv[i] == nmax && lane + 32 * i < ne ? lane + 32 * i : first;
+            kp = (int)__reduce_min_sync(0xFFFFFFFFu, (unsigned)first);
+        } else {
+#pragma unroll
+            for (int i = 0; i < kSearchEdges / 32; ++i) {
+                const int k = lane + 32 * i;
+                if (k < ne) s_w[warp][k] = search_play_weight(nv[i], nmax, a.tau);
+            }
+            __syncwarp();
+            if (lane == 0) kp = search_play_sample([&](int k) { return s_w[warp][k]; }, ne, policy_uniform(rng(a.seed, a.env_id0 + (uint64_t)t, root.ctr)));
+        }
+    }
+    if (lane != 0) return;
+    SmemBoard b{s_b[warp], 1};
+    b.load(a.envs + t);
+    Meta m; m.load(a.envs + t);
+    const int ai = kp >= 0 ? d.act[eb0 + kp] : 0, from = ai / 90, to = ai % 90;
+    if (a.actions) a.actions[t] = kp >= 0 ? policy_index(from, to, policy_flip(m.player, a.view)) : -1;
+    policy_apply(b, m, a.envs, t, kp >= 0, from, to, a.auto_reset, a.reward, a.done, a.winner, a.captured, a.valid);
+}
+
+// Dirichlet(alpha) noise mixed into the priors of every expanded root with at least one edge (xq_search_root_noise_device), one warp per
+// tree: the lanes draw the log-Gamma variates of edges k = lane + 32 i (search_log_gamma), the maximum is a shuffle reduction, the
+// exponentials go through shared memory where lane 0 sums them in list order; every lane then divides its edges, writes eta and mixes it
+// into the priors in place (search_mix).  The arithmetic is search_dirichlet's.
+__global__ void __launch_bounds__(32 * kPlayWarps) search_noise_kernel(SearchDev d, float alpha, float eps, uint64_t seed, uint64_t env_id0,
+                                                                      const uint8_t* __restrict__ mask, float* __restrict__ noise_out) {
+    __shared__ float s_e[kPlayWarps][kSearchEdges];
+    __shared__ float s_sum[kPlayWarps];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t t = (int64_t)blockIdx.x * kPlayWarps + warp;
+    if (t >= d.n) return;
+    const int64_t g0 = t * d.cap, eb0 = g0 * kSearchEdges;
+    const int ne = (!mask || mask[t]) && d.expanded[g0] ? d.nedges[g0] : 0;
+    float* out = noise_out ? noise_out + t * kSearchEdges : nullptr;
+    if (ne == 0) {
+        if (out) for (int k = lane; k < kSearchEdges; k += 32) out[k] = 0.f;
+        return;
+    }
+    const uint64_t base = rng(seed, env_id0 + (uint64_t)t, d.rec[g0].ctr);
+    float lg[kSearchEdges / 32];
+    float m = -INFINITY;
+#pragma unroll
+    for (int i = 0; i < kSearchEdges / 32; ++i) {
+        const int k = lane + 32 * i;
+        lg[i] = k < ne ? search_log_gamma(base, k, alpha) : -INFINITY;
+        m = fmaxf(m, lg[i]);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) m = fmaxf(m, __shfl_xor_sync(0xFFFFFFFFu, m, off));
+#pragma unroll
+    for (int i = 0; i < kSearchEdges / 32; ++i) {
+        const int k = lane + 32 * i;
+        if (k < ne) s_e[warp][k] = search_noise_exp(lg[i], m);
+    }
+    __syncwarp();
+    if (lane == 0) {
+        float s = 0.f;
+        for (int k = 0; k < ne; ++k) s = s_add(s, s_e[warp][k]);
+        s_sum[warp] = s;
+    }
+    __syncwarp();
+    const float s = s_sum[warp];
+#pragma unroll
+    for (int i = 0; i < kSearchEdges / 32; ++i) {
+        const int k = lane + 32 * i;
+        const float eta = k < ne ? s_div(s_e[warp][k], s) : 0.f;
+        if (k < ne) d.P[eb0 + k] = search_mix(d.P[eb0 + k], eta, eps);
+        if (out) out[k] = eta;
+    }
+}
+
 }  // namespace xq
 
 // ==========================================================================================
@@ -622,6 +738,34 @@ int xq_search_root_device(xq_search_t s, int view, int32_t* visits_dev, float* q
     if (reinterpret_cast<uintptr_t>(visits_dev) & 15u) return fail(XQ_ERR_INVALID, "xq_search_root_device: visits must be 16-byte aligned");
     if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_root_device: the search was never reset (xq_search_reset)");
     search_root_kernel<<<(unsigned)s->d.n, kRootThreads, 0, E.stream>>>(s->d, view, visits_dev, q_dev, best_dev);
+    XQ_LAUNCH_CHECK();
+    return XQ_OK;
+}
+
+int xq_search_play_device(xq_search_t s, float temperature, int sample_plies, int view, int auto_reset, int64_t* actions_dev, int32_t* reward_dev,
+                          uint8_t* done_dev, uint8_t* winner_dev, uint8_t* captured_dev, uint8_t* valid_dev) {
+    EnvInfo E;
+    if (int rc = enter(s, &E, "xq_search_play_device")) return rc;
+    if (!(temperature >= 0.f && temperature <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_search_play_device: temperature must be finite and >= 0");
+    if (sample_plies < 0) return fail(XQ_ERR_INVALID, "xq_search_play_device: sample_plies %d < 0", sample_plies);
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_search_play_device: view %d", view);
+    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_play_device: the search was never reset (xq_search_reset)");
+    if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_search_play_device: the last selection was not expanded and backed up");
+    const PlayArgs a{E.d_envs, E.env_id0, E.seed, temperature, sample_plies, view, auto_reset,
+                     actions_dev, reward_dev, done_dev, winner_dev, captured_dev, valid_dev};
+    search_play_kernel<<<grid_of(s->d.n, kPlayWarps), 32 * kPlayWarps, 0, E.stream>>>(s->d, a);
+    XQ_LAUNCH_CHECK();
+    return XQ_OK;
+}
+
+int xq_search_root_noise_device(xq_search_t s, float alpha, float eps, uint64_t seed, const uint8_t* mask_dev, float* noise_out_dev) {
+    EnvInfo E;
+    if (int rc = enter(s, &E, "xq_search_root_noise_device")) return rc;
+    if (!(alpha > 0.f && alpha <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_search_root_noise_device: alpha must be finite and > 0");
+    if (!(eps >= 0.f && eps <= 1.f)) return fail(XQ_ERR_INVALID, "xq_search_root_noise_device: eps must be in [0, 1]");
+    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_root_noise_device: the search was never reset (xq_search_reset)");
+    if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_search_root_noise_device: the last selection was not expanded and backed up");
+    search_noise_kernel<<<grid_of(s->d.n, kPlayWarps), 32 * kPlayWarps, 0, E.stream>>>(s->d, alpha, eps, seed, E.env_id0, mask_dev, noise_out_dev);
     XQ_LAUNCH_CHECK();
     return XQ_OK;
 }

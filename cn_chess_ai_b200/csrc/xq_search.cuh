@@ -1,6 +1,7 @@
 // xq_search.cuh -- host-compilable helpers of the batched tree search (xq_search.cu; include/xq.h: xq_search_*): the PUCT score of an
 // edge and its arg-max order, the priors of a freshly expanded node, the root-noise mix, the value cleaning, the backup along a path, and
-// the membership and renumbering of a tree re-rooted after a move (xq_search_advance).
+// the membership and renumbering of a tree re-rooted after a move (xq_search_advance), the visit-count choice of the move to play
+// (xq_search_play_device) and the Dirichlet draw of the root noise (xq_search_root_noise_device).
 //
 // The arithmetic is spelled with explicitly rounded operations (__fmul_rn and friends on the device; plain operators on the host, where
 // tests/hostsim/search_shim.cpp is compiled with -ffp-contract=off) so that no multiply-add is contracted and numpy can restate every
@@ -139,6 +140,68 @@ XQ_HD int search_membership(int count, int m, const int32_t* parent, uint32_t* b
 // the new index of kept node j
 XQ_HD int search_new_index(const uint32_t* bits, const int32_t* prefix, int j) {
     return prefix[j >> 5] + popc32(bits[j >> 5] & ((1u << (j & 31)) - 1u));
+}
+
+// ---- play: the move from the root's visit counts (xq_search_play_device) ----
+// weight of a root edge with n visits, nmax the root's largest count (> 0): n exactly at tau == 1 (every weight and sum an integer below
+// 2^24, exact in f32); otherwise exp(log(n / nmax) / tau), 0 for n == 0
+XQ_HD float search_play_weight(int n, int nmax, float tau) {
+    if (tau == 1.f) return (float)n;
+    return n > 0 ? expf(s_div(logf(s_div((float)n, (float)nmax)), tau)) : 0.f;
+}
+// the sampled edge among n: S = the weights w(k) summed in list order, the first k whose running sum exceeds u * S, else (rounding) the last
+// edge with a positive weight; -1 if none has one
+template <class W>
+XQ_HD int search_play_sample(W&& w, int n, float u) {
+    float s = 0.f;
+    for (int k = 0; k < n; ++k) s = s_add(s, w(k));
+    const float thr = s_mul(u, s);
+    float run = 0.f;
+    int last = -1;
+    for (int k = 0; k < n; ++k) {
+        const float x = w(k);
+        run = s_add(run, x);
+        if (run > thr) return k;
+        last = x > 0.f ? k : last;
+    }
+    return last;
+}
+
+// ---- root noise: Dirichlet(alpha) over a root's edges (xq_search_root_noise_device) ----
+// Word j of edge k: xq_rng(base, k, j), base = xq_rng(seed, global env id, root ctr).  A uniform from the 24-bit field f at bit `lo` is
+// (f + 1) * 2^-24 in (0, 1] (exact in f32, never 0, so every log is finite).  Word 0: the boost uniform Ub (bits 40..63).  Candidate i
+// (i = 0 .. 31): word 1 + 2i gives a Box-Muller normal z = sqrt(-2 log u1) * cos(2 pi u2) (u1 bits 40..63, u2 bits 16..39), word 2 + 2i the
+// acceptance uniform Ua (bits 40..63).  Marsaglia-Tsang at shape a = alpha + 1: d = a - 1/3, c = 1 / sqrt(9 d), v = (1 + c z)^3, accepted
+// when v > 0 and log Ua < ((0.5 z^2 + d) - d v) + d log v.  After 32 rejected candidates the last one with v > 0 is used (v = 1 if none
+// had); at a rejection rate below 5 % per candidate this never happens in practice.  Gamma(alpha) = d v Ub^(1 / alpha), kept in log space.
+constexpr int kGammaTries = 32;
+XQ_HD float search_u24(uint64_t x, int lo) { return s_mul(s_add((float)((uint32_t)(x >> lo) & 0xFFFFFFu), 1.f), 5.9604644775390625e-8f); }
+// log of the Gamma(alpha) draw of edge k: log(d v) + log(Ub) / alpha
+XQ_HD float search_log_gamma(uint64_t base, int k, float alpha) {
+    const float d = s_add(s_add(alpha, 1.f), -1.f / 3.f);
+    const float c = s_div(1.f, s_sqrt(s_mul(9.f, d)));
+    float v = 1.f;
+    for (int i = 0; i < kGammaTries; ++i) {
+        const uint64_t xn = rng(base, (uint64_t)k, (uint32_t)(1 + 2 * i));
+        const float z = s_mul(s_sqrt(s_mul(-2.f, logf(search_u24(xn, 40)))), cosf(s_mul(6.28318548f, search_u24(xn, 16))));
+        const float t = s_add(1.f, s_mul(c, z));
+        const float cand = s_mul(s_mul(t, t), t);
+        if (!(cand > 0.f)) continue;
+        v = cand;
+        const float ua = search_u24(rng(base, (uint64_t)k, (uint32_t)(2 + 2 * i)), 40);
+        if (logf(ua) < s_add(s_add(s_add(s_mul(0.5f, s_mul(z, z)), d), -s_mul(d, v)), s_mul(d, logf(v)))) break;
+    }
+    return s_add(logf(s_mul(d, v)), s_div(logf(search_u24(rng(base, (uint64_t)k, 0u), 40)), alpha));
+}
+// exp(lg - m) of one edge, m the largest lg of the root (all -inf: 1 for every edge, so that eta stays defined)
+XQ_HD float search_noise_exp(float lg, float m) { return m == -INFINITY ? 1.f : expf(s_add(lg, -m)); }
+// eta[0 .. n) of one root (n >= 1): eta_k = exp(lg_k - max) / S, S summed in list order.  Host restatement of the noise kernel.
+XQ_HD void search_dirichlet(uint64_t base, int n, float alpha, float* eta) {
+    float m = -INFINITY;
+    for (int k = 0; k < n; ++k) { eta[k] = search_log_gamma(base, k, alpha); m = fmaxf(m, eta[k]); }
+    float s = 0.f;
+    for (int k = 0; k < n; ++k) { eta[k] = search_noise_exp(eta[k], m); s = s_add(s, eta[k]); }
+    for (int k = 0; k < n; ++k) eta[k] = s_div(eta[k], s);
 }
 
 }  // namespace xq

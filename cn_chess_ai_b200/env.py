@@ -210,6 +210,18 @@ class BatchedSearch:
     def root_device(self, view, visits_ptr, q_ptr, best_ptr):
         check(self._L.xq_search_root_device(self._h, view, visits_ptr, q_ptr, best_ptr))
 
+    def play_device(self, temperature, sample_plies, view, auto_reset, actions_ptr=None, reward_ptr=None, done_ptr=None, winner_ptr=None,
+                    captured_ptr=None, valid_ptr=None):
+        """xq_search_play_device: one move per tree from its root's visit counts (greedy, or sampled with N^(1/temperature) for the first
+        sample_plies plies), played on the env"""
+        check(self._L.xq_search_play_device(self._h, float(temperature), int(sample_plies), view, 1 if auto_reset else 0, actions_ptr, reward_ptr,
+                                            done_ptr, winner_ptr, captured_ptr, valid_ptr))
+
+    def root_noise_device(self, alpha, eps, seed, mask_ptr=None, noise_out_ptr=None):
+        """xq_search_root_noise_device: Dirichlet(alpha) noise drawn over each expanded root's edges and mixed into its priors; mask u8 [n]
+        or None, noise_out f32 [n][128] (list order) or None"""
+        check(self._L.xq_search_root_noise_device(self._h, float(alpha), float(eps), int(seed), mask_ptr, noise_out_ptr))
+
     def get_tree(self, tree):
         """synchronous read-back of one tree: (nodes SEARCH_NODE_DTYPE [n_nodes], edges SEARCH_EDGE_DTYPE [n_nodes][128])"""
         cap = self.max_simulations + 1

@@ -9,9 +9,9 @@ from collections import namedtuple
 
 import torch
 
-from ._lib import POLICY_ACTIONS
+from ._lib import POLICY_ACTIONS, SEARCH_MAX_EDGES
 from .env import BatchedSearch
-from .torch_env import _OBS_DTYPES, _SCORE_DTYPES, _view
+from .torch_env import _OBS_DTYPES, _SCORE_DTYPES, StepResult, _view
 
 SelectResult = namedtuple("SelectResult", "status winner reward depth")
 RootResult = namedtuple("RootResult", "visits q best")
@@ -29,6 +29,7 @@ class TorchSearch:
         self.device = tenv.device
         self.search = BatchedSearch(tenv.env, max_simulations)
         self.max_simulations = self.search.max_simulations
+        self._kept = None          # kept int32 [n] of the last advance(); None after reset(): every root was rebuilt
 
     def close(self):
         self.search.close()
@@ -36,6 +37,7 @@ class TorchSearch:
     def reset(self):
         self.tenv._enter()
         self.search.reset()
+        self._kept = None
 
     def advance(self, min_free, root_noise=None, noise_eps=0.25, view="side"):
         """instead of reset() after a move: every tree is re-rooted at its env's current board, keeping the subtree (and its statistics)
@@ -49,6 +51,7 @@ class TorchSearch:
         self.tenv._enter()
         kept = torch.empty(self.n, dtype=torch.int32, device=self.device)
         self.search.advance_device(min_free, None if root_noise is None else root_noise.data_ptr(), noise_eps, v, kept.data_ptr())
+        self._kept = kept
         return kept
 
     def select(self, c_puct=1.5, fpu=0.0):
@@ -104,6 +107,35 @@ class TorchSearch:
         self.search.root_device(v, visits.data_ptr(), q.data_ptr(), best.data_ptr())
         return RootResult(visits, q, best)
 
+    def play(self, temperature=1.0, sample_plies=30, view="side", auto_reset=True):
+        """one move per env from its root's visit counts, played on the env: sampled with probability N^(1 / temperature) while the root's
+        move_count < sample_plies, the most-visited edge afterwards or at temperature 0.  A root that is not its env's board or has no
+        visited edge plays nothing (action -1, valid 0).  Returns a TorchEnv.step StepResult (logp None): actions int64 (frame of `view`),
+        reward i32, done / winner / captured / valid uint8 -- the input of TorchExamples.finish.  The trees are not changed: advance()
+        re-roots them at the played moves."""
+        v = _view(view)
+        self.tenv._enter()
+        actions = torch.empty(self.n, dtype=torch.int64, device=self.device)
+        reward = torch.empty(self.n, dtype=torch.int32, device=self.device)
+        done, winner, captured, valid = (torch.empty(self.n, dtype=torch.uint8, device=self.device) for _ in range(4))
+        self.search.play_device(temperature, sample_plies, v, auto_reset, actions.data_ptr(), reward.data_ptr(), done.data_ptr(),
+                                winner.data_ptr(), captured.data_ptr(), valid.data_ptr())
+        return StepResult(actions, None, reward, done, winner, captured, valid)
+
+    def root_noise(self, alpha, eps=0.25, seed=0, mask=None, want_noise=False):
+        """Dirichlet(alpha) noise drawn by the library over the edges of every expanded root (or of the envs where mask, bool / uint8 [n],
+        is set) and mixed into its priors: P <- (1 - eps) P + eps eta.  The draw depends on the seed, the global env id and the root's
+        ply counter only.  Returns eta f32 [n, 128] in the root's edge order (0 past its edges and for trees left alone) with want_noise,
+        else None."""
+        m = None
+        if mask is not None:
+            self.tenv._check(mask, "mask", [torch.bool, torch.uint8], (self.n,))
+            m = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
+        self.tenv._enter()
+        out = torch.empty((self.n, SEARCH_MAX_EDGES), dtype=torch.float32, device=self.device) if want_noise else None
+        self.search.root_noise_device(alpha, eps, seed, None if m is None else m.data_ptr(), None if out is None else out.data_ptr())
+        return out
+
     @staticmethod
     def outcome_values(status, winner, aux, cap_value=0.0):
         """a default value of terminal leaves, from the leaf's side to move (aux[:, 0], absolute colour): +1 / -1 when a General was
@@ -116,13 +148,20 @@ class TorchSearch:
         return torch.where(status == NO_LEGAL_ACTION, torch.full_like(v, -1.0), v)
 
     def run(self, evaluate, n_simulations, c_puct=1.5, fpu=0.0, temperature=1.0, root_noise=None, noise_eps=0.25, view="side",
-            obs_dtype=torch.bfloat16, cap_value=0.0, reset=True):
+            obs_dtype=torch.bfloat16, cap_value=0.0, reset=True, dirichlet_alpha=None, dirichlet_eps=0.25, noise_seed=0):
         """reset + n_simulations simulations: evaluate(planes) -> (scores [n, 8100], values [n]) is called once per simulation on the
         leaves; at terminal leaves outcome_values replaces the network's value.  reset=False continues from the current trees (after
-        advance(), or to add simulations to this move's search).  Returns root(view)."""
+        advance(), or to add simulations to this move's search).  dirichlet_alpha: root_noise(dirichlet_alpha, dirichlet_eps, noise_seed)
+        once per root and move -- before the first simulation on the roots the last advance() kept, after it on the roots reset() or
+        advance() rebuilt (expanded by the first simulation).  Returns root(view)."""
         if reset:
             self.reset()
-        for _ in range(n_simulations):
+        kept = None if self._kept is None else self._kept > 0
+        if dirichlet_alpha is not None and kept is not None:
+            self.root_noise(dirichlet_alpha, dirichlet_eps, noise_seed, mask=kept)
+        for i in range(n_simulations):
+            if i == 1 and dirichlet_alpha is not None:
+                self.root_noise(dirichlet_alpha, dirichlet_eps, noise_seed, mask=None if kept is None else ~kept)
             sel = self.select(c_puct, fpu)
             planes, aux = self.observe(obs_dtype, view)
             scores, values = evaluate(planes)

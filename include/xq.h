@@ -226,7 +226,7 @@ int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dty
  * Expansion (status 0 only): scores [n][8100] (f32 / bf16, in the frame of `view`, cleaned as in xq_env_policy_step_device; only legal
  * entries are read) give P_k = exp((l_k - m) / T) / S, S summed in list order, uniform 1 / count if every legal score is -inf.  At the root
  * only, with root_noise_dev [n][8100] f32 (finite; e.g. Dirichlet noise the caller draws over the legal mask):
- * P <- (1 - eps) * P + eps * noise[index].  The library draws no random numbers.
+ * P <- (1 - eps) * P + eps * noise[index].  Expansion draws no random numbers; xq_search_root_noise_device draws the noise in the library.
  * Backup (every status): the caller's value of the leaf, from the leaf's side to move, NaN -> 0, clamped to [-1, 1]; going up,
  * v <- -v, the edge gets N += 1 and W += v, every node on the path N_node += 1.  The library has no value convention for terminal leaves.
  *
@@ -297,6 +297,36 @@ int xq_search_expand_backup_device(xq_search_t s, const void* scores_dev, int sc
  * int64 [n] = policy index (frame of `view`) of the most-visited root edge, first in list order on ties, -1 when no edge was visited --
  * the input of xq_env_policy_step_device with XQ_PICK_GIVEN. */
 int xq_search_root_device(xq_search_t s, int view, int32_t* visits_dev, float* q_dev, int64_t* best_dev);
+/* One move per tree from its root's visit counts, played on the search's env (asynchronous on its stream).  A tree whose root record
+ * differs in any of its 64 bytes from its env's current record (as xq_examples_record_device compares them), or whose root has no visited
+ * edge, plays nothing: the env steps as xq_env_step_device with XQ_ACTION_NONE (action -1, valid 0, board unchanged).  Otherwise:
+ *  greedy, when temperature == 0 or the root's move_count >= sample_plies: the most-visited root edge, first in list order on ties
+ *    (best_dev of xq_search_root_device);
+ *  sampled otherwise: w_k = N_k at temperature 1 (exact), else expf(logf(N_k / N_max) / temperature) in f32 (0 for N_k = 0); S = the w_k
+ *    summed in list order; u = (float)(xq_rng(seed, env_id0 + e, rec.ctr) >> 40) * 2^-24, the draw of XQ_PICK_SAMPLE; the first edge whose
+ *    running sum exceeds u*S is played (the last edge with w > 0 if rounding leaves none).  Results do not depend on sharding.
+ * The step is bit for bit xq_env_policy_step_device (XQ_PICK_GIVEN) with that edge's action: record, reward, done, winner, captured, valid
+ * and auto_reset.  actions_dev int64 [n] = the played policy index in the frame of `view` (-1 none); reward i32, done / winner / captured /
+ * valid u8 [n]; every output may be NULL.  The tree is not touched: the next xq_search_advance re-roots it at the played child.
+ * temperature finite and >= 0, sample_plies >= 0 (XQ_ERR_INVALID otherwise); allowed after a reset when no selection is pending
+ * (XQ_ERR_STATE otherwise, as xq_search_advance). */
+int xq_search_play_device(xq_search_t s, float temperature, int sample_plies, int view, int auto_reset, int64_t* actions_dev, int32_t* reward_dev,
+                          uint8_t* done_dev, uint8_t* winner_dev, uint8_t* captured_dev, uint8_t* valid_dev);
+/* Dirichlet(alpha) exploration noise drawn by the library and mixed into the priors of every root that is expanded with at least one edge,
+ * or of those with mask_dev[e] != 0 (u8 [n]; NULL = all): P_k <- (1 - eps) * P_k + eps * eta_k, the expression of the dense root_noise_dev
+ * path.  eta is drawn over the root's n_edges edges in list order from words xq_rng(xq_rng(seed, env_id0 + e, root ctr), k, j) of edge k:
+ * it depends only on the seed, the global env id, the root's ply counter and the edge, not on sharding or n.  A uniform from the 24-bit
+ * field f of a word at bit b is (f + 1) * 2^-24, in (0, 1].  Word 0 (bits 40..63): the boost uniform Ub.  Candidate i = 0 .. 31: word
+ * 1 + 2i gives z = sqrt(-2 log u1) * cos(2 pi u2) (u1 from bits 40..63, u2 from bits 16..39), word 2 + 2i the acceptance uniform Ua (bits
+ * 40..63).  Marsaglia-Tsang at shape a = alpha + 1, d = a - 1/3, c = 1 / sqrt(9 d), v = (1 + c z)^3: the first candidate with v > 0 and
+ * log Ua < ((0.5 z^2 + d) - d v) + d log v is taken; after 32 rejected candidates the last with v > 0 (v = 1 if none) is used, which at a
+ * rejection rate below 5 % never happens in practice.  lg_k = log(d v) + log(Ub) / alpha (Gamma(alpha) = Gamma(alpha + 1) Ub^(1/alpha),
+ * kept in log space so that tiny alpha does not underflow); eta_k = exp(lg_k - max) / S, S summed in list order.  All arithmetic in f32
+ * with no contraction.  noise_out_dev f32 [n][128] or NULL: eta in list order, 0 past n_edges and in whole rows of trees not noised.
+ * Trees outside the mask or with an unexpanded root are not changed.  alpha finite and > 0, eps in [0, 1] (XQ_ERR_INVALID otherwise);
+ * allowed after a reset when no selection is pending (XQ_ERR_STATE otherwise).  Neither call uses device memory beyond
+ * xq_search_bytes_per_tree. */
+int xq_search_root_noise_device(xq_search_t s, float alpha, float eps, uint64_t seed, const uint8_t* mask_dev, float* noise_out_dev);
 /* synchronous read-back of one tree: nodes_host[max_simulations + 1], edges_host [max_simulations + 1][128] (may be NULL; edges past a
  * node's n_edges have action -1 and child -1), *n_nodes = nodes in the tree */
 int xq_search_get_tree(xq_search_t s, int64_t tree, xq_search_node* nodes_host, xq_search_edge* edges_host, int32_t* n_nodes);
