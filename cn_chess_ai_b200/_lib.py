@@ -27,6 +27,7 @@ VIEW_ABSOLUTE, VIEW_SIDE_TO_MOVE = 0, 1
 PICK_GREEDY, PICK_SAMPLE, PICK_GIVEN = 0, 1, 2
 SEARCH_MAX_EDGES = 128    # edge slots per search-tree node (include/xq.h: XQ_SEARCH_MAX_EDGES)
 SEARCH_ADVANCE_MAX_SIMULATIONS = 65536    # largest max_simulations xq_search_advance takes (include/xq.h)
+SEARCH_MAX_LEAVES = 32    # largest max_leaves of a search, leaves of one selection (include/xq.h: XQ_SEARCH_MAX_LEAVES)
 SEARCH_NODE_DTYPE = np.dtype([("rec", ENV_DTYPE), ("parent", "<i4"), ("visits", "<i4"), ("reward", "<i4"), ("depth", "<i4"),
                               ("parent_edge", "u1"), ("n_edges", "u1"), ("expanded", "u1"), ("status", "u1"), ("winner", "u1"),
                               ("reserved", "u1", (3,))])
@@ -93,11 +94,14 @@ def lib():
     L.xq_env_legal_mask_device.argtypes = [_P, _P, C.c_int, C.c_int]
     L.xq_env_policy_step_device.argtypes = [_P, _P, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int] + [_P] * 7
     L.xq_search_create.argtypes = [_P, C.c_int, C.POINTER(_P)]
+    L.xq_search_create_ex.argtypes = [_P, C.c_int, C.c_int, C.POINTER(_P)]
     L.xq_search_destroy.argtypes = [_P]
     L.xq_search_bytes_per_tree.argtypes = [C.c_int, C.POINTER(C.c_int64)]
+    L.xq_search_bytes_per_tree_ex.argtypes = [C.c_int, C.c_int, C.POINTER(C.c_int64)]
     L.xq_search_reset.argtypes = [_P]
     L.xq_search_advance.argtypes = [_P, C.c_int, _P, C.c_float, C.c_int, _P]
     L.xq_search_select_device.argtypes = [_P, C.c_float, C.c_float, _P, _P, _P, _P]
+    L.xq_search_select_leaves_device.argtypes = [_P, C.c_int, C.c_float, C.c_float, C.c_float, _P, _P, _P, _P]
     L.xq_search_leaves_device.argtypes = [_P, C.POINTER(_P)]
     L.xq_search_observe_leaves_device.argtypes = [_P, _P, C.c_int, C.c_int, _P]
     L.xq_search_expand_backup_device.argtypes = [_P, _P, C.c_int, C.c_float, C.c_int, _P, _P, C.c_float]

@@ -11,6 +11,9 @@
 // search_expand_lane_kernel: one thread per tree, the structure of policy_step_lane_kernel: the generator stages the legal scores into
 //   a [list index][thread] shared row, the priors are taken over that row in list order, the backup walks the parent pointers.
 //   Boards the generator refuses go to search_expand_generic_kernel (all_actions, thread per board).
+// search_select_leaves_kernel: one warp per tree, the L descents of a multi-leaf selection in order with virtual loss (in-flight counts
+//   from the earlier descents' edges, kept per depth in shared memory); search_expand_slots_kernel / search_expand_generic_slots_kernel:
+//   one thread per (tree, slot) for the expansions, the backups of a tree in slot order by the thread of its slot 0.
 // search_root_kernel: one CTA per tree, the dense visit row built in shared memory and written with 16-byte stores.
 // search_advance_kernel: one warp per tree, re-roots the tree at the played child in place (membership bitmap in shared memory).
 // search_play_kernel: one warp per tree, the move from the root's visit counts and the env's step with it.
@@ -228,6 +231,32 @@ __global__ void __launch_bounds__(32 * kAdvWarps) search_advance_kernel(SearchDe
     }
 }
 
+// node nw of tree t as the child of `node` through edge bk: the parent's record after the action, exactly as xq_env_step_device
+// (auto_reset = 0) makes it (one thread; sb a 12-word shared board)
+__device__ __forceinline__ void search_make_child(const SearchDev& d, int64_t t, int64_t g0, int node, int bk, int nw, uint32_t* sb) {
+    const int64_t g = g0 + node, eb = g * kSearchEdges;
+    const int a = d.act[eb + bk];
+    const int64_t gn = g0 + nw;
+    SmemBoard b{sb, 1};
+    b.load(d.rec + g);
+    Meta m; m.load(d.rec + g);
+    const int mover = m.player;
+    apply_move(b, m, a / 90, a % 90);
+    m.ctr++;
+    uint32_t wd[12];
+#pragma unroll
+    for (int i = 0; i < 12; ++i) wd[i] = b.base[i];
+    const WordSummary s = summarize_words(wd);
+    uint8_t term, win;
+    search_status(s, m.move_count, term, win);
+    const int diff = mover == RED ? s.mat_red - s.mat_black : s.mat_black - s.mat_red;
+    b.store(d.rec + gn); m.store(d.rec + gn);
+    d.parent[gn] = node; d.pedge[gn] = (uint8_t)bk; d.visits[gn] = 0; d.reward[gn] = reward_from_material(diff, m.move_count);
+    d.depth[gn] = d.depth[g] + 1; d.nedges[gn] = 0; d.expanded[gn] = 0; d.term[gn] = term; d.winner[gn] = win;
+    d.child[eb + bk] = nw;
+    d.count[t] = nw + 1;
+}
+
 __global__ void __launch_bounds__(32 * kSelWarps) search_select_kernel(SearchDev d, float c_puct, float fpu, uint8_t* __restrict__ status,
                                                                       uint8_t* __restrict__ winner, int32_t* __restrict__ reward,
                                                                       int32_t* __restrict__ depth) {
@@ -258,30 +287,8 @@ __global__ void __launch_bounds__(32 * kSelWarps) search_select_kernel(SearchDev
         bk = __shfl_sync(0xFFFFFFFFu, bk, 0);
         const int child = d.child[eb + bk];
         if (child >= 0) { node = child; continue; }
-        // a new child: the parent's record after the action, exactly as xq_env_step_device (auto_reset = 0) makes it
         const int nw = d.count[t];
-        if (lane == 0) {
-            const int a = d.act[eb + bk];
-            const int64_t gn = g0 + nw;
-            SmemBoard b{s_b[warp], 1};
-            b.load(d.rec + g);
-            Meta m; m.load(d.rec + g);
-            const int mover = m.player;
-            apply_move(b, m, a / 90, a % 90);
-            m.ctr++;
-            uint32_t wd[12];
-#pragma unroll
-            for (int i = 0; i < 12; ++i) wd[i] = b.base[i];
-            const WordSummary s = summarize_words(wd);
-            uint8_t term, win;
-            search_status(s, m.move_count, term, win);
-            const int diff = mover == RED ? s.mat_red - s.mat_black : s.mat_black - s.mat_red;
-            b.store(d.rec + gn); m.store(d.rec + gn);
-            d.parent[gn] = node; d.pedge[gn] = (uint8_t)bk; d.visits[gn] = 0; d.reward[gn] = reward_from_material(diff, m.move_count);
-            d.depth[gn] = d.depth[g] + 1; d.nedges[gn] = 0; d.expanded[gn] = 0; d.term[gn] = term; d.winner[gn] = win;
-            d.child[eb + bk] = nw;
-            d.count[t] = nw + 1;
-        }
+        if (lane == 0) search_make_child(d, t, g0, node, bk, nw, s_b[warp]);
         leaf = nw;
         break;
     }
@@ -295,6 +302,87 @@ __global__ void __launch_bounds__(32 * kSelWarps) search_select_kernel(SearchDev
             if (winner) winner[t] = d.winner[g];
             if (reward) reward[t] = d.reward[g];
             if (depth) depth[t] = d.depth[g];
+        }
+    }
+}
+
+// Multi-leaf selection (xq_search_select_leaves_device), one warp per tree: the L descents k = 0 .. L - 1 in order, each by the rules of
+// search_select_kernel with the scores of search_puct_vl.  Lane k' stands for descent k' once it has ended: it holds that descent's leaf
+// and its alive bit (search_inflight_node); the list index of the edge each descent took at depth dep is s_path[dep][k'] (depth < 200:
+// a node at move 200 is terminal).  At a node the alive lanes add their edge to the warp's count row s_cnt (integer atomics: the counts
+// do not depend on the order), the scoring lanes read it, and the alive lanes clear their entries again.  The slab changes only by child
+// creation, as in search_select_kernel.  A descent that ends at an open leaf (unexpanded, not terminal) an earlier one ended at is a
+// duplicate: status 4, leaf index -1 for the expand kernel.
+constexpr int kSelLeavesWarps = 4;      // trees per CTA of the multi-leaf select kernel
+
+__global__ void __launch_bounds__(32 * kSelLeavesWarps) search_select_leaves_kernel(SearchDev d, int L, float c_puct, float fpu, float vl,
+                                                                                    uint8_t* __restrict__ status, uint8_t* __restrict__ winner,
+                                                                                    int32_t* __restrict__ reward, int32_t* __restrict__ depth) {
+    __shared__ uint32_t s_b[kSelLeavesWarps][12];
+    __shared__ uint8_t s_path[kSelLeavesWarps][XQ_MAX_MOVES][32];
+    __shared__ int32_t s_cnt[kSelLeavesWarps][kSearchEdges];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t t = (int64_t)blockIdx.x * kSelLeavesWarps + warp;
+    if (t >= d.n) return;
+    for (int e = lane; e < kSearchEdges; e += 32) s_cnt[warp][e] = 0;
+    __syncwarp();
+    const int64_t g0 = t * d.cap;
+    int mine = -1;                      // lane k: the leaf of descent k
+    for (int k = 0; k < L; ++k) {
+        bool alive = lane < k;
+        int node = 0, dep = 0, leaf;
+        for (;;) {
+            const int64_t g = g0 + node;
+            if (!d.expanded[g] || d.term[g]) { leaf = node; break; }
+            const int ne = d.nedges[g];
+            const int cj = popc32(__ballot_sync(0xFFFFFFFFu, alive));
+            if (alive) atomicAdd(&s_cnt[warp][s_path[warp][dep][lane]], 1);
+            __syncwarp();
+            const float sq = search_sqrt_visits(d.visits[g] + cj);
+            const int64_t eb = g * kSearchEdges;
+            float bs = 0.f;
+            int bk = -1;
+            for (int e = lane; e < ne; e += 32) {
+                const float v = search_puct_vl(d.P[eb + e], d.N[eb + e], d.W[eb + e], s_cnt[warp][e], vl, c_puct, fpu, sq);
+                if (search_better(v, e, bs, bk)) { bs = v; bk = e; }
+            }
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) {
+                const float os = __shfl_xor_sync(0xFFFFFFFFu, bs, off);
+                const int ok = __shfl_xor_sync(0xFFFFFFFFu, bk, off);
+                if (ok >= 0 && search_better(os, ok, bs, bk)) { bs = os; bk = ok; }
+            }
+            bk = __shfl_sync(0xFFFFFFFFu, bk, 0);
+            __syncwarp();
+            if (alive) {
+                const int e = s_path[warp][dep][lane];
+                s_cnt[warp][e] = 0;
+                alive = e == bk;
+            }
+            if (lane == 0) s_path[warp][dep][k] = (uint8_t)bk;
+            __syncwarp();
+            ++dep;
+            const int child = d.child[eb + bk];
+            if (child >= 0) { node = child; continue; }
+            const int nw = d.count[t];
+            if (lane == 0) search_make_child(d, t, g0, node, bk, nw, s_b[warp]);
+            leaf = nw;
+            break;
+        }
+        __syncwarp();
+        const int64_t g = g0 + leaf, i = t * L + k;
+        const bool open = !d.expanded[g] && !d.term[g];
+        const bool dup = __any_sync(0xFFFFFFFFu, lane < k && mine == leaf) && open;
+        if (lane == k) mine = leaf;
+        if (lane < 4) {
+            reinterpret_cast<uint4*>(d.leaf_rec + i)[lane] = reinterpret_cast<const uint4*>(d.rec + g)[lane];
+            if (lane == 0) {
+                d.leaf[i] = dup ? -1 : leaf;
+                if (status) status[i] = dup ? 4 : d.term[g];
+                if (winner) winner[i] = d.winner[g];
+                if (reward) reward[i] = d.reward[g];
+                if (depth) depth[i] = d.depth[g];
+            }
         }
     }
 }
@@ -323,22 +411,16 @@ __device__ __forceinline__ void search_write_edges(const SearchDev& d, const Exp
     if (n == 0) d.term[g] = 3;
 }
 
+// Expansion of leaf `leaf` of tree t from the leaf record and score row `slot` (slot = t at one leaf per tree), one thread: the structure
+// of policy_step_lane_kernel (the generator stages the legal scores into the [list index][thread] shared row s_row).  Returns 1 when the
+// generator refuses the board and the generic kernel has to expand it.
 template <int SDT>
-__global__ void __launch_bounds__(kExpBoards) search_expand_lane_kernel(SearchDev d, ExpandArgs a) {
-    __shared__ uint8_t s_slot[32 * kExpBoards];
-    __shared__ uint32_t s_geo[kGeoWords];
-    __shared__ uint32_t s_view[kViewWords * kExpBoards];
-    __shared__ float s_row[XQ_MAX_ACTIONS * kExpBoards];       // [list index][thread]: the raw scores of the legal actions
-    const int tid = threadIdx.x;
-    const int64_t t = (int64_t)blockIdx.x * kExpBoards + tid;
-    for (int i = tid; i < kGeoWords; i += kExpBoards) s_geo[i] = geo_word(i);
-    __syncthreads();
-    if (t >= d.n) return;
-    const int leaf = d.leaf[t];
-    const int64_t g0 = t * d.cap, g = g0 + leaf;
+__device__ __forceinline__ uint8_t search_expand_lane(const SearchDev& d, const ExpandArgs& a, int64_t t, int64_t slot, int leaf, int tid,
+                                                      uint8_t* s_slot, const uint32_t* s_geo, uint32_t* s_view, float* s_row) {
+    const int64_t g = t * d.cap + leaf;
     uint8_t generic = 0;
     if (!d.expanded[g] && d.term[g] == 0) {
-        const uint4* rec = reinterpret_cast<const uint4*>(d.leaf_rec + t);
+        const uint4* rec = reinterpret_cast<const uint4*>(d.leaf_rec + slot);
         uint32_t w[12];
 #pragma unroll
         for (int i = 0; i < 3; ++i) { const uint4 v = rec[i]; w[4 * i] = v.x; w[4 * i + 1] = v.y; w[4 * i + 2] = v.z; w[4 * i + 3] = v.w; }
@@ -346,7 +428,7 @@ __global__ void __launch_bounds__(kExpBoards) search_expand_lane_kernel(SearchDe
         LaneGen lg;
         if (policy_lane_gen(w, player, s_view + tid, s_slot + tid, kExpBoards, s_geo, lg)) {
             const bool flip = policy_flip(player, a.view);
-            const void* sc = static_cast<const uint8_t*>(a.scores) + t * XQ_POLICY_ACTIONS * (SDT == XQ_DTYPE_BF16 ? 2 : 4);
+            const void* sc = static_cast<const uint8_t*>(a.scores) + slot * XQ_POLICY_ACTIONS * (SDT == XQ_DTYPE_BF16 ? 2 : 4);
             const int64_t eb = g * kSearchEdges;
             const int cnt = policy_lane_emit(lg, player, [&](int idx, int from, int to) {
                 s_row[idx * kExpBoards + tid] = search_score<SDT>(sc, policy_index(from, to, flip));
@@ -361,23 +443,63 @@ __global__ void __launch_bounds__(kExpBoards) search_expand_lane_kernel(SearchDe
             generic = 1;
         }
     }
-    d.nonstd[t] = generic;      // the generic kernel expands it; the backup below does not touch the new node's edges
-    search_backup(leaf, a.values[t], d.parent + g0, d.pedge + g0, d.visits + g0, d.N + g0 * kSearchEdges, d.W + g0 * kSearchEdges);
+    return generic;
 }
 
 template <int SDT>
-__global__ void __launch_bounds__(kThreads) search_expand_generic_kernel(SearchDev d, ExpandArgs a) {
-    __shared__ uint32_t s_board[12 * kThreads];
-    const int64_t t = (int64_t)blockIdx.x * kThreads + threadIdx.x;
-    if (t >= d.n || !d.nonstd[t]) return;
+__global__ void __launch_bounds__(kExpBoards) search_expand_lane_kernel(SearchDev d, ExpandArgs a) {
+    __shared__ uint8_t s_slot[32 * kExpBoards];
+    __shared__ uint32_t s_geo[kGeoWords];
+    __shared__ uint32_t s_view[kViewWords * kExpBoards];
+    __shared__ float s_row[XQ_MAX_ACTIONS * kExpBoards];       // [list index][thread]: the raw scores of the legal actions
+    const int tid = threadIdx.x;
+    const int64_t t = (int64_t)blockIdx.x * kExpBoards + tid;
+    for (int i = tid; i < kGeoWords; i += kExpBoards) s_geo[i] = geo_word(i);
+    __syncthreads();
+    if (t >= d.n) return;
     const int leaf = d.leaf[t];
+    const int64_t g0 = t * d.cap;
+    // the generic kernel expands a refused board; the backup below does not touch the new node's edges
+    d.nonstd[t] = search_expand_lane<SDT>(d, a, t, t, leaf, tid, s_slot, s_geo, s_view, s_row);
+    search_backup(leaf, a.values[t], d.parent + g0, d.pedge + g0, d.visits + g0, d.N + g0 * kSearchEdges, d.W + g0 * kSearchEdges);
+}
+
+// Expansion and backup after a multi-leaf selection of L slots per tree (slot i = t * L + k), one thread per slot: each status-0 slot
+// expands its leaf as search_expand_lane_kernel does (its score row i, the noise row t at the root); the thread of slot 0 then backs up
+// the tree's non-duplicate slots in slot order.  Expansions write only edges of unexpanded leaves, backups only edges of expanded
+// ancestors and N_node, so the two need no ordering between threads and the result is that of "expand, then back up in slot order".
+template <int SDT>
+__global__ void __launch_bounds__(kExpBoards) search_expand_slots_kernel(SearchDev d, ExpandArgs a, int L) {
+    __shared__ uint8_t s_slot[32 * kExpBoards];
+    __shared__ uint32_t s_geo[kGeoWords];
+    __shared__ uint32_t s_view[kViewWords * kExpBoards];
+    __shared__ float s_row[XQ_MAX_ACTIONS * kExpBoards];
+    const int tid = threadIdx.x;
+    const int64_t i = (int64_t)blockIdx.x * kExpBoards + tid;
+    for (int j = tid; j < kGeoWords; j += kExpBoards) s_geo[j] = geo_word(j);
+    __syncthreads();
+    if (i >= d.n * L) return;
+    const int64_t t = i / L;
+    const int leaf = d.leaf[i];          // -1: a duplicate slot
+    d.nonstd[i] = leaf >= 0 ? search_expand_lane<SDT>(d, a, t, i, leaf, tid, s_slot, s_geo, s_view, s_row) : 0;
+    if (i != t * L) return;
+    const int64_t g0 = t * d.cap;
+    for (int k = 0; k < L; ++k) {
+        const int lf = d.leaf[i + k];
+        if (lf >= 0) search_backup(lf, a.values[i + k], d.parent + g0, d.pedge + g0, d.visits + g0, d.N + g0 * kSearchEdges, d.W + g0 * kSearchEdges);
+    }
+}
+
+// Expansion of a board the generator refuses (all_actions, one thread): leaf `leaf` of tree t from the record and score row of slot i
+template <int SDT>
+__device__ __forceinline__ void search_expand_generic(const SearchDev& d, const ExpandArgs& a, int64_t t, int64_t i, int leaf, uint32_t* sb) {
     const int64_t g = t * d.cap + leaf, eb = g * kSearchEdges;
-    SmemBoard b{s_board + threadIdx.x, kThreads};
-    b.load(d.leaf_rec + t);
-    Meta mt; mt.load(d.leaf_rec + t);
+    SmemBoard b{sb, kThreads};
+    b.load(d.leaf_rec + i);
+    Meta mt; mt.load(d.leaf_rec + i);
     const int player = mt.player;
     const bool flip = policy_flip(player, a.view);
-    const void* sc = static_cast<const uint8_t*>(a.scores) + t * XQ_POLICY_ACTIONS * (SDT == XQ_DTYPE_BF16 ? 2 : 4);
+    const void* sc = static_cast<const uint8_t*>(a.scores) + i * XQ_POLICY_ACTIONS * (SDT == XQ_DTYPE_BF16 ? 2 : 4);
     // the first 128 actions in list order; a player byte > 1 owns no piece
     auto each_action = [&](auto&& f) {
         int c = 0;
@@ -393,6 +515,23 @@ __global__ void __launch_bounds__(kThreads) search_expand_generic_kernel(SearchD
     search_write_edges(d, a, t, g, leaf == 0, flip,
                        [&](auto&& f) { each_action([&](int from, int to) { f(policy_clean(search_score<SDT>(sc, policy_index(from, to, flip)))); }); },
                        cnt, best.m);
+}
+
+template <int SDT>
+__global__ void __launch_bounds__(kThreads) search_expand_generic_kernel(SearchDev d, ExpandArgs a) {
+    __shared__ uint32_t s_board[12 * kThreads];
+    const int64_t t = (int64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (t >= d.n || !d.nonstd[t]) return;
+    search_expand_generic<SDT>(d, a, t, t, d.leaf[t], s_board + threadIdx.x);
+}
+
+// the slots of a multi-leaf selection that search_expand_slots_kernel left to the generic generator
+template <int SDT>
+__global__ void __launch_bounds__(kThreads) search_expand_generic_slots_kernel(SearchDev d, ExpandArgs a, int L) {
+    __shared__ uint32_t s_board[12 * kThreads];
+    const int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (i >= d.n * L || !d.nonstd[i]) return;
+    search_expand_generic<SDT>(d, a, i / L, i, d.leaf[i], s_board + threadIdx.x);
 }
 
 __global__ void __launch_bounds__(kRootThreads) search_root_kernel(SearchDev d, int view, int32_t* __restrict__ visits, float* __restrict__ q,
@@ -553,6 +692,8 @@ struct xq_search_s {
     xq_env_t env = nullptr;
     int device = 0;
     int max_sims = 0;
+    int max_leaves = 1;
+    int leaves = 1;                // slots per tree of the last selection
     int sims = 0;
     int phase = 0;                 // 0 never reset, 1 ready for select, 2 selected (observe / leaves / expand_backup)
     bool maybe_nonstd = false;     // the env had injected boards at the reset: leaves may need the generic kernel
@@ -563,8 +704,9 @@ struct xq_search_s {
 namespace {
 constexpr size_t kNodeBytes = sizeof(xq_env_rec) + 4 * 4 + 5;                               // record, 4 int32, 5 bytes
 constexpr size_t kEdgeBytes = 4 + 4 + 4 + 4 + 2;                                              // P, N, W, child, action
-constexpr size_t kTreeBytes = sizeof(xq_env_rec) + 4 + 4 + 1;                                 // leaf record, node count, leaf, generic flag
-static_assert(kNodeBytes == 85 && kEdgeBytes == 18, "include/xq.h documents these sizes");
+constexpr size_t kSlotBytes = sizeof(xq_env_rec) + 4 + 1;                                     // per leaf slot: leaf record, leaf, generic flag
+constexpr size_t kTreeBytes = 4 + kSlotBytes;                                                  // node count and one slot
+static_assert(kNodeBytes == 85 && kEdgeBytes == 18 && kSlotBytes == 69, "include/xq.h documents these sizes");
 
 inline unsigned grid_of(int64_t n, int per_block) { return (unsigned)((n + per_block - 1) / per_block); }
 
@@ -586,23 +728,27 @@ int xq::search_roots(xq_search_t s, SearchRoots* out) {
 
 extern "C" {
 
-int xq_search_create(xq_env_t env, int max_simulations, xq_search_t* out) {
+int xq_search_create(xq_env_t env, int max_simulations, xq_search_t* out) { return xq_search_create_ex(env, max_simulations, 1, out); }
+
+int xq_search_create_ex(xq_env_t env, int max_simulations, int max_leaves, xq_search_t* out) {
     if (!out || !env) return fail(XQ_ERR_INVALID, "xq_search_create: null env or out");
     if (max_simulations < 1 || max_simulations > (1 << 24)) return fail(XQ_ERR_INVALID, "xq_search_create: max_simulations %d (1 .. 2^24)", max_simulations);
+    if (max_leaves < 1 || max_leaves > XQ_SEARCH_MAX_LEAVES)
+        return fail(XQ_ERR_INVALID, "xq_search_create_ex: max_leaves %d (1 .. %d)", max_leaves, XQ_SEARCH_MAX_LEAVES);
     EnvInfo E;
     if (int rc = env_info(env, &E)) return rc;
     XQ_CUDA(cudaSetDevice(E.device));
     xq_search_s* s = new (std::nothrow) xq_search_s();
     if (!s) return fail(XQ_ERR_NOMEM, "xq_search_create: out of host memory");
-    s->env = env; s->device = E.device; s->max_sims = max_simulations;
-    const int64_t n = E.n, cap = (int64_t)max_simulations + 1, nodes = n * cap, edges = nodes * kSearchEdges;
+    s->env = env; s->device = E.device; s->max_sims = max_simulations; s->max_leaves = max_leaves;
+    const int64_t n = E.n, cap = (int64_t)max_simulations + 1, nodes = n * cap, edges = nodes * kSearchEdges, slots = n * max_leaves;
     // one slab, every array 16-byte aligned
     size_t off = 0;
     auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
     const size_t o_rec = take(sizeof(xq_env_rec) * nodes), o_parent = take(4 * nodes), o_visits = take(4 * nodes), o_reward = take(4 * nodes),
                  o_depth = take(4 * nodes), o_pedge = take(nodes), o_nedges = take(nodes), o_exp = take(nodes), o_term = take(nodes),
                  o_win = take(nodes), o_P = take(4 * edges), o_N = take(4 * edges), o_W = take(4 * edges), o_child = take(4 * edges),
-                 o_act = take(2 * edges), o_count = take(4 * n), o_leaf = take(4 * n), o_leafrec = take(sizeof(xq_env_rec) * n), o_ns = take(n);
+                 o_act = take(2 * edges), o_count = take(4 * n), o_leaf = take(4 * slots), o_leafrec = take(sizeof(xq_env_rec) * slots), o_ns = take(slots);
     if (cudaMalloc(&s->slab, off) != cudaSuccess) {
         cudaGetLastError();
         delete s;
@@ -632,9 +778,13 @@ int xq_search_destroy(xq_search_t s) {
     return XQ_OK;
 }
 
-int xq_search_bytes_per_tree(int max_simulations, int64_t* bytes) {
-    if (!bytes || max_simulations < 1) return fail(XQ_ERR_INVALID, "xq_search_bytes_per_tree: bad arguments");
-    *bytes = (int64_t)(max_simulations + 1) * (int64_t)(kNodeBytes + kSearchEdges * kEdgeBytes) + (int64_t)kTreeBytes;
+int xq_search_bytes_per_tree(int max_simulations, int64_t* bytes) { return xq_search_bytes_per_tree_ex(max_simulations, 1, bytes); }
+
+int xq_search_bytes_per_tree_ex(int max_simulations, int max_leaves, int64_t* bytes) {
+    if (!bytes || max_simulations < 1 || max_leaves < 1 || max_leaves > XQ_SEARCH_MAX_LEAVES)
+        return fail(XQ_ERR_INVALID, "xq_search_bytes_per_tree: bad arguments");
+    *bytes = (int64_t)(max_simulations + 1) * (int64_t)(kNodeBytes + kSearchEdges * kEdgeBytes) + (int64_t)kTreeBytes +
+             (int64_t)(max_leaves - 1) * (int64_t)kSlotBytes;
     return XQ_OK;
 }
 
@@ -673,16 +823,30 @@ int xq_search_advance(xq_search_t s, int min_free, const float* root_noise_dev, 
 
 int xq_search_select_device(xq_search_t s, float c_puct, float fpu, uint8_t* status_dev, uint8_t* winner_dev, int32_t* reward_dev,
                             int32_t* depth_dev) {
+    return xq_search_select_leaves_device(s, 1, c_puct, fpu, 0.f, status_dev, winner_dev, reward_dev, depth_dev);
+}
+
+int xq_search_select_leaves_device(xq_search_t s, int leaves, float c_puct, float fpu, float virtual_loss, uint8_t* status_dev,
+                                   uint8_t* winner_dev, int32_t* reward_dev, int32_t* depth_dev) {
     EnvInfo E;
     if (int rc = enter(s, &E, "xq_search_select_device")) return rc;
+    if (leaves < 1 || leaves > s->max_leaves) return fail(XQ_ERR_INVALID, "xq_search_select_leaves_device: leaves %d (1 .. %d)", leaves, s->max_leaves);
     if (!(c_puct >= 0.f && c_puct <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_search_select_device: c_puct must be finite and >= 0");
     if (!(fpu >= -FLT_MAX && fpu <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_search_select_device: fpu must be finite");
+    if (!(virtual_loss >= 0.f && virtual_loss <= FLT_MAX))
+        return fail(XQ_ERR_INVALID, "xq_search_select_leaves_device: virtual_loss must be finite and >= 0");
     if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_select_device: the search was never reset (xq_search_reset)");
     if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_search_select_device: the last selection was not expanded and backed up");
-    if (s->sims >= s->max_sims) return fail(XQ_ERR_STATE, "xq_search_select_device: %d simulations since the reset, the capacity", s->sims);
-    search_select_kernel<<<grid_of(s->d.n, kSelWarps), 32 * kSelWarps, 0, E.stream>>>(s->d, c_puct, fpu, status_dev, winner_dev, reward_dev, depth_dev);
+    if (s->sims + leaves > s->max_sims)
+        return fail(XQ_ERR_STATE, "xq_search_select_device: %d simulations since the reset, %d more pass the capacity %d", s->sims, leaves, s->max_sims);
+    if (leaves == 1)
+        search_select_kernel<<<grid_of(s->d.n, kSelWarps), 32 * kSelWarps, 0, E.stream>>>(s->d, c_puct, fpu, status_dev, winner_dev, reward_dev, depth_dev);
+    else
+        search_select_leaves_kernel<<<grid_of(s->d.n, kSelLeavesWarps), 32 * kSelLeavesWarps, 0, E.stream>>>(s->d, leaves, c_puct, fpu, virtual_loss,
+                                                                                                            status_dev, winner_dev, reward_dev, depth_dev);
     XQ_LAUNCH_CHECK();
-    s->sims++;
+    s->sims += leaves;
+    s->leaves = leaves;
     s->phase = 2;
     return XQ_OK;
 }
@@ -702,7 +866,7 @@ int xq_search_observe_leaves_device(xq_search_t s, void* planes_dev, int dtype, 
     if ((reinterpret_cast<uintptr_t>(planes_dev) & 15u) || (reinterpret_cast<uintptr_t>(aux_dev) & 15u))
         return fail(XQ_ERR_INVALID, "xq_search_observe_leaves_device: planes and aux must be 16-byte aligned");
     if (s->phase != 2) return fail(XQ_ERR_STATE, "xq_search_observe_leaves_device: no selection since the last expand_backup / reset");
-    XQ_CUDA(launch_observe(s->d.leaf_rec, s->d.n, planes_dev, dtype, view, aux_dev, E.stream));
+    XQ_CUDA(launch_observe(s->d.leaf_rec, s->d.n * s->leaves, planes_dev, dtype, view, aux_dev, E.stream));
     return XQ_OK;
 }
 
@@ -719,6 +883,20 @@ int xq_search_expand_backup_device(xq_search_t s, const void* scores_dev, int sc
     if (s->phase != 2) return fail(XQ_ERR_STATE, "xq_search_expand_backup_device: no selection since the last expand_backup / reset");
     const ExpandArgs a{scores_dev, temperature, view, values_dev, root_noise_dev, noise_eps};
     const bool bf16 = scores_dtype == XQ_DTYPE_BF16;
+    const int L = s->leaves;
+    if (L > 1) {
+        const int64_t slots = s->d.n * L;
+        if (bf16) search_expand_slots_kernel<XQ_DTYPE_BF16><<<grid_of(slots, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a, L);
+        else search_expand_slots_kernel<XQ_DTYPE_F32><<<grid_of(slots, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a, L);
+        XQ_LAUNCH_CHECK();
+        if (s->maybe_nonstd) {
+            if (bf16) search_expand_generic_slots_kernel<XQ_DTYPE_BF16><<<grid_of(slots, kThreads), kThreads, 0, E.stream>>>(s->d, a, L);
+            else search_expand_generic_slots_kernel<XQ_DTYPE_F32><<<grid_of(slots, kThreads), kThreads, 0, E.stream>>>(s->d, a, L);
+            XQ_LAUNCH_CHECK();
+        }
+        s->phase = 1;
+        return XQ_OK;
+    }
     if (bf16) search_expand_lane_kernel<XQ_DTYPE_BF16><<<grid_of(s->d.n, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a);
     else search_expand_lane_kernel<XQ_DTYPE_F32><<<grid_of(s->d.n, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a);
     XQ_LAUNCH_CHECK();

@@ -1,7 +1,8 @@
 // xq_search.cuh -- host-compilable helpers of the batched tree search (xq_search.cu; include/xq.h: xq_search_*): the PUCT score of an
-// edge and its arg-max order, the priors of a freshly expanded node, the root-noise mix, the value cleaning, the backup along a path, and
-// the membership and renumbering of a tree re-rooted after a move (xq_search_advance), the visit-count choice of the move to play
-// (xq_search_play_device) and the Dirichlet draw of the root noise (xq_search_root_noise_device).
+// edge (with virtual loss: search_puct_vl) and its arg-max order, the in-flight counting of a multi-leaf selection, the priors of a
+// freshly expanded node, the root-noise mix, the value cleaning, the backup along a path, and the membership and renumbering of a tree
+// re-rooted after a move (xq_search_advance), the visit-count choice of the move to play (xq_search_play_device) and the Dirichlet draw
+// of the root noise (xq_search_root_noise_device).
 //
 // The arithmetic is spelled with explicitly rounded operations (__fmul_rn and friends on the device; plain operators on the host, where
 // tests/hostsim/search_shim.cpp is compiled with -ffp-contract=off) so that no multiply-add is contracted and numpy can restate every
@@ -54,6 +55,16 @@ XQ_HD float search_puct(float p, int n, float w, float c_puct, float fpu, float 
     return s_add(q, u);
 }
 XQ_HD float search_sqrt_visits(int n_node) { return s_sqrt((float)n_node); }
+// Q + U with virtual loss (xq_search_select_leaves_device): c = the earlier descents of this selection through the edge, vl the virtual
+// loss; N' = N + c, W' = c > 0 ? W - vl * c : W, Q = N' > 0 ? W' / N' : fpu, U = ((c_puct * P) * sqrt_n) / (1 + N'), sqrt_n =
+// sqrt(N_node + c_node) of the parent.  At c = 0 this is search_puct bit for bit.
+XQ_HD float search_puct_vl(float p, int n, float w, int c, float vl, float c_puct, float fpu, float sqrt_n) {
+    const int nv = n + c;
+    const float wv = c > 0 ? s_add(w, -s_mul(vl, (float)c)) : w;
+    const float q = nv > 0 ? s_div(wv, (float)nv) : fpu;
+    const float u = s_div(s_mul(s_mul(c_puct, p), sqrt_n), (float)(1 + nv));
+    return s_add(q, u);
+}
 // the arg-max order of selection: a larger score, or an equal one at a smaller list index (strict >, DQN::selectAction)
 XQ_HD bool search_better(float a, int ia, float b, int ib) { return ib < 0 || a > b || (a == b && ia < ib); }
 
@@ -93,6 +104,24 @@ XQ_HD void search_backup(int leaf, float value, const int32_t* parent, const uin
         node_visits[p] += 1;
         j = p;
     }
+}
+
+// ---- multi-leaf selection: the in-flight counts of descent k (xq_search_select_leaves_device) ----
+// The earlier descents k' < k of the selection are lanes of the select-leaves warp.  Each keeps the list index of the edge it took at every
+// depth (path[d][k'], d = plies below the root) and an "alive" bit: its path has taken the same edges as descent k so far, i.e. it went
+// through descent k's current node (a tree: a node is its edge sequence from the root).  At an expanded, non-terminal node at depth d,
+// c_e = the alive lanes whose edge at d is e, and c_node = the alive lanes; an alive lane stays alive if its edge at d is the one descent
+// k takes.  Host restatement of the lanes: alive and counts for one node; returns the new alive mask after descent k took edge `taken`.
+XQ_HD uint32_t search_inflight_node(uint32_t alive, const uint8_t* path_d, int taken, int32_t* counts, int* c_node) {
+    uint32_t next = 0;
+    *c_node = 0;
+    for (int l = 0; l < 32; ++l) {
+        if (!(alive >> l & 1u)) continue;
+        counts[path_d[l]] += 1;
+        *c_node += 1;
+        if (path_d[l] == taken) next |= 1u << l;
+    }
+    return next;
 }
 
 // ---- advance: re-rooting a tree at node m (0, or a child of the root) in place ----

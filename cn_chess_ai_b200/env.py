@@ -153,24 +153,25 @@ class BatchedEnv:
         return out
 
 
-def search_bytes_per_tree(max_simulations):
-    """device memory one tree of a BatchedSearch with this capacity takes"""
+def search_bytes_per_tree(max_simulations, max_leaves=1):
+    """device memory one tree of a BatchedSearch with this capacity (and up to max_leaves leaves per selection) takes"""
     b = C.c_int64()
-    check(lib().xq_search_bytes_per_tree(max_simulations, C.byref(b)))
+    check(lib().xq_search_bytes_per_tree_ex(max_simulations, max_leaves, C.byref(b)))
     return b.value
 
 
 class BatchedSearch:
-    """xq_search_*: one PUCT tree per env of `env` (a BatchedEnv), capacity max_simulations simulations per reset.  Raw device pointers
-    (ints), asynchronous on the env's stream; close() before the env is closed."""
+    """xq_search_*: one PUCT tree per env of `env` (a BatchedEnv), capacity max_simulations simulations per reset, up to max_leaves
+    leaves per tree in one selection.  Raw device pointers (ints), asynchronous on the env's stream; close() before the env is closed."""
 
-    def __init__(self, env, max_simulations):
+    def __init__(self, env, max_simulations, max_leaves=1):
         self._L = lib()
         self._h = C.c_void_p()
-        check(self._L.xq_search_create(env.handle, max_simulations, C.byref(self._h)))
+        check(self._L.xq_search_create_ex(env.handle, max_simulations, max_leaves, C.byref(self._h)))
         self.env = env
         self.n = env.n
         self.max_simulations = int(max_simulations)
+        self.max_leaves = int(max_leaves)
 
     def close(self):
         if self._h:
@@ -194,8 +195,13 @@ class BatchedSearch:
     def select_device(self, c_puct, fpu, status_ptr=None, winner_ptr=None, reward_ptr=None, depth_ptr=None):
         check(self._L.xq_search_select_device(self._h, float(c_puct), float(fpu), status_ptr, winner_ptr, reward_ptr, depth_ptr))
 
+    def select_leaves_device(self, leaves, c_puct, fpu, virtual_loss, status_ptr=None, winner_ptr=None, reward_ptr=None, depth_ptr=None):
+        """xq_search_select_leaves_device: `leaves` leaves per tree with virtual loss; outputs [n][leaves]"""
+        check(self._L.xq_search_select_leaves_device(self._h, int(leaves), float(c_puct), float(fpu), float(virtual_loss), status_ptr,
+                                                     winner_ptr, reward_ptr, depth_ptr))
+
     def leaves_device(self):
-        """device address of the [n] leaf records of the last selection"""
+        """device address of the [n * L] leaf records of the last selection of L leaves"""
         p = C.c_void_p()
         check(self._L.xq_search_leaves_device(self._h, C.byref(p)))
         return p.value

@@ -1,8 +1,9 @@
 """TorchSearch: batched PUCT tree search (one tree per env) for a policy/value network written in PyTorch, on the device
 (include/xq.h: xq_search_*).
 
-Each simulation selects one leaf per tree, observes all leaves at once, calls the network once on them and hands its scores and values
-back; selection, child creation, expansion and backup run in the library's kernels on torch's current stream.  Actions and visit counts
+Each simulation selects one leaf per tree (or, with select_leaves, several per tree with virtual loss), observes all leaves at once, calls
+the network once on them and hands its scores and values back; selection, child creation, expansion and backup run in the library's
+kernels on torch's current stream.  Actions and visit counts
 use the policy indices from * 90 + to of TorchEnv, in the frame of `view`.
 """
 from collections import namedtuple
@@ -16,19 +17,22 @@ from .torch_env import _OBS_DTYPES, _SCORE_DTYPES, StepResult, _view
 SelectResult = namedtuple("SelectResult", "status winner reward depth")
 RootResult = namedtuple("RootResult", "visits q best")
 
-# leaf status (xq_search_select_device)
-NEEDS_EVALUATION, GENERAL_CAPTURED, MOVE_CAP, NO_LEGAL_ACTION = 0, 1, 2, 3
+# leaf status (xq_search_select_device; DUPLICATE only from xq_search_select_leaves_device)
+NEEDS_EVALUATION, GENERAL_CAPTURED, MOVE_CAP, NO_LEGAL_ACTION, DUPLICATE = 0, 1, 2, 3, 4
 
 
 class TorchSearch:
-    """max_simulations simulations per reset on the envs of `tenv` (a TorchEnv); the roots are the envs' boards at reset()"""
+    """max_simulations simulations per reset on the envs of `tenv` (a TorchEnv); the roots are the envs' boards at reset().  max_leaves:
+    the most leaves per tree one select_leaves() call may take (1 .. 32)"""
 
-    def __init__(self, tenv, max_simulations):
+    def __init__(self, tenv, max_simulations, max_leaves=1):
         self.tenv = tenv
         self.n = tenv.n
         self.device = tenv.device
-        self.search = BatchedSearch(tenv.env, max_simulations)
+        self.search = BatchedSearch(tenv.env, max_simulations, max_leaves)
         self.max_simulations = self.search.max_simulations
+        self.max_leaves = self.search.max_leaves
+        self._rows = self.n        # leaf rows of the last selection: n * leaves
         self._kept = None          # kept int32 [n] of the last advance(); None after reset(): every root was rebuilt
 
     def close(self):
@@ -60,13 +64,27 @@ class TorchSearch:
         status, winner = (torch.empty(self.n, dtype=torch.uint8, device=self.device) for _ in range(2))
         reward, depth = (torch.empty(self.n, dtype=torch.int32, device=self.device) for _ in range(2))
         self.search.select_device(c_puct, fpu, status.data_ptr(), winner.data_ptr(), reward.data_ptr(), depth.data_ptr())
+        self._rows = self.n
+        return SelectResult(status, winner, reward, depth)
+
+    def select_leaves(self, leaves, c_puct=1.5, fpu=0.0, virtual_loss=1.0):
+        """`leaves` leaves per tree in one call, descents in order with virtual loss (include/xq.h): SelectResult of tensors [n, leaves];
+        status DUPLICATE (4) marks a slot that ended at the open leaf of an earlier slot.  leaves(), observe() and expand_backup() then
+        take or return n * leaves rows, slot k of tree t at row t * leaves + k.  Spends `leaves` of the search's simulations."""
+        self.tenv._enter()
+        shape = (self.n, int(leaves))
+        status, winner = (torch.empty(shape, dtype=torch.uint8, device=self.device) for _ in range(2))
+        reward, depth = (torch.empty(shape, dtype=torch.int32, device=self.device) for _ in range(2))
+        self.search.select_leaves_device(leaves, c_puct, fpu, virtual_loss, status.data_ptr(), winner.data_ptr(), reward.data_ptr(),
+                                         depth.data_ptr())
+        self._rows = self.n * int(leaves)
         return SelectResult(status, winner, reward, depth)
 
     def leaves(self):
-        """the leaf records of the last selection as a uint8 [n, 64] tensor aliasing the library's buffer (xq_env_rec each; valid until
-        the next select: clone() to keep them)"""
+        """the leaf records of the last selection as a uint8 [rows, 64] tensor aliasing the library's buffer (xq_env_rec each, rows = n
+        after select(), n * leaves after select_leaves(); valid until the next select: clone() to keep them)"""
         ptr = self.search.leaves_device()
-        n = self.n
+        n = self._rows
 
         class _Leaves:
             __cuda_array_interface__ = {"shape": (n, 64), "typestr": "|u1", "data": (ptr, False), "version": 3, "strides": None}
@@ -74,22 +92,23 @@ class TorchSearch:
         return torch.as_tensor(_Leaves(), device=self.device)
 
     def observe(self, dtype=torch.bfloat16, view="side"):
-        """the leaves as TorchEnv.observe shows envs: (planes [n, 14, 10, 9], aux int32 [n, 4])"""
+        """the leaves as TorchEnv.observe shows envs: (planes [rows, 14, 10, 9], aux int32 [rows, 4]), rows as in leaves()"""
         if dtype not in _OBS_DTYPES:
             raise ValueError(f"dtype must be one of {list(_OBS_DTYPES)}")
         v = _view(view)
         self.tenv._enter()
-        planes = torch.empty((self.n, 14, 10, 9), dtype=dtype, device=self.device)
-        aux = torch.empty((self.n, 4), dtype=torch.int32, device=self.device)
+        planes = torch.empty((self._rows, 14, 10, 9), dtype=dtype, device=self.device)
+        aux = torch.empty((self._rows, 4), dtype=torch.int32, device=self.device)
         self.search.observe_leaves_device(planes.data_ptr(), _OBS_DTYPES[dtype], v, aux.data_ptr())
         return planes, aux
 
     def expand_backup(self, scores, values, temperature=1.0, root_noise=None, noise_eps=0.25, view="side"):
-        """scores [n, 8100] (f32 / bf16, frame of `view`) expand the leaves that need evaluation; values f32 [n] (from each leaf's side
-        to move) are backed up for every leaf.  root_noise f32 [n, 8100]: mixed into the root's priors when the root is expanded."""
+        """scores [rows, 8100] (f32 / bf16, frame of `view`) expand the leaves that need evaluation; values f32 [rows] (from each leaf's
+        side to move) are backed up for every leaf but duplicates (rows as in leaves()).  root_noise f32 [n, 8100]: mixed into the
+        root's priors when the root is expanded."""
         v = _view(view)
-        self.tenv._check(scores, "scores", list(_SCORE_DTYPES), (self.n, POLICY_ACTIONS))
-        self.tenv._check(values, "values", [torch.float32], (self.n,))
+        self.tenv._check(scores, "scores", list(_SCORE_DTYPES), (self._rows, POLICY_ACTIONS))
+        self.tenv._check(values, "values", [torch.float32], (self._rows,))
         if root_noise is not None:
             self.tenv._check(root_noise, "root_noise", [torch.float32], (self.n, POLICY_ACTIONS))
         self.tenv._enter()
@@ -139,7 +158,8 @@ class TorchSearch:
     @staticmethod
     def outcome_values(status, winner, aux, cap_value=0.0):
         """a default value of terminal leaves, from the leaf's side to move (aux[:, 0], absolute colour): +1 / -1 when a General was
-        captured and the side to move is / is not the winner, cap_value at the move cap, -1 without a legal action, 0 elsewhere"""
+        captured and the side to move is / is not the winner, cap_value at the move cap, -1 without a legal action, 0 elsewhere
+        (duplicates included)"""
         player = aux[:, 0].to(torch.int32)
         won = torch.where(winner.to(torch.int32) == player, 1.0, -1.0)
         v = torch.zeros(status.shape, dtype=torch.float32, device=status.device)
@@ -148,24 +168,31 @@ class TorchSearch:
         return torch.where(status == NO_LEGAL_ACTION, torch.full_like(v, -1.0), v)
 
     def run(self, evaluate, n_simulations, c_puct=1.5, fpu=0.0, temperature=1.0, root_noise=None, noise_eps=0.25, view="side",
-            obs_dtype=torch.bfloat16, cap_value=0.0, reset=True, dirichlet_alpha=None, dirichlet_eps=0.25, noise_seed=0):
-        """reset + n_simulations simulations: evaluate(planes) -> (scores [n, 8100], values [n]) is called once per simulation on the
-        leaves; at terminal leaves outcome_values replaces the network's value.  reset=False continues from the current trees (after
+            obs_dtype=torch.bfloat16, cap_value=0.0, reset=True, dirichlet_alpha=None, dirichlet_eps=0.25, noise_seed=0, leaves=1,
+            virtual_loss=1.0):
+        """reset + n_simulations simulations: evaluate(planes) -> (scores [rows, 8100], values [rows]) is called once per selection on
+        its leaves; at terminal leaves outcome_values replaces the network's value.  reset=False continues from the current trees (after
         advance(), or to add simulations to this move's search).  dirichlet_alpha: root_noise(dirichlet_alpha, dirichlet_eps, noise_seed)
         once per root and move -- before the first simulation on the roots the last advance() kept, after it on the roots reset() or
-        advance() rebuilt (expanded by the first simulation).  Returns root(view)."""
+        advance() rebuilt (expanded by the first simulation).  leaves > 1: after the first simulation (one leaf per tree, which expands
+        rebuilt roots) the rest go in select_leaves(leaves, virtual_loss=virtual_loss) calls, the last one smaller, so evaluate sees
+        n * leaves planes; n_simulations counts the selected slots.  Returns root(view)."""
         if reset:
             self.reset()
         kept = None if self._kept is None else self._kept > 0
         if dirichlet_alpha is not None and kept is not None:
             self.root_noise(dirichlet_alpha, dirichlet_eps, noise_seed, mask=kept)
-        for i in range(n_simulations):
+        i = 0
+        while i < n_simulations:
             if i == 1 and dirichlet_alpha is not None:
                 self.root_noise(dirichlet_alpha, dirichlet_eps, noise_seed, mask=None if kept is None else ~kept)
-            sel = self.select(c_puct, fpu)
+            k = 1 if i == 0 else min(leaves, n_simulations - i)
+            sel = self.select(c_puct, fpu) if k == 1 else self.select_leaves(k, c_puct, fpu, virtual_loss)
+            status, winner = sel.status.reshape(-1), sel.winner.reshape(-1)
             planes, aux = self.observe(obs_dtype, view)
             scores, values = evaluate(planes)
-            values = values.reshape(self.n).to(torch.float32).contiguous()
-            values = torch.where(sel.status != NEEDS_EVALUATION, self.outcome_values(sel.status, sel.winner, aux, cap_value), values)
+            values = values.reshape(self._rows).to(torch.float32).contiguous()
+            values = torch.where(status != NEEDS_EVALUATION, self.outcome_values(status, winner, aux, cap_value), values)
             self.expand_backup(scores.contiguous(), values, temperature, root_noise, noise_eps, view)
+            i += k
         return self.root(view)

@@ -215,7 +215,7 @@ int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dty
  * what xq_env_step_device (auto_reset = 0) makes of the parent's record and the edge's action (move_count, player, scores, ctr included).
  * Edges are a node's legal actions in reference list order (xq_env_legal_moves; the first 128), each with the prior P, the visit count N,
  * the value sum W (from the side to move at the parent) and the child.  N_node = simulations whose path contained the node, leaf included.
- * Selection (one leaf per tree per simulation, no virtual loss), from the root: a node not yet expanded, or terminal, is the leaf;
+ * Selection (one leaf per tree per simulation; xq_search_select_leaves_device below selects several with virtual loss), from the root: a node not yet expanded, or terminal, is the leaf;
  * otherwise the edge with the largest Q + U, ties to the smaller list index, in f32 with no contraction, in this order:
  *   Q = N > 0 ? W / N : fpu,   U = ((c_puct * P) * sqrt(N_node)) / (1 + N).
  * If that edge has no child yet, the child is made and is the leaf: a simulation adds at most one node per tree.
@@ -234,7 +234,31 @@ int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dty
  * else is XQ_ERR_STATE, as is a select past max_simulations since the reset (past min_free since an xq_search_advance, which may
  * take the place of the reset).  root_device and get_tree work at any time after a reset.
  * Memory: (max_simulations + 1) x 2,389 + 73 bytes per tree (xq_search_bytes_per_tree): per node a record, 21 bytes of node state and
- * 128 edge slots of 18 bytes (P, N, W, child, action); per tree the leaf record and 9 bytes. */
+ * 128 edge slots of 18 bytes (P, N, W, child, action); per tree the leaf record and 9 bytes.  A search made with max_leaves
+ * (xq_search_create_ex) keeps max_leaves leaf slots of 69 bytes (leaf record, leaf index, generic flag) per tree:
+ * (max_simulations + 1) x 2,389 + 4 + 69 x max_leaves bytes (xq_search_bytes_per_tree_ex).
+ *
+ * Multi-leaf selection (xq_search_select_leaves_device) of L leaves, 1 <= L <= max_leaves <= XQ_SEARCH_MAX_LEAVES: L descents per
+ * tree, k = 0 .. L - 1, in order, each from the root by the rules above, with two changes.
+ *  Score with virtual loss vl (finite, >= 0).  During descent k, at an expanded, non-terminal node j, c_e = the earlier descents k' < k of
+ *  this call whose path went through edge e of j, c_j = sum of c_e; N' = N + c_e, W' = c_e > 0 ? W - vl * c_e : W,
+ *    Q = N' > 0 ? W' / N' : fpu,   U = ((c_puct * P) * sqrt(N_node + c_j)) / (1 + N'),
+ *  Q + U, ties to the smaller list index, f32 with no contraction (at c_e = c_j = 0 exactly the score above).  Virtual loss does not
+ *  change the tree: N, W and N_node change only in the backup; the in-flight counts live inside the call.  A descent makes at most one
+ *  node, as before.
+ *  Duplicates.  A descent that ends at a node that is unexpanded and not terminal, where an earlier descent of the call also ended (always
+ *  the case for descents 1 .. L - 1 on the first call after a reset: every descent stops at the unexpanded root), is a duplicate slot:
+ *  leaf status 4, with the winner, reward and depth of its leaf.  Terminal leaves (status 1 / 2 / 3) reached again are ordinary slots.
+ *  Outputs status / winner / reward / depth are [n][L], row-major by tree; the leaf records of xq_search_leaves_device and the planes of
+ *  xq_search_observe_leaves_device are the n * L slots, slot k of tree t at row t * L + k.
+ *  Expand + backup after it reads scores [n * L][8100] and values [n * L]: for k = 0 .. L - 1 of each tree, in order, a status-0 slot
+ *  expands its leaf from row t * L + k (the root noise row t applies when that leaf is the root), and every slot except a duplicate backs
+ *  up its value.  Duplicate slots read neither scores nor values.  Expansions write only edges of unexpanded leaves and backups only edges
+ *  of expanded ancestors, so the result is bit for bit "expand every status-0 slot, then back up in slot order", whatever the thread
+ *  schedule.
+ *  Budget: a selection spends L of the allowed selects (max_simulations since a reset, min_free since an xq_search_advance), duplicates
+ *  included; one that would pass the budget is XQ_ERR_STATE.  Every slot makes at most one node, so xq_search_advance's guarantee holds.
+ *  L = 1 is xq_search_select_device bit for bit (the same kernels). */
 typedef struct xq_search_s* xq_search_t;
 #define XQ_SEARCH_MAX_EDGES 128
 typedef struct {
@@ -258,10 +282,14 @@ typedef struct {
     int32_t child;        /* node index, -1 none */
 } xq_search_edge;         /* 20 B */
 
-/* capacity max_simulations + 1 nodes per tree; XQ_ERR_NOMEM when the device memory cannot be had.  The trees are empty until a reset. */
+/* capacity max_simulations + 1 nodes per tree; XQ_ERR_NOMEM when the device memory cannot be had.  The trees are empty until a reset.
+ * xq_search_create is xq_search_create_ex with max_leaves 1; max_leaves (1 .. XQ_SEARCH_MAX_LEAVES) bounds the leaves of one selection. */
+#define XQ_SEARCH_MAX_LEAVES 32
 int xq_search_create(xq_env_t env, int max_simulations, xq_search_t* out);
+int xq_search_create_ex(xq_env_t env, int max_simulations, int max_leaves, xq_search_t* out);
 int xq_search_destroy(xq_search_t s);
 int xq_search_bytes_per_tree(int max_simulations, int64_t* bytes);
+int xq_search_bytes_per_tree_ex(int max_simulations, int max_leaves, int64_t* bytes);
 /* roots = the env's current records (read in stream order), every tree empty, simulation count 0 */
 int xq_search_reset(xq_search_t s);
 /* Subtree reuse between moves.  Re-root every tree at the node whose record equals its env's current record (read in stream order): the
@@ -284,12 +312,18 @@ int xq_search_advance(xq_search_t s, int min_free, const float* root_noise_dev, 
 /* one leaf per tree; c_puct finite and >= 0, fpu finite.  Outputs [n] (any may be NULL): status u8, winner u8, reward i32, depth i32 */
 int xq_search_select_device(xq_search_t s, float c_puct, float fpu, uint8_t* status_dev, uint8_t* winner_dev, int32_t* reward_dev,
                             int32_t* depth_dev);
-/* device address of the [n] leaf records of the last selection (valid until the next select) */
+/* `leaves` leaves per tree with virtual loss (multi-leaf selection above): leaves in 1 .. max_leaves and virtual_loss finite and >= 0
+ * (XQ_ERR_INVALID otherwise), the other checks of xq_search_select_device.  Outputs [n][leaves] (any may be NULL): status u8 (4 for a
+ * duplicate slot), winner u8, reward i32, depth i32 */
+int xq_search_select_leaves_device(xq_search_t s, int leaves, float c_puct, float fpu, float virtual_loss, uint8_t* status_dev,
+                                   uint8_t* winner_dev, int32_t* reward_dev, int32_t* depth_dev);
+/* device address of the [n * L] leaf records of the last selection of L leaves (valid until the next select) */
 int xq_search_leaves_device(xq_search_t s, void** leaf_recs_dev);
 /* xq_env_observe_device on the leaf records: same planes / aux contract */
 int xq_search_observe_leaves_device(xq_search_t s, void* planes_dev, int dtype, int view, int32_t* aux_dev);
 /* expansion of the status-0 leaves and backup of every leaf: scores_dev [n][8100] (scores_dtype f32 / bf16), temperature finite > 0,
- * values_dev f32 [n] (required), root_noise_dev f32 [n][8100] or NULL, noise_eps in [0, 1] */
+ * values_dev f32 [n] (required), root_noise_dev f32 [n][8100] or NULL, noise_eps in [0, 1].  After a selection of L leaves: scores
+ * [n * L][8100] and values [n * L], duplicate slots neither expanded nor backed up */
 int xq_search_expand_backup_device(xq_search_t s, const void* scores_dev, int scores_dtype, float temperature, int view,
                                    const float* values_dev, const float* root_noise_dev, float noise_eps);
 /* per root (any output may be NULL): visits_dev int32 [n][8100] (16-byte aligned) = the root edges' N at their policy indices in the frame
