@@ -109,6 +109,15 @@ def lib():
     L.xq_search_play_device.argtypes = [_P, C.c_float, C.c_int, C.c_int, C.c_int] + [_P] * 6
     L.xq_search_root_noise_device.argtypes = [_P, C.c_float, C.c_float, C.c_uint64, _P, _P]
     L.xq_search_get_tree.argtypes = [_P, C.c_int64, _P, _P, C.POINTER(C.c_int32)]
+    L.xq_gumbel_create.argtypes = [_P, C.c_int, C.POINTER(_P)]
+    L.xq_gumbel_destroy.argtypes = [_P]
+    L.xq_gumbel_bytes.argtypes = [C.c_int64, C.c_int, C.POINTER(C.c_int64)]
+    L.xq_gumbel_begin_device.argtypes = [_P, _P, C.c_int, C.c_float, C.c_int, _P, C.c_int, C.c_uint64, C.c_float, C.c_float]
+    L.xq_gumbel_select_device.argtypes = [_P, C.c_int, C.c_float, C.c_float, C.c_float, _P, _P, _P, _P]
+    L.xq_gumbel_root_device.argtypes = [_P, C.c_int, _P, _P]
+    L.xq_gumbel_play_device.argtypes = [_P, C.c_int, C.c_int] + [_P] * 6
+    L.xq_gumbel_get.argtypes = [_P, C.c_int64, _P, _P, _P, _P, _P, _P]
+    L.xq_examples_record_gumbel_device.argtypes = [_P, _P, _P]
     L.xq_examples_create.argtypes = [_P, C.c_int64, C.c_int, C.POINTER(_P)]
     L.xq_examples_destroy.argtypes = [_P]
     L.xq_examples_bytes.argtypes = [C.c_int64, C.c_int64, C.c_int, C.POINTER(C.c_int64)]

@@ -47,6 +47,9 @@ struct SearchRoots {
     const xq_env_rec* rec; const uint8_t *nedges, *expanded; const int32_t* N; const float* W; const int16_t* act;
 };
 int search_roots(xq_search_t s, SearchRoots* out);
+// xq_examples_record_gumbel_device: the call checks of a begun Gumbel search on env `env`, its roots, and the improved-policy weights of
+// every root ([n][128], edge k at t * 128 + k) launched on the env's stream
+int gumbel_weights(xq_gumbel_t g, xq_env_t env, SearchRoots* roots, const uint32_t** w);
 
 // ---- device helpers ---------------------------------------------------------------------------
 #if defined(__CUDACC__)

@@ -49,8 +49,11 @@ struct ExDev {
     ExCounters* ctr;
 };
 
+// WEIGHTS: the visits field takes the Gumbel improved-policy weights wts[t * 128 + k] instead of N (xq_examples_record_gumbel_device)
+template <bool WEIGHTS>
 __global__ void __launch_bounds__(32 * kRecWarps) examples_record_kernel(ExDev b, SearchRoots r, const xq_env_rec* __restrict__ envs,
-                                                                        const uint8_t* __restrict__ mask, uint64_t env_id0) {
+                                                                        const uint8_t* __restrict__ mask, uint64_t env_id0,
+                                                                        const uint32_t* __restrict__ wts) {
     __shared__ __align__(16) xq_example s_ex[kRecWarps];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int64_t t = (int64_t)blockIdx.x * kRecWarps + warp;
@@ -76,18 +79,22 @@ __global__ void __launch_bounds__(32 * kRecWarps) examples_record_kernel(ExDev b
     // 2. the edges, coalesced; q summed in list order as search_root_kernel sums it
     const int ne = r.expanded[g] ? r.nedges[g] : 0;
     float w[kSearchEdges / 32];
-    uint32_t tot = 0;
+    uint32_t tot = 0, sn = 0;           // sum of visits[], and sum of N for q (the same sum unless WEIGHTS)
 #pragma unroll
     for (int i = 0; i < kSearchEdges / 32; ++i) {
         const int k = lane + 32 * i;
         const bool live = k < ne;
-        const uint32_t v = live ? (uint32_t)r.N[eb + k] : 0u;
+        const uint32_t nk = live ? (uint32_t)r.N[eb + k] : 0u;
+        const uint32_t v = WEIGHTS ? (live ? wts[t * kSearchEdges + k] : 0u) : nk;
         w[i] = live ? r.W[eb + k] : 0.f;
         x.action[k] = live ? r.act[eb + k] : (int16_t)-1;
         x.visits[k] = v;
         tot += v;
+        if (WEIGHTS) sn += nk;
     }
     tot = __reduce_add_sync(0xFFFFFFFFu, tot);
+    if (WEIGHTS) sn = __reduce_add_sync(0xFFFFFFFFu, sn);
+    const uint32_t qn = WEIGHTS ? sn : tot;
     float sw = 0.f;
 #pragma unroll
     for (int i = 0; i < kSearchEdges / 32; ++i) {
@@ -99,7 +106,7 @@ __global__ void __launch_bounds__(32 * kRecWarps) examples_record_kernel(ExDev b
     }
     if (lane == 0) {
         x.env = env_id0 + (uint64_t)t; x.game = 0; x.ply = (uint16_t)slot; x.n_edges = (uint8_t)ne; x.reserved0 = 0;
-        x.z = 0.f; x.q = tot > 0 ? s_div(sw, (float)(int)tot) : NAN; x.total_visits = tot; x.reserved1 = 0;
+        x.z = 0.f; x.q = qn > 0 ? s_div(sw, (float)(int)qn) : NAN; x.total_visits = tot; x.reserved1 = 0;
         b.staged[t] = slot + 1;
     }
     __syncwarp();
@@ -328,7 +335,19 @@ int xq_examples_record_device(xq_examples_t b, xq_search_t s, const uint8_t* mas
     if (r.env != b->env) return fail(XQ_ERR_INVALID, "xq_examples_record_device: the search is on another env handle");
     if (r.phase == 0) return fail(XQ_ERR_STATE, "xq_examples_record_device: the search was never reset (xq_search_reset)");
     if (r.phase == 2) return fail(XQ_ERR_STATE, "xq_examples_record_device: the last selection was not expanded and backed up");
-    examples_record_kernel<<<grid_of(b->d.n, kRecWarps), 32 * kRecWarps, 0, E.stream>>>(b->d, r, E.d_envs, mask_dev, E.env_id0);
+    examples_record_kernel<false><<<grid_of(b->d.n, kRecWarps), 32 * kRecWarps, 0, E.stream>>>(b->d, r, E.d_envs, mask_dev, E.env_id0, nullptr);
+    XQ_LAUNCH_CHECK();
+    return XQ_OK;
+}
+
+int xq_examples_record_gumbel_device(xq_examples_t b, xq_gumbel_t g, const uint8_t* mask_dev) {
+    EnvInfo E;
+    if (int rc = enter(b, &E, "xq_examples_record_gumbel_device")) return rc;
+    if (!g) return fail(XQ_ERR_INVALID, "xq_examples_record_gumbel_device: null Gumbel state");
+    SearchRoots r;
+    const uint32_t* w = nullptr;
+    if (int rc = gumbel_weights(g, b->env, &r, &w)) return rc;
+    examples_record_kernel<true><<<grid_of(b->d.n, kRecWarps), 32 * kRecWarps, 0, E.stream>>>(b->d, r, E.d_envs, mask_dev, E.env_id0, w);
     XQ_LAUNCH_CHECK();
     return XQ_OK;
 }

@@ -18,9 +18,12 @@
 // search_advance_kernel: one warp per tree, re-roots the tree at the played child in place (membership bitmap in shared memory).
 // search_play_kernel: one warp per tree, the move from the root's visit counts and the env's step with it.
 // search_noise_kernel: one warp per tree, Dirichlet noise drawn over the root's edges and mixed into its priors.
+// Gumbel root search (xq_gumbel_*): gumbel_expand_root_kernel / gumbel_init_kernel begin a move, search_select_leaves_kernel<GumbelDev>
+//   selects with the Gumbel root rule, gumbel_root_kernel / gumbel_play_kernel / gumbel_weights_kernel read the improved policy and action.
 #include <string.h>
 
 #include <new>
+#include <type_traits>
 #include <vector>
 
 #include "xq_common.cuh"
@@ -314,19 +317,181 @@ __global__ void __launch_bounds__(32 * kSelWarps) search_select_kernel(SearchDev
 // creation, as in search_select_kernel.  A descent that ends at an open leaf (unexpanded, not terminal) an earlier one ended at is a
 // duplicate: status 4, leaf index -1 for the expand kernel.
 constexpr int kSelLeavesWarps = 4;      // trees per CTA of the multi-leaf select kernel
+constexpr int kGumbelSlots = kSearchEdges / 32;      // root edges per lane: k = lane + 32 i
 
-__global__ void __launch_bounds__(32 * kSelLeavesWarps) search_select_leaves_kernel(SearchDev d, int L, float c_puct, float fpu, float vl,
+// The state of a Gumbel root search (xq_gumbel_*), per tree t: the Gumbel g and logit log P of root edge k at t * 128 + k, N0 (the edge's
+// N at begin) likewise, the considered bitmap as 4 words (bit l of word i: edge 32 i + l), the cleaned root value and m_t (0: the root
+// had no edge at begin); the integer weights of the improved policy (scratch of xq_examples_record_gumbel_device).  c_visit, c_scale, the
+// simulations of the move and the Gumbel selections since begin are the same for every tree.
+struct GumbelDev {
+    float *g, *logit; int32_t* n0; uint32_t* cons; float* vhat; int32_t* m; uint32_t* w;
+    float c_visit, c_scale; int sims, n_sims;
+};
+struct GumbelNone {};                 // the PUCT root of search_select_leaves_kernel
+
+// A root as the lanes of a warp see it (edges k = lane + 32 i): the improved-policy logits z = logit + sigma, the root-rule scores
+// (g + logit) + sigma, the visits this move n = N - N0 and the considered bits.  The arithmetic is gumbel_root_scores' (xq_search.cuh):
+// the list-order sums of v_mix are lane 0's walk over two 128-float shared scratch rows (sa, sb), the integer sums and the min / max are
+// warp reductions.
+struct GumbelRoot {
+    int ne, mt; uint32_t cons;
+    float z[kGumbelSlots], score[kGumbelSlots]; int n[kGumbelSlots];
+};
+
+__device__ __forceinline__ void gumbel_root_warp(const SearchDev& d, const GumbelDev& G, int64_t t, int lane, float* sa, float* sb,
+                                                 GumbelRoot& r) {
+    const int64_t eb0 = t * d.cap * kSearchEdges, gb = t * kSearchEdges;
+    r.mt = G.m[t];
+    const int ne = r.mt > 0 ? d.nedges[t * d.cap] : 0;
+    r.ne = ne;
+    int N[kGumbelSlots];
+    float q[kGumbelSlots], pp[kGumbelSlots], pq[kGumbelSlots];
+    int sn = 0, nmax = 0;
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) {
+        const int k = lane + 32 * i;
+        const bool live = k < ne;
+        N[i] = live ? d.N[eb0 + k] : 0;
+        q[i] = N[i] > 0 ? s_div(d.W[eb0 + k], (float)N[i]) : 0.f;
+        pp[i] = N[i] > 0 ? fmaxf(d.P[eb0 + k], FLT_MIN) : 0.f;
+        pq[i] = s_mul(pp[i], q[i]);
+        sn += N[i];
+        nmax = max(nmax, N[i]);
+    }
+    sn = __reduce_add_sync(0xFFFFFFFFu, sn);
+    nmax = __reduce_max_sync(0xFFFFFFFFu, nmax);
+    // the visited edges are those with P' > 0 (an unvisited edge's entries are 0)
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) { sa[lane + 32 * i] = pp[i]; sb[lane + 32 * i] = pq[i]; }
+    __syncwarp();
+    float sp = 0.f, sq = 0.f;
+    if (lane == 0)
+        for (int k = 0; k < ne; ++k)
+            if (sa[k] > 0.f) { sp = s_add(sp, sa[k]); sq = s_add(sq, sb[k]); }
+    sp = __shfl_sync(0xFFFFFFFFu, sp, 0);
+    sq = __shfl_sync(0xFFFFFFFFu, sq, 0);
+    const float vm = gumbel_vmix_of(sn, sp, sq, G.vhat[t]);
+    float mn = INFINITY, mx = -INFINITY;
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) {
+        if (lane + 32 * i >= ne) continue;
+        if (N[i] <= 0) q[i] = vm;
+        mn = fminf(mn, q[i]); mx = fmaxf(mx, q[i]);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        mn = fminf(mn, __shfl_xor_sync(0xFFFFFFFFu, mn, off));
+        mx = fmaxf(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, off));
+    }
+    r.cons = 0;
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) {
+        const int k = lane + 32 * i;
+        r.z[i] = -INFINITY; r.score[i] = -INFINITY; r.n[i] = 0;
+        if (k >= ne) continue;
+        const float sg = gumbel_sigma(q[i], mn, mx, nmax, G.c_visit, G.c_scale), lg = G.logit[gb + k];
+        r.z[i] = s_add(lg, sg);
+        r.score[i] = s_add(s_add(G.g[gb + k], lg), sg);
+        r.n[i] = N[i] - G.n0[gb + k];
+        r.cons |= (G.cons[t * 4 + i] >> lane & 1u) << i;
+    }
+}
+
+// the root rule of descent k (gumbel_pick) from the root's scores sc and visits this move nv (-1 for an edge not considered) in shared
+// memory: cnt = n + the in-flight count of the call's earlier descents (s_cnt); returns the edge
+__device__ __forceinline__ int gumbel_pick_warp(const float* sc, const int32_t* nv, const int32_t* s_cnt, int target, int lane) {
+    int cnt[kGumbelSlots];
+    bool hit = false;
+    int least = 0x7FFFFFFF;
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) {
+        const int e = lane + 32 * i;
+        cnt[i] = nv[e] >= 0 ? nv[e] + s_cnt[e] : -1;
+        if (cnt[i] >= 0) { hit = hit || cnt[i] == target; least = min(least, cnt[i]); }
+    }
+    const int want = __any_sync(0xFFFFFFFFu, hit) ? target : __reduce_min_sync(0xFFFFFFFFu, least);
+    float bs = 0.f;
+    int bk = -1;
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i)
+        if (cnt[i] == want && search_better(sc[lane + 32 * i], lane + 32 * i, bs, bk)) { bs = sc[lane + 32 * i]; bk = lane + 32 * i; }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        const float os = __shfl_xor_sync(0xFFFFFFFFu, bs, off);
+        const int ok = __shfl_xor_sync(0xFFFFFFFFu, bk, off);
+        if (ok >= 0 && search_better(os, ok, bs, bk)) { bs = os; bk = ok; }
+    }
+    return __shfl_sync(0xFFFFFFFFu, bk, 0);
+}
+
+// the action (gumbel_action): the considered edge with the most visits this move, then the larger score, then the smaller index; -1 none
+__device__ __forceinline__ int gumbel_action_warp(const GumbelRoot& r, int lane) {
+    int bk = -1, bn = 0;
+    float bs = 0.f;
+    auto better = [](int n1, float s1, int k1, int n2, float s2, int k2) {
+        return k1 >= 0 && (k2 < 0 || n1 > n2 || (n1 == n2 && search_better(s1, k1, s2, k2)));
+    };
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i)
+        if ((r.cons >> i & 1u) && r.n[i] > 0 && better(r.n[i], r.score[i], lane + 32 * i, bn, bs, bk)) { bk = lane + 32 * i; bn = r.n[i]; bs = r.score[i]; }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        const float os = __shfl_xor_sync(0xFFFFFFFFu, bs, off);
+        const int ok = __shfl_xor_sync(0xFFFFFFFFu, bk, off), on = __shfl_xor_sync(0xFFFFFFFFu, bn, off);
+        if (better(on, os, ok, bn, bs, bk)) { bs = os; bk = ok; bn = on; }
+    }
+    return __shfl_sync(0xFFFFFFFFu, bk, 0);
+}
+
+// the improved policy of the lanes' edges: p_i = exp(z_i - max z) / S, S summed in list order (gumbel_exp)
+__device__ __forceinline__ void gumbel_policy_warp(const GumbelRoot& r, int lane, float* sa, float (&p)[kGumbelSlots]) {
+    float zm = -INFINITY;
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) zm = fmaxf(zm, r.z[i]);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) zm = fmaxf(zm, __shfl_xor_sync(0xFFFFFFFFu, zm, off));
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) p[i] = lane + 32 * i < r.ne ? gumbel_exp(r.z[i], zm) : 0.f;
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) sa[lane + 32 * i] = p[i];
+    __syncwarp();
+    float s = 0.f;
+    if (lane == 0)
+        for (int k = 0; k < r.ne; ++k) s = s_add(s, sa[k]);
+    s = __shfl_sync(0xFFFFFFFFu, s, 0);
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) p[i] = s_div(p[i], s);
+}
+
+// GumbelDev as ROOT: the Gumbel root rule at depth 0 (xq_gumbel_select_device), below it PUCT with virtual loss as before
+template <class ROOT>
+__global__ void __launch_bounds__(32 * kSelLeavesWarps, std::is_same<ROOT, GumbelNone>::value ? 0 : 1) search_select_leaves_kernel(SearchDev d, int L, float c_puct, float fpu, float vl,
                                                                                     uint8_t* __restrict__ status, uint8_t* __restrict__ winner,
-                                                                                    int32_t* __restrict__ reward, int32_t* __restrict__ depth) {
+                                                                                    int32_t* __restrict__ reward, int32_t* __restrict__ depth,
+                                                                                    ROOT root) {
+    constexpr bool kGumbel = !std::is_same<ROOT, GumbelNone>::value;
     __shared__ uint32_t s_b[kSelLeavesWarps][12];
     __shared__ uint8_t s_path[kSelLeavesWarps][XQ_MAX_MOVES][32];
     __shared__ int32_t s_cnt[kSelLeavesWarps][kSearchEdges];
+    __shared__ float s_gsc[kGumbel ? kSelLeavesWarps : 1][kSearchEdges];      // Gumbel: the root's scores and visits this move
+    __shared__ int32_t s_gnv[kGumbel ? kSelLeavesWarps : 1][kSearchEdges];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int64_t t = (int64_t)blockIdx.x * kSelLeavesWarps + warp;
     if (t >= d.n) return;
     for (int e = lane; e < kSearchEdges; e += 32) s_cnt[warp][e] = 0;
-    __syncwarp();
     const int64_t g0 = t * d.cap;
+    int mt = 0;
+    if constexpr (kGumbel) {
+        GumbelRoot gr;
+        gumbel_root_warp(d, root, t, lane, s_gsc[warp], reinterpret_cast<float*>(s_gnv[warp]), gr);
+        mt = gr.mt;
+#pragma unroll
+        for (int i = 0; i < kGumbelSlots; ++i) {
+            s_gsc[warp][lane + 32 * i] = gr.score[i];
+            s_gnv[warp][lane + 32 * i] = gr.cons >> i & 1u ? gr.n[i] : -1;
+        }
+    }
+    __syncwarp();
     int mine = -1;                      // lane k: the leaf of descent k
     for (int k = 0; k < L; ++k) {
         bool alive = lane < k;
@@ -338,21 +503,26 @@ __global__ void __launch_bounds__(32 * kSelLeavesWarps) search_select_leaves_ker
             const int cj = popc32(__ballot_sync(0xFFFFFFFFu, alive));
             if (alive) atomicAdd(&s_cnt[warp][s_path[warp][dep][lane]], 1);
             __syncwarp();
-            const float sq = search_sqrt_visits(d.visits[g] + cj);
+            const bool groot = kGumbel && dep == 0;         // the Gumbel root rule instead of PUCT
+            const float sq = groot ? 0.f : search_sqrt_visits(d.visits[g] + cj);
             const int64_t eb = g * kSearchEdges;
             float bs = 0.f;
             int bk = -1;
-            for (int e = lane; e < ne; e += 32) {
-                const float v = search_puct_vl(d.P[eb + e], d.N[eb + e], d.W[eb + e], s_cnt[warp][e], vl, c_puct, fpu, sq);
-                if (search_better(v, e, bs, bk)) { bs = v; bk = e; }
-            }
+            if (groot) {
+                if constexpr (kGumbel) bk = gumbel_pick_warp(s_gsc[warp], s_gnv[warp], s_cnt[warp], gumbel_seq(mt, root.n_sims, root.sims + k), lane);
+            } else {
+                for (int e = lane; e < ne; e += 32) {
+                    const float v = search_puct_vl(d.P[eb + e], d.N[eb + e], d.W[eb + e], s_cnt[warp][e], vl, c_puct, fpu, sq);
+                    if (search_better(v, e, bs, bk)) { bs = v; bk = e; }
+                }
 #pragma unroll
-            for (int off = 16; off > 0; off >>= 1) {
-                const float os = __shfl_xor_sync(0xFFFFFFFFu, bs, off);
-                const int ok = __shfl_xor_sync(0xFFFFFFFFu, bk, off);
-                if (ok >= 0 && search_better(os, ok, bs, bk)) { bs = os; bk = ok; }
+                for (int off = 16; off > 0; off >>= 1) {
+                    const float os = __shfl_xor_sync(0xFFFFFFFFu, bs, off);
+                    const int ok = __shfl_xor_sync(0xFFFFFFFFu, bk, off);
+                    if (ok >= 0 && search_better(os, ok, bs, bk)) { bs = os; bk = ok; }
+                }
+                bk = __shfl_sync(0xFFFFFFFFu, bk, 0);
             }
-            bk = __shfl_sync(0xFFFFFFFFu, bk, 0);
             __syncwarp();
             if (alive) {
                 const int e = s_path[warp][dep][lane];
@@ -681,6 +851,149 @@ __global__ void __launch_bounds__(32 * kPlayWarps) search_noise_kernel(SearchDev
     }
 }
 
+
+// ---- Gumbel root search (xq_gumbel_*) ----
+// gumbel_expand_root_kernel: the unexpanded, non-terminal roots expanded and backed up as expand_backup does a root leaf after a select
+//   (the root record staged in the tree's leaf slot, search_expand_lane, search_backup; refused boards to search_expand_generic_kernel).
+// gumbel_init_kernel: one warp per tree: the Gumbel and logit of every root edge, the considered set (the key rows in shared memory, each
+//   lane ranks its edges: gumbel_considered), N0 and the root value.
+// gumbel_root_kernel: one CTA per tree, as search_root_kernel: warp 0 computes the improved policy and the action, the dense row is built
+//   in shared memory and written with 16-byte stores.  gumbel_play_kernel: search_play_kernel with the Gumbel action.
+// gumbel_weights_kernel: one warp per tree, the integer weights of xq_examples_record_gumbel_device.
+template <int SDT>
+__global__ void __launch_bounds__(kExpBoards) gumbel_expand_root_kernel(SearchDev d, ExpandArgs a) {
+    __shared__ uint8_t s_slot[32 * kExpBoards];
+    __shared__ uint32_t s_geo[kGeoWords];
+    __shared__ uint32_t s_view[kViewWords * kExpBoards];
+    __shared__ float s_row[XQ_MAX_ACTIONS * kExpBoards];
+    const int tid = threadIdx.x;
+    const int64_t t = (int64_t)blockIdx.x * kExpBoards + tid;
+    for (int i = tid; i < kGeoWords; i += kExpBoards) s_geo[i] = geo_word(i);
+    __syncthreads();
+    if (t >= d.n) return;
+    const int64_t g0 = t * d.cap;
+    uint8_t generic = 0;
+    if (!d.expanded[g0] && d.term[g0] == 0) {
+#pragma unroll
+        for (int i = 0; i < 4; ++i) reinterpret_cast<uint4*>(d.leaf_rec + t)[i] = reinterpret_cast<const uint4*>(d.rec + g0)[i];
+        d.leaf[t] = 0;
+        generic = search_expand_lane<SDT>(d, a, t, t, 0, tid, s_slot, s_geo, s_view, s_row);
+        search_backup(0, a.values[t], d.parent + g0, d.pedge + g0, d.visits + g0, d.N + g0 * kSearchEdges, d.W + g0 * kSearchEdges);
+    }
+    d.nonstd[t] = generic;
+}
+
+constexpr int kGumbelWarps = 4;       // trees per CTA of the Gumbel init, play and weights kernels
+
+__global__ void __launch_bounds__(32 * kGumbelWarps) gumbel_init_kernel(SearchDev d, GumbelDev G, int max_considered, uint64_t seed,
+                                                                       uint64_t env_id0, const float* __restrict__ values) {
+    __shared__ float s_key[kGumbelWarps][kSearchEdges];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t t = (int64_t)blockIdx.x * kGumbelWarps + warp;
+    if (t >= d.n) return;
+    const int64_t g0 = t * d.cap, eb0 = g0 * kSearchEdges, gb = t * kSearchEdges;
+    const int ne = d.expanded[g0] ? d.nedges[g0] : 0, mt = min(max_considered, ne);
+    const uint64_t base = rng(seed, env_id0 + (uint64_t)t, d.rec[g0].ctr);
+    float gv[kGumbelSlots], lg[kGumbelSlots];
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) {
+        const int k = lane + 32 * i;
+        gv[i] = k < ne ? gumbel_draw(base, k) : 0.f;
+        lg[i] = k < ne ? logf(d.P[eb0 + k]) : 0.f;
+        if (k < ne) s_key[warp][k] = s_add(gv[i], lg[i]);
+    }
+    __syncwarp();
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) {
+        const int k = lane + 32 * i;
+        const uint32_t word = __ballot_sync(0xFFFFFFFFu, k < ne && gumbel_considered(s_key[warp], ne, mt, k));
+        G.g[gb + k] = gv[i]; G.logit[gb + k] = lg[i];
+        G.n0[gb + k] = k < ne ? d.N[eb0 + k] : 0;
+        if (lane == 0) G.cons[t * 4 + i] = word;
+    }
+    if (lane == 0) { G.vhat[t] = search_clean_value(values[t]); G.m[t] = mt; }
+}
+
+__global__ void __launch_bounds__(kRootThreads) gumbel_root_kernel(SearchDev d, GumbelDev G, int view, float* __restrict__ policy,
+                                                                  int64_t* __restrict__ action) {
+    __shared__ __align__(16) float s_p[XQ_POLICY_ACTIONS];
+    __shared__ float s_scr[2][kSearchEdges];
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int64_t t = blockIdx.x, g = t * d.cap, eb = g * kSearchEdges;
+    const bool flip = policy_flip(d.rec[g].player, view);
+    if (policy) {
+        for (int i = tid; i < XQ_POLICY_ACTIONS / 4; i += kRootThreads) reinterpret_cast<float4*>(s_p)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+        __syncthreads();
+    }
+    if (tid < 32) {
+        GumbelRoot r;
+        gumbel_root_warp(d, G, t, lane, s_scr[0], s_scr[1], r);
+        if (policy) {
+            float p[kGumbelSlots];
+            gumbel_policy_warp(r, lane, s_scr[0], p);
+#pragma unroll
+            for (int i = 0; i < kGumbelSlots; ++i) {
+                const int k = lane + 32 * i;
+                if (k < r.ne) { const int ai = d.act[eb + k]; s_p[flip ? XQ_POLICY_ACTIONS - 1 - ai : ai] = p[i]; }
+            }
+        }
+        const int kp = gumbel_action_warp(r, lane);
+        if (action && lane == 0) {
+            const int ai = kp >= 0 ? d.act[eb + kp] : -1;
+            action[t] = kp < 0 ? -1 : (flip ? XQ_POLICY_ACTIONS - 1 - ai : ai);
+        }
+    }
+    if (policy) {
+        __syncthreads();
+        float4* dst = reinterpret_cast<float4*>(policy + t * XQ_POLICY_ACTIONS);
+        for (int i = tid; i < XQ_POLICY_ACTIONS / 4; i += kRootThreads) dst[i] = reinterpret_cast<const float4*>(s_p)[i];
+    }
+}
+
+__global__ void __launch_bounds__(32 * kGumbelWarps) gumbel_play_kernel(SearchDev d, GumbelDev G, PlayArgs a) {
+    __shared__ uint32_t s_b[kGumbelWarps][12];
+    __shared__ float s_scr[kGumbelWarps][2][kSearchEdges];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t t = (int64_t)blockIdx.x * kGumbelWarps + warp;
+    if (t >= d.n) return;
+    const int64_t g0 = t * d.cap, eb0 = g0 * kSearchEdges;
+    bool diff = false;
+    if (lane < 4) {
+        const uint4 rv = reinterpret_cast<const uint4*>(d.rec + g0)[lane], ev = reinterpret_cast<const uint4*>(a.envs + t)[lane];
+        diff = rv.x != ev.x || rv.y != ev.y || rv.z != ev.z || rv.w != ev.w;
+    }
+    const bool stale = __any_sync(0xFFFFFFFFu, diff);
+    int kp = -1;
+    if (!stale) {
+        GumbelRoot r;
+        gumbel_root_warp(d, G, t, lane, s_scr[warp][0], s_scr[warp][1], r);
+        kp = gumbel_action_warp(r, lane);
+    }
+    if (lane != 0) return;
+    SmemBoard b{s_b[warp], 1};
+    b.load(a.envs + t);
+    Meta m; m.load(a.envs + t);
+    const int ai = kp >= 0 ? d.act[eb0 + kp] : 0, from = ai / 90, to = ai % 90;
+    if (a.actions) a.actions[t] = kp >= 0 ? policy_index(from, to, policy_flip(m.player, a.view)) : -1;
+    policy_apply(b, m, a.envs, t, kp >= 0, from, to, a.auto_reset, a.reward, a.done, a.winner, a.captured, a.valid);
+}
+
+__global__ void __launch_bounds__(32 * kGumbelWarps) gumbel_weights_kernel(SearchDev d, GumbelDev G) {
+    __shared__ float s_scr[kGumbelWarps][2][kSearchEdges];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t t = (int64_t)blockIdx.x * kGumbelWarps + warp;
+    if (t >= d.n) return;
+    GumbelRoot r;
+    gumbel_root_warp(d, G, t, lane, s_scr[warp][0], s_scr[warp][1], r);
+    float p[kGumbelSlots];
+    gumbel_policy_warp(r, lane, s_scr[warp][0], p);
+#pragma unroll
+    for (int i = 0; i < kGumbelSlots; ++i) {
+        const int k = lane + 32 * i;
+        if (k < r.ne) G.w[t * kSearchEdges + k] = gumbel_weight(p[i]);
+    }
+}
+
 }  // namespace xq
 
 // ==========================================================================================
@@ -696,6 +1009,7 @@ struct xq_search_s {
     int leaves = 1;                // slots per tree of the last selection
     int sims = 0;
     int phase = 0;                 // 0 never reset, 1 ready for select, 2 selected (observe / leaves / expand_backup)
+    uint64_t roots = 0;            // resets and advances so far: a Gumbel state begun on other roots is stale
     bool maybe_nonstd = false;     // the env had injected boards at the reset: leaves may need the generic kernel
     void* slab = nullptr;
     SearchDev d{};
@@ -718,6 +1032,9 @@ int enter(xq_search_t s, EnvInfo* E, const char* fn) {
 }
 bool valid_view(int v) { return v == XQ_VIEW_ABSOLUTE || v == XQ_VIEW_SIDE_TO_MOVE; }
 }  // namespace
+
+static int select_leaves(xq_search_t s, int leaves, float c_puct, float fpu, float virtual_loss, uint8_t* status_dev, uint8_t* winner_dev,
+                         int32_t* reward_dev, int32_t* depth_dev, const GumbelDev* G);
 
 int xq::search_roots(xq_search_t s, SearchRoots* out) {
     if (!s) return fail(XQ_ERR_INVALID, "null search handle");
@@ -796,6 +1113,7 @@ int xq_search_reset(xq_search_t s) {
     s->maybe_nonstd = E.maybe_nonstd;
     s->sims = 0;
     s->phase = 1;
+    s->roots++;
     return XQ_OK;
 }
 
@@ -818,6 +1136,7 @@ int xq_search_advance(xq_search_t s, int min_free, const float* root_noise_dev, 
     s->maybe_nonstd = s->maybe_nonstd || E.maybe_nonstd;      // kept boards descend from the old roots
     s->sims = s->max_sims - min_free;
     s->phase = 1;
+    s->roots++;
     return XQ_OK;
 }
 
@@ -828,6 +1147,14 @@ int xq_search_select_device(xq_search_t s, float c_puct, float fpu, uint8_t* sta
 
 int xq_search_select_leaves_device(xq_search_t s, int leaves, float c_puct, float fpu, float virtual_loss, uint8_t* status_dev,
                                    uint8_t* winner_dev, int32_t* reward_dev, int32_t* depth_dev) {
+    return select_leaves(s, leaves, c_puct, fpu, virtual_loss, status_dev, winner_dev, reward_dev, depth_dev, nullptr);
+}
+
+}  // extern "C"
+
+// the selection of xq_search_select_leaves_device, with the Gumbel root rule when G is given (xq_gumbel_select_device)
+static int select_leaves(xq_search_t s, int leaves, float c_puct, float fpu, float virtual_loss, uint8_t* status_dev, uint8_t* winner_dev,
+                         int32_t* reward_dev, int32_t* depth_dev, const GumbelDev* G) {
     EnvInfo E;
     if (int rc = enter(s, &E, "xq_search_select_device")) return rc;
     if (leaves < 1 || leaves > s->max_leaves) return fail(XQ_ERR_INVALID, "xq_search_select_leaves_device: leaves %d (1 .. %d)", leaves, s->max_leaves);
@@ -839,17 +1166,23 @@ int xq_search_select_leaves_device(xq_search_t s, int leaves, float c_puct, floa
     if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_search_select_device: the last selection was not expanded and backed up");
     if (s->sims + leaves > s->max_sims)
         return fail(XQ_ERR_STATE, "xq_search_select_device: %d simulations since the reset, %d more pass the capacity %d", s->sims, leaves, s->max_sims);
-    if (leaves == 1)
+    if (G)
+        search_select_leaves_kernel<<<grid_of(s->d.n, kSelLeavesWarps), 32 * kSelLeavesWarps, 0, E.stream>>>(s->d, leaves, c_puct, fpu, virtual_loss,
+                                                                                                            status_dev, winner_dev, reward_dev, depth_dev, *G);
+    else if (leaves == 1)
         search_select_kernel<<<grid_of(s->d.n, kSelWarps), 32 * kSelWarps, 0, E.stream>>>(s->d, c_puct, fpu, status_dev, winner_dev, reward_dev, depth_dev);
     else
         search_select_leaves_kernel<<<grid_of(s->d.n, kSelLeavesWarps), 32 * kSelLeavesWarps, 0, E.stream>>>(s->d, leaves, c_puct, fpu, virtual_loss,
-                                                                                                            status_dev, winner_dev, reward_dev, depth_dev);
+                                                                                                            status_dev, winner_dev, reward_dev, depth_dev,
+                                                                                                            GumbelNone{});
     XQ_LAUNCH_CHECK();
     s->sims += leaves;
     s->leaves = leaves;
     s->phase = 2;
     return XQ_OK;
 }
+
+extern "C" {
 
 int xq_search_leaves_device(xq_search_t s, void** leaf_recs_dev) {
     if (!s || !leaf_recs_dev) return fail(XQ_ERR_INVALID, "xq_search_leaves_device: null argument");
@@ -995,6 +1328,188 @@ int xq_search_get_tree(xq_search_t s, int64_t tree, xq_search_node* nodes_host, 
         }
     }
     *n_nodes = cnt;
+    return XQ_OK;
+}
+
+}  // extern "C"
+
+// ==========================================================================================
+// Gumbel root search (xq_gumbel_*)
+// ==========================================================================================
+struct xq_gumbel_s {
+    xq_search_t s = nullptr;
+    int device = 0;
+    int max_considered = 0;
+    bool begun = false;
+    uint64_t roots = 0;            // the search's xq_search_s::roots at begin
+    void* slab = nullptr;
+    GumbelDev G{};
+};
+
+namespace {
+constexpr size_t kGumbelTreeBytes = 4 * kSearchEdges * 4 + 4 * 4 + 4 + 4;      // g, logit, N0, weights; the bitmap, v, m
+static_assert(kGumbelTreeBytes == 2072, "include/xq.h documents 2,072 B per tree");
+
+// the slab of xq_gumbel_create: its seven arrays, each 256-byte aligned (offsets o[0 .. 6]); returns the total
+size_t gumbel_slab(int64_t n, size_t* o) {
+    const int64_t edges = n * kSearchEdges;
+    const size_t sizes[7] = {(size_t)(4 * edges), (size_t)(4 * edges), (size_t)(4 * edges), (size_t)(4 * edges), (size_t)(16 * n), (size_t)(4 * n),
+                             (size_t)(4 * n)};
+    size_t off = 0;
+    for (int i = 0; i < 7; ++i) { o[i] = off; off += (sizes[i] + 255) & ~(size_t)255; }
+    return off;
+}
+
+// the state is current: begun on the search's present roots (no reset / advance since)
+int gumbel_ready(xq_gumbel_t g, EnvInfo* E, const char* fn) {
+    if (!g) return fail(XQ_ERR_INVALID, "%s: null handle", fn);
+    if (int rc = enter(g->s, E, fn)) return rc;
+    if (!g->begun || g->roots != g->s->roots) return fail(XQ_ERR_STATE, "%s: no xq_gumbel_begin_device since the last reset / advance", fn);
+    return XQ_OK;
+}
+}  // namespace
+
+int xq::gumbel_weights(xq_gumbel_t g, xq_env_t env, SearchRoots* roots, const uint32_t** w) {
+    EnvInfo E;
+    if (!g) return fail(XQ_ERR_INVALID, "xq_examples_record_gumbel_device: null Gumbel state");
+    if (g->s->env != env) return fail(XQ_ERR_INVALID, "xq_examples_record_gumbel_device: the search is on another env handle");
+    if (int rc = gumbel_ready(g, &E, "xq_examples_record_gumbel_device")) return rc;
+    if (g->s->phase == 2) return fail(XQ_ERR_STATE, "xq_examples_record_gumbel_device: the last selection was not expanded and backed up");
+    gumbel_weights_kernel<<<grid_of(g->s->d.n, kGumbelWarps), 32 * kGumbelWarps, 0, E.stream>>>(g->s->d, g->G);
+    XQ_LAUNCH_CHECK();
+    *w = g->G.w;
+    return search_roots(g->s, roots);
+}
+
+extern "C" {
+
+int xq_gumbel_bytes(int64_t n_trees, int max_simulations, int64_t* bytes) {
+    if (!bytes || n_trees < 1 || max_simulations < 1 || max_simulations > (1 << 24)) return fail(XQ_ERR_INVALID, "xq_gumbel_bytes: bad arguments");
+    size_t o[7];
+    *bytes = (int64_t)gumbel_slab(n_trees, o);
+    return XQ_OK;
+}
+
+int xq_gumbel_create(xq_search_t s, int max_considered, xq_gumbel_t* out) {
+    if (!out || !s) return fail(XQ_ERR_INVALID, "xq_gumbel_create: null search or out");
+    if (max_considered < 1 || max_considered > kSearchEdges)
+        return fail(XQ_ERR_INVALID, "xq_gumbel_create: max_considered %d (1 .. %d)", max_considered, kSearchEdges);
+    EnvInfo E;
+    if (int rc = enter(s, &E, "xq_gumbel_create")) return rc;
+    xq_gumbel_s* g = new (std::nothrow) xq_gumbel_s();
+    if (!g) return fail(XQ_ERR_NOMEM, "xq_gumbel_create: out of host memory");
+    g->s = s; g->device = E.device; g->max_considered = max_considered;
+    const int64_t n = s->d.n;
+    size_t o[7];
+    const size_t off = gumbel_slab(n, o);
+    if (cudaMalloc(&g->slab, off) != cudaSuccess) {
+        cudaGetLastError();
+        delete g;
+        return fail(XQ_ERR_NOMEM, "xq_gumbel_create: %lld trees need %.2f GB of device memory", (long long)n, off / 1e9);
+    }
+    char* b = static_cast<char*>(g->slab);
+    GumbelDev& G = g->G;
+    G.g = reinterpret_cast<float*>(b + o[0]); G.logit = reinterpret_cast<float*>(b + o[1]); G.n0 = reinterpret_cast<int32_t*>(b + o[2]);
+    G.w = reinterpret_cast<uint32_t*>(b + o[3]); G.cons = reinterpret_cast<uint32_t*>(b + o[4]); G.vhat = reinterpret_cast<float*>(b + o[5]);
+    G.m = reinterpret_cast<int32_t*>(b + o[6]);
+    *out = g;
+    return XQ_OK;
+}
+
+int xq_gumbel_destroy(xq_gumbel_t g) {
+    if (!g) return XQ_OK;
+    cudaSetDevice(g->device);
+    cudaFree(g->slab);             // synchronises with the work still queued on the env's stream
+    delete g;
+    return XQ_OK;
+}
+
+int xq_gumbel_begin_device(xq_gumbel_t g, const void* scores_dev, int scores_dtype, float temperature, int view, const float* root_value_dev,
+                           int n_simulations, uint64_t seed, float c_visit, float c_scale) {
+    EnvInfo E;
+    if (!g) return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: null handle");
+    xq_search_t s = g->s;
+    if (int rc = enter(s, &E, "xq_gumbel_begin_device")) return rc;
+    if (!scores_dev || !root_value_dev) return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: scores and root values are required");
+    if (scores_dtype != XQ_DTYPE_F32 && scores_dtype != XQ_DTYPE_BF16)
+        return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: scores_dtype %d (f32 or bf16)", scores_dtype);
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: view %d", view);
+    if (!(temperature > 0.f && temperature <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: temperature must be finite and > 0");
+    if (n_simulations < 1 || n_simulations > s->max_sims)
+        return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: n_simulations %d (1 .. %d)", n_simulations, s->max_sims);
+    if (!(c_visit >= 0.f && c_visit <= FLT_MAX) || !(c_scale >= 0.f && c_scale <= FLT_MAX))
+        return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: c_visit and c_scale must be finite and >= 0");
+    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_gumbel_begin_device: the search was never reset (xq_search_reset)");
+    if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_gumbel_begin_device: the last selection was not expanded and backed up");
+    const ExpandArgs a{scores_dev, temperature, view, root_value_dev, nullptr, 0.f};
+    const bool bf16 = scores_dtype == XQ_DTYPE_BF16;
+    if (bf16) gumbel_expand_root_kernel<XQ_DTYPE_BF16><<<grid_of(s->d.n, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a);
+    else gumbel_expand_root_kernel<XQ_DTYPE_F32><<<grid_of(s->d.n, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a);
+    XQ_LAUNCH_CHECK();
+    if (s->maybe_nonstd) {
+        if (bf16) search_expand_generic_kernel<XQ_DTYPE_BF16><<<grid_of(s->d.n, kThreads), kThreads, 0, E.stream>>>(s->d, a);
+        else search_expand_generic_kernel<XQ_DTYPE_F32><<<grid_of(s->d.n, kThreads), kThreads, 0, E.stream>>>(s->d, a);
+        XQ_LAUNCH_CHECK();
+    }
+    g->G.c_visit = c_visit; g->G.c_scale = c_scale; g->G.sims = 0; g->G.n_sims = n_simulations;
+    gumbel_init_kernel<<<grid_of(s->d.n, kGumbelWarps), 32 * kGumbelWarps, 0, E.stream>>>(s->d, g->G, g->max_considered, seed, E.env_id0,
+                                                                                         root_value_dev);
+    XQ_LAUNCH_CHECK();
+    g->begun = true;
+    g->roots = s->roots;
+    return XQ_OK;
+}
+
+int xq_gumbel_select_device(xq_gumbel_t g, int leaves, float c_puct, float fpu, float virtual_loss, uint8_t* status_dev, uint8_t* winner_dev,
+                            int32_t* reward_dev, int32_t* depth_dev) {
+    EnvInfo E;
+    if (int rc = gumbel_ready(g, &E, "xq_gumbel_select_device")) return rc;
+    if (leaves < 1 || leaves > g->s->max_leaves) return fail(XQ_ERR_INVALID, "xq_gumbel_select_device: leaves %d (1 .. %d)", leaves, g->s->max_leaves);
+    if (g->G.sims + leaves > g->G.n_sims)
+        return fail(XQ_ERR_STATE, "xq_gumbel_select_device: %d of the %d simulations of this move done, %d more pass them", g->G.sims, g->G.n_sims,
+                    leaves);
+    if (int rc = select_leaves(g->s, leaves, c_puct, fpu, virtual_loss, status_dev, winner_dev, reward_dev, depth_dev, &g->G)) return rc;
+    g->G.sims += leaves;
+    return XQ_OK;
+}
+
+int xq_gumbel_root_device(xq_gumbel_t g, int view, float* policy_dev, int64_t* action_dev) {
+    EnvInfo E;
+    if (int rc = gumbel_ready(g, &E, "xq_gumbel_root_device")) return rc;
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_gumbel_root_device: view %d", view);
+    if (reinterpret_cast<uintptr_t>(policy_dev) & 15u) return fail(XQ_ERR_INVALID, "xq_gumbel_root_device: policy must be 16-byte aligned");
+    if (g->s->phase == 2) return fail(XQ_ERR_STATE, "xq_gumbel_root_device: the last selection was not expanded and backed up");
+    gumbel_root_kernel<<<(unsigned)g->s->d.n, kRootThreads, 0, E.stream>>>(g->s->d, g->G, view, policy_dev, action_dev);
+    XQ_LAUNCH_CHECK();
+    return XQ_OK;
+}
+
+int xq_gumbel_play_device(xq_gumbel_t g, int view, int auto_reset, int64_t* actions_dev, int32_t* reward_dev, uint8_t* done_dev,
+                          uint8_t* winner_dev, uint8_t* captured_dev, uint8_t* valid_dev) {
+    EnvInfo E;
+    if (int rc = gumbel_ready(g, &E, "xq_gumbel_play_device")) return rc;
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_gumbel_play_device: view %d", view);
+    if (g->s->phase == 2) return fail(XQ_ERR_STATE, "xq_gumbel_play_device: the last selection was not expanded and backed up");
+    const PlayArgs a{E.d_envs, E.env_id0, E.seed, 0.f, 0, view, auto_reset, actions_dev, reward_dev, done_dev, winner_dev, captured_dev, valid_dev};
+    gumbel_play_kernel<<<grid_of(g->s->d.n, kGumbelWarps), 32 * kGumbelWarps, 0, E.stream>>>(g->s->d, g->G, a);
+    XQ_LAUNCH_CHECK();
+    return XQ_OK;
+}
+
+int xq_gumbel_get(xq_gumbel_t g, int64_t tree, float* gumbel_host, float* logit_host, int32_t* n0_host, uint32_t* considered_host,
+                  float* root_value_host, int32_t* m_host) {
+    EnvInfo E;
+    if (int rc = gumbel_ready(g, &E, "xq_gumbel_get")) return rc;
+    if (tree < 0 || tree >= g->s->d.n) return fail(XQ_ERR_INVALID, "xq_gumbel_get: tree %lld of %lld", (long long)tree, (long long)g->s->d.n);
+    const GumbelDev& G = g->G;
+    const int64_t e0 = tree * kSearchEdges;
+    if (gumbel_host) XQ_CUDA(cudaMemcpyAsync(gumbel_host, G.g + e0, 4 * kSearchEdges, cudaMemcpyDeviceToHost, E.stream));
+    if (logit_host) XQ_CUDA(cudaMemcpyAsync(logit_host, G.logit + e0, 4 * kSearchEdges, cudaMemcpyDeviceToHost, E.stream));
+    if (n0_host) XQ_CUDA(cudaMemcpyAsync(n0_host, G.n0 + e0, 4 * kSearchEdges, cudaMemcpyDeviceToHost, E.stream));
+    if (considered_host) XQ_CUDA(cudaMemcpyAsync(considered_host, G.cons + tree * 4, 16, cudaMemcpyDeviceToHost, E.stream));
+    if (root_value_host) XQ_CUDA(cudaMemcpyAsync(root_value_host, G.vhat + tree, 4, cudaMemcpyDeviceToHost, E.stream));
+    if (m_host) XQ_CUDA(cudaMemcpyAsync(m_host, G.m + tree, 4, cudaMemcpyDeviceToHost, E.stream));
+    XQ_CUDA(cudaStreamSynchronize(E.stream));
     return XQ_OK;
 }
 

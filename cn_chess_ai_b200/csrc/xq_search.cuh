@@ -1,8 +1,8 @@
 // xq_search.cuh -- host-compilable helpers of the batched tree search (xq_search.cu; include/xq.h: xq_search_*): the PUCT score of an
 // edge (with virtual loss: search_puct_vl) and its arg-max order, the in-flight counting of a multi-leaf selection, the priors of a
 // freshly expanded node, the root-noise mix, the value cleaning, the backup along a path, and the membership and renumbering of a tree
-// re-rooted after a move (xq_search_advance), the visit-count choice of the move to play (xq_search_play_device) and the Dirichlet draw
-// of the root noise (xq_search_root_noise_device).
+// re-rooted after a move (xq_search_advance), the visit-count choice of the move to play (xq_search_play_device), the Dirichlet draw
+// of the root noise (xq_search_root_noise_device), and the Gumbel root search (xq_gumbel_*).
 //
 // The arithmetic is spelled with explicitly rounded operations (__fmul_rn and friends on the device; plain operators on the host, where
 // tests/hostsim/search_shim.cpp is compiled with -ffp-contract=off) so that no multiply-add is contracted and numpy can restate every
@@ -231,6 +231,108 @@ XQ_HD void search_dirichlet(uint64_t base, int n, float alpha, float* eta) {
     float s = 0.f;
     for (int k = 0; k < n; ++k) { eta[k] = search_noise_exp(eta[k], m); s = s_add(s, eta[k]); }
     for (int k = 0; k < n; ++k) eta[k] = s_div(eta[k], s);
+}
+
+// ---- Gumbel root search: sampled root actions, Sequential Halving, completed-Q targets (xq_gumbel_*) ----
+// Gumbel of edge k: g = -log(-log u), u = (f + 0.5) * 2^-24 from the 24-bit field f at bits 40..63 of xq_rng(base, k, 128), base =
+// xq_rng(seed, global env id, root ctr); word 128 keeps the draw apart from the root noise's words 0 .. 64.
+constexpr uint32_t kGumbelWord = 128;
+XQ_HD float gumbel_draw(uint64_t base, int k) {
+    const float u = s_mul(s_add((float)((uint32_t)(rng(base, (uint64_t)k, kGumbelWord) >> 40)), 0.5f), 5.9604644775390625e-8f);
+    return -logf(-logf(u));
+}
+// the root-rule order: a larger score, or an equal one at a smaller list index (search_better)
+// considered set: edge k is among the top m by key (g + logit), ties to the smaller list index, iff fewer than m edges come before it
+XQ_HD bool gumbel_considered(const float* key, int n, int m, int k) {
+    int before = 0;
+    for (int b = 0; b < n; ++b) before += (key[b] > key[k] || (key[b] == key[k] && b < k)) ? 1 : 0;
+    return before < m;
+}
+// entry i of the Sequential Halving visit sequence of m considered actions and n simulations (mctx's
+// get_sequence_of_considered_visits): m <= 1 gives i; otherwise log2max = ceil(log2 m), and each phase adds
+// max(1, n / (log2max * m_cur)) rounds of one visit to each of the first m_cur actions (whose counts are equal, c), so an entry at offset
+// p of a phase is c + p / m_cur; after a phase m_cur = max(2, m_cur / 2).  The sequence is n entries long; i < n.
+XQ_HD int gumbel_seq(int m, int n, int i) {
+    if (m <= 1) return i;
+    int log2max = 0;
+    while ((1 << log2max) < m) ++log2max;
+    int mc = m, c = 0;
+    for (;;) {
+        const int q = n / (log2max * mc), rounds = q > 1 ? q : 1;
+        if ((int64_t)i < (int64_t)rounds * mc) return c + i / mc;
+        i -= rounds * mc;
+        c += rounds;
+        mc = mc / 2 > 2 ? mc / 2 : 2;
+    }
+}
+// Completed Q of a root with n edges (N, W the edges' statistics, P the stored priors, vhat the cleaned root value), from the root's side:
+//   q_k = W_k / N_k when N_k > 0, else v_mix = (vhat + SN * (sq / sp)) / (1 + SN), SN = sum N, sp = sum over visited edges of
+//   P'_b = max(P_b, FLT_MIN), sq = sum over visited edges of P'_b * q_b (both in list order); v_mix = vhat when no edge is visited.
+XQ_HD float gumbel_vmix_of(int sn, float sp, float sq, float vhat) {
+    return sn > 0 ? s_div(s_add(vhat, s_mul((float)sn, s_div(sq, sp))), (float)(sn + 1)) : vhat;
+}
+XQ_HD float gumbel_vmix(const int32_t* N, const float* W, const float* P, int n, float vhat) {
+    int sn = 0;
+    float sp = 0.f, sq = 0.f;
+    for (int k = 0; k < n; ++k) {
+        if (N[k] <= 0) continue;
+        sn += N[k];
+        const float p = fmaxf(P[k], FLT_MIN);
+        sp = s_add(sp, p);
+        sq = s_add(sq, s_mul(p, s_div(W[k], (float)N[k])));
+    }
+    return gumbel_vmix_of(sn, sp, sq, vhat);
+}
+// sigma of an edge with completed q, over the root's min / max completed q and largest N: q^ = (q - min) / max(max - min, 1e-8),
+// sigma = ((c_visit + N_max) * c_scale) * q^
+XQ_HD float gumbel_sigma(float q, float mn, float mx, int nmax, float c_visit, float c_scale) {
+    const float qh = s_div(s_add(q, -mn), fmaxf(s_add(mx, -mn), 1e-8f));
+    return s_mul(s_mul(s_add(c_visit, (float)nmax), c_scale), qh);
+}
+// z_k = logit_k + sigma_k (the improved policy's logits) and score_k = (g_k + logit_k) + sigma_k (the root rule's) of a root of n edges
+XQ_HD void gumbel_root_scores(const int32_t* N, const float* W, const float* P, const float* g, const float* logit, int n, float vhat,
+                              float c_visit, float c_scale, float* z, float* score) {
+    const float vm = gumbel_vmix(N, W, P, n, vhat);
+    float mn = INFINITY, mx = -INFINITY;
+    int nmax = 0;
+    for (int k = 0; k < n; ++k) {
+        const float q = N[k] > 0 ? s_div(W[k], (float)N[k]) : vm;
+        mn = fminf(mn, q); mx = fmaxf(mx, q);
+        nmax = N[k] > nmax ? N[k] : nmax;
+    }
+    for (int k = 0; k < n; ++k) {
+        const float q = N[k] > 0 ? s_div(W[k], (float)N[k]) : vm;
+        const float sg = gumbel_sigma(q, mn, mx, nmax, c_visit, c_scale);
+        z[k] = s_add(logit[k], sg);
+        score[k] = s_add(s_add(g[k], logit[k]), sg);
+    }
+}
+// the improved policy pi'_k = exp(z_k - max z) / S, S summed in list order; its integer weight round-to-nearest-even(pi' * 2^24)
+XQ_HD float gumbel_exp(float z, float zmax) { return expf(s_add(z, -zmax)); }
+XQ_HD uint32_t gumbel_weight(float p) { return (uint32_t)rintf(s_mul(p, 16777216.f)); }
+// the root rule of one descent: among considered edges (cons) whose count this move (n_k + in-flight c_k: cnt) equals `target`, the
+// largest score, ties to the smaller list index; if none has that count, the considered edges with the fewest, then the same order
+XQ_HD int gumbel_pick(const bool* cons, const int* cnt, const float* score, int n, int target) {
+    bool hit = false;
+    int least = 0x7FFFFFFF;
+    for (int k = 0; k < n; ++k)
+        if (cons[k]) { hit = hit || cnt[k] == target; least = cnt[k] < least ? cnt[k] : least; }
+    const int want = hit ? target : least;
+    int bk = -1;
+    float bs = 0.f;
+    for (int k = 0; k < n; ++k)
+        if (cons[k] && cnt[k] == want && search_better(score[k], k, bs, bk)) { bs = score[k]; bk = k; }
+    return bk;
+}
+// the action to play: the considered edge with the most visits this move, ties by score, then list index; -1 when none was visited
+XQ_HD int gumbel_action(const bool* cons, const int* nv, const float* score, int n) {
+    int bk = -1, bn = 0;
+    float bs = 0.f;
+    for (int k = 0; k < n; ++k) {
+        if (!cons[k] || nv[k] <= 0) continue;
+        if (bk < 0 || nv[k] > bn || (nv[k] == bn && search_better(score[k], k, bs, bk))) { bk = k; bn = nv[k]; bs = score[k]; }
+    }
+    return bk;
 }
 
 }  // namespace xq

@@ -238,6 +238,69 @@ class BatchedSearch:
         return nodes[:cnt.value].copy(), edges[:cnt.value].copy()
 
 
+def gumbel_bytes(n_trees, max_simulations):
+    """device memory a BatchedGumbel on a search of n_trees trees allocates"""
+    b = C.c_int64()
+    check(lib().xq_gumbel_bytes(int(n_trees), int(max_simulations), C.byref(b)))
+    return b.value
+
+
+class BatchedGumbel:
+    """xq_gumbel_*: the Gumbel root-search state of `search` (a BatchedSearch): Gumbel-top-k sampled root actions, Sequential Halving
+    over them, and the completed-Q improved policy.  Raw device pointers (ints), asynchronous on the env's stream; close() before the
+    search is closed."""
+
+    def __init__(self, search, max_considered=16):
+        self._L = lib()
+        self._h = C.c_void_p()
+        check(self._L.xq_gumbel_create(search._h, int(max_considered), C.byref(self._h)))
+        self.search = search
+        self.n = search.n
+        self.max_considered = int(max_considered)
+
+    def close(self):
+        if self._h:
+            self._L.xq_gumbel_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def begin_device(self, scores_ptr, scores_dtype, temperature, view, values_ptr, n_simulations, seed, c_visit=50.0, c_scale=0.1):
+        """xq_gumbel_begin_device: expand the unexpanded roots from scores [n][8100], then draw the Gumbels, the considered sets, N0 and
+        the root values (f32 [n]) of this move's n_simulations"""
+        check(self._L.xq_gumbel_begin_device(self._h, scores_ptr, scores_dtype, float(temperature), view, values_ptr, int(n_simulations),
+                                             int(seed), float(c_visit), float(c_scale)))
+
+    def select_device(self, leaves, c_puct, fpu, virtual_loss, status_ptr=None, winner_ptr=None, reward_ptr=None, depth_ptr=None):
+        """xq_gumbel_select_device: xq_search_select_leaves_device with the Gumbel root rule; outputs [n][leaves]"""
+        check(self._L.xq_gumbel_select_device(self._h, int(leaves), float(c_puct), float(fpu), float(virtual_loss), status_ptr, winner_ptr,
+                                              reward_ptr, depth_ptr))
+
+    def root_device(self, view, policy_ptr=None, action_ptr=None):
+        """xq_gumbel_root_device: the improved policy f32 [n][8100] and the action to play int64 [n] (-1 none)"""
+        check(self._L.xq_gumbel_root_device(self._h, view, policy_ptr, action_ptr))
+
+    def play_device(self, view, auto_reset, actions_ptr=None, reward_ptr=None, done_ptr=None, winner_ptr=None, captured_ptr=None, valid_ptr=None):
+        """xq_gumbel_play_device: the action of root_device played on the env"""
+        check(self._L.xq_gumbel_play_device(self._h, view, 1 if auto_reset else 0, actions_ptr, reward_ptr, done_ptr, winner_ptr, captured_ptr,
+                                            valid_ptr))
+
+    def get(self, tree):
+        """synchronous read-back of one tree's state: dict of gumbel, logit (f32 [128]), n0 (int32 [128]), considered (bool [128]),
+        root_value (float) and m (int)"""
+        g, lg = np.zeros(SEARCH_MAX_EDGES, np.float32), np.zeros(SEARCH_MAX_EDGES, np.float32)
+        n0 = np.zeros(SEARCH_MAX_EDGES, np.int32)
+        cons = np.zeros(4, np.uint32)
+        v, m = C.c_float(), C.c_int32()
+        check(self._L.xq_gumbel_get(self._h, int(tree), ptr(g), ptr(lg), ptr(n0), ptr(cons), C.byref(v), C.byref(m)))
+        bits = ((cons[:, None] >> np.arange(32, dtype=np.uint32)[None, :]) & 1).reshape(-1).astype(bool)
+        return {"gumbel": g, "logit": lg, "n0": n0, "considered": bits, "root_value": v.value, "m": m.value}
+
+
 def examples_bytes(n_envs, capacity, max_game_examples):
     """device memory a BatchedExamples of this size allocates (the sampling scratch aside)"""
     b = C.c_int64()
@@ -273,6 +336,11 @@ class BatchedExamples:
     def record_device(self, search, mask_ptr=None):
         """xq_examples_record_device: one example of every root of `search` (a BatchedSearch on the same env), u8 [n] mask or None"""
         check(self._L.xq_examples_record_device(self._h, search._h, mask_ptr))
+
+    def record_gumbel_device(self, gumbel, mask_ptr=None):
+        """xq_examples_record_gumbel_device: record_device with the improved-policy weights round(pi' * 2^24) of `gumbel` (a BatchedGumbel
+        on a search of the same env) in the visits field"""
+        check(self._L.xq_examples_record_gumbel_device(self._h, gumbel._h, mask_ptr))
 
     def end_games_device(self, ended_ptr, result_ptr):
         """xq_examples_end_games_device: ended u8 [n], result f32 [n] from Red's side"""

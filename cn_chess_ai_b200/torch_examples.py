@@ -46,6 +46,13 @@ class TorchExamples:
         self.tenv._enter()
         self.examples.record_device(search.search, None if m is None else m.data_ptr())
 
+    def record_gumbel(self, gumbel, mask=None):
+        """record() after a Gumbel search (a TorchGumbel on the same envs): the stored visits are the integer weights
+        round(pi'_k * 2^24) of the improved policy, so sample() gives pi' (within about 2^-24) as the policy target"""
+        m = None if mask is None else self._flags(mask, "mask")
+        self.tenv._enter()
+        self.examples.record_gumbel_device(gumbel.gumbel, None if m is None else m.data_ptr())
+
     def end_games(self, ended, result_red):
         """commit the staged examples of the envs where ended (bool / uint8 [n]) is set; result_red f32 [n] is each game's result from
         Red's side (NaN -> 0, clamped to [-1, 1]); an example's z is the result from its side to move"""

@@ -11,7 +11,7 @@ from collections import namedtuple
 import torch
 
 from ._lib import POLICY_ACTIONS, SEARCH_MAX_EDGES
-from .env import BatchedSearch
+from .env import BatchedGumbel, BatchedSearch
 from .torch_env import _OBS_DTYPES, _SCORE_DTYPES, StepResult, _view
 
 SelectResult = namedtuple("SelectResult", "status winner reward depth")
@@ -194,5 +194,96 @@ class TorchSearch:
             values = values.reshape(self._rows).to(torch.float32).contiguous()
             values = torch.where(status != NEEDS_EVALUATION, self.outcome_values(status, winner, aux, cap_value), values)
             self.expand_backup(scores.contiguous(), values, temperature, root_noise, noise_eps, view)
+            i += k
+        return self.root(view)
+
+
+GumbelRootResult = namedtuple("GumbelRootResult", "policy action")
+
+
+class TorchGumbel:
+    """Gumbel root search (Danihelka et al., ICLR 2022; include/xq.h: xq_gumbel_*) on a TorchSearch: each move begin() samples up to
+    max_considered (1 .. 128) root actions per tree without replacement (Gumbel-top-k), select() splits the move's simulations among them
+    by Sequential Halving, root() gives the improved policy pi' = softmax(logits + sigma(completed Q)) -- the policy target -- and the
+    action to play, play() plays it.  Below the root, selection is the search's PUCT (with virtual loss for several leaves)."""
+
+    def __init__(self, search, max_considered=16):
+        self.tsearch = search
+        self.tenv = search.tenv
+        self.n = search.n
+        self.device = search.device
+        self.gumbel = BatchedGumbel(search.search, max_considered)
+        self.max_considered = self.gumbel.max_considered
+
+    def close(self):
+        self.gumbel.close()
+
+    def begin(self, scores, values, n_simulations, seed=0, temperature=1.0, c_visit=50.0, c_scale=0.1, view="side"):
+        """after the search's reset() / advance(): scores [n, 8100] (f32 / bf16, frame of `view`) and values f32 [n] of the network on the
+        roots (TorchEnv.observe).  Unexpanded roots are expanded and backed up from them, as a first simulation would; then every tree
+        draws its Gumbels from (seed, env id, root ply counter), picks its considered actions and keeps the root value for the completed
+        Q.  n_simulations: the selected slots of this move."""
+        v = _view(view)
+        self.tenv._check(scores, "scores", list(_SCORE_DTYPES), (self.n, POLICY_ACTIONS))
+        self.tenv._check(values, "values", [torch.float32], (self.n,))
+        self.tenv._enter()
+        self.gumbel.begin_device(scores.data_ptr(), _SCORE_DTYPES[scores.dtype], temperature, v, values.data_ptr(), n_simulations, seed,
+                                 c_visit, c_scale)
+
+    def select(self, leaves=1, c_puct=1.5, fpu=0.0, virtual_loss=1.0):
+        """TorchSearch.select_leaves with the Gumbel root rule: SelectResult of tensors [n, leaves]; the search's leaves(), observe() and
+        expand_backup() follow as after select_leaves"""
+        ts = self.tsearch
+        self.tenv._enter()
+        shape = (self.n, int(leaves))
+        status, winner = (torch.empty(shape, dtype=torch.uint8, device=self.device) for _ in range(2))
+        reward, depth = (torch.empty(shape, dtype=torch.int32, device=self.device) for _ in range(2))
+        self.gumbel.select_device(leaves, c_puct, fpu, virtual_loss, status.data_ptr(), winner.data_ptr(), reward.data_ptr(), depth.data_ptr())
+        ts._rows = self.n * int(leaves)
+        return SelectResult(status, winner, reward, depth)
+
+    def root(self, view="side"):
+        """GumbelRootResult: policy f32 [n, 8100] (pi' in the frame of `view`, zero rows for roots without edges), action int64 [n] (the
+        considered action with the most visits this move, -1 without one: the input of TorchEnv.step(actions=action, pick="given"))"""
+        v = _view(view)
+        self.tenv._enter()
+        policy = torch.empty((self.n, POLICY_ACTIONS), dtype=torch.float32, device=self.device)
+        action = torch.empty(self.n, dtype=torch.int64, device=self.device)
+        self.gumbel.root_device(v, policy.data_ptr(), action.data_ptr())
+        return GumbelRootResult(policy, action)
+
+    def play(self, view="side", auto_reset=True):
+        """root().action played on every env, as TorchSearch.play steps (a stale root or no action plays nothing): StepResult"""
+        v = _view(view)
+        self.tenv._enter()
+        actions = torch.empty(self.n, dtype=torch.int64, device=self.device)
+        reward = torch.empty(self.n, dtype=torch.int32, device=self.device)
+        done, winner, captured, valid = (torch.empty(self.n, dtype=torch.uint8, device=self.device) for _ in range(4))
+        self.gumbel.play_device(v, auto_reset, actions.data_ptr(), reward.data_ptr(), done.data_ptr(), winner.data_ptr(), captured.data_ptr(),
+                                valid.data_ptr())
+        return StepResult(actions, None, reward, done, winner, captured, valid)
+
+    def run(self, evaluate, n_simulations, seed=0, c_puct=1.5, fpu=0.0, temperature=1.0, c_visit=50.0, c_scale=0.1, view="side",
+            obs_dtype=torch.bfloat16, cap_value=0.0, leaves=1, virtual_loss=1.0, reset=True):
+        """one move's Gumbel search: reset() (reset=False: continue from advance()), evaluate(planes) -> (scores, values) once on the env
+        boards (TorchEnv.observe) for begin(), then n_simulations selections in select(leaves) calls, the last one smaller, each
+        evaluated once with outcome_values at terminal leaves as TorchSearch.run does.  Returns root(view)."""
+        ts = self.tsearch
+        if reset:
+            ts.reset()
+        planes, _ = self.tenv.observe(obs_dtype, view)
+        scores, values = evaluate(planes)
+        self.begin(scores.contiguous(), values.reshape(self.n).to(torch.float32).contiguous(), n_simulations, seed, temperature, c_visit,
+                   c_scale, view)
+        i = 0
+        while i < n_simulations:
+            k = min(leaves, n_simulations - i)
+            sel = self.select(k, c_puct, fpu, virtual_loss)
+            status, winner = sel.status.reshape(-1), sel.winner.reshape(-1)
+            planes, aux = ts.observe(obs_dtype, view)
+            scores, values = evaluate(planes)
+            values = values.reshape(ts._rows).to(torch.float32).contiguous()
+            values = torch.where(status != NEEDS_EVALUATION, ts.outcome_values(status, winner, aux, cap_value), values)
+            ts.expand_backup(scores.contiguous(), values, temperature, None, 0.0, view)
             i += k
         return self.root(view)

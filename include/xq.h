@@ -365,6 +365,71 @@ int xq_search_root_noise_device(xq_search_t s, float alpha, float eps, uint64_t 
  * node's n_edges have action -1 and child -1), *n_nodes = nodes in the tree */
 int xq_search_get_tree(xq_search_t s, int64_t tree, xq_search_node* nodes_host, xq_search_edge* edges_host, int32_t* n_nodes);
 
+/* ---- Gumbel root search (Danihelka et al., "Policy improvement by planning with Gumbel", ICLR 2022; mctx's gumbel_muzero_policy) ----
+ * A root rule beside PUCT for small simulation budgets: m root actions sampled without replacement by the Gumbel-top-k trick, the
+ * simulations split among them by Sequential Halving, the survivor played, and the improved policy pi' = softmax(logits + sigma(completed
+ * Q)) as the policy target.  The state is a separate object bound to one search (destroy it before the search); below the root,
+ * selection stays PUCT (with virtual loss when several leaves are selected), with the same child creation, statuses, duplicates and
+ * budget.  All arithmetic is f32 with no contraction; for one tree, with root edges k = 0 .. n_edges - 1 in list order:
+ *  logit  l_k = logf(P_k), P_k the root's stored prior at begin.
+ *  Gumbel g_k = -logf(-logf(u_k)), u_k = (f + 0.5) * 2^-24, f = bits 40..63 of xq_rng(xq_rng(seed, env_id0 + e, root ctr), k, 128): word 128
+ *    is apart from the root noise's words 0 .. 64 (xq_search_root_noise_device); the draw does not depend on sharding or n.
+ *  Considered set: the m_t = min(max_considered, n_edges) edges with the largest g_k + l_k, ties to the smaller list index.
+ *  Visits this move: n_k = N_k - N0_k, N0_k the edge's N at begin (so a subtree kept by xq_search_advance does not break the schedule).
+ *  Completed Q, from the root's side (W is from the side to move at the parent): q_k = W_k / N_k when N_k > 0, else
+ *    v_mix = (v + SN * (sq / sp)) / (1 + SN), SN = sum of N, sp = sum over visited edges of P'_b = max(P_b, FLT_MIN), sq = the sum of
+ *    P'_b * q_b over them (both sums in list order), v the root value given to begin (NaN -> 0, clamped to [-1, 1]); v_mix = v when no edge
+ *    is visited.  q^_k = (q_k - min) / max(max - min, 1e-8), min and max over the root's edges.
+ *    sigma_k = ((c_visit + max_b N_b) * c_scale) * q^_k; mctx's defaults are c_visit = 50, c_scale = 0.1.
+ *  Schedule: seq = mctx's get_sequence_of_considered_visits(m_t, n_simulations): for m_t <= 1 it is 0, 1, 2, ...; otherwise
+ *    log2max = ceil(log2 m_t), m_cur = m_t, and each phase adds max(1, n_simulations / (log2max * m_cur)) rounds of one visit to each of
+ *    the first m_cur entries (one entry per visit: the entry's count before it), then m_cur = max(2, m_cur / 2); truncated to
+ *    n_simulations entries.
+ *  Root rule of Gumbel simulation i (counted since begin; descent k of a call of L leaves is i = done + k), c_k = the earlier descents of
+ *    the call through edge k: among considered edges with n_k + c_k == seq[i], the largest (g_k + l_k) + sigma_k, ties to the smaller list
+ *    index; if no considered edge has that count (a duplicate slot did not back up), the considered edges with the fewest n_k + c_k, in
+ *    the same order.  sigma uses the tree's N and W (virtual loss does not change them).
+ *  Action to play: the considered edge with the largest n_k, ties to the larger (g + l) + sigma, then the smaller list index; none when
+ *    every considered n_k is 0.
+ *  Improved policy: pi'_k = expf(z_k - max z) / S, z_k = l_k + sigma_k, S summed in list order over all root edges.
+ * Call order: xq_search_reset or xq_search_advance, then xq_gumbel_begin_device, then n_simulations selections through
+ * xq_gumbel_select_device (each followed by the unchanged leaves / observe_leaves / expand_backup), then root / play / record.  Every call
+ * but begin returns XQ_ERR_STATE when there was no begin since the search's last reset / advance; select, root, play and record also
+ * while a selection is pending, and select past n_simulations.  XQ_ERR_INVALID for bad arguments.
+ * Memory (xq_gumbel_bytes, exact): 2,072 bytes per tree -- g, l, N0 and a weight row of 128 x 4 bytes, the considered bitmap (16 bytes), v
+ * and m_t -- in seven arrays each rounded up to 256 bytes (under 1.8 KB in all); the simulation counts are the same for every tree and held
+ * on the host.  The schedule is computed, not stored, so the size does not
+ * depend on max_simulations (checked to be 1 .. 2^24).  xq_search_bytes_per_tree is unchanged. */
+typedef struct xq_gumbel_s* xq_gumbel_t;
+/* max_considered 1 .. 128; XQ_ERR_NOMEM when the device memory cannot be had */
+int xq_gumbel_create(xq_search_t s, int max_considered, xq_gumbel_t* out);
+int xq_gumbel_destroy(xq_gumbel_t g);
+int xq_gumbel_bytes(int64_t n_trees, int max_simulations, int64_t* bytes);
+/* Begin the move's Gumbel search.  Every unexpanded, non-terminal root is expanded from its row of scores_dev [n][8100] (f32 / bf16,
+ * frame of `view`, temperature finite > 0) and backed up with root_value_dev[e] (f32 [n], from the root's side to move), bit for bit what
+ * a select that stops at the root followed by xq_search_expand_backup_device makes of it; then every tree draws g, picks its considered
+ * set and records N0 and v (root_value_dev, cleaned).  One network call on the n root boards supplies both.  Not a select: it spends no
+ * budget and makes no node.  n_simulations 1 .. max_simulations (the Gumbel selections of this move), c_visit and c_scale finite >= 0;
+ * allowed after a reset / advance when no selection is pending. */
+int xq_gumbel_begin_device(xq_gumbel_t g, const void* scores_dev, int scores_dtype, float temperature, int view, const float* root_value_dev,
+                           int n_simulations, uint64_t seed, float c_visit, float c_scale);
+/* xq_search_select_leaves_device (leaves 1 .. max_leaves, the same outputs and checks) with the Gumbel root rule; spends `leaves` of the
+ * search's budget and of n_simulations */
+int xq_gumbel_select_device(xq_gumbel_t g, int leaves, float c_puct, float fpu, float virtual_loss, uint8_t* status_dev, uint8_t* winner_dev,
+                            int32_t* reward_dev, int32_t* depth_dev);
+/* policy_dev f32 [n][8100] (16-byte aligned) or NULL: pi' at the root edges' policy indices in the frame of `view`, 0 elsewhere (a zero
+ * row for a root without edges); action_dev int64 [n] or NULL: the action to play (frame of `view`), -1 for a root without edges or
+ * without a visit this move */
+int xq_gumbel_root_device(xq_gumbel_t g, int view, float* policy_dev, int64_t* action_dev);
+/* plays the action of xq_gumbel_root_device on the search's env: the step is bit for bit xq_search_play_device's (xq_env_policy_step_device
+ * with XQ_PICK_GIVEN), stale-root rule included; outputs as xq_search_play_device's.  The tree is not touched. */
+int xq_gumbel_play_device(xq_gumbel_t g, int view, int auto_reset, int64_t* actions_dev, int32_t* reward_dev, uint8_t* done_dev,
+                          uint8_t* winner_dev, uint8_t* captured_dev, uint8_t* valid_dev);
+/* synchronous read-back of one tree's state (tests, inspection): g, l and N0 [128] (0 past the root's edges), the considered bitmap [4]
+ * (bit l of word i: edge 32 i + l), v and m_t (0: the root had no edge at begin); any pointer may be NULL */
+int xq_gumbel_get(xq_gumbel_t g, int64_t tree, float* gumbel_host, float* logit_host, int32_t* n0_host, uint32_t* considered_host,
+                  float* root_value_host, int32_t* m_host);
+
 /* ---- device-resident self-play example buffer: the training data of an AlphaZero-style policy/value network ----
  * Bound to one env handle (asynchronous on its stream and device, unless a call says otherwise; destroy it before the env).  Each move,
  * xq_examples_record_device stores one example per tree of a search on that env: the root's record and its root edges' actions and visit
@@ -411,6 +476,11 @@ int xq_examples_bytes(int64_t n_envs, int64_t capacity, int max_game_examples, i
  * step, or a missing xq_search_advance) is not recorded and counts as stale.  Recording an env twice in one game (after a rejected move)
  * stores two examples. */
 int xq_examples_record_device(xq_examples_t b, xq_search_t s, const uint8_t* mask_dev);
+/* xq_examples_record_device for the search of a begun Gumbel state (same checks, same example), except that visits[k] holds the integer
+ * weight w_k = round-to-nearest-even(pi'_k * 2^24) of the improved policy (xq_gumbel_root_device) and total_visits the sum of the w_k:
+ * such examples carry weights, not visit counts, and xq_examples_sample_device gives w_k / sum w.  sum w is 2^24 within a few units (each
+ * weight is rounded on its own), so the target is within (1.5 + pi'_k |sum w - 2^24|) 2^-24 of pi'_k. */
+int xq_examples_record_gumbel_device(xq_examples_t b, xq_gumbel_t g, const uint8_t* mask_dev);
 /* envs with ended_dev[e] != 0 (u8 [n], required) commit their staged examples to the ring with z from result_dev[e] (f32 [n], required,
  * Red's side) and their game number; their staging areas empty and their game counts advance */
 int xq_examples_end_games_device(xq_examples_t b, const uint8_t* ended_dev, const float* result_dev);
