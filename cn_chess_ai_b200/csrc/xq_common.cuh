@@ -40,16 +40,34 @@ struct EnvInfo {
 int env_info(xq_env_t h, EnvInfo* out);
 void env_advance_event_ply(xq_env_t h, uint32_t plies);   // the collector applied `plies` more plies
 void** env_scratch_slot(xq_env_t h, void (*free_fn)(void*));   // the env handle's slot for the collector's scratch; free_fn runs when the handle is destroyed
-// what the example buffer (xq_examples.cu) reads of a search (xq_search.cu): its env, call state and the root rows of its slab
+// what the example buffer (xq_examples.cu) reads of a search (xq_search.cu): the root rows of its slab
 struct SearchRoots {
-    xq_env_t env; int phase;         // phase: 0 never reset, 1 ready, 2 a selection pending
     int64_t n; int cap;              // node j of tree t at g = t * cap + j; edge k of node g at g * 128 + k
     const xq_env_rec* rec; const uint8_t *nedges, *expanded; const int32_t* N; const float* W; const int16_t* act;
 };
-int search_roots(xq_search_t s, SearchRoots* out);
+// the roots of search s for the caller fn, which records them for the envs of `env`: the search must be on `env`, reset, and have no
+// selection pending
+int search_roots(xq_search_t s, xq_env_t env, const char* fn, SearchRoots* out);
 // xq_examples_record_gumbel_device: the call checks of a begun Gumbel search on env `env`, its roots, and the improved-policy weights of
 // every root ([n][128], edge k at t * 128 + k) launched on the env's stream
 int gumbel_weights(xq_gumbel_t g, xq_env_t env, SearchRoots* roots, const uint32_t** w);
+
+// ---- host helpers of the C ABI -----------------------------------------------------------------
+inline unsigned grid_of(int64_t n, int per_block) { return (unsigned)((n + per_block - 1) / per_block); }
+inline bool valid_view(int view) { return view == XQ_VIEW_ABSOLUTE || view == XQ_VIEW_SIDE_TO_MOVE; }
+inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+// A handle's device slab, carved into arrays that each start on a 256-byte boundary.  A handle lays its slab out in one function, run
+// first with base nullptr to count the bytes and then on the allocation to set its pointers, so the size and the offsets agree.
+struct Slab {
+    char* base;
+    size_t bytes = 0;
+    template <class T> T* take(size_t count) {
+        T* p = reinterpret_cast<T*>(reinterpret_cast<uintptr_t>(base) + bytes);
+        bytes += (sizeof(T) * count + 255) & ~(size_t)255;
+        return p;
+    }
+};
 
 // ---- device helpers ---------------------------------------------------------------------------
 #if defined(__CUDACC__)

@@ -134,7 +134,6 @@ __global__ void __launch_bounds__(128) select_greedy_f64(const double* __restric
     }
 }
 
-static inline unsigned blocks(int64_t n, int per) { return (unsigned)((n + per - 1) / per); }
 
 static int dqn_reserve(xq_dqn_s* h, int64_t n) {
     if (n <= h->cap) return XQ_OK;
@@ -152,7 +151,7 @@ static int dqn_forward_dev(xq_dqn_s* h, const double* W, const double* B, int64_
     size_t ofs = 0;
     for (int l = 0; l < h->L; ++l) {
         const int in = h->layers[l], on = h->layers[l + 1];
-        fwd_layer_f64<<<blocks(n * on * 32, 256), 256, 0, h->stream>>>(W + h->wofs[l], B + h->bofs[l], h->d_act + ofs, (int64_t)h->act_stride,
+        fwd_layer_f64<<<grid_of(n * on * 32, 256), 256, 0, h->stream>>>(W + h->wofs[l], B + h->bofs[l], h->d_act + ofs, (int64_t)h->act_stride,
                                                                        h->d_act + ofs + in, keep_z ? h->d_z + ofs + in : nullptr,
                                                                        (int64_t)h->act_stride, in, on, n);
         XQ_LAUNCH_CHECK();
@@ -169,27 +168,27 @@ static int dqn_backprop_dev(xq_dqn_s* h, double lr) {
     for (int l = 0; l <= h->L; ++l) { aofs[l] = o; o += h->layers[l]; }
     const int Lo = h->L - 1;
     double* delta = h->d_delta;   // deltas use the same per-layer offsets as activations
-    out_delta_f64<<<blocks(h->layers[Lo + 1], 256), 256, 0, h->stream>>>(h->d_act + aofs[Lo + 1], h->d_target, h->d_z + aofs[Lo + 1],
+    out_delta_f64<<<grid_of(h->layers[Lo + 1], 256), 256, 0, h->stream>>>(h->d_act + aofs[Lo + 1], h->d_target, h->d_z + aofs[Lo + 1],
                                                                          delta + aofs[Lo + 1], h->layers[Lo + 1]);
     XQ_LAUNCH_CHECK();
     for (int l = Lo - 1; l >= 0; --l) {
         const int width = h->layers[l + 1], prev = h->layers[l], next = h->layers[l + 2];
         const double* Wn = h->d_w + h->wofs[l + 1];
         if (h->mode == XQ_DQN_AS_WRITTEN) {
-            hidden_delta_as_written_f64<<<blocks(width, 128), 128, 0, h->stream>>>(Wn, (size_t)width * next, delta + aofs[l + 2], next,
+            hidden_delta_as_written_f64<<<grid_of(width, 128), 128, 0, h->stream>>>(Wn, (size_t)width * next, delta + aofs[l + 2], next,
                                                                                    h->d_z + aofs[l + 1], delta + aofs[l + 1], width, prev);
             XQ_LAUNCH_CHECK();
         } else {
             XQ_CUDA(cudaMemsetAsync(h->d_tmp, 0, sizeof(double) * width, h->stream));
-            hidden_delta_partial_f64<<<blocks(next, 32), 256, 0, h->stream>>>(Wn, delta + aofs[l + 2], h->d_tmp, width, next);
+            hidden_delta_partial_f64<<<grid_of(next, 32), 256, 0, h->stream>>>(Wn, delta + aofs[l + 2], h->d_tmp, width, next);
             XQ_LAUNCH_CHECK();
-            hidden_delta_finish_f64<<<blocks(width, 128), 128, 0, h->stream>>>(h->d_tmp, h->d_z + aofs[l + 1], delta + aofs[l + 1], width);
+            hidden_delta_finish_f64<<<grid_of(width, 128), 128, 0, h->stream>>>(h->d_tmp, h->d_z + aofs[l + 1], delta + aofs[l + 1], width);
             XQ_LAUNCH_CHECK();
         }
     }
     for (int l = 0; l < h->L; ++l) {   // every delta was taken from the pre-update weights (src/dqn.cu:429-447)
         const int in = h->layers[l], on = h->layers[l + 1];
-        update_f64<<<blocks((int64_t)in * on, 256), 256, 0, h->stream>>>(h->d_w + h->wofs[l], h->d_b + h->bofs[l], h->d_act + aofs[l],
+        update_f64<<<grid_of((int64_t)in * on, 256), 256, 0, h->stream>>>(h->d_w + h->wofs[l], h->d_b + h->bofs[l], h->d_act + aofs[l],
                                                                          delta + aofs[l + 1], lr, in, on);
         XQ_LAUNCH_CHECK();
     }

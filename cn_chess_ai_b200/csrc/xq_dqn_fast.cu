@@ -1490,7 +1490,6 @@ static inline DwPush dw_push(Fast* f, bool apply, bool fused = false) {
     return p;
 }
 
-static inline unsigned blocks(int64_t n, int per) { return (unsigned)((n + per - 1) / per); }
 
 void dqn_fast_destroy(xq_dqn_s* h) {
     Fast* f = h->fast;
@@ -1593,12 +1592,12 @@ static int ensure_fast(xq_dqn_s* h) {
     if (int rc = fast_init(h)) return rc;
     Fast* f = h->fast;
     if (!h->fast_current) {
-        f64_to_fast_kernel<<<blocks((int64_t)kOut * kHid, 256), 256, 0, h->stream>>>(h->d_w, h->d_b, f->W0T, f->b0, f->W1, f->b1, f->W1bf, f->W1lo);
+        f64_to_fast_kernel<<<grid_of((int64_t)kOut * kHid, 256), 256, 0, h->stream>>>(h->d_w, h->d_b, f->W0T, f->b0, f->W1, f->b1, f->W1bf, f->W1lo);
         XQ_LAUNCH_CHECK();
         h->fast_current = true; ++f->w_version;
     }
     if (!f->target_current) {
-        f64_to_fast_kernel<<<blocks((int64_t)kOut * kHid, 256), 256, 0, h->stream>>>(h->d_tw, h->d_tb, f->tW0T, f->tb0, f->tW1, f->tb1, f->tW1bf, (__nv_bfloat16*)nullptr);
+        f64_to_fast_kernel<<<grid_of((int64_t)kOut * kHid, 256), 256, 0, h->stream>>>(h->d_tw, h->d_tb, f->tW0T, f->tb0, f->tW1, f->tb1, f->tW1bf, (__nv_bfloat16*)nullptr);
         XQ_LAUNCH_CHECK();
         f->target_current = true;
     }
@@ -1608,7 +1607,7 @@ static int ensure_fast(xq_dqn_s* h) {
 int dqn_ensure_f64(xq_dqn_s* h) {
     if (h->f64_current || !h->fast) return XQ_OK;
     Fast* f = h->fast;
-    fast_to_f64_kernel<<<blocks((int64_t)kOut * kHid, 256), 256, 0, h->stream>>>(h->d_w, h->d_b, f->W0T, f->b0, f->W1, f->b1);
+    fast_to_f64_kernel<<<grid_of((int64_t)kOut * kHid, 256), 256, 0, h->stream>>>(h->d_w, h->d_b, f->W0T, f->b0, f->W1, f->b1);
     XQ_LAUNCH_CHECK();
     h->f64_current = true;
     return XQ_OK;
@@ -1678,7 +1677,7 @@ int dqn_q90_device(xq_dqn_s* h, const xq_env_rec* envs_dev, int64_t n, float* q9
     // `carried`: the caller's act_team_kernel has already brought the sums, the remembered boards and h(s) of these n envs up to date
     // (tail of the previous ply of the same xq_selfplay_collect call); only valid while nothing else could have touched them
     if (!(carried && !fresh_all && n == f->act_carried_n)) {
-        l0_act_kernel<<<blocks(n, 32), 256, 0, stream>>>(envs_dev, n, f->W0Q, f->b0Q, reinterpret_cast<const float*>(f->actMax + 2), f->actZ, f->actPrev, fresh_all,
+        l0_act_kernel<<<grid_of(n, 32), 256, 0, stream>>>(envs_dev, n, f->W0Q, f->b0Q, reinterpret_cast<const float*>(f->actMax + 2), f->actZ, f->actPrev, fresh_all,
                                                         f->actHhi, f->actHlo);
         XQ_LAUNCH_CHECK();
     }
@@ -1741,7 +1740,7 @@ int xq_dqn_forward_boards(xq_dqn_t h, const xq_env_rec* boards_host, int64_t n, 
     Fast* f = h->fast;
     if (n > f->q_cap) { cudaFree(f->q); f->q = nullptr; f->q_cap = 0; XQ_CUDA(cudaMalloc(&f->q, sizeof(float) * n * kOut)); f->q_cap = n; }
     XQ_CUDA(cudaMemcpyAsync(f->boards, boards_host, sizeof(xq_env_rec) * n, cudaMemcpyHostToDevice, h->stream));
-    l0_forward_kernel<<<blocks(n * 32, 256), 256, 0, h->stream>>>(reinterpret_cast<const uint8_t*>(f->boards), sizeof(xq_env_rec), n, f->W0T, f->b0, f->Hbf, nullptr);
+    l0_forward_kernel<<<grid_of(n * 32, 256), 256, 0, h->stream>>>(reinterpret_cast<const uint8_t*>(f->boards), sizeof(xq_env_rec), n, f->W0T, f->b0, f->Hbf, nullptr);
     XQ_LAUNCH_CHECK();
     if (int rc = fast_maps(h, n)) return rc;
     if (int rc = launch_gemm(h, EPI_STORE_TANH, f->tmH, f->tmW1, f->b1, n, f->q)) return rc;
@@ -1775,13 +1774,13 @@ int td_update_core(xq_dqn_s* h, const BatchRef& ref, int64_t n, int use_target_n
     // Four kernels chained with programmatic dependent launch: each one's set-up (barriers, TMEM, operand tiles that do not
     // depend on its predecessor) overlaps the predecessor's tail.
     // 1. h(s) with the online net; h(s') with the online (ChessAI::train) or target (DQN::train) net; compact batch
-    XQ_CUDA(launch_pdl(l0_pair_kernel, dim3(blocks(n, kL0Warps)), dim3(kL0Warps * 32), 0, h->stream, 1, ref, n, f->W0T, f->b0,
+    XQ_CUDA(launch_pdl(l0_pair_kernel, dim3(grid_of(n, kL0Warps)), dim3(kL0Warps * 32), 0, h->stream, 1, ref, n, f->W0T, f->b0,
                        use_target_net ? f->tW0T : f->W0T, use_target_net ? f->tb0 : f->b0, f->Hf, f->H2bf, f->cb, ld, f->info_slots,
                        kInfoSlots * 4, 3));
     // 2. max_a z(s')[a] over all 8100 outputs
     if (int rc = launch_gemm(h, EPI_ROWMAX, f->tmH2, use_target_net ? f->tmTW1 : f->tmW1, use_target_net ? f->tb1 : f->b1, n, nullptr)) return rc;
     // 3. TD error, delta0, delta1 h
-    XQ_CUDA(launch_pdl(td_delta_kernel, dim3(blocks(n * 32, 256)), dim3(256), 0, h->stream, 1, f->cb, n, f->Hf, f->W1, f->b1, f->zpart, ld, kParts,
+    XQ_CUDA(launch_pdl(td_delta_kernel, dim3(grid_of(n * 32, 256)), dim3(256), 0, h->stream, 1, f->cb, n, f->Hf, f->W1, f->b1, f->zpart, ld, kParts,
                        (float)h->gamma, h->mode, f->d0hi, f->d0lo, f->ghi, f->glo, ld, f->info_slots));
     // 4. dW0 / db0 / dW1 / db1 contraction, cluster reduction and the SGD step (or the compact gradient)
     XQ_CUDA(launch_pdl(dw_gemm_kernel, dim3(kDwMTiles, kDwSplits), dim3(kDwThreads), kDwSmem, h->stream, kDwSplits, f->tmD0hi, f->tmD0lo, f->tmGhi,
@@ -1844,7 +1843,7 @@ int dqn_td_update_pipelined(xq_dqn_s* h, const void* ring, int64_t size, uint64_
     auto aux_l0 = [&](int i) -> int {
         const int slot = i & 1;
         const BatchRef ref{reinterpret_cast<const uint8_t*>(ring), size, seed, counter0 + (uint32_t)i, 1};
-        XQ_CUDA(launch_pdl(l0_pair_kernel, dim3(blocks(n, kL0Warps)), dim3(kL0Warps * 32), 0, aux, 1, ref, n, f->W0T, f->b0, f->tW0T, f->tb0, f->Hf,
+        XQ_CUDA(launch_pdl(l0_pair_kernel, dim3(grid_of(n, kL0Warps)), dim3(kL0Warps * 32), 0, aux, 1, ref, n, f->W0T, f->b0, f->tW0T, f->tb0, f->Hf,
                            slot ? f->H2bf_b : f->H2bf, f->cb, ld, f->info_slots, 0, 2));
         return XQ_OK;
     };
@@ -1867,12 +1866,12 @@ int dqn_td_update_pipelined(xq_dqn_s* h, const void* ring, int64_t size, uint64_
         const int slot = i & 1;
         const BatchRef ref{reinterpret_cast<const uint8_t*>(ring), size, seed, counter0 + (uint32_t)i, 1};
         if (i + 1 < n_updates) if (int rc = aux_l0(i + 1)) return rc;
-        XQ_CUDA(launch_pdl(l0_pair_kernel, dim3(blocks(n, kL0Warps)), dim3(kL0Warps * 32), 0, main, 1, ref, n, f->W0T, f->b0, f->tW0T, f->tb0, f->Hf,
+        XQ_CUDA(launch_pdl(l0_pair_kernel, dim3(grid_of(n, kL0Warps)), dim3(kL0Warps * 32), 0, main, 1, ref, n, f->W0T, f->b0, f->tW0T, f->tb0, f->Hf,
                            f->H2bf, f->cb, ld, f->info_slots, kInfoSlots * 4, 1));
         XQ_CUDA(cudaStreamWaitEvent(main, f->ev_aux[slot], 0));  // the row-max partials of this update
         XQ_CUDA(cudaEventRecord(f->ev_td[slot], main));
         if (i + 1 < n_updates) if (int rc = aux_gemm(i + 1, f->ev_td[slot])) return rc;
-        XQ_CUDA(launch_pdl(td_delta_kernel, dim3(blocks(n * 32, 256)), dim3(256), 0, main, 1, f->cb, n, f->Hf, f->W1, f->b1, slot ? f->zpart_b : f->zpart,
+        XQ_CUDA(launch_pdl(td_delta_kernel, dim3(grid_of(n * 32, 256)), dim3(256), 0, main, 1, f->cb, n, f->Hf, f->W1, f->b1, slot ? f->zpart_b : f->zpart,
                            ld, kParts, (float)h->gamma, h->mode, f->d0hi, f->d0lo, f->ghi, f->glo, ld, f->info_slots));
         // multi-GPU: the contraction exchanges the gradient and applies the SGD step itself
         XQ_CUDA(launch_pdl(dw_gemm_kernel, dim3(kDwMTiles, kDwSplits), dim3(kDwThreads), kDwSmem, main, kDwSplits, f->tmD0hi, f->tmD0lo, f->tmGhi,
@@ -1925,7 +1924,7 @@ int xq_dqn_apply_grads(xq_dqn_t h, double lr) {
     if (int rc = ensure_fast(h)) return rc;
     Fast* f = h->fast;
     if (lr <= 0) lr = h->lr;
-    apply_kernel<<<blocks(kGradSize, 256), 256, 0, h->stream>>>(f->W0T, f->b0, f->W1, f->b1, f->W1bf, f->W1lo, cur_grad(f), (float)lr);
+    apply_kernel<<<grid_of(kGradSize, 256), 256, 0, h->stream>>>(f->W0T, f->b0, f->W1, f->b1, f->W1bf, f->W1lo, cur_grad(f), (float)lr);
     XQ_LAUNCH_CHECK();
     h->f64_current = false; ++f->w_version;
     return XQ_OK;
@@ -1995,7 +1994,7 @@ int dqn_exchange_apply(xq_dqn_s* h, double lr) {
     PeerPtrs pp;
     for (int r = 0; r < kMaxRanks; ++r) pp.p[r] = f->peer[r];
     ++f->epoch;
-    XQ_CUDA(launch_pdl(grad_exchange_apply_kernel, dim3(blocks(kGradPad / 4, 256)), dim3(256), 0, h->stream, 1, pp, f->rank, f->world, f->parity, f->epoch, f->W0T,
+    XQ_CUDA(launch_pdl(grad_exchange_apply_kernel, dim3(grid_of(kGradPad / 4, 256)), dim3(256), 0, h->stream, 1, pp, f->rank, f->world, f->parity, f->epoch, f->W0T,
                        f->b0, f->W1, f->b1, f->W1bf, f->W1lo, (float)lr, f->timeout_ticks, f->status_dev));
     f->parity ^= 1;
     h->f64_current = false; ++f->w_version;

@@ -313,7 +313,6 @@ struct xq_env_s {
     bool async_dirty = false;                                   // asynchronous work on `stream` since the last synchronisation of the handle
 };
 
-static inline unsigned grid_for(int64_t n, int per_block) { return (unsigned)((n + per_block - 1) / per_block); }
 
 namespace xq {
 cudaError_t launch_rollout_team(xq_env_rec* envs, int64_t n, uint64_t env_id0, uint64_t seed, int n_plies, xq_trace_rec* trace,
@@ -339,7 +338,7 @@ static int launch_legal_moves(xq_env_s* h) {
     if (team) XQ_CUDA(launch_legal_moves_team(h->d_envs, h->n, h->d_u8[0], h->d_lists, h->d_nonstd, h->stream));
     else XQ_CUDA(launch_legal_moves_lane(h->d_envs, h->n, h->d_u8[0], h->d_lists, h->d_nonstd, h->stream));
     if (h->maybe_nonstd) {
-        legal_moves_kernel<<<grid_for(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->d_u8[0], h->d_lists, h->d_nonstd);
+        legal_moves_kernel<<<grid_of(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->d_u8[0], h->d_lists, h->d_nonstd);
         XQ_LAUNCH_CHECK();
     }
     return XQ_OK;
@@ -369,7 +368,7 @@ static int launch_rollout(xq_env_s* h, int n_plies, xq_trace_rec* d_trace, const
     if (rollout_team(h->n) == 1) XQ_CUDA(launch_rollout_lane(h->d_envs, h->n, h->env_id0, h->seed, n_plies, d_trace, h->d_stats, h->d_nonstd, h->stream, src, mirror));
     else XQ_CUDA(launch_rollout_team(h->d_envs, h->n, h->env_id0, h->seed, n_plies, d_trace, h->d_stats, h->d_nonstd, h->stream, src, mirror));
     if (h->maybe_nonstd) {
-        rollout_random_kernel<<<grid_for(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->env_id0, h->seed, n_plies, d_trace,
+        rollout_random_kernel<<<grid_of(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->env_id0, h->seed, n_plies, d_trace,
                                                                                     h->d_stats, h->d_nonstd, mirror);
         XQ_LAUNCH_CHECK();
     }
@@ -377,7 +376,7 @@ static int launch_rollout(xq_env_s* h, int n_plies, xq_trace_rec* d_trace, const
 }
 // device alias of a pinned, mapped, 16-byte aligned host buffer (cudaHostAlloc / cudaHostRegister under unified addressing), or null
 static void* mapped_alias(const void* host) {
-    if (!host || (reinterpret_cast<uintptr_t>(host) & 15u)) return nullptr;
+    if (!host || !aligned16(host)) return nullptr;
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, host) != cudaSuccess) { cudaGetLastError(); return nullptr; }
     return a.type == cudaMemoryTypeHost ? a.devicePointer : nullptr;
@@ -457,7 +456,7 @@ int xq_env_create(int64_t n_envs, int device, uint64_t seed, uint64_t env_id0, x
     if (e == cudaSuccess) e = cudaMalloc(&h->d_nonstd, (size_t)n_envs);
     if (e == cudaSuccess) e = cudaMemsetAsync(h->d_stats, 0, sizeof(xq_env_stats), h->stream);
     if (e != cudaSuccess) { xq_env_destroy(h); return fail(XQ_ERR_CUDA, "xq_env_create: %s", cudaGetErrorString(e)); }
-    reset_kernel<<<grid_for(4 * n_envs, 256), 256, 0, h->stream>>>(h->d_envs, n_envs, nullptr, 1);
+    reset_kernel<<<grid_of(4 * n_envs, 256), 256, 0, h->stream>>>(h->d_envs, n_envs, nullptr, 1);
     ++g_launches;
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
@@ -489,7 +488,7 @@ int xq_env_device_boards(xq_env_t h, void** p) { if (!h || !p) return fail(XQ_ER
 int xq_env_reset(xq_env_t h, const uint8_t* mask_host) {
     XQ_ENV_ENTER(h);
     if (mask_host) XQ_CUDA(cudaMemcpyAsync(h->d_u8[0], mask_host, (size_t)h->n, cudaMemcpyHostToDevice, h->stream));
-    reset_kernel<<<grid_for(4 * h->n, 256), 256, 0, h->stream>>>(h->d_envs, h->n, mask_host ? h->d_u8[0] : nullptr, 0);
+    reset_kernel<<<grid_of(4 * h->n, 256), 256, 0, h->stream>>>(h->d_envs, h->n, mask_host ? h->d_u8[0] : nullptr, 0);
     XQ_LAUNCH_CHECK();
     XQ_CUDA(cudaStreamSynchronize(h->stream));
     return XQ_OK;
@@ -525,7 +524,7 @@ int xq_env_legal_moves_strict(xq_env_t h, uint8_t* counts_host, xq_action* actio
     XQ_ENV_ENTER(h);
     if (!counts_host || !actions_host) return fail(XQ_ERR_INVALID, "xq_env_legal_moves_strict: null output");
     if (!h->d_lists) XQ_CUDA(cudaMalloc(&h->d_lists, sizeof(uint32_t) * 64 * h->n));
-    legal_moves_strict_kernel<<<grid_for(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->d_u8[0], h->d_lists);
+    legal_moves_strict_kernel<<<grid_of(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->d_u8[0], h->d_lists);
     XQ_LAUNCH_CHECK();
     XQ_CUDA(cudaMemcpyAsync(counts_host, h->d_u8[0], (size_t)h->n, cudaMemcpyDeviceToHost, h->stream));
     XQ_CUDA(cudaMemcpyAsync(actions_host, h->d_lists, sizeof(uint32_t) * 64 * h->n, cudaMemcpyDeviceToHost, h->stream));
@@ -537,7 +536,7 @@ int xq_env_valid_moves(xq_env_t h, int row, int col, uint8_t* counts_host, uint8
     XQ_ENV_ENTER(h);
     if (!counts_host || !to_host) return fail(XQ_ERR_INVALID, "xq_env_valid_moves: null output");
     if (!h->d_lists) XQ_CUDA(cudaMalloc(&h->d_lists, sizeof(uint32_t) * 64 * h->n));
-    valid_moves_kernel<<<grid_for(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, row, col, h->d_u8[0], reinterpret_cast<uint8_t*>(h->d_lists));
+    valid_moves_kernel<<<grid_of(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, row, col, h->d_u8[0], reinterpret_cast<uint8_t*>(h->d_lists));
     XQ_LAUNCH_CHECK();
     XQ_CUDA(cudaMemcpyAsync(counts_host, h->d_u8[0], (size_t)h->n, cudaMemcpyDeviceToHost, h->stream));
     XQ_CUDA(cudaMemcpyAsync(to_host, h->d_lists, (size_t)20 * h->n, cudaMemcpyDeviceToHost, h->stream));
@@ -549,7 +548,7 @@ int xq_env_is_valid_move(xq_env_t h, const int32_t* moves_host, uint8_t* valid_h
     XQ_ENV_ENTER(h);
     if (!moves_host || !valid_host) return fail(XQ_ERR_INVALID, "xq_env_is_valid_move: null pointer");
     XQ_CUDA(cudaMemcpyAsync(h->d_i32, moves_host, sizeof(int32_t) * 4 * h->n, cudaMemcpyHostToDevice, h->stream));
-    is_valid_kernel<<<grid_for(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, reinterpret_cast<const int4*>(h->d_i32), h->d_u8[0]);
+    is_valid_kernel<<<grid_of(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, reinterpret_cast<const int4*>(h->d_i32), h->d_u8[0]);
     XQ_LAUNCH_CHECK();
     XQ_CUDA(cudaMemcpyAsync(valid_host, h->d_u8[0], (size_t)h->n, cudaMemcpyDeviceToHost, h->stream));
     XQ_CUDA(cudaStreamSynchronize(h->stream));
@@ -561,7 +560,7 @@ int xq_env_step(xq_env_t h, const xq_action* actions_host, int32_t* reward_host,
     XQ_ENV_ENTER(h);
     if (!actions_host) return fail(XQ_ERR_INVALID, "xq_env_step: null actions");
     XQ_CUDA(cudaMemcpyAsync(h->d_actions, actions_host, sizeof(uint16_t) * h->n, cudaMemcpyHostToDevice, h->stream));
-    step_kernel<<<grid_for(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->d_actions, h->d_i32, h->d_u8[0], h->d_u8[1],
+    step_kernel<<<grid_of(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, h->d_actions, h->d_i32, h->d_u8[0], h->d_u8[1],
                                                                       h->d_u8[2], h->d_u8[3], auto_reset);
     XQ_LAUNCH_CHECK();
     if (reward_host) XQ_CUDA(cudaMemcpyAsync(reward_host, h->d_i32, sizeof(int32_t) * h->n, cudaMemcpyDeviceToHost, h->stream));
@@ -593,7 +592,7 @@ int xq_env_step_device(xq_env_t h, const void* actions_dev, int auto_reset, void
     XQ_ENV_ENTER(h);
     const uint16_t* a = actions_dev ? static_cast<const uint16_t*>(actions_dev) : h->d_actions;
     h->async_dirty = true;
-    step_kernel<<<grid_for(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, a, h->d_i32, h->d_u8[1], h->d_u8[2], h->d_u8[3], h->d_u8[4], auto_reset);
+    step_kernel<<<grid_of(h->n, kThreads), kThreads, 0, h->stream>>>(h->d_envs, h->n, a, h->d_i32, h->d_u8[1], h->d_u8[2], h->d_u8[3], h->d_u8[4], auto_reset);
     XQ_LAUNCH_CHECK();
     if (reward_dev) *reward_dev = h->d_i32;
     if (done_dev) *done_dev = h->d_u8[1];
@@ -759,7 +758,7 @@ int xq_env_state_onehot(xq_env_t h, double* out_host) {
     XQ_ENV_ENTER(h);
     if (!out_host) return fail(XQ_ERR_INVALID, "xq_env_state_onehot: null output");
     if (!h->d_state) XQ_CUDA(cudaMalloc(&h->d_state, sizeof(double) * XQ_STATE_SIZE * h->n));
-    state_onehot_kernel<<<grid_for(32 * h->n, 256), 256, 0, h->stream>>>(h->d_envs, h->n, h->d_state);
+    state_onehot_kernel<<<grid_of(32 * h->n, 256), 256, 0, h->stream>>>(h->d_envs, h->n, h->d_state);
     XQ_LAUNCH_CHECK();
     XQ_CUDA(cudaMemcpyAsync(out_host, h->d_state, sizeof(double) * XQ_STATE_SIZE * h->n, cudaMemcpyDeviceToHost, h->stream));
     XQ_CUDA(cudaStreamSynchronize(h->stream));

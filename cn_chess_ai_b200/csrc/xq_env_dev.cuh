@@ -1,5 +1,5 @@
-// xq_env_dev.cuh -- device helpers shared by the thread-per-board kernels (xq_env.cu, xq_selfplay.cu) and the board steps of the policy
-// and search kernels (xq_policy.cu, xq_search.cu).
+// xq_env_dev.cuh -- device helpers shared by the thread-per-board kernels (xq_env.cu, xq_selfplay.cu), the board steps of the policy
+// and search kernels (xq_policy.cu, xq_search.cu) and the root check of the search and example kernels (xq_search.cu, xq_examples.cu).
 #pragma once
 #include "xq_common.cuh"
 #include "xq_bitboard.cuh"
@@ -92,6 +92,18 @@ __device__ __forceinline__ void policy_apply(SmemBoard& b, Meta& m, xq_env_rec* 
     if (valid) valid[env] = ok ? 1 : 0;
     if (over && auto_reset) { reset_board(b); m.reset(); }
     if (ok || (over && auto_reset)) { b.store(envs + env); m.store(envs + env); }
+}
+
+// one warp: whether a search root's 64-byte record is no longer its env's, on every lane.  Lanes 0-3 compare a 16-byte word each and hand
+// it back in keep[lane] when keep is given.
+__device__ __forceinline__ bool root_stale_warp(const xq_env_rec* root, const xq_env_rec* env, int lane, uint4* keep = nullptr) {
+    bool diff = false;
+    if (lane < 4) {
+        const uint4 rv = reinterpret_cast<const uint4*>(root)[lane], ev = reinterpret_cast<const uint4*>(env)[lane];
+        diff = rv.x != ev.x || rv.y != ev.y || rv.z != ev.z || rv.w != ev.w;
+        if (keep) keep[lane] = rv;
+    }
+    return __any_sync(0xFFFFFFFFu, diff);
 }
 
 

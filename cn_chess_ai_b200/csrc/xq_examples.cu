@@ -21,6 +21,7 @@
 #include <vector>
 
 #include "xq_common.cuh"
+#include "xq_env_dev.cuh"
 #include "xq_examples.cuh"
 
 static_assert(sizeof(xq_example) == xq::kExampleBytes && sizeof(xq_example) % 32 == 0, "include/xq.h documents 864 B");
@@ -61,13 +62,7 @@ __global__ void __launch_bounds__(32 * kRecWarps) examples_record_kernel(ExDev b
     const int64_t g = t * r.cap, eb = g * kSearchEdges;
     xq_example& x = s_ex[warp];
     // 1. the root is the env's current board, all 64 bytes
-    bool diff = false;
-    if (lane < 4) {
-        const uint4 rv = reinterpret_cast<const uint4*>(r.rec + g)[lane], ev = reinterpret_cast<const uint4*>(envs + t)[lane];
-        diff = rv.x != ev.x || rv.y != ev.y || rv.z != ev.z || rv.w != ev.w;
-        reinterpret_cast<uint4*>(&x.rec)[lane] = rv;
-    }
-    if (__any_sync(0xFFFFFFFFu, diff)) {
+    if (root_stale_warp(r.rec + g, envs + t, lane, reinterpret_cast<uint4*>(&x.rec))) {
         if (lane == 0) atomicAdd(&b.ctr->stale, 1ull);
         return;
     }
@@ -243,16 +238,19 @@ struct xq_examples_s {
 
 namespace {
 
-inline size_t round256(size_t b) { return (b + 255) & ~(size_t)255; }
-// the slab of xq_examples_create, every array 256-byte aligned; false when the size does not fit
-bool slab_bytes(int64_t n, int64_t capacity, int maxg, size_t* bytes) {
+// the slab of an example buffer for n envs (Slab); false when it does not fit in memory
+bool ex_slab(ExDev& d, void* base, int64_t n, int64_t capacity, int maxg, size_t* bytes) {
     const double ex = ((double)capacity + (double)n * (double)maxg) * kExampleBytes;
     if (ex > 9.0e18) return false;
-    *bytes = round256(sizeof(xq_example) * (size_t)capacity) + round256(sizeof(xq_example) * (size_t)n * (size_t)maxg) +
-             3 * round256(4 * (size_t)n) + round256(8 * (size_t)n) + round256(sizeof(ExCounters));
+    Slab b{static_cast<char*>(base)};
+    d.ring = b.take<xq_example>((size_t)capacity);
+    d.staging = b.take<xq_example>((size_t)n * (size_t)maxg);
+    d.staged = b.take<uint32_t>(n); d.games = b.take<uint32_t>(n); d.game_at = b.take<uint32_t>(n);
+    d.off = b.take<int64_t>(n);
+    d.ctr = b.take<ExCounters>(1);
+    *bytes = b.bytes;
     return true;
 }
-inline unsigned grid_of(int64_t n, int per_block) { return (unsigned)((n + per_block - 1) / per_block); }
 int enter(xq_examples_t b, EnvInfo* E, const char* fn) {
     if (!b) return fail(XQ_ERR_INVALID, "%s: null handle", fn);
     if (int rc = env_info(b->env, E)) return rc;
@@ -265,8 +263,9 @@ extern "C" {
 
 int xq_examples_bytes(int64_t n_envs, int64_t capacity, int max_game_examples, int64_t* bytes) {
     size_t s = 0;
+    ExDev d;
     if (!bytes || n_envs < 1 || capacity < 1 || max_game_examples < 1 || max_game_examples > 65535 ||
-        !slab_bytes(n_envs, capacity, max_game_examples, &s))
+        !ex_slab(d, nullptr, n_envs, capacity, max_game_examples, &s))
         return fail(XQ_ERR_INVALID, "xq_examples_bytes: bad arguments");
     *bytes = (int64_t)s;
     return XQ_OK;
@@ -280,7 +279,8 @@ int xq_examples_create(xq_env_t env, int64_t capacity, int max_game_examples, xq
     EnvInfo E;
     if (int rc = env_info(env, &E)) return rc;
     size_t bytes = 0;
-    if (!slab_bytes(E.n, capacity, max_game_examples, &bytes)) return fail(XQ_ERR_NOMEM, "xq_examples_create: the buffer does not fit in memory");
+    ExDev d{};
+    if (!ex_slab(d, nullptr, E.n, capacity, max_game_examples, &bytes)) return fail(XQ_ERR_NOMEM, "xq_examples_create: the buffer does not fit in memory");
     XQ_CUDA(cudaSetDevice(E.device));
     xq_examples_s* b = new (std::nothrow) xq_examples_s();
     if (!b) return fail(XQ_ERR_NOMEM, "xq_examples_create: out of host memory");
@@ -292,19 +292,9 @@ int xq_examples_create(xq_env_t env, int64_t capacity, int max_game_examples, xq
         delete b;
         return fail(XQ_ERR_NOMEM, "xq_examples_create: %.2f GB of device memory not available", bytes / 1e9);
     }
-    const int64_t n = E.n;
-    char* p = static_cast<char*>(b->slab);
-    size_t off = 0;
-    auto take = [&](size_t sz) { char* q = p + off; off += round256(sz); return q; };
-    ExDev& d = b->d;
-    d.n = n; d.capacity = capacity; d.maxg = max_game_examples;
-    d.ring = reinterpret_cast<xq_example*>(take(sizeof(xq_example) * (size_t)capacity));
-    d.staging = reinterpret_cast<xq_example*>(take(sizeof(xq_example) * (size_t)n * (size_t)max_game_examples));
-    d.staged = reinterpret_cast<uint32_t*>(take(4 * (size_t)n));
-    d.games = reinterpret_cast<uint32_t*>(take(4 * (size_t)n));
-    d.game_at = reinterpret_cast<uint32_t*>(take(4 * (size_t)n));
-    d.off = reinterpret_cast<int64_t*>(take(8 * (size_t)n));
-    d.ctr = reinterpret_cast<ExCounters*>(take(sizeof(ExCounters)));
+    ex_slab(d, b->slab, E.n, capacity, max_game_examples, &bytes);
+    d.n = E.n; d.capacity = capacity; d.maxg = max_game_examples;
+    b->d = d;
     // the ring reads back as zeros before it is written; the counters and per-env words start at 0
     cudaError_t e = cudaMemsetAsync(b->slab, 0, bytes, E.stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(E.stream);
@@ -331,10 +321,7 @@ int xq_examples_record_device(xq_examples_t b, xq_search_t s, const uint8_t* mas
     if (int rc = enter(b, &E, "xq_examples_record_device")) return rc;
     if (!s) return fail(XQ_ERR_INVALID, "xq_examples_record_device: null search");
     SearchRoots r;
-    if (int rc = search_roots(s, &r)) return rc;
-    if (r.env != b->env) return fail(XQ_ERR_INVALID, "xq_examples_record_device: the search is on another env handle");
-    if (r.phase == 0) return fail(XQ_ERR_STATE, "xq_examples_record_device: the search was never reset (xq_search_reset)");
-    if (r.phase == 2) return fail(XQ_ERR_STATE, "xq_examples_record_device: the last selection was not expanded and backed up");
+    if (int rc = search_roots(s, b->env, "xq_examples_record_device", &r)) return rc;
     examples_record_kernel<false><<<grid_of(b->d.n, kRecWarps), 32 * kRecWarps, 0, E.stream>>>(b->d, r, E.d_envs, mask_dev, E.env_id0, nullptr);
     XQ_LAUNCH_CHECK();
     return XQ_OK;
@@ -378,10 +365,10 @@ int xq_examples_sample_device(xq_examples_t b, int64_t batch, uint64_t seed, uin
     EnvInfo E;
     if (int rc = enter(b, &E, "xq_examples_sample_device")) return rc;
     if (batch <= 0 || batch > 0x7FFFFFFF) return fail(XQ_ERR_INVALID, "xq_examples_sample_device: batch %lld", (long long)batch);
-    if (view != XQ_VIEW_ABSOLUTE && view != XQ_VIEW_SIDE_TO_MOVE) return fail(XQ_ERR_INVALID, "xq_examples_sample_device: view %d", view);
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_examples_sample_device: view %d", view);
     if (dtype < XQ_DTYPE_F32 || dtype > XQ_DTYPE_U8) return fail(XQ_ERR_INVALID, "xq_examples_sample_device: dtype %d", dtype);
     if (!planes_dev || !policy_dev) return fail(XQ_ERR_INVALID, "xq_examples_sample_device: planes and policy are required");
-    if ((reinterpret_cast<uintptr_t>(planes_dev) & 15u) || (reinterpret_cast<uintptr_t>(policy_dev) & 15u) || (reinterpret_cast<uintptr_t>(mask_dev) & 7u))
+    if (!aligned16(planes_dev) || !aligned16(policy_dev) || (reinterpret_cast<uintptr_t>(mask_dev) & 7u))
         return fail(XQ_ERR_INVALID, "xq_examples_sample_device: planes and policy must be 16-byte aligned, mask 8-byte aligned");
     if (batch > b->recs_cap) {      // grows on the env's stream; cudaFree waits for the work that used the old scratch
         cudaFree(b->recs); b->recs = nullptr; b->recs_cap = 0;

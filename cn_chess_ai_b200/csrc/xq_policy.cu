@@ -262,8 +262,6 @@ cudaError_t launch_observe(const xq_env_rec* recs, int64_t n, void* planes, int 
 // ==========================================================================================
 using namespace xq;
 
-static inline unsigned policy_grid(int64_t n, int per_block) { return (unsigned)((n + per_block - 1) / per_block); }
-static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 extern "C" {
 
@@ -271,11 +269,11 @@ int xq_env_observe_device(xq_env_t h, void* planes_dev, int dtype, int view, int
     EnvInfo E;
     if (int rc = env_info(h, &E)) return rc;
     if (dtype < XQ_DTYPE_F32 || dtype > XQ_DTYPE_U8) return fail(XQ_ERR_INVALID, "xq_env_observe_device: dtype %d", dtype);
-    if (view != XQ_VIEW_ABSOLUTE && view != XQ_VIEW_SIDE_TO_MOVE) return fail(XQ_ERR_INVALID, "xq_env_observe_device: view %d", view);
-    if (!aligned16(planes_dev) || (reinterpret_cast<uintptr_t>(aux_dev) & 15u)) return fail(XQ_ERR_INVALID, "xq_env_observe_device: planes and aux must be 16-byte aligned");
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_env_observe_device: view %d", view);
+    if (!aligned16(planes_dev) || !aligned16(aux_dev)) return fail(XQ_ERR_INVALID, "xq_env_observe_device: planes and aux must be 16-byte aligned");
     XQ_CUDA(cudaSetDevice(E.device));
     uint8_t* p = static_cast<uint8_t*>(planes_dev);
-    const unsigned grid = policy_grid(E.n, kObsBoards);
+    const unsigned grid = grid_of(E.n, kObsBoards);
     if (dtype == XQ_DTYPE_F32) observe_kernel<XQ_DTYPE_F32><<<grid, kObsThreads, 0, E.stream>>>(E.d_envs, E.n, p, view, aux_dev);
     else if (dtype == XQ_DTYPE_BF16) observe_kernel<XQ_DTYPE_BF16><<<grid, kObsThreads, 0, E.stream>>>(E.d_envs, E.n, p, view, aux_dev);
     else observe_kernel<XQ_DTYPE_U8><<<grid, kObsThreads, 0, E.stream>>>(E.d_envs, E.n, p, view, aux_dev);
@@ -287,14 +285,14 @@ int xq_env_legal_mask_device(xq_env_t h, void* mask_dev, int packed, int view) {
     EnvInfo E;
     if (int rc = env_info(h, &E)) return rc;
     if (!mask_dev || !aligned16(mask_dev)) return fail(XQ_ERR_INVALID, "xq_env_legal_mask_device: the mask must be a 16-byte aligned device buffer");
-    if (view != XQ_VIEW_ABSOLUTE && view != XQ_VIEW_SIDE_TO_MOVE) return fail(XQ_ERR_INVALID, "xq_env_legal_mask_device: view %d", view);
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_env_legal_mask_device: view %d", view);
     XQ_CUDA(cudaSetDevice(E.device));
     uint8_t* out = static_cast<uint8_t*>(mask_dev);
-    if (packed) mask_lane_kernel<false><<<policy_grid(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(E.d_envs, E.n, out, view, E.d_nonstd);
-    else mask_lane_kernel<true><<<policy_grid(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(E.d_envs, E.n, out, view, E.d_nonstd);
+    if (packed) mask_lane_kernel<false><<<grid_of(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(E.d_envs, E.n, out, view, E.d_nonstd);
+    else mask_lane_kernel<true><<<grid_of(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(E.d_envs, E.n, out, view, E.d_nonstd);
     XQ_LAUNCH_CHECK();
     if (E.maybe_nonstd) {      // injected boards (xq_env_set_boards) may have a piece set or a player byte the generator does not take
-        mask_generic_kernel<<<policy_grid(E.n, kThreads), kThreads, 0, E.stream>>>(E.d_envs, E.n, out, packed ? 1 : 0, view, E.d_nonstd);
+        mask_generic_kernel<<<grid_of(E.n, kThreads), kThreads, 0, E.stream>>>(E.d_envs, E.n, out, packed ? 1 : 0, view, E.d_nonstd);
         XQ_LAUNCH_CHECK();
     }
     return XQ_OK;
@@ -306,7 +304,7 @@ int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dty
     EnvInfo E;
     if (int rc = env_info(h, &E)) return rc;
     if (pick < XQ_PICK_GREEDY || pick > XQ_PICK_GIVEN) return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: pick %d", pick);
-    if (view != XQ_VIEW_ABSOLUTE && view != XQ_VIEW_SIDE_TO_MOVE) return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: view %d", view);
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: view %d", view);
     if (scores_dev && scores_dtype != XQ_DTYPE_F32 && scores_dtype != XQ_DTYPE_BF16)
         return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: scores_dtype %d (f32 or bf16)", scores_dtype);
     if (pick != XQ_PICK_GIVEN && !scores_dev) return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: GREEDY and SAMPLE need scores");
@@ -317,12 +315,12 @@ int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dty
     const PolicyArgs a{E.d_envs, E.n, E.env_id0, E.seed, scores_dev, pick, temperature, view, auto_reset,
                        actions_dev, logp_dev, reward_dev, done_dev, winner_dev, captured_dev, valid_dev};
     const bool bf16 = scores_dev && scores_dtype == XQ_DTYPE_BF16;
-    if (bf16) policy_step_lane_kernel<XQ_DTYPE_BF16><<<policy_grid(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(a, E.d_nonstd);
-    else policy_step_lane_kernel<XQ_DTYPE_F32><<<policy_grid(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(a, E.d_nonstd);
+    if (bf16) policy_step_lane_kernel<XQ_DTYPE_BF16><<<grid_of(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(a, E.d_nonstd);
+    else policy_step_lane_kernel<XQ_DTYPE_F32><<<grid_of(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(a, E.d_nonstd);
     XQ_LAUNCH_CHECK();
     if (E.maybe_nonstd) {
-        if (bf16) policy_step_generic_kernel<XQ_DTYPE_BF16><<<policy_grid(E.n, kThreads), kThreads, 0, E.stream>>>(a, E.d_nonstd);
-        else policy_step_generic_kernel<XQ_DTYPE_F32><<<policy_grid(E.n, kThreads), kThreads, 0, E.stream>>>(a, E.d_nonstd);
+        if (bf16) policy_step_generic_kernel<XQ_DTYPE_BF16><<<grid_of(E.n, kThreads), kThreads, 0, E.stream>>>(a, E.d_nonstd);
+        else policy_step_generic_kernel<XQ_DTYPE_F32><<<grid_of(E.n, kThreads), kThreads, 0, E.stream>>>(a, E.d_nonstd);
         XQ_LAUNCH_CHECK();
     }
     return XQ_OK;

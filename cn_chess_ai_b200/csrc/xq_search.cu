@@ -260,6 +260,17 @@ __device__ __forceinline__ void search_make_child(const SearchDev& d, int64_t t,
     d.count[t] = nw + 1;
 }
 
+// the warp's best edge by search_better from each lane's best (bs, bk; bk = -1: none), on every lane
+__device__ __forceinline__ int search_best_warp(float bs, int bk) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        const float os = __shfl_xor_sync(0xFFFFFFFFu, bs, off);
+        const int ok = __shfl_xor_sync(0xFFFFFFFFu, bk, off);
+        if (ok >= 0 && search_better(os, ok, bs, bk)) { bs = os; bk = ok; }
+    }
+    return __shfl_sync(0xFFFFFFFFu, bk, 0);
+}
+
 __global__ void __launch_bounds__(32 * kSelWarps) search_select_kernel(SearchDev d, float c_puct, float fpu, uint8_t* __restrict__ status,
                                                                       uint8_t* __restrict__ winner, int32_t* __restrict__ reward,
                                                                       int32_t* __restrict__ depth) {
@@ -281,13 +292,7 @@ __global__ void __launch_bounds__(32 * kSelWarps) search_select_kernel(SearchDev
             const float v = search_puct(d.P[eb + k], d.N[eb + k], d.W[eb + k], c_puct, fpu, sq);
             if (search_better(v, k, bs, bk)) { bs = v; bk = k; }
         }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            const float os = __shfl_xor_sync(0xFFFFFFFFu, bs, off);
-            const int ok = __shfl_xor_sync(0xFFFFFFFFu, bk, off);
-            if (ok >= 0 && search_better(os, ok, bs, bk)) { bs = os; bk = ok; }
-        }
-        bk = __shfl_sync(0xFFFFFFFFu, bk, 0);
+        bk = search_best_warp(bs, bk);
         const int child = d.child[eb + bk];
         if (child >= 0) { node = child; continue; }
         const int nw = d.count[t];
@@ -415,13 +420,7 @@ __device__ __forceinline__ int gumbel_pick_warp(const float* sc, const int32_t* 
 #pragma unroll
     for (int i = 0; i < kGumbelSlots; ++i)
         if (cnt[i] == want && search_better(sc[lane + 32 * i], lane + 32 * i, bs, bk)) { bs = sc[lane + 32 * i]; bk = lane + 32 * i; }
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-        const float os = __shfl_xor_sync(0xFFFFFFFFu, bs, off);
-        const int ok = __shfl_xor_sync(0xFFFFFFFFu, bk, off);
-        if (ok >= 0 && search_better(os, ok, bs, bk)) { bs = os; bk = ok; }
-    }
-    return __shfl_sync(0xFFFFFFFFu, bk, 0);
+    return search_best_warp(bs, bk);
 }
 
 // the action (gumbel_action): the considered edge with the most visits this move, then the larger score, then the smaller index; -1 none
@@ -515,13 +514,7 @@ __global__ void __launch_bounds__(32 * kSelLeavesWarps, std::is_same<ROOT, Gumbe
                     const float v = search_puct_vl(d.P[eb + e], d.N[eb + e], d.W[eb + e], s_cnt[warp][e], vl, c_puct, fpu, sq);
                     if (search_better(v, e, bs, bk)) { bs = v; bk = e; }
                 }
-#pragma unroll
-                for (int off = 16; off > 0; off >>= 1) {
-                    const float os = __shfl_xor_sync(0xFFFFFFFFu, bs, off);
-                    const int ok = __shfl_xor_sync(0xFFFFFFFFu, bk, off);
-                    if (ok >= 0 && search_better(os, ok, bs, bk)) { bs = os; bk = ok; }
-                }
-                bk = __shfl_sync(0xFFFFFFFFu, bk, 0);
+                bk = search_best_warp(bs, bk);
             }
             __syncwarp();
             if (alive) {
@@ -704,6 +697,20 @@ __global__ void __launch_bounds__(kThreads) search_expand_generic_slots_kernel(S
     search_expand_generic<SDT>(d, a, i / L, i, d.leaf[i], s_board + threadIdx.x);
 }
 
+// The dense 8,100-entry row of a root (one CTA of kRootThreads per tree): root_row_zero clears the shared row with 16-byte stores, the
+// kernel scatters the root's edges into it at their view-flipped action indices, root_row_store streams it out with 16-byte stores.
+template <class T>
+__device__ __forceinline__ void root_row_zero(T* row) {
+    for (int i = threadIdx.x; i < XQ_POLICY_ACTIONS / 4; i += kRootThreads) reinterpret_cast<uint4*>(row)[i] = make_uint4(0u, 0u, 0u, 0u);
+    __syncthreads();
+}
+
+template <class T>
+__device__ __forceinline__ void root_row_store(const T* row, T* dst) {
+    __syncthreads();
+    for (int i = threadIdx.x; i < XQ_POLICY_ACTIONS / 4; i += kRootThreads) reinterpret_cast<uint4*>(dst)[i] = reinterpret_cast<const uint4*>(row)[i];
+}
+
 __global__ void __launch_bounds__(kRootThreads) search_root_kernel(SearchDev d, int view, int32_t* __restrict__ visits, float* __restrict__ q,
                                                                   int64_t* __restrict__ best) {
     __shared__ __align__(16) int32_t s_v[XQ_POLICY_ACTIONS];
@@ -712,12 +719,9 @@ __global__ void __launch_bounds__(kRootThreads) search_root_kernel(SearchDev d, 
     const int ne = d.expanded[g] ? d.nedges[g] : 0;
     const bool flip = policy_flip(d.rec[g].player, view);
     if (visits) {
-        for (int i = tid; i < XQ_POLICY_ACTIONS / 4; i += kRootThreads) reinterpret_cast<int4*>(s_v)[i] = make_int4(0, 0, 0, 0);
-        __syncthreads();
+        root_row_zero(s_v);
         for (int k = tid; k < ne; k += kRootThreads) { const int ai = d.act[eb + k]; s_v[flip ? XQ_POLICY_ACTIONS - 1 - ai : ai] = d.N[eb + k]; }
-        __syncthreads();
-        int4* dst = reinterpret_cast<int4*>(visits + t * XQ_POLICY_ACTIONS);
-        for (int i = tid; i < XQ_POLICY_ACTIONS / 4; i += kRootThreads) dst[i] = reinterpret_cast<const int4*>(s_v)[i];
+        root_row_store(s_v, visits + t * XQ_POLICY_ACTIONS);
     }
     if (tid == 0) {
         // sums in list order; the most-visited edge, first in list order, none while no edge is visited
@@ -750,6 +754,17 @@ struct PlayArgs {
     int64_t* actions; int32_t* reward; uint8_t *done, *winner, *captured, *valid;
 };
 
+// env t steps with action act[kp] of its root's edges (kp < 0: no action) exactly as xq_env_policy_step_device (GIVEN) steps, one thread
+// (sb a 12-word shared board)
+__device__ __forceinline__ void search_play_step(const PlayArgs& a, int64_t t, const int16_t* act, int kp, uint32_t* sb) {
+    SmemBoard b{sb, 1};
+    b.load(a.envs + t);
+    Meta m; m.load(a.envs + t);
+    const int ai = kp >= 0 ? act[kp] : 0, from = ai / 90, to = ai % 90;
+    if (a.actions) a.actions[t] = kp >= 0 ? policy_index(from, to, policy_flip(m.player, a.view)) : -1;
+    policy_apply(b, m, a.envs, t, kp >= 0, from, to, a.auto_reset, a.reward, a.done, a.winner, a.captured, a.valid);
+}
+
 __global__ void __launch_bounds__(32 * kPlayWarps) search_play_kernel(SearchDev d, PlayArgs a) {
     __shared__ uint32_t s_b[kPlayWarps][12];
     __shared__ float s_w[kPlayWarps][kSearchEdges];
@@ -757,12 +772,7 @@ __global__ void __launch_bounds__(32 * kPlayWarps) search_play_kernel(SearchDev 
     const int64_t t = (int64_t)blockIdx.x * kPlayWarps + warp;
     if (t >= d.n) return;
     const int64_t g0 = t * d.cap, eb0 = g0 * kSearchEdges;
-    bool diff = false;
-    if (lane < 4) {
-        const uint4 rv = reinterpret_cast<const uint4*>(d.rec + g0)[lane], ev = reinterpret_cast<const uint4*>(a.envs + t)[lane];
-        diff = rv.x != ev.x || rv.y != ev.y || rv.z != ev.z || rv.w != ev.w;
-    }
-    const bool stale = __any_sync(0xFFFFFFFFu, diff);
+    const bool stale = root_stale_warp(d.rec + g0, a.envs + t, lane);
     const int ne = !stale && d.expanded[g0] ? d.nedges[g0] : 0;
     int nv[kSearchEdges / 32];
     int nmax = 0;
@@ -791,13 +801,7 @@ __global__ void __launch_bounds__(32 * kPlayWarps) search_play_kernel(SearchDev 
             if (lane == 0) kp = search_play_sample([&](int k) { return s_w[warp][k]; }, ne, policy_uniform(rng(a.seed, a.env_id0 + (uint64_t)t, root.ctr)));
         }
     }
-    if (lane != 0) return;
-    SmemBoard b{s_b[warp], 1};
-    b.load(a.envs + t);
-    Meta m; m.load(a.envs + t);
-    const int ai = kp >= 0 ? d.act[eb0 + kp] : 0, from = ai / 90, to = ai % 90;
-    if (a.actions) a.actions[t] = kp >= 0 ? policy_index(from, to, policy_flip(m.player, a.view)) : -1;
-    policy_apply(b, m, a.envs, t, kp >= 0, from, to, a.auto_reset, a.reward, a.done, a.winner, a.captured, a.valid);
+    if (lane == 0) search_play_step(a, t, d.act + eb0, kp, s_b[warp]);
 }
 
 // Dirichlet(alpha) noise mixed into the priors of every expanded root with at least one edge (xq_search_root_noise_device), one warp per
@@ -921,10 +925,7 @@ __global__ void __launch_bounds__(kRootThreads) gumbel_root_kernel(SearchDev d, 
     const int tid = threadIdx.x, lane = tid & 31;
     const int64_t t = blockIdx.x, g = t * d.cap, eb = g * kSearchEdges;
     const bool flip = policy_flip(d.rec[g].player, view);
-    if (policy) {
-        for (int i = tid; i < XQ_POLICY_ACTIONS / 4; i += kRootThreads) reinterpret_cast<float4*>(s_p)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-        __syncthreads();
-    }
+    if (policy) root_row_zero(s_p);
     if (tid < 32) {
         GumbelRoot r;
         gumbel_root_warp(d, G, t, lane, s_scr[0], s_scr[1], r);
@@ -943,11 +944,7 @@ __global__ void __launch_bounds__(kRootThreads) gumbel_root_kernel(SearchDev d, 
             action[t] = kp < 0 ? -1 : (flip ? XQ_POLICY_ACTIONS - 1 - ai : ai);
         }
     }
-    if (policy) {
-        __syncthreads();
-        float4* dst = reinterpret_cast<float4*>(policy + t * XQ_POLICY_ACTIONS);
-        for (int i = tid; i < XQ_POLICY_ACTIONS / 4; i += kRootThreads) dst[i] = reinterpret_cast<const float4*>(s_p)[i];
-    }
+    if (policy) root_row_store(s_p, policy + t * XQ_POLICY_ACTIONS);
 }
 
 __global__ void __launch_bounds__(32 * kGumbelWarps) gumbel_play_kernel(SearchDev d, GumbelDev G, PlayArgs a) {
@@ -957,25 +954,14 @@ __global__ void __launch_bounds__(32 * kGumbelWarps) gumbel_play_kernel(SearchDe
     const int64_t t = (int64_t)blockIdx.x * kGumbelWarps + warp;
     if (t >= d.n) return;
     const int64_t g0 = t * d.cap, eb0 = g0 * kSearchEdges;
-    bool diff = false;
-    if (lane < 4) {
-        const uint4 rv = reinterpret_cast<const uint4*>(d.rec + g0)[lane], ev = reinterpret_cast<const uint4*>(a.envs + t)[lane];
-        diff = rv.x != ev.x || rv.y != ev.y || rv.z != ev.z || rv.w != ev.w;
-    }
-    const bool stale = __any_sync(0xFFFFFFFFu, diff);
+    const bool stale = root_stale_warp(d.rec + g0, a.envs + t, lane);
     int kp = -1;
     if (!stale) {
         GumbelRoot r;
         gumbel_root_warp(d, G, t, lane, s_scr[warp][0], s_scr[warp][1], r);
         kp = gumbel_action_warp(r, lane);
     }
-    if (lane != 0) return;
-    SmemBoard b{s_b[warp], 1};
-    b.load(a.envs + t);
-    Meta m; m.load(a.envs + t);
-    const int ai = kp >= 0 ? d.act[eb0 + kp] : 0, from = ai / 90, to = ai % 90;
-    if (a.actions) a.actions[t] = kp >= 0 ? policy_index(from, to, policy_flip(m.player, a.view)) : -1;
-    policy_apply(b, m, a.envs, t, kp >= 0, from, to, a.auto_reset, a.reward, a.done, a.winner, a.captured, a.valid);
+    if (lane == 0) search_play_step(a, t, d.act + eb0, kp, s_b[warp]);
 }
 
 __global__ void __launch_bounds__(32 * kGumbelWarps) gumbel_weights_kernel(SearchDev d, GumbelDev G) {
@@ -1022,24 +1008,68 @@ constexpr size_t kSlotBytes = sizeof(xq_env_rec) + 4 + 1;                       
 constexpr size_t kTreeBytes = 4 + kSlotBytes;                                                  // node count and one slot
 static_assert(kNodeBytes == 85 && kEdgeBytes == 18 && kSlotBytes == 69, "include/xq.h documents these sizes");
 
-inline unsigned grid_of(int64_t n, int per_block) { return (unsigned)((n + per_block - 1) / per_block); }
-
 int enter(xq_search_t s, EnvInfo* E, const char* fn) {
     if (!s) return fail(XQ_ERR_INVALID, "%s: null handle", fn);
     if (int rc = env_info(s->env, E)) return rc;
     XQ_CUDA(cudaSetDevice(E->device));
     return XQ_OK;
 }
-bool valid_view(int v) { return v == XQ_VIEW_ABSOLUTE || v == XQ_VIEW_SIDE_TO_MOVE; }
+
+// The call order, as entry point fn needs it: kReset, a reset since create; kReady, also no selection pending (the last one was expanded
+// and backed up); kSelected, a selection pending.
+enum Need { kReset, kReady, kSelected };
+int check_phase(const xq_search_s* s, const char* fn, Need need) {
+    if (need == kSelected) return s->phase == 2 ? XQ_OK : fail(XQ_ERR_STATE, "%s: no selection since the last expand_backup / reset", fn);
+    if (s->phase == 0) return fail(XQ_ERR_STATE, "%s: the search was never reset (xq_search_reset)", fn);
+    if (need == kReady && s->phase == 2) return fail(XQ_ERR_STATE, "%s: the last selection was not expanded and backed up", fn);
+    return XQ_OK;
+}
+
+// the slab of a search of n trees of cap nodes with max_leaves slots per tree (Slab); returns its bytes
+size_t search_slab(SearchDev& d, void* base, int64_t n, int64_t cap, int max_leaves) {
+    const int64_t nodes = n * cap, edges = nodes * kSearchEdges, slots = n * max_leaves;
+    Slab b{static_cast<char*>(base)};
+    d.rec = b.take<xq_env_rec>(nodes);
+    d.parent = b.take<int32_t>(nodes); d.visits = b.take<int32_t>(nodes); d.reward = b.take<int32_t>(nodes); d.depth = b.take<int32_t>(nodes);
+    d.pedge = b.take<uint8_t>(nodes); d.nedges = b.take<uint8_t>(nodes); d.expanded = b.take<uint8_t>(nodes); d.term = b.take<uint8_t>(nodes);
+    d.winner = b.take<uint8_t>(nodes);
+    d.P = b.take<float>(edges); d.N = b.take<int32_t>(edges); d.W = b.take<float>(edges); d.child = b.take<int32_t>(edges);
+    d.act = b.take<int16_t>(edges);
+    d.count = b.take<int32_t>(n); d.leaf = b.take<int32_t>(slots); d.leaf_rec = b.take<xq_env_rec>(slots); d.nonstd = b.take<uint8_t>(slots);
+    return b.bytes;
+}
+
+// The expansion and backup of the L slots per tree of the leaf buffer (for the Gumbel begin, `roots`, of every unexpanded root, L = 1),
+// then the generic kernel for the boards the generator refused.  One leaf per tree has its own kernels: the slots kernels at L = 1 are
+// measurably slower.
+template <int SDT>
+int launch_expand(const xq_search_s* s, cudaStream_t stream, const ExpandArgs& a, int L, bool roots) {
+    const int64_t n = s->d.n;
+    if (roots) gumbel_expand_root_kernel<SDT><<<grid_of(n, kExpBoards), kExpBoards, 0, stream>>>(s->d, a);
+    else if (L == 1) search_expand_lane_kernel<SDT><<<grid_of(n, kExpBoards), kExpBoards, 0, stream>>>(s->d, a);
+    else search_expand_slots_kernel<SDT><<<grid_of(n * L, kExpBoards), kExpBoards, 0, stream>>>(s->d, a, L);
+    XQ_LAUNCH_CHECK();
+    if (s->maybe_nonstd) {
+        if (L == 1) search_expand_generic_kernel<SDT><<<grid_of(n, kThreads), kThreads, 0, stream>>>(s->d, a);
+        else search_expand_generic_slots_kernel<SDT><<<grid_of(n * L, kThreads), kThreads, 0, stream>>>(s->d, a, L);
+        XQ_LAUNCH_CHECK();
+    }
+    return XQ_OK;
+}
+int launch_expand(const xq_search_s* s, cudaStream_t stream, const ExpandArgs& a, int scores_dtype, int L, bool roots) {
+    return scores_dtype == XQ_DTYPE_BF16 ? launch_expand<XQ_DTYPE_BF16>(s, stream, a, L, roots) : launch_expand<XQ_DTYPE_F32>(s, stream, a, L, roots);
+}
 }  // namespace
 
 static int select_leaves(xq_search_t s, int leaves, float c_puct, float fpu, float virtual_loss, uint8_t* status_dev, uint8_t* winner_dev,
                          int32_t* reward_dev, int32_t* depth_dev, const GumbelDev* G);
 
-int xq::search_roots(xq_search_t s, SearchRoots* out) {
+int xq::search_roots(xq_search_t s, xq_env_t env, const char* fn, SearchRoots* out) {
     if (!s) return fail(XQ_ERR_INVALID, "null search handle");
+    if (s->env != env) return fail(XQ_ERR_INVALID, "%s: the search is on another env handle", fn);
+    if (int rc = check_phase(s, fn, kReady)) return rc;
     const SearchDev& d = s->d;
-    *out = SearchRoots{s->env, s->phase, d.n, d.cap, d.rec, d.nedges, d.expanded, d.N, d.W, d.act};
+    *out = SearchRoots{d.n, d.cap, d.rec, d.nedges, d.expanded, d.N, d.W, d.act};
     return XQ_OK;
 }
 
@@ -1058,31 +1088,15 @@ int xq_search_create_ex(xq_env_t env, int max_simulations, int max_leaves, xq_se
     xq_search_s* s = new (std::nothrow) xq_search_s();
     if (!s) return fail(XQ_ERR_NOMEM, "xq_search_create: out of host memory");
     s->env = env; s->device = E.device; s->max_sims = max_simulations; s->max_leaves = max_leaves;
-    const int64_t n = E.n, cap = (int64_t)max_simulations + 1, nodes = n * cap, edges = nodes * kSearchEdges, slots = n * max_leaves;
-    // one slab, every array 16-byte aligned
-    size_t off = 0;
-    auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-    const size_t o_rec = take(sizeof(xq_env_rec) * nodes), o_parent = take(4 * nodes), o_visits = take(4 * nodes), o_reward = take(4 * nodes),
-                 o_depth = take(4 * nodes), o_pedge = take(nodes), o_nedges = take(nodes), o_exp = take(nodes), o_term = take(nodes),
-                 o_win = take(nodes), o_P = take(4 * edges), o_N = take(4 * edges), o_W = take(4 * edges), o_child = take(4 * edges),
-                 o_act = take(2 * edges), o_count = take(4 * n), o_leaf = take(4 * slots), o_leafrec = take(sizeof(xq_env_rec) * slots), o_ns = take(slots);
-    if (cudaMalloc(&s->slab, off) != cudaSuccess) {
+    const int64_t n = E.n, cap = (int64_t)max_simulations + 1;
+    const size_t bytes = search_slab(s->d, nullptr, n, cap, max_leaves);
+    if (cudaMalloc(&s->slab, bytes) != cudaSuccess) {
         cudaGetLastError();
         delete s;
-        return fail(XQ_ERR_NOMEM, "xq_search_create: %lld trees x %d simulations need %.1f GB of device memory", (long long)n, max_simulations, off / 1e9);
+        return fail(XQ_ERR_NOMEM, "xq_search_create: %lld trees x %d simulations need %.1f GB of device memory", (long long)n, max_simulations, bytes / 1e9);
     }
-    char* b = static_cast<char*>(s->slab);
-    SearchDev& d = s->d;
-    d.n = n; d.cap = (int)cap;
-    d.rec = reinterpret_cast<xq_env_rec*>(b + o_rec);
-    d.parent = reinterpret_cast<int32_t*>(b + o_parent); d.visits = reinterpret_cast<int32_t*>(b + o_visits);
-    d.reward = reinterpret_cast<int32_t*>(b + o_reward); d.depth = reinterpret_cast<int32_t*>(b + o_depth);
-    d.pedge = reinterpret_cast<uint8_t*>(b + o_pedge); d.nedges = reinterpret_cast<uint8_t*>(b + o_nedges);
-    d.expanded = reinterpret_cast<uint8_t*>(b + o_exp); d.term = reinterpret_cast<uint8_t*>(b + o_term); d.winner = reinterpret_cast<uint8_t*>(b + o_win);
-    d.P = reinterpret_cast<float*>(b + o_P); d.N = reinterpret_cast<int32_t*>(b + o_N); d.W = reinterpret_cast<float*>(b + o_W);
-    d.child = reinterpret_cast<int32_t*>(b + o_child); d.act = reinterpret_cast<int16_t*>(b + o_act);
-    d.count = reinterpret_cast<int32_t*>(b + o_count); d.leaf = reinterpret_cast<int32_t*>(b + o_leaf);
-    d.leaf_rec = reinterpret_cast<xq_env_rec*>(b + o_leafrec); d.nonstd = reinterpret_cast<uint8_t*>(b + o_ns);
+    search_slab(s->d, s->slab, n, cap, max_leaves);
+    s->d.n = n; s->d.cap = (int)cap;
     *out = s;
     return XQ_OK;
 }
@@ -1125,8 +1139,7 @@ int xq_search_advance(xq_search_t s, int min_free, const float* root_noise_dev, 
     if (min_free < 1 || min_free > s->max_sims) return fail(XQ_ERR_INVALID, "xq_search_advance: min_free %d (1 .. %d)", min_free, s->max_sims);
     if (!(noise_eps >= 0.f && noise_eps <= 1.f)) return fail(XQ_ERR_INVALID, "xq_search_advance: noise_eps must be in [0, 1]");
     if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_search_advance: view %d", view);
-    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_advance: the search was never reset (xq_search_reset)");
-    if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_search_advance: the last selection was not expanded and backed up");
+    if (int rc = check_phase(s, "xq_search_advance", kReady)) return rc;
     // per warp (tree) the membership bitmap and one prefix count per 32-node word: cap / 4 bytes
     const size_t smem = (size_t)kAdvWarps * 2 * 4 * (size_t)((s->d.cap + 31) / 32);
     if (smem > 48 * 1024) XQ_CUDA(cudaFuncSetAttribute(search_advance_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1162,8 +1175,7 @@ static int select_leaves(xq_search_t s, int leaves, float c_puct, float fpu, flo
     if (!(fpu >= -FLT_MAX && fpu <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_search_select_device: fpu must be finite");
     if (!(virtual_loss >= 0.f && virtual_loss <= FLT_MAX))
         return fail(XQ_ERR_INVALID, "xq_search_select_leaves_device: virtual_loss must be finite and >= 0");
-    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_select_device: the search was never reset (xq_search_reset)");
-    if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_search_select_device: the last selection was not expanded and backed up");
+    if (int rc = check_phase(s, "xq_search_select_device", kReady)) return rc;
     if (s->sims + leaves > s->max_sims)
         return fail(XQ_ERR_STATE, "xq_search_select_device: %d simulations since the reset, %d more pass the capacity %d", s->sims, leaves, s->max_sims);
     if (G)
@@ -1186,7 +1198,7 @@ extern "C" {
 
 int xq_search_leaves_device(xq_search_t s, void** leaf_recs_dev) {
     if (!s || !leaf_recs_dev) return fail(XQ_ERR_INVALID, "xq_search_leaves_device: null argument");
-    if (s->phase != 2) return fail(XQ_ERR_STATE, "xq_search_leaves_device: no selection since the last expand_backup / reset");
+    if (int rc = check_phase(s, "xq_search_leaves_device", kSelected)) return rc;
     *leaf_recs_dev = s->d.leaf_rec;
     return XQ_OK;
 }
@@ -1196,9 +1208,9 @@ int xq_search_observe_leaves_device(xq_search_t s, void* planes_dev, int dtype, 
     if (int rc = enter(s, &E, "xq_search_observe_leaves_device")) return rc;
     if (dtype < XQ_DTYPE_F32 || dtype > XQ_DTYPE_U8) return fail(XQ_ERR_INVALID, "xq_search_observe_leaves_device: dtype %d", dtype);
     if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_search_observe_leaves_device: view %d", view);
-    if ((reinterpret_cast<uintptr_t>(planes_dev) & 15u) || (reinterpret_cast<uintptr_t>(aux_dev) & 15u))
+    if (!aligned16(planes_dev) || !aligned16(aux_dev))
         return fail(XQ_ERR_INVALID, "xq_search_observe_leaves_device: planes and aux must be 16-byte aligned");
-    if (s->phase != 2) return fail(XQ_ERR_STATE, "xq_search_observe_leaves_device: no selection since the last expand_backup / reset");
+    if (int rc = check_phase(s, "xq_search_observe_leaves_device", kSelected)) return rc;
     XQ_CUDA(launch_observe(s->d.leaf_rec, s->d.n * s->leaves, planes_dev, dtype, view, aux_dev, E.stream));
     return XQ_OK;
 }
@@ -1213,31 +1225,9 @@ int xq_search_expand_backup_device(xq_search_t s, const void* scores_dev, int sc
     if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_search_expand_backup_device: view %d", view);
     if (!(temperature > 0.f && temperature <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_search_expand_backup_device: temperature must be finite and > 0");
     if (!(noise_eps >= 0.f && noise_eps <= 1.f)) return fail(XQ_ERR_INVALID, "xq_search_expand_backup_device: noise_eps must be in [0, 1]");
-    if (s->phase != 2) return fail(XQ_ERR_STATE, "xq_search_expand_backup_device: no selection since the last expand_backup / reset");
+    if (int rc = check_phase(s, "xq_search_expand_backup_device", kSelected)) return rc;
     const ExpandArgs a{scores_dev, temperature, view, values_dev, root_noise_dev, noise_eps};
-    const bool bf16 = scores_dtype == XQ_DTYPE_BF16;
-    const int L = s->leaves;
-    if (L > 1) {
-        const int64_t slots = s->d.n * L;
-        if (bf16) search_expand_slots_kernel<XQ_DTYPE_BF16><<<grid_of(slots, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a, L);
-        else search_expand_slots_kernel<XQ_DTYPE_F32><<<grid_of(slots, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a, L);
-        XQ_LAUNCH_CHECK();
-        if (s->maybe_nonstd) {
-            if (bf16) search_expand_generic_slots_kernel<XQ_DTYPE_BF16><<<grid_of(slots, kThreads), kThreads, 0, E.stream>>>(s->d, a, L);
-            else search_expand_generic_slots_kernel<XQ_DTYPE_F32><<<grid_of(slots, kThreads), kThreads, 0, E.stream>>>(s->d, a, L);
-            XQ_LAUNCH_CHECK();
-        }
-        s->phase = 1;
-        return XQ_OK;
-    }
-    if (bf16) search_expand_lane_kernel<XQ_DTYPE_BF16><<<grid_of(s->d.n, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a);
-    else search_expand_lane_kernel<XQ_DTYPE_F32><<<grid_of(s->d.n, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a);
-    XQ_LAUNCH_CHECK();
-    if (s->maybe_nonstd) {
-        if (bf16) search_expand_generic_kernel<XQ_DTYPE_BF16><<<grid_of(s->d.n, kThreads), kThreads, 0, E.stream>>>(s->d, a);
-        else search_expand_generic_kernel<XQ_DTYPE_F32><<<grid_of(s->d.n, kThreads), kThreads, 0, E.stream>>>(s->d, a);
-        XQ_LAUNCH_CHECK();
-    }
+    if (int rc = launch_expand(s, E.stream, a, scores_dtype, s->leaves, false)) return rc;
     s->phase = 1;
     return XQ_OK;
 }
@@ -1246,8 +1236,8 @@ int xq_search_root_device(xq_search_t s, int view, int32_t* visits_dev, float* q
     EnvInfo E;
     if (int rc = enter(s, &E, "xq_search_root_device")) return rc;
     if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_search_root_device: view %d", view);
-    if (reinterpret_cast<uintptr_t>(visits_dev) & 15u) return fail(XQ_ERR_INVALID, "xq_search_root_device: visits must be 16-byte aligned");
-    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_root_device: the search was never reset (xq_search_reset)");
+    if (!aligned16(visits_dev)) return fail(XQ_ERR_INVALID, "xq_search_root_device: visits must be 16-byte aligned");
+    if (int rc = check_phase(s, "xq_search_root_device", kReset)) return rc;
     search_root_kernel<<<(unsigned)s->d.n, kRootThreads, 0, E.stream>>>(s->d, view, visits_dev, q_dev, best_dev);
     XQ_LAUNCH_CHECK();
     return XQ_OK;
@@ -1260,8 +1250,7 @@ int xq_search_play_device(xq_search_t s, float temperature, int sample_plies, in
     if (!(temperature >= 0.f && temperature <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_search_play_device: temperature must be finite and >= 0");
     if (sample_plies < 0) return fail(XQ_ERR_INVALID, "xq_search_play_device: sample_plies %d < 0", sample_plies);
     if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_search_play_device: view %d", view);
-    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_play_device: the search was never reset (xq_search_reset)");
-    if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_search_play_device: the last selection was not expanded and backed up");
+    if (int rc = check_phase(s, "xq_search_play_device", kReady)) return rc;
     const PlayArgs a{E.d_envs, E.env_id0, E.seed, temperature, sample_plies, view, auto_reset,
                      actions_dev, reward_dev, done_dev, winner_dev, captured_dev, valid_dev};
     search_play_kernel<<<grid_of(s->d.n, kPlayWarps), 32 * kPlayWarps, 0, E.stream>>>(s->d, a);
@@ -1274,8 +1263,7 @@ int xq_search_root_noise_device(xq_search_t s, float alpha, float eps, uint64_t 
     if (int rc = enter(s, &E, "xq_search_root_noise_device")) return rc;
     if (!(alpha > 0.f && alpha <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_search_root_noise_device: alpha must be finite and > 0");
     if (!(eps >= 0.f && eps <= 1.f)) return fail(XQ_ERR_INVALID, "xq_search_root_noise_device: eps must be in [0, 1]");
-    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_root_noise_device: the search was never reset (xq_search_reset)");
-    if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_search_root_noise_device: the last selection was not expanded and backed up");
+    if (int rc = check_phase(s, "xq_search_root_noise_device", kReady)) return rc;
     search_noise_kernel<<<grid_of(s->d.n, kPlayWarps), 32 * kPlayWarps, 0, E.stream>>>(s->d, alpha, eps, seed, E.env_id0, mask_dev, noise_out_dev);
     XQ_LAUNCH_CHECK();
     return XQ_OK;
@@ -1286,7 +1274,7 @@ int xq_search_get_tree(xq_search_t s, int64_t tree, xq_search_node* nodes_host, 
     if (int rc = enter(s, &E, "xq_search_get_tree")) return rc;
     if (tree < 0 || tree >= s->d.n) return fail(XQ_ERR_INVALID, "xq_search_get_tree: tree %lld of %lld", (long long)tree, (long long)s->d.n);
     if (!nodes_host || !n_nodes) return fail(XQ_ERR_INVALID, "xq_search_get_tree: nodes and n_nodes are required");
-    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_search_get_tree: the search was never reset (xq_search_reset)");
+    if (int rc = check_phase(s, "xq_search_get_tree", kReset)) return rc;
     const SearchDev& d = s->d;
     const int64_t cap = d.cap, g0 = tree * cap;
     int32_t cnt = 0;
@@ -1350,14 +1338,13 @@ namespace {
 constexpr size_t kGumbelTreeBytes = 4 * kSearchEdges * 4 + 4 * 4 + 4 + 4;      // g, logit, N0, weights; the bitmap, v, m
 static_assert(kGumbelTreeBytes == 2072, "include/xq.h documents 2,072 B per tree");
 
-// the slab of xq_gumbel_create: its seven arrays, each 256-byte aligned (offsets o[0 .. 6]); returns the total
-size_t gumbel_slab(int64_t n, size_t* o) {
-    const int64_t edges = n * kSearchEdges;
-    const size_t sizes[7] = {(size_t)(4 * edges), (size_t)(4 * edges), (size_t)(4 * edges), (size_t)(4 * edges), (size_t)(16 * n), (size_t)(4 * n),
-                             (size_t)(4 * n)};
-    size_t off = 0;
-    for (int i = 0; i < 7; ++i) { o[i] = off; off += (sizes[i] + 255) & ~(size_t)255; }
-    return off;
+// the slab of the Gumbel state of n trees (Slab); returns its bytes
+size_t gumbel_slab(GumbelDev& G, void* base, int64_t n) {
+    const size_t edges = (size_t)n * kSearchEdges;
+    Slab b{static_cast<char*>(base)};
+    G.g = b.take<float>(edges); G.logit = b.take<float>(edges); G.n0 = b.take<int32_t>(edges); G.w = b.take<uint32_t>(edges);
+    G.cons = b.take<uint32_t>(4 * (size_t)n); G.vhat = b.take<float>(n); G.m = b.take<int32_t>(n);
+    return b.bytes;
 }
 
 // the state is current: begun on the search's present roots (no reset / advance since)
@@ -1374,19 +1361,19 @@ int xq::gumbel_weights(xq_gumbel_t g, xq_env_t env, SearchRoots* roots, const ui
     if (!g) return fail(XQ_ERR_INVALID, "xq_examples_record_gumbel_device: null Gumbel state");
     if (g->s->env != env) return fail(XQ_ERR_INVALID, "xq_examples_record_gumbel_device: the search is on another env handle");
     if (int rc = gumbel_ready(g, &E, "xq_examples_record_gumbel_device")) return rc;
-    if (g->s->phase == 2) return fail(XQ_ERR_STATE, "xq_examples_record_gumbel_device: the last selection was not expanded and backed up");
+    if (int rc = search_roots(g->s, env, "xq_examples_record_gumbel_device", roots)) return rc;
     gumbel_weights_kernel<<<grid_of(g->s->d.n, kGumbelWarps), 32 * kGumbelWarps, 0, E.stream>>>(g->s->d, g->G);
     XQ_LAUNCH_CHECK();
     *w = g->G.w;
-    return search_roots(g->s, roots);
+    return XQ_OK;
 }
 
 extern "C" {
 
 int xq_gumbel_bytes(int64_t n_trees, int max_simulations, int64_t* bytes) {
     if (!bytes || n_trees < 1 || max_simulations < 1 || max_simulations > (1 << 24)) return fail(XQ_ERR_INVALID, "xq_gumbel_bytes: bad arguments");
-    size_t o[7];
-    *bytes = (int64_t)gumbel_slab(n_trees, o);
+    GumbelDev G;
+    *bytes = (int64_t)gumbel_slab(G, nullptr, n_trees);
     return XQ_OK;
 }
 
@@ -1400,18 +1387,13 @@ int xq_gumbel_create(xq_search_t s, int max_considered, xq_gumbel_t* out) {
     if (!g) return fail(XQ_ERR_NOMEM, "xq_gumbel_create: out of host memory");
     g->s = s; g->device = E.device; g->max_considered = max_considered;
     const int64_t n = s->d.n;
-    size_t o[7];
-    const size_t off = gumbel_slab(n, o);
-    if (cudaMalloc(&g->slab, off) != cudaSuccess) {
+    const size_t bytes = gumbel_slab(g->G, nullptr, n);
+    if (cudaMalloc(&g->slab, bytes) != cudaSuccess) {
         cudaGetLastError();
         delete g;
-        return fail(XQ_ERR_NOMEM, "xq_gumbel_create: %lld trees need %.2f GB of device memory", (long long)n, off / 1e9);
+        return fail(XQ_ERR_NOMEM, "xq_gumbel_create: %lld trees need %.2f GB of device memory", (long long)n, bytes / 1e9);
     }
-    char* b = static_cast<char*>(g->slab);
-    GumbelDev& G = g->G;
-    G.g = reinterpret_cast<float*>(b + o[0]); G.logit = reinterpret_cast<float*>(b + o[1]); G.n0 = reinterpret_cast<int32_t*>(b + o[2]);
-    G.w = reinterpret_cast<uint32_t*>(b + o[3]); G.cons = reinterpret_cast<uint32_t*>(b + o[4]); G.vhat = reinterpret_cast<float*>(b + o[5]);
-    G.m = reinterpret_cast<int32_t*>(b + o[6]);
+    gumbel_slab(g->G, g->slab, n);
     *out = g;
     return XQ_OK;
 }
@@ -1439,18 +1421,9 @@ int xq_gumbel_begin_device(xq_gumbel_t g, const void* scores_dev, int scores_dty
         return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: n_simulations %d (1 .. %d)", n_simulations, s->max_sims);
     if (!(c_visit >= 0.f && c_visit <= FLT_MAX) || !(c_scale >= 0.f && c_scale <= FLT_MAX))
         return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: c_visit and c_scale must be finite and >= 0");
-    if (s->phase == 0) return fail(XQ_ERR_STATE, "xq_gumbel_begin_device: the search was never reset (xq_search_reset)");
-    if (s->phase == 2) return fail(XQ_ERR_STATE, "xq_gumbel_begin_device: the last selection was not expanded and backed up");
+    if (int rc = check_phase(s, "xq_gumbel_begin_device", kReady)) return rc;
     const ExpandArgs a{scores_dev, temperature, view, root_value_dev, nullptr, 0.f};
-    const bool bf16 = scores_dtype == XQ_DTYPE_BF16;
-    if (bf16) gumbel_expand_root_kernel<XQ_DTYPE_BF16><<<grid_of(s->d.n, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a);
-    else gumbel_expand_root_kernel<XQ_DTYPE_F32><<<grid_of(s->d.n, kExpBoards), kExpBoards, 0, E.stream>>>(s->d, a);
-    XQ_LAUNCH_CHECK();
-    if (s->maybe_nonstd) {
-        if (bf16) search_expand_generic_kernel<XQ_DTYPE_BF16><<<grid_of(s->d.n, kThreads), kThreads, 0, E.stream>>>(s->d, a);
-        else search_expand_generic_kernel<XQ_DTYPE_F32><<<grid_of(s->d.n, kThreads), kThreads, 0, E.stream>>>(s->d, a);
-        XQ_LAUNCH_CHECK();
-    }
+    if (int rc = launch_expand(s, E.stream, a, scores_dtype, 1, true)) return rc;
     g->G.c_visit = c_visit; g->G.c_scale = c_scale; g->G.sims = 0; g->G.n_sims = n_simulations;
     gumbel_init_kernel<<<grid_of(s->d.n, kGumbelWarps), 32 * kGumbelWarps, 0, E.stream>>>(s->d, g->G, g->max_considered, seed, E.env_id0,
                                                                                          root_value_dev);
@@ -1477,8 +1450,8 @@ int xq_gumbel_root_device(xq_gumbel_t g, int view, float* policy_dev, int64_t* a
     EnvInfo E;
     if (int rc = gumbel_ready(g, &E, "xq_gumbel_root_device")) return rc;
     if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_gumbel_root_device: view %d", view);
-    if (reinterpret_cast<uintptr_t>(policy_dev) & 15u) return fail(XQ_ERR_INVALID, "xq_gumbel_root_device: policy must be 16-byte aligned");
-    if (g->s->phase == 2) return fail(XQ_ERR_STATE, "xq_gumbel_root_device: the last selection was not expanded and backed up");
+    if (!aligned16(policy_dev)) return fail(XQ_ERR_INVALID, "xq_gumbel_root_device: policy must be 16-byte aligned");
+    if (int rc = check_phase(g->s, "xq_gumbel_root_device", kReady)) return rc;
     gumbel_root_kernel<<<(unsigned)g->s->d.n, kRootThreads, 0, E.stream>>>(g->s->d, g->G, view, policy_dev, action_dev);
     XQ_LAUNCH_CHECK();
     return XQ_OK;
@@ -1489,7 +1462,7 @@ int xq_gumbel_play_device(xq_gumbel_t g, int view, int auto_reset, int64_t* acti
     EnvInfo E;
     if (int rc = gumbel_ready(g, &E, "xq_gumbel_play_device")) return rc;
     if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_gumbel_play_device: view %d", view);
-    if (g->s->phase == 2) return fail(XQ_ERR_STATE, "xq_gumbel_play_device: the last selection was not expanded and backed up");
+    if (int rc = check_phase(g->s, "xq_gumbel_play_device", kReady)) return rc;
     const PlayArgs a{E.d_envs, E.env_id0, E.seed, 0.f, 0, view, auto_reset, actions_dev, reward_dev, done_dev, winner_dev, captured_dev, valid_dev};
     gumbel_play_kernel<<<grid_of(g->s->d.n, kGumbelWarps), 32 * kGumbelWarps, 0, E.stream>>>(g->s->d, g->G, a);
     XQ_LAUNCH_CHECK();

@@ -189,7 +189,6 @@ static void free_scratch(void* p) {
     delete s;
 }
 
-static inline unsigned blocks(int64_t n, int per) { return (unsigned)((n + per - 1) / per); }
 static int reserve_scratch(xq_env_t env, int64_t n, SelfplayScratch** out) {
     void** slot = env_scratch_slot(env, free_scratch);
     if (!*slot) {
@@ -224,10 +223,10 @@ static int launch_act(bool apply, const EnvInfo& ei, const float* q90, uint32_t 
                             ei.d_events, ei.d_event_count, ei.event_cap, event_ply, ei.d_nonstd, carry, event_env0, ei.stream));
     if (ei.maybe_nonstd) {
         if (apply)
-            act_kernel<true><<<blocks(ei.n, kThreads), kThreads, 0, ei.stream>>>(ei.d_envs, ei.n, ei.env_id0, ei.seed, q90, thr, train_done, actions, ring, ring_cap,
+            act_kernel<true><<<grid_of(ei.n, kThreads), kThreads, 0, ei.stream>>>(ei.d_envs, ei.n, ei.env_id0, ei.seed, q90, thr, train_done, actions, ring, ring_cap,
                                                                                 ring_pos, stats, ei.d_events, ei.d_event_count, ei.event_cap, event_ply, ei.d_nonstd);
         else
-            act_kernel<false><<<blocks(ei.n, kThreads), kThreads, 0, ei.stream>>>(ei.d_envs, ei.n, ei.env_id0, ei.seed, q90, thr, train_done, actions, ring, ring_cap,
+            act_kernel<false><<<grid_of(ei.n, kThreads), kThreads, 0, ei.stream>>>(ei.d_envs, ei.n, ei.env_id0, ei.seed, q90, thr, train_done, actions, ring, ring_cap,
                                                                                  ring_pos, stats, ei.d_events, ei.d_event_count, ei.event_cap, event_ply, ei.d_nonstd);
         XQ_LAUNCH_CHECK();
     }
@@ -305,7 +304,7 @@ static int replay_sample_dev(xq_replay_t r, int64_t batch, uint64_t seed, uint32
         XQ_CUDA(cudaMalloc(&r->d_index, sizeof(int64_t) * batch));
         r->batch_cap = batch;
     }
-    sample_kernel<<<blocks(batch * 32, 256), 256, 0, stream>>>(r->d_ring, size, batch, seed, counter, r->d_batch, want_index ? r->d_index : nullptr);
+    sample_kernel<<<grid_of(batch * 32, 256), 256, 0, stream>>>(r->d_ring, size, batch, seed, counter, r->d_batch, want_index ? r->d_index : nullptr);
     XQ_LAUNCH_CHECK();
     return XQ_OK;
 }

@@ -61,24 +61,24 @@ class TorchSearch:
     def select(self, c_puct=1.5, fpu=0.0):
         """one leaf per tree: SelectResult of tensors [n]: status / winner uint8, reward / depth int32"""
         self.tenv._enter()
-        status, winner = (torch.empty(self.n, dtype=torch.uint8, device=self.device) for _ in range(2))
-        reward, depth = (torch.empty(self.n, dtype=torch.int32, device=self.device) for _ in range(2))
-        self.search.select_device(c_puct, fpu, status.data_ptr(), winner.data_ptr(), reward.data_ptr(), depth.data_ptr())
+        sel = self._select_outputs(self.n)
+        self.search.select_device(c_puct, fpu, *(t.data_ptr() for t in sel))
         self._rows = self.n
-        return SelectResult(status, winner, reward, depth)
+        return sel
 
     def select_leaves(self, leaves, c_puct=1.5, fpu=0.0, virtual_loss=1.0):
         """`leaves` leaves per tree in one call, descents in order with virtual loss (include/xq.h): SelectResult of tensors [n, leaves];
         status DUPLICATE (4) marks a slot that ended at the open leaf of an earlier slot.  leaves(), observe() and expand_backup() then
         take or return n * leaves rows, slot k of tree t at row t * leaves + k.  Spends `leaves` of the search's simulations."""
         self.tenv._enter()
-        shape = (self.n, int(leaves))
-        status, winner = (torch.empty(shape, dtype=torch.uint8, device=self.device) for _ in range(2))
-        reward, depth = (torch.empty(shape, dtype=torch.int32, device=self.device) for _ in range(2))
-        self.search.select_leaves_device(leaves, c_puct, fpu, virtual_loss, status.data_ptr(), winner.data_ptr(), reward.data_ptr(),
-                                         depth.data_ptr())
+        sel = self._select_outputs((self.n, int(leaves)))
+        self.search.select_leaves_device(leaves, c_puct, fpu, virtual_loss, *(t.data_ptr() for t in sel))
         self._rows = self.n * int(leaves)
-        return SelectResult(status, winner, reward, depth)
+        return sel
+
+    def _select_outputs(self, shape):
+        """the SelectResult tensors a select call fills: status / winner uint8, reward / depth int32 of `shape`"""
+        return SelectResult(*(torch.empty(shape, dtype=dt, device=self.device) for dt in (torch.uint8, torch.uint8, torch.int32, torch.int32)))
 
     def leaves(self):
         """the leaf records of the last selection as a uint8 [rows, 64] tensor aliasing the library's buffer (xq_env_rec each, rows = n
@@ -134,12 +134,14 @@ class TorchSearch:
         re-roots them at the played moves."""
         v = _view(view)
         self.tenv._enter()
-        actions = torch.empty(self.n, dtype=torch.int64, device=self.device)
-        reward = torch.empty(self.n, dtype=torch.int32, device=self.device)
-        done, winner, captured, valid = (torch.empty(self.n, dtype=torch.uint8, device=self.device) for _ in range(4))
-        self.search.play_device(temperature, sample_plies, v, auto_reset, actions.data_ptr(), reward.data_ptr(), done.data_ptr(),
-                                winner.data_ptr(), captured.data_ptr(), valid.data_ptr())
-        return StepResult(actions, None, reward, done, winner, captured, valid)
+        res = self._step_outputs()
+        self.search.play_device(temperature, sample_plies, v, auto_reset, *(t.data_ptr() for t in res if t is not None))
+        return res
+
+    def _step_outputs(self):
+        """the StepResult tensors [n] a play call fills: actions int64, logp None, reward int32, done / winner / captured / valid uint8"""
+        empty = lambda dt: torch.empty(self.n, dtype=dt, device=self.device)      # noqa: E731
+        return StepResult(empty(torch.int64), None, empty(torch.int32), *(empty(torch.uint8) for _ in range(4)))
 
     def root_noise(self, alpha, eps=0.25, seed=0, mask=None, want_noise=False):
         """Dirichlet(alpha) noise drawn by the library over the edges of every expanded root (or of the envs where mask, bool / uint8 [n],
@@ -188,14 +190,19 @@ class TorchSearch:
                 self.root_noise(dirichlet_alpha, dirichlet_eps, noise_seed, mask=None if kept is None else ~kept)
             k = 1 if i == 0 else min(leaves, n_simulations - i)
             sel = self.select(c_puct, fpu) if k == 1 else self.select_leaves(k, c_puct, fpu, virtual_loss)
-            status, winner = sel.status.reshape(-1), sel.winner.reshape(-1)
-            planes, aux = self.observe(obs_dtype, view)
-            scores, values = evaluate(planes)
-            values = values.reshape(self._rows).to(torch.float32).contiguous()
-            values = torch.where(status != NEEDS_EVALUATION, self.outcome_values(status, winner, aux, cap_value), values)
-            self.expand_backup(scores.contiguous(), values, temperature, root_noise, noise_eps, view)
+            self._simulate(sel, evaluate, temperature, root_noise, noise_eps, view, obs_dtype, cap_value)
             i += k
         return self.root(view)
+
+    def _simulate(self, sel, evaluate, temperature, root_noise, noise_eps, view, obs_dtype, cap_value):
+        """the rest of a simulation after the selection `sel`: its leaves observed and evaluated once, outcome_values at terminal leaves,
+        expand_backup"""
+        status, winner = sel.status.reshape(-1), sel.winner.reshape(-1)
+        planes, aux = self.observe(obs_dtype, view)
+        scores, values = evaluate(planes)
+        values = values.reshape(self._rows).to(torch.float32).contiguous()
+        values = torch.where(status != NEEDS_EVALUATION, self.outcome_values(status, winner, aux, cap_value), values)
+        self.expand_backup(scores.contiguous(), values, temperature, root_noise, noise_eps, view)
 
 
 GumbelRootResult = namedtuple("GumbelRootResult", "policy action")
@@ -235,12 +242,10 @@ class TorchGumbel:
         expand_backup() follow as after select_leaves"""
         ts = self.tsearch
         self.tenv._enter()
-        shape = (self.n, int(leaves))
-        status, winner = (torch.empty(shape, dtype=torch.uint8, device=self.device) for _ in range(2))
-        reward, depth = (torch.empty(shape, dtype=torch.int32, device=self.device) for _ in range(2))
-        self.gumbel.select_device(leaves, c_puct, fpu, virtual_loss, status.data_ptr(), winner.data_ptr(), reward.data_ptr(), depth.data_ptr())
+        sel = ts._select_outputs((self.n, int(leaves)))
+        self.gumbel.select_device(leaves, c_puct, fpu, virtual_loss, *(t.data_ptr() for t in sel))
         ts._rows = self.n * int(leaves)
-        return SelectResult(status, winner, reward, depth)
+        return sel
 
     def root(self, view="side"):
         """GumbelRootResult: policy f32 [n, 8100] (pi' in the frame of `view`, zero rows for roots without edges), action int64 [n] (the
@@ -256,12 +261,9 @@ class TorchGumbel:
         """root().action played on every env, as TorchSearch.play steps (a stale root or no action plays nothing): StepResult"""
         v = _view(view)
         self.tenv._enter()
-        actions = torch.empty(self.n, dtype=torch.int64, device=self.device)
-        reward = torch.empty(self.n, dtype=torch.int32, device=self.device)
-        done, winner, captured, valid = (torch.empty(self.n, dtype=torch.uint8, device=self.device) for _ in range(4))
-        self.gumbel.play_device(v, auto_reset, actions.data_ptr(), reward.data_ptr(), done.data_ptr(), winner.data_ptr(), captured.data_ptr(),
-                                valid.data_ptr())
-        return StepResult(actions, None, reward, done, winner, captured, valid)
+        res = self.tsearch._step_outputs()
+        self.gumbel.play_device(v, auto_reset, *(t.data_ptr() for t in res if t is not None))
+        return res
 
     def run(self, evaluate, n_simulations, seed=0, c_puct=1.5, fpu=0.0, temperature=1.0, c_visit=50.0, c_scale=0.1, view="side",
             obs_dtype=torch.bfloat16, cap_value=0.0, leaves=1, virtual_loss=1.0, reset=True):
@@ -278,12 +280,6 @@ class TorchGumbel:
         i = 0
         while i < n_simulations:
             k = min(leaves, n_simulations - i)
-            sel = self.select(k, c_puct, fpu, virtual_loss)
-            status, winner = sel.status.reshape(-1), sel.winner.reshape(-1)
-            planes, aux = ts.observe(obs_dtype, view)
-            scores, values = evaluate(planes)
-            values = values.reshape(ts._rows).to(torch.float32).contiguous()
-            values = torch.where(status != NEEDS_EVALUATION, ts.outcome_values(status, winner, aux, cap_value), values)
-            ts.expand_backup(scores.contiguous(), values, temperature, None, 0.0, view)
+            ts._simulate(self.select(k, c_puct, fpu, virtual_loss), evaluate, temperature, None, 0.0, view, obs_dtype, cap_value)
             i += k
         return self.root(view)
