@@ -1647,6 +1647,7 @@ int dqn_q90_device(xq_dqn_s* h, const xq_env_rec* envs_dev, int64_t n, float* q9
     if (n > f->act_cap) {
         cudaFree(f->actHhi); cudaFree(f->actHlo); cudaFree(f->actZ); cudaFree(f->actPrev);
         f->actHhi = f->actHlo = nullptr; f->actZ = nullptr; f->actPrev = nullptr; f->act_cap = 0; f->act_rows = 0; f->actz_version = 0;
+        f->act_sub_n = -1;      // the half-range maps of dqn_q90_half pointed into the freed buffers
         const int64_t rows = (n + BM - 1) / BM * BM;
         XQ_CUDA(cudaMalloc(&f->actHhi, sizeof(__nv_bfloat16) * rows * kHid)); XQ_CUDA(cudaMalloc(&f->actHlo, sizeof(__nv_bfloat16) * rows * kHid));
         XQ_CUDA(cudaMalloc(&f->actZ, sizeof(int32_t) * n * kHid)); XQ_CUDA(cudaMalloc(&f->actPrev, sizeof(uint32_t) * n * 12));

@@ -345,6 +345,8 @@ int xq_selfplay_collect(xq_dqn_t h, xq_env_t env, xq_replay_t r, int n_plies, do
     EnvInfo ei;
     if (int rc = env_info(env, &ei)) return rc;
     if (ei.device != h->device || (r && r->device != h->device)) return fail(XQ_ERR_INVALID, "xq_selfplay_collect: handles live on different devices");
+    // one ply writes slots ring_pos + env (mod capacity) from every env at once: a smaller ring would take several envs' records in one slot
+    if (r && r->capacity < ei.n) return fail(XQ_ERR_INVALID, "xq_selfplay_collect: the replay ring holds fewer transitions than one ply");
     XQ_CUDA(cudaSetDevice(h->device));
     { FastWeights fw; if (int rc = dqn_fast_weights(h, &fw)) return rc; }      // refresh the FP32 / BF16 copies on h->stream before ordering after it
     SelfplayScratch* sc;

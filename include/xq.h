@@ -512,7 +512,8 @@ int xq_examples_get(xq_examples_t b, int64_t first, int64_t n, xq_example* out_h
  *      (summation order and FMA contraction differ in the last ulps).
  *  (2) batched BF16 tensor-core path for the {1260,128,8100} self-play network, fed by packed boards:
  *      xq_dqn_forward_boards, xq_dqn_act, xq_dqn_td_update.  FP32 master weights, BF16 MMA operands, FP32
- *      accumulation.  Tolerance vs the FP64 oracle: |dQ| <= 2e-3 abs. */
+ *      accumulation.  Tolerance vs the FP64 oracle: |dQ| <= 2e-3 abs; xq_dqn_act and xq_selfplay_collect act on a
+ *      tighter Q(s)[0..95] (see xq_dqn_act). */
 typedef struct xq_dqn_s* xq_dqn_t;
 enum { XQ_DQN_AS_WRITTEN = 0, XQ_DQN_CORRECTED = 1 };   /* hidden-layer delta: src/dqn.cu:406-427 as written, or W^T.delta (SURVEY F7) */
 
@@ -616,12 +617,19 @@ int xq_replay_sample(xq_replay_t r, int64_t batch, uint64_t seed, uint32_t count
 
 /* DQN::selectAction for every env at once (src/dqn.cpp:24-56 over ChessAI::getAllValidActions): coin31/idx31 come from
  * xq_rng(seed, env_id, ctr); explore: list[idx31 % n]; exploit: FIRST action maximising Q(s)[action.to] (strict >).
- * Nothing is applied.  q_host (optional) [n][96]: Q(s)[0..89] as used for the choice. */
+ * Nothing is applied.  q_host (optional) [n][96]: Q(s)[0..89] as used for the choice.
+ * Q is computed from a fixed-point layer-0 sum (scale 2^k from max |W0|, |b0| per weight version) and a split-precision
+ * (BF16 hi + lo, FP32 accumulation) layer 1.  Every entry of Q(s)[0..95] stays within the per-entry error bound stated in
+ * tests/act_oracle.py of the FP64 network: (occupied squares + 1) x 2^-(k+1) per hidden unit from the rounding of the table,
+ * the FP32 weight copies, the SFU tanh, the hi + lo splits of h and W1 and the FP32 accumulation.  At the U(-0.05, 0.05)
+ * initialisation that bound is below 2e-5; it grows with the weights. */
 int xq_dqn_act(xq_dqn_t h, xq_env_t env, double eps, xq_action* actions_host, float* q_host);
 /* n_plies of epsilon-greedy self-play on every env, device-resident and asynchronous: per ply the body of ChessAI::train
  * (src/chessai.cpp:96-119) up to the transition (s, a, r, s', done), which is written to the replay ring (r may be NULL);
  * terminal envs restart.  train_done != 0: done = checkGameOver() || moveCount+1 >= 200 (train, :119), else checkGameOver()
- * (startSelfPlay, :227).  Env statistics accumulate in the env handle (xq_env_get_stats). */
+ * (startSelfPlay, :227).  Env statistics accumulate in the env handle (xq_env_get_stats).
+ * The ring must hold at least one ply (capacity >= n_envs): a smaller ring returns XQ_ERR_INVALID before anything is enqueued,
+ * and the ring, the boards and the statistics are left as they were. */
 int xq_selfplay_collect(xq_dqn_t h, xq_env_t env, xq_replay_t r, int n_plies, double eps, int train_done);
 /* sample `batch` transitions from the ring and run xq_dqn_td_update_device on them, all on the device */
 int xq_dqn_td_update_replay(xq_dqn_t h, xq_replay_t r, int64_t batch, uint64_t seed, uint32_t counter, int use_target_net, double lr,

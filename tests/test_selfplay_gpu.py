@@ -205,17 +205,43 @@ def test_two_stream_collector_plies(xq, O, oracle_lib):
     """At >= 4,096 envs per stream the collector cuts the env range in parts that run their [contraction -> act] chains on 2..4 streams
     (xq_selfplay_collect).  Same transitions, same finished-game events (with the env index of the whole range) and same final boards as
     the step-by-step path: GPU act (same Q, same draws) + oracle rules."""
+    two_stream_collect_vs_stepwise(xq, O, oracle_lib, 16500, 44, 16500 * 44)     # not a multiple of 128: the second half ends in partial tiles / CTAs
+
+
+def test_two_stream_collector_ring_wraps_inside_each_half(xq, O, oracle_lib):
+    """The same at 65,613 envs (513 tiles: several per CTA of the contraction, a partial last tile) with a ring of 3n + 40,000 transitions:
+    within 12 plies the ring wraps inside the first half at one ply and inside the second half at another, and it must hold what sequential
+    inserts of the plies would leave."""
+    two_stream_collect_vs_stepwise(xq, O, oracle_lib, 65613, 12, 3 * 65613 + 40000)
+
+
+def two_stream_collect_vs_stepwise(xq, O, oracle_lib, n, plies, capacity):
+    """One collect of `plies` plies over n envs into a ring of `capacity` against the step-by-step path; the expected ring is that of
+    sequential inserts.  Afterwards the Q the act kernels' carried sums give is checked against FP64 for every env (tests/act_oracle.py)."""
+    import act_oracle as AO
     from cn_chess_ai_b200.trainer import drain_game_events, enable_game_events
-    n, plies, seed, eps = 16500, 44, 17, 0.6            # not a multiple of 128: the second half ends in partial tiles / CTAs
+    seed, eps = 17, 0.6
     w, b = rand_params(31)
     net = xq.DQN(LAYERS); net.set_params(w, b)
     envA = xq.BatchedEnv(n, seed=seed, env_id0=1000)
-    rb = xq.ReplayBuffer(n * plies)
+    rb = xq.ReplayBuffer(capacity)
     enable_game_events(envA, n * plies)
     xq.collect(net, envA, rb, plies, eps, train_done=True)
     envA.sync()
     events, dropped = drain_game_events(envA)
-    ring = rb.get(0, n * plies).reshape(plies, n)
+    # sequential inserts: ply p writes slots (p n + env) % capacity; keep the last writer of each slot
+    slot = (np.arange(plies)[:, None] * n + np.arange(n)[None, :]) % capacity
+    owner = np.full(capacity, -1)
+    np.maximum.at(owner, slot.ravel(), np.arange(plies * n))
+    alive = (owner[slot] == np.arange(plies * n).reshape(plies, n))
+    half = ((n + 1) // 2 + 127) // 128 * 128
+    head = np.arange(plies) * n % capacity
+    wraps = capacity - head
+    if capacity < plies * n:
+        assert ((wraps > 0) & (wraps < half)).any() and ((wraps > half) & (wraps < n)).any()     # a wrap inside each half
+    ring_all = rb.get()
+    assert (ring_all[owner < 0].view(np.uint8) == 0).all()
+    ring = ring_all[slot]
     envB = xq.BatchedEnv(n, seed=seed, env_id0=1000)
     ref = O.new_envs(n)
     finished = []
@@ -224,9 +250,9 @@ def test_two_stream_collector_plies(xq, O, oracle_lib):
         before = ref.copy()
         r0 = np.zeros(n, np.int32); d0, w0, c0, v0 = (np.zeros(n, np.uint8) for _ in range(4))
         oracle_lib.xqo_batch_step(ref.ctypes.data, n, actions, r0, d0, w0, c0, v0)
-        t = ring[p]
-        assert (t["action"] == actions).all() and (t["reward"] == r0).all(), p
-        assert t["s"].tobytes() == before["sq"].tobytes() and t["s2"].tobytes() == ref["sq"].tobytes(), p
+        t, k = ring[p], alive[p]
+        assert (t["action"][k] == actions[k]).all() and (t["reward"][k] == r0[k]).all(), p
+        assert t["s"][k].tobytes() == before["sq"][k].tobytes() and t["s2"][k].tobytes() == ref["sq"][k].tobytes(), p
         for i in np.nonzero(d0)[0]:
             finished.append((p, int(i), int(ref[i]["red_score"]), int(ref[i]["black_score"])))
             oracle_lib.xqo_reset(ref[i:i + 1].ctypes.data)
@@ -234,6 +260,10 @@ def test_two_stream_collector_plies(xq, O, oracle_lib):
     assert envA.get_boards().tobytes() == ref.tobytes()
     assert dropped == 0 and len(finished) > 20
     assert [(int(e["ply"]), int(e["env"]), int(e["red_score"]), int(e["black_score"])) for e in events] == finished
+    _, q = xq.act(net, envA, 0.0, want_q=True)
+    q64, h = AO.forward(ref, w, b)
+    err = np.abs(q[:, :96] - q64)
+    assert (err <= AO.bound(ref, w, b, h)).all(), err.max()
 
 
 def test_td_update_from_replay_matches_host_batch(xq, O):
