@@ -22,6 +22,7 @@ MAX_ACTIONS = 128
 STATE_SIZE = 1260
 POLICY_ACTIONS = 8100     # policy index = from * 90 + to (include/xq.h: XQ_POLICY_ACTIONS)
 MASK_WORDS = 254          # uint32 words of a packed legal-action mask
+COMPACT_ACTIONS = 128     # entries of a compact row: list entry k of a board (include/xq.h: XQ_COMPACT_ACTIONS)
 DTYPE_F32, DTYPE_BF16, DTYPE_U8 = 0, 1, 2
 VIEW_ABSOLUTE, VIEW_SIDE_TO_MOVE = 0, 1
 PICK_GREEDY, PICK_SAMPLE, PICK_GIVEN = 0, 1, 2
@@ -93,6 +94,8 @@ def lib():
     L.xq_env_observe_device.argtypes = [_P, _P, C.c_int, C.c_int, _P]
     L.xq_env_legal_mask_device.argtypes = [_P, _P, C.c_int, C.c_int]
     L.xq_env_policy_step_device.argtypes = [_P, _P, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int] + [_P] * 7
+    L.xq_env_legal_actions_device.argtypes = [_P, C.c_int, _P, _P]
+    L.xq_env_policy_step_compact_device.argtypes = [_P, _P, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int] + [_P] * 7
     L.xq_search_create.argtypes = [_P, C.c_int, C.POINTER(_P)]
     L.xq_search_create_ex.argtypes = [_P, C.c_int, C.c_int, C.POINTER(_P)]
     L.xq_search_destroy.argtypes = [_P]
@@ -105,6 +108,8 @@ def lib():
     L.xq_search_leaves_device.argtypes = [_P, C.POINTER(_P)]
     L.xq_search_observe_leaves_device.argtypes = [_P, _P, C.c_int, C.c_int, _P]
     L.xq_search_expand_backup_device.argtypes = [_P, _P, C.c_int, C.c_float, C.c_int, _P, _P, C.c_float]
+    L.xq_search_leaf_actions_device.argtypes = [_P, C.c_int, _P, _P]
+    L.xq_search_expand_backup_compact_device.argtypes = [_P, _P, C.c_int, C.c_float, _P]
     L.xq_search_root_device.argtypes = [_P, C.c_int, _P, _P, _P]
     L.xq_search_play_device.argtypes = [_P, C.c_float, C.c_int, C.c_int, C.c_int] + [_P] * 6
     L.xq_search_root_noise_device.argtypes = [_P, C.c_float, C.c_float, C.c_uint64, _P, _P]
@@ -113,6 +118,7 @@ def lib():
     L.xq_gumbel_destroy.argtypes = [_P]
     L.xq_gumbel_bytes.argtypes = [C.c_int64, C.c_int, C.POINTER(C.c_int64)]
     L.xq_gumbel_begin_device.argtypes = [_P, _P, C.c_int, C.c_float, C.c_int, _P, C.c_int, C.c_uint64, C.c_float, C.c_float]
+    L.xq_gumbel_begin_compact_device.argtypes = [_P, _P, C.c_int, C.c_float, _P, C.c_int, C.c_uint64, C.c_float, C.c_float]
     L.xq_gumbel_select_device.argtypes = [_P, C.c_int, C.c_float, C.c_float, C.c_float, _P, _P, _P, _P]
     L.xq_gumbel_root_device.argtypes = [_P, C.c_int, _P, _P]
     L.xq_gumbel_play_device.argtypes = [_P, C.c_int, C.c_int] + [_P] * 6
@@ -125,6 +131,7 @@ def lib():
     L.xq_examples_end_games_device.argtypes = [_P, _P, _P]
     L.xq_examples_discard_device.argtypes = [_P, _P]
     L.xq_examples_sample_device.argtypes = [_P, C.c_int64, C.c_uint64, C.c_uint32, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]
+    L.xq_examples_sample_compact_device.argtypes = [_P, C.c_int64, C.c_uint64, C.c_uint32, C.c_int, _P, C.c_int] + [_P] * 6
     L.xq_examples_info.argtypes = [_P] + [C.POINTER(C.c_int64)] * 6
     L.xq_examples_get.argtypes = [_P, C.c_int64, C.c_int64, _P]
     _lib = L

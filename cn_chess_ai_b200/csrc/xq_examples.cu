@@ -14,6 +14,7 @@
 //   binary search over the offsets, moves to the next env at its end, and copies one 864-byte example per step with z and game stamped.
 // examples_sample_kernel: one CTA per sample: the draw, the policy row and the packed mask built in shared memory and streamed out with
 //   16-byte (policy) and 8-byte (mask) stores, the record gathered for observe_kernel (launch_observe, xq_policy.cu).
+// examples_sample_compact_kernel: one warp per sample, the same draw and record; the compact action and policy rows with 16-byte stores.
 #include <stddef.h>
 
 #include <algorithm>
@@ -221,6 +222,41 @@ __global__ void __launch_bounds__(kSmpThreads) examples_sample_kernel(ExDev b, u
     }
 }
 
+// The compact form of examples_sample_kernel: one warp per sample; lane l writes entries 4 l .. 4 l + 3 of the sample's action and policy
+// rows (one 16-byte store each: the warp writes each 512-byte row in one coalesced sweep) from the example's action / visits rows.
+constexpr int kSmpWarps = 4;
+__global__ void __launch_bounds__(32 * kSmpWarps) examples_sample_compact_kernel(ExDev b, int64_t batch, uint64_t seed, uint32_t counter, int view,
+                                                                               xq_env_rec* __restrict__ recs, int32_t* __restrict__ actions,
+                                                                               float* __restrict__ policy, uint8_t* __restrict__ counts,
+                                                                               float* __restrict__ value, float* __restrict__ q,
+                                                                               int64_t* __restrict__ index) {
+    const int lane = threadIdx.x & 31;
+    const int64_t i = (int64_t)blockIdx.x * kSmpWarps + (threadIdx.x >> 5);
+    if (i >= batch) return;
+    const int64_t total = (int64_t)b.ctr->total, size = total < b.capacity ? total : b.capacity;
+    const int64_t idx = ex_sample_index(seed, i, counter, size);
+    const xq_example* x = idx >= 0 ? b.ring + idx : nullptr;
+    if (lane < 4) reinterpret_cast<uint4*>(recs + i)[lane] = x ? reinterpret_cast<const uint4*>(&x->rec)[lane] : make_uint4(0u, 0u, 0u, 0u);
+    const int ne = x ? x->n_edges : 0, player = x ? x->rec.player : 0;
+    const uint32_t tot = x ? x->total_visits : 0u;
+    int32_t a[4];
+    float p[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        const int k = 4 * lane + j;
+        a[j] = k < ne ? ex_view_index(x->action[k], player, view) : -1;
+        p[j] = k < ne ? ex_policy(x->visits[k], tot) : 0.f;
+    }
+    reinterpret_cast<int4*>(actions + i * XQ_COMPACT_ACTIONS)[lane] = make_int4(a[0], a[1], a[2], a[3]);
+    reinterpret_cast<float4*>(policy + i * XQ_COMPACT_ACTIONS)[lane] = make_float4(p[0], p[1], p[2], p[3]);
+    if (lane == 0) {
+        if (counts) counts[i] = (uint8_t)ne;
+        if (value) value[i] = x ? x->z : NAN;
+        if (q) q[i] = x ? x->q : NAN;
+        if (index) index[i] = idx;
+    }
+}
+
 }  // namespace xq
 
 // ==========================================================================================
@@ -360,6 +396,22 @@ int xq_examples_discard_device(xq_examples_t b, const uint8_t* mask_dev) {
     return XQ_OK;
 }
 
+}  // extern "C"
+
+namespace {
+// the record scratch of a batch of `batch` samples (grown on the env's stream; cudaFree waits for the work that used the old scratch)
+int sample_scratch(xq_examples_t b, int64_t batch) {
+    if (batch > b->recs_cap) {
+        cudaFree(b->recs); b->recs = nullptr; b->recs_cap = 0;
+        XQ_CUDA(cudaMalloc(&b->recs, sizeof(xq_env_rec) * (size_t)batch));
+        b->recs_cap = batch;
+    }
+    return XQ_OK;
+}
+}  // namespace
+
+extern "C" {
+
 int xq_examples_sample_device(xq_examples_t b, int64_t batch, uint64_t seed, uint32_t counter, int view, void* planes_dev, int dtype,
                               float* policy_dev, float* value_dev, float* q_dev, uint32_t* mask_dev, int64_t* index_dev) {
     EnvInfo E;
@@ -370,15 +422,30 @@ int xq_examples_sample_device(xq_examples_t b, int64_t batch, uint64_t seed, uin
     if (!planes_dev || !policy_dev) return fail(XQ_ERR_INVALID, "xq_examples_sample_device: planes and policy are required");
     if (!aligned16(planes_dev) || !aligned16(policy_dev) || (reinterpret_cast<uintptr_t>(mask_dev) & 7u))
         return fail(XQ_ERR_INVALID, "xq_examples_sample_device: planes and policy must be 16-byte aligned, mask 8-byte aligned");
-    if (batch > b->recs_cap) {      // grows on the env's stream; cudaFree waits for the work that used the old scratch
-        cudaFree(b->recs); b->recs = nullptr; b->recs_cap = 0;
-        XQ_CUDA(cudaMalloc(&b->recs, sizeof(xq_env_rec) * (size_t)batch));
-        b->recs_cap = batch;
-    }
+    if (int rc = sample_scratch(b, batch)) return rc;
     examples_sample_kernel<<<(unsigned)batch, kSmpThreads, 0, E.stream>>>(b->d, seed, counter, view, b->recs, policy_dev, value_dev, q_dev, mask_dev,
                                                                          index_dev);
     XQ_LAUNCH_CHECK();
     XQ_CUDA(launch_observe(b->recs, batch, planes_dev, dtype, view, nullptr, E.stream));
+    return XQ_OK;
+}
+
+int xq_examples_sample_compact_device(xq_examples_t b, int64_t batch, uint64_t seed, uint32_t counter, int view, void* planes_dev, int dtype,
+                                      int32_t* actions_dev, float* policy_dev, uint8_t* counts_dev, float* value_dev, float* q_dev,
+                                      int64_t* index_dev) {
+    EnvInfo E;
+    if (int rc = enter(b, &E, "xq_examples_sample_compact_device")) return rc;
+    if (batch <= 0 || batch > 0x7FFFFFFF) return fail(XQ_ERR_INVALID, "xq_examples_sample_compact_device: batch %lld", (long long)batch);
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_examples_sample_compact_device: view %d", view);
+    if (planes_dev && (dtype < XQ_DTYPE_F32 || dtype > XQ_DTYPE_U8)) return fail(XQ_ERR_INVALID, "xq_examples_sample_compact_device: dtype %d", dtype);
+    if (!actions_dev || !policy_dev) return fail(XQ_ERR_INVALID, "xq_examples_sample_compact_device: actions and policy are required");
+    if (!aligned16(planes_dev) || !aligned16(actions_dev) || !aligned16(policy_dev))
+        return fail(XQ_ERR_INVALID, "xq_examples_sample_compact_device: planes, actions and policy must be 16-byte aligned");
+    if (int rc = sample_scratch(b, batch)) return rc;
+    examples_sample_compact_kernel<<<grid_of(batch, kSmpWarps), 32 * kSmpWarps, 0, E.stream>>>(b->d, batch, seed, counter, view, b->recs, actions_dev,
+                                                                                                policy_dev, counts_dev, value_dev, q_dev, index_dev);
+    XQ_LAUNCH_CHECK();
+    if (planes_dev) XQ_CUDA(launch_observe(b->recs, batch, planes_dev, dtype, view, nullptr, E.stream));
     return XQ_OK;
 }
 

@@ -1,5 +1,5 @@
 // xq_policy.cu -- device-resident interface for a policy that is not the library's DQN (include/xq.h: xq_env_observe_device,
-// xq_env_legal_mask_device, xq_env_policy_step_device).
+// xq_env_legal_mask_device, xq_env_legal_actions_device, xq_env_policy_step_device and its compact form).
 //
 // observe_kernel: the record -> [14][10][9] planes (f32 / bf16 / u8) + aux; write-bound, so a CTA stages 32 records in shared memory and
 //   streams the 32 contiguous rows as one flat run of 16-byte stores (a row is 5,040 / 2,520 / 1,260 B: not a multiple of 16, the run is).
@@ -8,7 +8,10 @@
 //   16-byte stores, either as they are (packed) or expanded to one byte per index (dense: 8,100 B per board written once, no memset).
 // policy_step_lane_kernel: the same generator; the score of each legal action is read once (only legal entries are touched) into a
 //   [list index][thread] row of shared memory, the choice runs over that row in reference list order (policy_choose), the played
-//   action is decoded with lane_select_kth and applied exactly as step_kernel (xq_env.cu) applies an xq_action.
+//   action is decoded with lane_select_kth and applied exactly as step_kernel (xq_env.cu) applies an xq_action.  The score rows are
+//   dense ([n][8100], read at the policy index) or compact ([n][128], read at the list index): a template parameter of the step kernels.
+// actions_lane_kernel: the same generator, the compact list of each board (policy indices in list order) staged per thread in shared
+//   memory and written as one flat run of 16-byte stores; also over the leaf records of a search (launch_legal_actions).
 // Boards the generator cannot take (a non-standard piece set, or a player byte > 1) are flagged and handled by the generic thread-per-board
 // kernels on all_actions (xq_rules.cuh), with the same choice in list order.
 #include "xq_common.cuh"
@@ -152,6 +155,82 @@ __global__ void __launch_bounds__(kThreads) mask_generic_kernel(const xq_env_rec
     }
 }
 
+// ---- compact action lists ---------------------------------------------------------------------------------------------------------
+// actions_lane_kernel: the generator's list of each board, entry k = its policy index, into a per-thread row of shared memory (row stride
+// kActRow: odd, so the thread-major writes are conflict-free); the CTA's rows go out as one flat run of 16-byte stores, -1 past the count.
+constexpr int kActRow = XQ_COMPACT_ACTIONS + 1;
+__global__ void __launch_bounds__(kPolBoards) actions_lane_kernel(const xq_env_rec* __restrict__ recs, int64_t n, int32_t* __restrict__ actions,
+                                                                 uint8_t* __restrict__ counts, int view, uint8_t* __restrict__ nonstd) {
+    __shared__ uint8_t s_slot[32 * kPolBoards];
+    __shared__ uint32_t s_geo[kGeoWords];
+    __shared__ uint32_t s_view[kViewWords * kPolBoards];
+    __shared__ int32_t s_list[kPolBoards * kActRow];
+    __shared__ int s_cnt[kPolBoards];
+    const int tid = threadIdx.x;
+    const int64_t env0 = (int64_t)blockIdx.x * kPolBoards, env = env0 + tid;
+    for (int i = tid; i < kGeoWords; i += kPolBoards) s_geo[i] = geo_word(i);
+    __syncthreads();
+    int cnt = 0;
+    if (env < n) {
+        const uint4* rec = reinterpret_cast<const uint4*>(recs + env);
+        uint32_t w[12];
+#pragma unroll
+        for (int i = 0; i < 3; ++i) { const uint4 v = rec[i]; w[4 * i] = v.x; w[4 * i + 1] = v.y; w[4 * i + 2] = v.z; w[4 * i + 3] = v.w; }
+        const int player = (int)((rec[3].x >> 16) & 0xFFu);
+        LaneGen g;
+        const bool ok = policy_lane_gen(w, player, s_view + tid, s_slot + tid, kPolBoards, s_geo, g);
+        nonstd[env] = ok ? 0 : 1;      // its row is written here as an empty list; the generic kernel rewrites it
+        if (ok) {
+            const bool flip = policy_flip(player, view);
+            int32_t* row = s_list + tid * kActRow;
+            cnt = policy_lane_emit(g, player, [&](int idx, int from, int to) { if (idx < XQ_COMPACT_ACTIONS) row[idx] = policy_index(from, to, flip); });
+            cnt = min(cnt, XQ_COMPACT_ACTIONS);
+        }
+        if (counts) counts[env] = (uint8_t)cnt;
+    }
+    s_cnt[tid] = cnt;
+    __syncthreads();
+    const int live = (int)min((int64_t)kPolBoards, n - env0);
+    int4* dst = reinterpret_cast<int4*>(actions + env0 * XQ_COMPACT_ACTIONS);
+    for (int c = tid; c < live * (XQ_COMPACT_ACTIONS / 4); c += kPolBoards) {      // entries 4 (c % 32) .. + 3 of board c / 32
+        const int e = c / (XQ_COMPACT_ACTIONS / 4), k = (c % (XQ_COMPACT_ACTIONS / 4)) * 4, ce = s_cnt[e];
+        const int32_t* row = s_list + e * kActRow + k;
+        dst[c] = make_int4(k < ce ? row[0] : -1, k + 1 < ce ? row[1] : -1, k + 2 < ce ? row[2] : -1, k + 3 < ce ? row[3] : -1);
+    }
+}
+
+// the boards the lane kernel flagged: all_actions, one thread per board, the whole row rewritten
+__global__ void __launch_bounds__(kThreads) actions_generic_kernel(const xq_env_rec* __restrict__ recs, int64_t n, int32_t* __restrict__ actions,
+                                                                  uint8_t* __restrict__ counts, int view, const uint8_t* __restrict__ only) {
+    __shared__ uint32_t s_board[12 * kThreads];
+    const int64_t env = (int64_t)blockIdx.x * kThreads + threadIdx.x;
+    if (env >= n || !only[env]) return;
+    SmemBoard b{s_board + threadIdx.x, kThreads};
+    b.load(recs + env);
+    Meta m; m.load(recs + env);
+    const bool flip = policy_flip(m.player, view);
+    int32_t* row = actions + env * XQ_COMPACT_ACTIONS;
+    int k = 0;
+    if ((unsigned)m.player <= 1u)
+        all_actions(b, m.player, [&](int from, int to) { if (k < XQ_COMPACT_ACTIONS) row[k++] = policy_index(from, to, flip); });
+    if (counts) counts[env] = (uint8_t)k;
+    for (int i = k; i < XQ_COMPACT_ACTIONS; ++i) row[i] = -1;
+}
+
+// the compact lists of any array of records (the envs of a handle, the leaves of a search); flags u8 [n] receives the lane kernel's
+// refusals, and the generic kernel runs on them when `generic` (the records may hold boards the generator refuses)
+cudaError_t launch_legal_actions(const xq_env_rec* recs, int64_t n, int32_t* actions, uint8_t* counts, int view, uint8_t* flags, bool generic,
+                                 cudaStream_t stream) {
+    actions_lane_kernel<<<grid_of(n, kPolBoards), kPolBoards, 0, stream>>>(recs, n, actions, counts, view, flags);
+    ++g_launches;
+    if (cudaError_t e = cudaGetLastError()) return e;
+    if (generic) {
+        actions_generic_kernel<<<grid_of(n, kThreads), kThreads, 0, stream>>>(recs, n, actions, counts, view, flags);
+        ++g_launches;
+    }
+    return cudaGetLastError();
+}
+
 // ---- policy step ------------------------------------------------------------------------------------------------------------------
 template <int SDT>
 __device__ __forceinline__ float load_score(const void* p, int64_t i) {
@@ -164,7 +243,7 @@ struct PolicyArgs {
     int64_t* actions; float* logp; int32_t* reward; uint8_t *done, *winner, *captured, *valid;
 };
 
-template <int SDT>
+template <int SDT, bool CMP>
 __global__ void __launch_bounds__(kPolBoards) policy_step_lane_kernel(PolicyArgs a, uint8_t* __restrict__ nonstd) {
     __shared__ uint8_t s_slot[32 * kPolBoards];
     __shared__ uint32_t s_geo[kGeoWords];
@@ -186,14 +265,14 @@ __global__ void __launch_bounds__(kPolBoards) policy_step_lane_kernel(PolicyArgs
     if (nonstd) nonstd[env] = ok ? 0 : 1;
     if (!ok) return;
     const bool flip = policy_flip(player, a.view);
-    const void* sc = a.scores ? static_cast<const uint8_t*>(a.scores) + env * XQ_POLICY_ACTIONS * (SDT == XQ_DTYPE_BF16 ? 2 : 4) : nullptr;
+    const void* sc = a.scores ? static_cast<const uint8_t*>(a.scores) + env * score_width<CMP>() * (SDT == XQ_DTYPE_BF16 ? 2 : 4) : nullptr;
     const int64_t given = a.pick == XQ_PICK_GIVEN ? a.actions[env] : -1;
     int given_k = -1;
     // the walk only stages the raw scores: its loads do not depend on each other and are in flight together (consuming each score in the
     // walk chained ~40 global-load latencies per board)
     const int cnt = policy_lane_emit(g, player, [&](int idx, int from, int to) {
         const int pi = policy_index(from, to, flip);
-        if (sc) s_row[idx * kPolBoards + tid] = load_score<SDT>(sc, pi);
+        if (sc) s_row[idx * kPolBoards + tid] = load_score<SDT>(sc, score_at<CMP>(idx, pi));
         given_k = pi == given ? idx : given_k;
     });
     auto each = [&](auto&& f) { for (int k = 0; k < cnt; ++k) f(policy_clean(s_row[k * kPolBoards + tid])); };
@@ -211,8 +290,9 @@ __global__ void __launch_bounds__(kPolBoards) policy_step_lane_kernel(PolicyArgs
     policy_apply(b, mt, a.envs, env, c.k >= 0, from, to, a.auto_reset, a.reward, a.done, a.winner, a.captured, a.valid);
 }
 
-// the boards the lane kernel flagged: all_actions enumerates the list in reference order (three or four times; rare boards)
-template <int SDT>
+// the boards the lane kernel flagged: all_actions enumerates the list in reference order (three or four times; rare boards); compact
+// scores cover the first XQ_COMPACT_ACTIONS actions, and the choice is among those
+template <int SDT, bool CMP>
 __global__ void __launch_bounds__(kThreads) policy_step_generic_kernel(PolicyArgs a, const uint8_t* __restrict__ only) {
     __shared__ uint32_t s_board[12 * kThreads];
     const int64_t env = (int64_t)blockIdx.x * kThreads + threadIdx.x;
@@ -222,23 +302,26 @@ __global__ void __launch_bounds__(kThreads) policy_step_generic_kernel(PolicyArg
     Meta mt; mt.load(a.envs + env);
     const int player = mt.player;
     const bool flip = policy_flip(player, a.view);
-    const void* sc = a.scores ? static_cast<const uint8_t*>(a.scores) + env * XQ_POLICY_ACTIONS * (SDT == XQ_DTYPE_BF16 ? 2 : 4) : nullptr;
+    const void* sc = a.scores ? static_cast<const uint8_t*>(a.scores) + env * score_width<CMP>() * (SDT == XQ_DTYPE_BF16 ? 2 : 4) : nullptr;
     const int64_t given = a.pick == XQ_PICK_GIVEN ? a.actions[env] : -1;
-    auto each_action = [&](auto&& f) { if ((unsigned)player <= 1u) all_actions(b, player, f); };      // a player byte > 1 owns no piece
+    auto each_action = [&](auto&& f) {      // f(list index, from, to); a player byte > 1 owns no piece
+        int k = 0;
+        if ((unsigned)player <= 1u) all_actions(b, player, [&](int from, int to) { if (!CMP || k < XQ_COMPACT_ACTIONS) f(k, from, to); ++k; });
+    };
     PolicyBest best{-INFINITY, -1};
     int cnt = 0, given_k = -1;
-    each_action([&](int from, int to) {
+    each_action([&](int k, int from, int to) {
         const int pi = policy_index(from, to, flip);
-        if (sc) best.offer(policy_clean(load_score<SDT>(sc, pi)), cnt);
+        if (sc) best.offer(policy_clean(load_score<SDT>(sc, score_at<CMP>(k, pi))), cnt);
         given_k = pi == given ? cnt : given_k;
         ++cnt;
     });
     const float u = a.pick == XQ_PICK_SAMPLE ? policy_uniform(rng(a.seed, a.env_id0 + (uint64_t)env, mt.ctr)) : 0.f;
     const PolicyChoice c = policy_choose(
-        [&](auto&& f) { each_action([&](int from, int to) { f(policy_clean(load_score<SDT>(sc, policy_index(from, to, flip)))); }); },
+        [&](auto&& f) { each_action([&](int k, int from, int to) { f(policy_clean(load_score<SDT>(sc, score_at<CMP>(k, policy_index(from, to, flip))))); }); },
         cnt, best, given_k, a.pick, sc != nullptr, a.logp != nullptr, a.t, u);
     int from = 0, to = 0, i = 0;
-    if (c.k >= 0) each_action([&](int f, int t) { if (i == c.k) { from = f; to = t; } ++i; });
+    if (c.k >= 0) each_action([&](int, int f, int t) { if (i == c.k) { from = f; to = t; } ++i; });
     if (a.pick != XQ_PICK_GIVEN && a.actions) a.actions[env] = c.k >= 0 ? policy_index(from, to, flip) : -1;
     if (a.logp) a.logp[env] = c.logp;
     policy_apply(b, mt, a.envs, env, c.k >= 0, from, to, a.auto_reset, a.reward, a.done, a.winner, a.captured, a.valid);
@@ -298,32 +381,65 @@ int xq_env_legal_mask_device(xq_env_t h, void* mask_dev, int packed, int view) {
     return XQ_OK;
 }
 
-int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dtype, int pick, float temperature, int view, int auto_reset,
-                              int64_t* actions_dev, float* logp_dev, int32_t* reward_dev, uint8_t* done_dev, uint8_t* winner_dev,
-                              uint8_t* captured_dev, uint8_t* valid_dev) {
+int xq_env_legal_actions_device(xq_env_t h, int view, int32_t* actions_dev, uint8_t* counts_dev) {
     EnvInfo E;
     if (int rc = env_info(h, &E)) return rc;
-    if (pick < XQ_PICK_GREEDY || pick > XQ_PICK_GIVEN) return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: pick %d", pick);
-    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: view %d", view);
+    if (!actions_dev || !aligned16(actions_dev)) return fail(XQ_ERR_INVALID, "xq_env_legal_actions_device: actions must be a 16-byte aligned device buffer");
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_env_legal_actions_device: view %d", view);
+    XQ_CUDA(cudaSetDevice(E.device));
+    XQ_CUDA(launch_legal_actions(E.d_envs, E.n, actions_dev, counts_dev, view, E.d_nonstd, E.maybe_nonstd, E.stream));
+    return XQ_OK;
+}
+
+}  // extern "C"
+
+namespace {
+// the checks and launches of xq_env_policy_step_device and its compact form (CMP: the score rows are compact)
+template <bool CMP>
+int policy_step(const char* fn, xq_env_t h, const void* scores_dev, int scores_dtype, int pick, float temperature, int view, int auto_reset,
+                int64_t* actions_dev, float* logp_dev, int32_t* reward_dev, uint8_t* done_dev, uint8_t* winner_dev, uint8_t* captured_dev,
+                uint8_t* valid_dev) {
+    EnvInfo E;
+    if (int rc = env_info(h, &E)) return rc;
+    if (pick < XQ_PICK_GREEDY || pick > XQ_PICK_GIVEN) return fail(XQ_ERR_INVALID, "%s: pick %d", fn, pick);
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "%s: view %d", fn, view);
     if (scores_dev && scores_dtype != XQ_DTYPE_F32 && scores_dtype != XQ_DTYPE_BF16)
-        return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: scores_dtype %d (f32 or bf16)", scores_dtype);
-    if (pick != XQ_PICK_GIVEN && !scores_dev) return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: GREEDY and SAMPLE need scores");
-    if (pick == XQ_PICK_GIVEN && !actions_dev) return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: GIVEN needs actions");
+        return fail(XQ_ERR_INVALID, "%s: scores_dtype %d (f32 or bf16)", fn, scores_dtype);
+    if (CMP && !aligned16(scores_dev)) return fail(XQ_ERR_INVALID, "%s: compact scores must be 16-byte aligned", fn);
+    if (pick != XQ_PICK_GIVEN && !scores_dev) return fail(XQ_ERR_INVALID, "%s: GREEDY and SAMPLE need scores", fn);
+    if (pick == XQ_PICK_GIVEN && !actions_dev) return fail(XQ_ERR_INVALID, "%s: GIVEN needs actions", fn);
     if ((pick == XQ_PICK_SAMPLE || (logp_dev && scores_dev)) && !(temperature > 0.f && temperature <= FLT_MAX))
-        return fail(XQ_ERR_INVALID, "xq_env_policy_step_device: temperature must be finite and > 0");
+        return fail(XQ_ERR_INVALID, "%s: temperature must be finite and > 0", fn);
     XQ_CUDA(cudaSetDevice(E.device));
     const PolicyArgs a{E.d_envs, E.n, E.env_id0, E.seed, scores_dev, pick, temperature, view, auto_reset,
                        actions_dev, logp_dev, reward_dev, done_dev, winner_dev, captured_dev, valid_dev};
     const bool bf16 = scores_dev && scores_dtype == XQ_DTYPE_BF16;
-    if (bf16) policy_step_lane_kernel<XQ_DTYPE_BF16><<<grid_of(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(a, E.d_nonstd);
-    else policy_step_lane_kernel<XQ_DTYPE_F32><<<grid_of(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(a, E.d_nonstd);
+    if (bf16) policy_step_lane_kernel<XQ_DTYPE_BF16, CMP><<<grid_of(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(a, E.d_nonstd);
+    else policy_step_lane_kernel<XQ_DTYPE_F32, CMP><<<grid_of(E.n, kPolBoards), kPolBoards, 0, E.stream>>>(a, E.d_nonstd);
     XQ_LAUNCH_CHECK();
     if (E.maybe_nonstd) {
-        if (bf16) policy_step_generic_kernel<XQ_DTYPE_BF16><<<grid_of(E.n, kThreads), kThreads, 0, E.stream>>>(a, E.d_nonstd);
-        else policy_step_generic_kernel<XQ_DTYPE_F32><<<grid_of(E.n, kThreads), kThreads, 0, E.stream>>>(a, E.d_nonstd);
+        if (bf16) policy_step_generic_kernel<XQ_DTYPE_BF16, CMP><<<grid_of(E.n, kThreads), kThreads, 0, E.stream>>>(a, E.d_nonstd);
+        else policy_step_generic_kernel<XQ_DTYPE_F32, CMP><<<grid_of(E.n, kThreads), kThreads, 0, E.stream>>>(a, E.d_nonstd);
         XQ_LAUNCH_CHECK();
     }
     return XQ_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dtype, int pick, float temperature, int view, int auto_reset,
+                              int64_t* actions_dev, float* logp_dev, int32_t* reward_dev, uint8_t* done_dev, uint8_t* winner_dev,
+                              uint8_t* captured_dev, uint8_t* valid_dev) {
+    return policy_step<false>("xq_env_policy_step_device", h, scores_dev, scores_dtype, pick, temperature, view, auto_reset, actions_dev, logp_dev,
+                              reward_dev, done_dev, winner_dev, captured_dev, valid_dev);
+}
+
+int xq_env_policy_step_compact_device(xq_env_t h, const void* scores_dev, int scores_dtype, int pick, float temperature, int view, int auto_reset,
+                                      int64_t* actions_dev, float* logp_dev, int32_t* reward_dev, uint8_t* done_dev, uint8_t* winner_dev,
+                                      uint8_t* captured_dev, uint8_t* valid_dev) {
+    return policy_step<true>("xq_env_policy_step_compact_device", h, scores_dev, scores_dtype, pick, temperature, view, auto_reset, actions_dev,
+                             logp_dev, reward_dev, done_dev, winner_dev, captured_dev, valid_dev);
 }
 
 }  // extern "C"

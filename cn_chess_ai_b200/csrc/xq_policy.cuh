@@ -17,6 +17,10 @@ namespace xq {
 XQ_HD bool policy_flip(int player, int view) { return view == XQ_VIEW_SIDE_TO_MOVE && player == BLACK; }
 // policy index of the absolute action (from, to) in the frame of the view (flip: rotated by 180 degrees, s -> 89 - s)
 XQ_HD int policy_index(int from, int to, bool flip) { return flip ? (89 - from) * 90 + (89 - to) : from * 90 + to; }
+// Where a score row holds the score of list entry k with policy index pi: a dense row (XQ_POLICY_ACTIONS wide) at pi, a compact row
+// (XQ_COMPACT_ACTIONS wide) at k.  The kernels that read scores take COMPACT as a template parameter.
+template <bool COMPACT> XQ_HD constexpr int score_width() { return COMPACT ? XQ_COMPACT_ACTIONS : XQ_POLICY_ACTIONS; }
+template <bool COMPACT> XQ_HD int score_at(int k, int pi) { return COMPACT ? k : pi; }
 // NaN never wins (it counts as -inf); +inf is clamped so that a softmax over it stays defined
 XQ_HD float policy_clean(float v) { return v != v ? -INFINITY : (v > FLT_MAX ? FLT_MAX : v); }
 // bf16 -> f32 is exact: the 16 bits are the high half of the f32

@@ -10,7 +10,8 @@
 //   summarize_words on the nibble board, as policy_apply does; the leaf record goes to the leaf buffer.
 // search_expand_lane_kernel: one thread per tree, the structure of policy_step_lane_kernel: the generator stages the legal scores into
 //   a [list index][thread] shared row, the priors are taken over that row in list order, the backup walks the parent pointers.
-//   Boards the generator refuses go to search_expand_generic_kernel (all_actions, thread per board).
+//   Boards the generator refuses go to search_expand_generic_kernel (all_actions, thread per board).  Every expand kernel reads dense score
+//   rows ([rows][8100] at the view's policy index) or compact ones ([rows][128] at the edge index), a template parameter (CMP).
 // search_select_leaves_kernel: one warp per tree, the L descents of a multi-leaf selection in order with virtual loss (in-flight counts
 //   from the earlier descents' edges, kept per depth in shared memory); search_expand_slots_kernel / search_expand_generic_slots_kernel:
 //   one thread per (tree, slot) for the expansions, the backups of a tree in slot order by the thread of its slot 0.
@@ -34,6 +35,8 @@
 namespace xq {
 
 cudaError_t launch_observe(const xq_env_rec* recs, int64_t n, void* planes, int dtype, int view, int32_t* aux, cudaStream_t stream);
+cudaError_t launch_legal_actions(const xq_env_rec* recs, int64_t n, int32_t* actions, uint8_t* counts, int view, uint8_t* flags, bool generic,
+                                 cudaStream_t stream);
 
 constexpr int kSelWarps = 4;       // trees per CTA of the select kernel
 constexpr int kExpBoards = 32;     // trees per CTA of the lane expand kernel
@@ -576,8 +579,8 @@ __device__ __forceinline__ void search_write_edges(const SearchDev& d, const Exp
 
 // Expansion of leaf `leaf` of tree t from the leaf record and score row `slot` (slot = t at one leaf per tree), one thread: the structure
 // of policy_step_lane_kernel (the generator stages the legal scores into the [list index][thread] shared row s_row).  Returns 1 when the
-// generator refuses the board and the generic kernel has to expand it.
-template <int SDT>
+// generator refuses the board and the generic kernel has to expand it.  CMP: the score rows are compact (entry k = edge k).
+template <int SDT, bool CMP>
 __device__ __forceinline__ uint8_t search_expand_lane(const SearchDev& d, const ExpandArgs& a, int64_t t, int64_t slot, int leaf, int tid,
                                                       uint8_t* s_slot, const uint32_t* s_geo, uint32_t* s_view, float* s_row) {
     const int64_t g = t * d.cap + leaf;
@@ -591,10 +594,10 @@ __device__ __forceinline__ uint8_t search_expand_lane(const SearchDev& d, const 
         LaneGen lg;
         if (policy_lane_gen(w, player, s_view + tid, s_slot + tid, kExpBoards, s_geo, lg)) {
             const bool flip = policy_flip(player, a.view);
-            const void* sc = static_cast<const uint8_t*>(a.scores) + slot * XQ_POLICY_ACTIONS * (SDT == XQ_DTYPE_BF16 ? 2 : 4);
+            const void* sc = static_cast<const uint8_t*>(a.scores) + slot * score_width<CMP>() * (SDT == XQ_DTYPE_BF16 ? 2 : 4);
             const int64_t eb = g * kSearchEdges;
             const int cnt = policy_lane_emit(lg, player, [&](int idx, int from, int to) {
-                s_row[idx * kExpBoards + tid] = search_score<SDT>(sc, policy_index(from, to, flip));
+                s_row[idx * kExpBoards + tid] = search_score<SDT>(sc, score_at<CMP>(idx, policy_index(from, to, flip)));
                 d.act[eb + idx] = (int16_t)(from * 90 + to);
             });
             auto each = [&](auto&& f) { for (int k = 0; k < cnt; ++k) f(policy_clean(s_row[k * kExpBoards + tid])); };
@@ -609,7 +612,7 @@ __device__ __forceinline__ uint8_t search_expand_lane(const SearchDev& d, const 
     return generic;
 }
 
-template <int SDT>
+template <int SDT, bool CMP>
 __global__ void __launch_bounds__(kExpBoards) search_expand_lane_kernel(SearchDev d, ExpandArgs a) {
     __shared__ uint8_t s_slot[32 * kExpBoards];
     __shared__ uint32_t s_geo[kGeoWords];
@@ -623,7 +626,7 @@ __global__ void __launch_bounds__(kExpBoards) search_expand_lane_kernel(SearchDe
     const int leaf = d.leaf[t];
     const int64_t g0 = t * d.cap;
     // the generic kernel expands a refused board; the backup below does not touch the new node's edges
-    d.nonstd[t] = search_expand_lane<SDT>(d, a, t, t, leaf, tid, s_slot, s_geo, s_view, s_row);
+    d.nonstd[t] = search_expand_lane<SDT, CMP>(d, a, t, t, leaf, tid, s_slot, s_geo, s_view, s_row);
     search_backup(leaf, a.values[t], d.parent + g0, d.pedge + g0, d.visits + g0, d.N + g0 * kSearchEdges, d.W + g0 * kSearchEdges);
 }
 
@@ -631,7 +634,7 @@ __global__ void __launch_bounds__(kExpBoards) search_expand_lane_kernel(SearchDe
 // expands its leaf as search_expand_lane_kernel does (its score row i, the noise row t at the root); the thread of slot 0 then backs up
 // the tree's non-duplicate slots in slot order.  Expansions write only edges of unexpanded leaves, backups only edges of expanded
 // ancestors and N_node, so the two need no ordering between threads and the result is that of "expand, then back up in slot order".
-template <int SDT>
+template <int SDT, bool CMP>
 __global__ void __launch_bounds__(kExpBoards) search_expand_slots_kernel(SearchDev d, ExpandArgs a, int L) {
     __shared__ uint8_t s_slot[32 * kExpBoards];
     __shared__ uint32_t s_geo[kGeoWords];
@@ -644,7 +647,7 @@ __global__ void __launch_bounds__(kExpBoards) search_expand_slots_kernel(SearchD
     if (i >= d.n * L) return;
     const int64_t t = i / L;
     const int leaf = d.leaf[i];          // -1: a duplicate slot
-    d.nonstd[i] = leaf >= 0 ? search_expand_lane<SDT>(d, a, t, i, leaf, tid, s_slot, s_geo, s_view, s_row) : 0;
+    d.nonstd[i] = leaf >= 0 ? search_expand_lane<SDT, CMP>(d, a, t, i, leaf, tid, s_slot, s_geo, s_view, s_row) : 0;
     if (i != t * L) return;
     const int64_t g0 = t * d.cap;
     for (int k = 0; k < L; ++k) {
@@ -654,7 +657,7 @@ __global__ void __launch_bounds__(kExpBoards) search_expand_slots_kernel(SearchD
 }
 
 // Expansion of a board the generator refuses (all_actions, one thread): leaf `leaf` of tree t from the record and score row of slot i
-template <int SDT>
+template <int SDT, bool CMP>
 __device__ __forceinline__ void search_expand_generic(const SearchDev& d, const ExpandArgs& a, int64_t t, int64_t i, int leaf, uint32_t* sb) {
     const int64_t g = t * d.cap + leaf, eb = g * kSearchEdges;
     SmemBoard b{sb, kThreads};
@@ -662,39 +665,39 @@ __device__ __forceinline__ void search_expand_generic(const SearchDev& d, const 
     Meta mt; mt.load(d.leaf_rec + i);
     const int player = mt.player;
     const bool flip = policy_flip(player, a.view);
-    const void* sc = static_cast<const uint8_t*>(a.scores) + i * XQ_POLICY_ACTIONS * (SDT == XQ_DTYPE_BF16 ? 2 : 4);
-    // the first 128 actions in list order; a player byte > 1 owns no piece
+    const void* sc = static_cast<const uint8_t*>(a.scores) + i * score_width<CMP>() * (SDT == XQ_DTYPE_BF16 ? 2 : 4);
+    // f(list index, from, to) for the first 128 actions in list order; a player byte > 1 owns no piece
     auto each_action = [&](auto&& f) {
         int c = 0;
-        if ((unsigned)player <= 1u) all_actions(b, player, [&](int from, int to) { if (c < kSearchEdges) f(from, to); ++c; });
+        if ((unsigned)player <= 1u) all_actions(b, player, [&](int from, int to) { if (c < kSearchEdges) f(c, from, to); ++c; });
     };
     PolicyBest best{-INFINITY, -1};
     int cnt = 0;
-    each_action([&](int from, int to) {
-        best.offer(policy_clean(search_score<SDT>(sc, policy_index(from, to, flip))), cnt);
+    each_action([&](int k, int from, int to) {
+        best.offer(policy_clean(search_score<SDT>(sc, score_at<CMP>(k, policy_index(from, to, flip)))), cnt);
         d.act[eb + cnt] = (int16_t)(from * 90 + to);
         ++cnt;
     });
     search_write_edges(d, a, t, g, leaf == 0, flip,
-                       [&](auto&& f) { each_action([&](int from, int to) { f(policy_clean(search_score<SDT>(sc, policy_index(from, to, flip)))); }); },
+                       [&](auto&& f) { each_action([&](int k, int from, int to) { f(policy_clean(search_score<SDT>(sc, score_at<CMP>(k, policy_index(from, to, flip))))); }); },
                        cnt, best.m);
 }
 
-template <int SDT>
+template <int SDT, bool CMP>
 __global__ void __launch_bounds__(kThreads) search_expand_generic_kernel(SearchDev d, ExpandArgs a) {
     __shared__ uint32_t s_board[12 * kThreads];
     const int64_t t = (int64_t)blockIdx.x * kThreads + threadIdx.x;
     if (t >= d.n || !d.nonstd[t]) return;
-    search_expand_generic<SDT>(d, a, t, t, d.leaf[t], s_board + threadIdx.x);
+    search_expand_generic<SDT, CMP>(d, a, t, t, d.leaf[t], s_board + threadIdx.x);
 }
 
 // the slots of a multi-leaf selection that search_expand_slots_kernel left to the generic generator
-template <int SDT>
+template <int SDT, bool CMP>
 __global__ void __launch_bounds__(kThreads) search_expand_generic_slots_kernel(SearchDev d, ExpandArgs a, int L) {
     __shared__ uint32_t s_board[12 * kThreads];
     const int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x;
     if (i >= d.n * L || !d.nonstd[i]) return;
-    search_expand_generic<SDT>(d, a, i / L, i, d.leaf[i], s_board + threadIdx.x);
+    search_expand_generic<SDT, CMP>(d, a, i / L, i, d.leaf[i], s_board + threadIdx.x);
 }
 
 // The dense 8,100-entry row of a root (one CTA of kRootThreads per tree): root_row_zero clears the shared row with 16-byte stores, the
@@ -864,7 +867,7 @@ __global__ void __launch_bounds__(32 * kPlayWarps) search_noise_kernel(SearchDev
 // gumbel_root_kernel: one CTA per tree, as search_root_kernel: warp 0 computes the improved policy and the action, the dense row is built
 //   in shared memory and written with 16-byte stores.  gumbel_play_kernel: search_play_kernel with the Gumbel action.
 // gumbel_weights_kernel: one warp per tree, the integer weights of xq_examples_record_gumbel_device.
-template <int SDT>
+template <int SDT, bool CMP>
 __global__ void __launch_bounds__(kExpBoards) gumbel_expand_root_kernel(SearchDev d, ExpandArgs a) {
     __shared__ uint8_t s_slot[32 * kExpBoards];
     __shared__ uint32_t s_geo[kGeoWords];
@@ -881,7 +884,7 @@ __global__ void __launch_bounds__(kExpBoards) gumbel_expand_root_kernel(SearchDe
 #pragma unroll
         for (int i = 0; i < 4; ++i) reinterpret_cast<uint4*>(d.leaf_rec + t)[i] = reinterpret_cast<const uint4*>(d.rec + g0)[i];
         d.leaf[t] = 0;
-        generic = search_expand_lane<SDT>(d, a, t, t, 0, tid, s_slot, s_geo, s_view, s_row);
+        generic = search_expand_lane<SDT, CMP>(d, a, t, t, 0, tid, s_slot, s_geo, s_view, s_row);
         search_backup(0, a.values[t], d.parent + g0, d.pedge + g0, d.visits + g0, d.N + g0 * kSearchEdges, d.W + g0 * kSearchEdges);
     }
     d.nonstd[t] = generic;
@@ -1042,22 +1045,26 @@ size_t search_slab(SearchDev& d, void* base, int64_t n, int64_t cap, int max_lea
 // The expansion and backup of the L slots per tree of the leaf buffer (for the Gumbel begin, `roots`, of every unexpanded root, L = 1),
 // then the generic kernel for the boards the generator refused.  One leaf per tree has its own kernels: the slots kernels at L = 1 are
 // measurably slower.
-template <int SDT>
+template <int SDT, bool CMP>
 int launch_expand(const xq_search_s* s, cudaStream_t stream, const ExpandArgs& a, int L, bool roots) {
     const int64_t n = s->d.n;
-    if (roots) gumbel_expand_root_kernel<SDT><<<grid_of(n, kExpBoards), kExpBoards, 0, stream>>>(s->d, a);
-    else if (L == 1) search_expand_lane_kernel<SDT><<<grid_of(n, kExpBoards), kExpBoards, 0, stream>>>(s->d, a);
-    else search_expand_slots_kernel<SDT><<<grid_of(n * L, kExpBoards), kExpBoards, 0, stream>>>(s->d, a, L);
+    if (roots) gumbel_expand_root_kernel<SDT, CMP><<<grid_of(n, kExpBoards), kExpBoards, 0, stream>>>(s->d, a);
+    else if (L == 1) search_expand_lane_kernel<SDT, CMP><<<grid_of(n, kExpBoards), kExpBoards, 0, stream>>>(s->d, a);
+    else search_expand_slots_kernel<SDT, CMP><<<grid_of(n * L, kExpBoards), kExpBoards, 0, stream>>>(s->d, a, L);
     XQ_LAUNCH_CHECK();
     if (s->maybe_nonstd) {
-        if (L == 1) search_expand_generic_kernel<SDT><<<grid_of(n, kThreads), kThreads, 0, stream>>>(s->d, a);
-        else search_expand_generic_slots_kernel<SDT><<<grid_of(n * L, kThreads), kThreads, 0, stream>>>(s->d, a, L);
+        if (L == 1) search_expand_generic_kernel<SDT, CMP><<<grid_of(n, kThreads), kThreads, 0, stream>>>(s->d, a);
+        else search_expand_generic_slots_kernel<SDT, CMP><<<grid_of(n * L, kThreads), kThreads, 0, stream>>>(s->d, a, L);
         XQ_LAUNCH_CHECK();
     }
     return XQ_OK;
 }
-int launch_expand(const xq_search_s* s, cudaStream_t stream, const ExpandArgs& a, int scores_dtype, int L, bool roots) {
-    return scores_dtype == XQ_DTYPE_BF16 ? launch_expand<XQ_DTYPE_BF16>(s, stream, a, L, roots) : launch_expand<XQ_DTYPE_F32>(s, stream, a, L, roots);
+// compact: the score rows are [rows][XQ_COMPACT_ACTIONS], entry k = edge k
+int launch_expand(const xq_search_s* s, cudaStream_t stream, const ExpandArgs& a, int scores_dtype, bool compact, int L, bool roots) {
+    if (compact) return scores_dtype == XQ_DTYPE_BF16 ? launch_expand<XQ_DTYPE_BF16, true>(s, stream, a, L, roots)
+                                                      : launch_expand<XQ_DTYPE_F32, true>(s, stream, a, L, roots);
+    return scores_dtype == XQ_DTYPE_BF16 ? launch_expand<XQ_DTYPE_BF16, false>(s, stream, a, L, roots)
+                                         : launch_expand<XQ_DTYPE_F32, false>(s, stream, a, L, roots);
 }
 }  // namespace
 
@@ -1215,21 +1222,50 @@ int xq_search_observe_leaves_device(xq_search_t s, void* planes_dev, int dtype, 
     return XQ_OK;
 }
 
-int xq_search_expand_backup_device(xq_search_t s, const void* scores_dev, int scores_dtype, float temperature, int view, const float* values_dev,
-                                   const float* root_noise_dev, float noise_eps) {
+int xq_search_leaf_actions_device(xq_search_t s, int view, int32_t* actions_dev, uint8_t* counts_dev) {
     EnvInfo E;
-    if (int rc = enter(s, &E, "xq_search_expand_backup_device")) return rc;
-    if (!scores_dev || !values_dev) return fail(XQ_ERR_INVALID, "xq_search_expand_backup_device: scores and values are required");
-    if (scores_dtype != XQ_DTYPE_F32 && scores_dtype != XQ_DTYPE_BF16)
-        return fail(XQ_ERR_INVALID, "xq_search_expand_backup_device: scores_dtype %d (f32 or bf16)", scores_dtype);
-    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_search_expand_backup_device: view %d", view);
-    if (!(temperature > 0.f && temperature <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_search_expand_backup_device: temperature must be finite and > 0");
-    if (!(noise_eps >= 0.f && noise_eps <= 1.f)) return fail(XQ_ERR_INVALID, "xq_search_expand_backup_device: noise_eps must be in [0, 1]");
-    if (int rc = check_phase(s, "xq_search_expand_backup_device", kSelected)) return rc;
+    if (int rc = enter(s, &E, "xq_search_leaf_actions_device")) return rc;
+    if (!actions_dev || !aligned16(actions_dev))
+        return fail(XQ_ERR_INVALID, "xq_search_leaf_actions_device: actions must be a 16-byte aligned device buffer");
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_search_leaf_actions_device: view %d", view);
+    if (int rc = check_phase(s, "xq_search_leaf_actions_device", kSelected)) return rc;
+    // the slots' generic flags are scratch here: expand_backup rewrites every one of them before its generic kernel reads them
+    XQ_CUDA(launch_legal_actions(s->d.leaf_rec, s->d.n * s->leaves, actions_dev, counts_dev, view, s->d.nonstd, s->maybe_nonstd, E.stream));
+    return XQ_OK;
+}
+
+}  // extern "C"
+
+namespace {
+// xq_search_expand_backup_device and its compact form (no view, no dense noise)
+int expand_backup(const char* fn, xq_search_t s, const void* scores_dev, int scores_dtype, float temperature, int view, const float* values_dev,
+                  const float* root_noise_dev, float noise_eps, bool compact) {
+    EnvInfo E;
+    if (int rc = enter(s, &E, fn)) return rc;
+    if (!scores_dev || !values_dev) return fail(XQ_ERR_INVALID, "%s: scores and values are required", fn);
+    if (scores_dtype != XQ_DTYPE_F32 && scores_dtype != XQ_DTYPE_BF16) return fail(XQ_ERR_INVALID, "%s: scores_dtype %d (f32 or bf16)", fn, scores_dtype);
+    if (compact && !aligned16(scores_dev)) return fail(XQ_ERR_INVALID, "%s: compact scores must be 16-byte aligned", fn);
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "%s: view %d", fn, view);
+    if (!(temperature > 0.f && temperature <= FLT_MAX)) return fail(XQ_ERR_INVALID, "%s: temperature must be finite and > 0", fn);
+    if (!(noise_eps >= 0.f && noise_eps <= 1.f)) return fail(XQ_ERR_INVALID, "%s: noise_eps must be in [0, 1]", fn);
+    if (int rc = check_phase(s, fn, kSelected)) return rc;
     const ExpandArgs a{scores_dev, temperature, view, values_dev, root_noise_dev, noise_eps};
-    if (int rc = launch_expand(s, E.stream, a, scores_dtype, s->leaves, false)) return rc;
+    if (int rc = launch_expand(s, E.stream, a, scores_dtype, compact, s->leaves, false)) return rc;
     s->phase = 1;
     return XQ_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int xq_search_expand_backup_device(xq_search_t s, const void* scores_dev, int scores_dtype, float temperature, int view, const float* values_dev,
+                                   const float* root_noise_dev, float noise_eps) {
+    return expand_backup("xq_search_expand_backup_device", s, scores_dev, scores_dtype, temperature, view, values_dev, root_noise_dev, noise_eps, false);
+}
+
+int xq_search_expand_backup_compact_device(xq_search_t s, const void* scores_dev, int scores_dtype, float temperature, const float* values_dev) {
+    return expand_backup("xq_search_expand_backup_compact_device", s, scores_dev, scores_dtype, temperature, XQ_VIEW_ABSOLUTE, values_dev, nullptr,
+                         0.f, true);
 }
 
 int xq_search_root_device(xq_search_t s, int view, int32_t* visits_dev, float* q_dev, int64_t* best_dev) {
@@ -1406,24 +1442,27 @@ int xq_gumbel_destroy(xq_gumbel_t g) {
     return XQ_OK;
 }
 
-int xq_gumbel_begin_device(xq_gumbel_t g, const void* scores_dev, int scores_dtype, float temperature, int view, const float* root_value_dev,
-                           int n_simulations, uint64_t seed, float c_visit, float c_scale) {
+}  // extern "C"
+
+namespace {
+// xq_gumbel_begin_device and its compact form
+int gumbel_begin(const char* fn, xq_gumbel_t g, const void* scores_dev, int scores_dtype, float temperature, int view, const float* root_value_dev,
+                 int n_simulations, uint64_t seed, float c_visit, float c_scale, bool compact) {
     EnvInfo E;
-    if (!g) return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: null handle");
+    if (!g) return fail(XQ_ERR_INVALID, "%s: null handle", fn);
     xq_search_t s = g->s;
-    if (int rc = enter(s, &E, "xq_gumbel_begin_device")) return rc;
-    if (!scores_dev || !root_value_dev) return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: scores and root values are required");
-    if (scores_dtype != XQ_DTYPE_F32 && scores_dtype != XQ_DTYPE_BF16)
-        return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: scores_dtype %d (f32 or bf16)", scores_dtype);
-    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: view %d", view);
-    if (!(temperature > 0.f && temperature <= FLT_MAX)) return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: temperature must be finite and > 0");
-    if (n_simulations < 1 || n_simulations > s->max_sims)
-        return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: n_simulations %d (1 .. %d)", n_simulations, s->max_sims);
+    if (int rc = enter(s, &E, fn)) return rc;
+    if (!scores_dev || !root_value_dev) return fail(XQ_ERR_INVALID, "%s: scores and root values are required", fn);
+    if (scores_dtype != XQ_DTYPE_F32 && scores_dtype != XQ_DTYPE_BF16) return fail(XQ_ERR_INVALID, "%s: scores_dtype %d (f32 or bf16)", fn, scores_dtype);
+    if (compact && !aligned16(scores_dev)) return fail(XQ_ERR_INVALID, "%s: compact scores must be 16-byte aligned", fn);
+    if (!valid_view(view)) return fail(XQ_ERR_INVALID, "%s: view %d", fn, view);
+    if (!(temperature > 0.f && temperature <= FLT_MAX)) return fail(XQ_ERR_INVALID, "%s: temperature must be finite and > 0", fn);
+    if (n_simulations < 1 || n_simulations > s->max_sims) return fail(XQ_ERR_INVALID, "%s: n_simulations %d (1 .. %d)", fn, n_simulations, s->max_sims);
     if (!(c_visit >= 0.f && c_visit <= FLT_MAX) || !(c_scale >= 0.f && c_scale <= FLT_MAX))
-        return fail(XQ_ERR_INVALID, "xq_gumbel_begin_device: c_visit and c_scale must be finite and >= 0");
-    if (int rc = check_phase(s, "xq_gumbel_begin_device", kReady)) return rc;
+        return fail(XQ_ERR_INVALID, "%s: c_visit and c_scale must be finite and >= 0", fn);
+    if (int rc = check_phase(s, fn, kReady)) return rc;
     const ExpandArgs a{scores_dev, temperature, view, root_value_dev, nullptr, 0.f};
-    if (int rc = launch_expand(s, E.stream, a, scores_dtype, 1, true)) return rc;
+    if (int rc = launch_expand(s, E.stream, a, scores_dtype, compact, 1, true)) return rc;
     g->G.c_visit = c_visit; g->G.c_scale = c_scale; g->G.sims = 0; g->G.n_sims = n_simulations;
     gumbel_init_kernel<<<grid_of(s->d.n, kGumbelWarps), 32 * kGumbelWarps, 0, E.stream>>>(s->d, g->G, g->max_considered, seed, E.env_id0,
                                                                                          root_value_dev);
@@ -1431,6 +1470,21 @@ int xq_gumbel_begin_device(xq_gumbel_t g, const void* scores_dev, int scores_dty
     g->begun = true;
     g->roots = s->roots;
     return XQ_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int xq_gumbel_begin_device(xq_gumbel_t g, const void* scores_dev, int scores_dtype, float temperature, int view, const float* root_value_dev,
+                           int n_simulations, uint64_t seed, float c_visit, float c_scale) {
+    return gumbel_begin("xq_gumbel_begin_device", g, scores_dev, scores_dtype, temperature, view, root_value_dev, n_simulations, seed, c_visit,
+                        c_scale, false);
+}
+
+int xq_gumbel_begin_compact_device(xq_gumbel_t g, const void* scores_dev, int scores_dtype, float temperature, const float* root_value_dev,
+                                   int n_simulations, uint64_t seed, float c_visit, float c_scale) {
+    return gumbel_begin("xq_gumbel_begin_compact_device", g, scores_dev, scores_dtype, temperature, XQ_VIEW_ABSOLUTE, root_value_dev, n_simulations,
+                        seed, c_visit, c_scale, true);
 }
 
 int xq_gumbel_select_device(xq_gumbel_t g, int leaves, float c_puct, float fpu, float virtual_loss, uint8_t* status_dev, uint8_t* winner_dev,

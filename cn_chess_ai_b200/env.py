@@ -147,6 +147,18 @@ class BatchedEnv:
         check(self._L.xq_env_policy_step_device(self._h, scores_ptr, scores_dtype, pick, float(temperature), view, 1 if auto_reset else 0,
                                                 actions_ptr, logp_ptr, reward_ptr, done_ptr, winner_ptr, captured_ptr, valid_ptr))
 
+    def legal_actions_device(self, actions_ptr, counts_ptr, view):
+        """xq_env_legal_actions_device: int32 [n][128] policy indices of each env's legal actions in list order (-1 past the count),
+        counts uint8 [n] or None"""
+        check(self._L.xq_env_legal_actions_device(self._h, view, actions_ptr, counts_ptr))
+
+    def policy_step_compact_device(self, scores_ptr, scores_dtype, pick, temperature, view, auto_reset, actions_ptr, logp_ptr=None,
+                                   reward_ptr=None, done_ptr=None, winner_ptr=None, captured_ptr=None, valid_ptr=None):
+        """xq_env_policy_step_compact_device: policy_step_device with compact scores [n][128] (entry k = list entry k)"""
+        check(self._L.xq_env_policy_step_compact_device(self._h, scores_ptr, scores_dtype, pick, float(temperature), view,
+                                                        1 if auto_reset else 0, actions_ptr, logp_ptr, reward_ptr, done_ptr, winner_ptr,
+                                                        captured_ptr, valid_ptr))
+
     def state_onehot(self):
         out = np.empty((self.n, STATE_SIZE), dtype=np.float64)
         check(self._L.xq_env_state_onehot(self._h, ptr(out)))
@@ -213,6 +225,14 @@ class BatchedSearch:
         check(self._L.xq_search_expand_backup_device(self._h, scores_ptr, scores_dtype, float(temperature), view, values_ptr, noise_ptr,
                                                      float(noise_eps)))
 
+    def leaf_actions_device(self, actions_ptr, counts_ptr, view):
+        """xq_search_leaf_actions_device: the compact lists int32 [n * L][128] (and counts uint8 [n * L] or None) of the leaf records"""
+        check(self._L.xq_search_leaf_actions_device(self._h, view, actions_ptr, counts_ptr))
+
+    def expand_backup_compact_device(self, scores_ptr, scores_dtype, temperature, values_ptr):
+        """xq_search_expand_backup_compact_device: expand_backup_device with compact scores [n * L][128] (entry k = edge k)"""
+        check(self._L.xq_search_expand_backup_compact_device(self._h, scores_ptr, scores_dtype, float(temperature), values_ptr))
+
     def root_device(self, view, visits_ptr, q_ptr, best_ptr):
         check(self._L.xq_search_root_device(self._h, view, visits_ptr, q_ptr, best_ptr))
 
@@ -274,6 +294,11 @@ class BatchedGumbel:
         the root values (f32 [n]) of this move's n_simulations"""
         check(self._L.xq_gumbel_begin_device(self._h, scores_ptr, scores_dtype, float(temperature), view, values_ptr, int(n_simulations),
                                              int(seed), float(c_visit), float(c_scale)))
+
+    def begin_compact_device(self, scores_ptr, scores_dtype, temperature, values_ptr, n_simulations, seed, c_visit=50.0, c_scale=0.1):
+        """xq_gumbel_begin_compact_device: begin_device with compact root scores [n][128] (entry k = root edge k)"""
+        check(self._L.xq_gumbel_begin_compact_device(self._h, scores_ptr, scores_dtype, float(temperature), values_ptr, int(n_simulations),
+                                                     int(seed), float(c_visit), float(c_scale)))
 
     def select_device(self, leaves, c_puct, fpu, virtual_loss, status_ptr=None, winner_ptr=None, reward_ptr=None, depth_ptr=None):
         """xq_gumbel_select_device: xq_search_select_leaves_device with the Gumbel root rule; outputs [n][leaves]"""
@@ -353,6 +378,12 @@ class BatchedExamples:
                       index_ptr=None):
         check(self._L.xq_examples_sample_device(self._h, int(batch), int(seed), int(counter), view, planes_ptr, dtype, policy_ptr, value_ptr,
                                                 q_ptr, mask_ptr, index_ptr))
+
+    def sample_compact_device(self, batch, seed, counter, view, planes_ptr, dtype, actions_ptr, policy_ptr, counts_ptr=None, value_ptr=None,
+                              q_ptr=None, index_ptr=None):
+        """xq_examples_sample_compact_device: sample_device's rows with compact actions int32 [batch][128] and policy f32 [batch][128]"""
+        check(self._L.xq_examples_sample_compact_device(self._h, int(batch), int(seed), int(counter), view, planes_ptr, dtype, actions_ptr,
+                                                        policy_ptr, counts_ptr, value_ptr, q_ptr, index_ptr))
 
     def info(self):
         """synchronous: dict of size, capacity, total_committed, pending, dropped, stale"""

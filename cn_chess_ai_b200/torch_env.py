@@ -4,14 +4,15 @@ all on the device (include/xq.h: xq_env_observe_device, xq_env_legal_mask_device
 Every call runs on torch.cuda.current_stream(device), allocates its outputs with torch and hands their data_ptr() to the library:
 nothing goes through host memory.  Actions are policy indices from * 90 + to (8,100 of them, the reference network's output width);
 with view="side" an env with Black to move is seen rotated by 180 degrees with the colours swapped, so that a network always plays
-"up the board" with its own pieces in channels 0..6.
+"up the board" with its own pieces in channels 0..6.  A network that scores only the legal actions uses compact rows instead:
+legal_actions() lists each board's actions (entry k = list entry k, 128 wide) and step_compact() takes scores in that order.
 """
 from collections import namedtuple
 
 import torch
 
-from ._lib import (DTYPE_BF16, DTYPE_F32, DTYPE_U8, MASK_WORDS, PICK_GIVEN, PICK_GREEDY, PICK_SAMPLE, POLICY_ACTIONS, VIEW_ABSOLUTE,
-                   VIEW_SIDE_TO_MOVE)
+from ._lib import (COMPACT_ACTIONS, DTYPE_BF16, DTYPE_F32, DTYPE_U8, MASK_WORDS, PICK_GIVEN, PICK_GREEDY, PICK_SAMPLE, POLICY_ACTIONS,
+                   VIEW_ABSOLUTE, VIEW_SIDE_TO_MOVE)
 from .env import BatchedEnv
 
 StepResult = namedtuple("StepResult", "actions logp reward done winner captured valid")
@@ -74,15 +75,34 @@ class TorchEnv:
         self.env.legal_mask_device(mask.data_ptr(), packed, v)
         return mask
 
+    def legal_actions(self, view="side"):
+        """(actions int32 [n, 128], counts uint8 [n]): entry k of a row is the policy index (frame of `view`) of the env's k-th legal
+        action in reference list order, -1 past the count -- the order of a compact score row (step_compact, TorchSearch)"""
+        v = _view(view)
+        self._enter()
+        actions = torch.empty((self.n, COMPACT_ACTIONS), dtype=torch.int32, device=self.device)
+        counts = torch.empty(self.n, dtype=torch.uint8, device=self.device)
+        self.env.legal_actions_device(actions.data_ptr(), counts.data_ptr(), v)
+        return actions, counts
+
     def step(self, scores=None, actions=None, pick="sample", temperature=1.0, view="side", auto_reset=True):
         """one ply: scores [n, 8100] (f32 / bf16) in the view's frame and/or actions int64 [n] (pick="given").  Returns StepResult of
         tensors: actions int64 (policy indices, -1 = no legal action), logp f32 (NaN without scores), reward i32, done / winner / captured / valid uint8."""
+        return self._step(scores, actions, pick, temperature, view, auto_reset, False)
+
+    def step_compact(self, scores=None, actions=None, pick="sample", temperature=1.0, view="side", auto_reset=True):
+        """step() with compact scores [n, 128] (f32 / bf16): entry k scores the env's k-th legal action (legal_actions(view)).  actions
+        (given and returned) are policy indices in the frame of `view`, as in step(); the same StepResult, bit for bit step()'s with the
+        dense row holding the compact entries at their policy indices."""
+        return self._step(scores, actions, pick, temperature, view, auto_reset, True)
+
+    def _step(self, scores, actions, pick, temperature, view, auto_reset, compact):
         if pick not in _PICKS:
             raise ValueError(f"pick must be one of {sorted(_PICKS)}, not {pick!r}")
         p, v = _PICKS[pick], _view(view)
         sdt = DTYPE_F32
         if scores is not None:
-            self._check(scores, "scores", list(_SCORE_DTYPES), (self.n, POLICY_ACTIONS))
+            self._check(scores, "scores", list(_SCORE_DTYPES), (self.n, COMPACT_ACTIONS if compact else POLICY_ACTIONS))
             sdt = _SCORE_DTYPES[scores.dtype]
         if p == PICK_GIVEN:
             if actions is None:
@@ -96,6 +116,7 @@ class TorchEnv:
         logp = torch.empty(self.n, dtype=torch.float32, device=self.device)
         reward = torch.empty(self.n, dtype=torch.int32, device=self.device)
         done, winner, captured, valid = (torch.empty(self.n, dtype=torch.uint8, device=self.device) for _ in range(4))
-        self.env.policy_step_device(None if scores is None else scores.data_ptr(), sdt, p, temperature, v, auto_reset, actions.data_ptr(),
-                                    logp.data_ptr(), reward.data_ptr(), done.data_ptr(), winner.data_ptr(), captured.data_ptr(), valid.data_ptr())
+        call = self.env.policy_step_compact_device if compact else self.env.policy_step_device
+        call(None if scores is None else scores.data_ptr(), sdt, p, temperature, v, auto_reset, actions.data_ptr(), logp.data_ptr(),
+             reward.data_ptr(), done.data_ptr(), winner.data_ptr(), captured.data_ptr(), valid.data_ptr())
         return StepResult(actions, logp, reward, done, winner, captured, valid)

@@ -9,11 +9,12 @@ from collections import namedtuple
 
 import torch
 
-from ._lib import MASK_WORDS, POLICY_ACTIONS
+from ._lib import COMPACT_ACTIONS, MASK_WORDS, POLICY_ACTIONS
 from .env import BatchedExamples
 from .torch_env import _OBS_DTYPES, _view
 
 Sample = namedtuple("Sample", "planes policy value q mask index")
+CompactSample = namedtuple("CompactSample", "planes actions policy counts value q index")
 
 # xq_env_rec piece codes of the Generals (StepResult.captured)
 RED_GENERAL, BLACK_GENERAL = 1, 8
@@ -84,19 +85,33 @@ class TorchExamples:
         self.tenv._enter()
         self.examples.discard_device(None if m is None else m.data_ptr())
 
-    def sample(self, batch, seed, counter, view="side", dtype=torch.bfloat16, want_mask=False):
+    def sample(self, batch, seed, counter, view="side", dtype=torch.bfloat16, want_mask=False, compact=False):
         """Sample of tensors: planes [batch, 14, 10, 9] (dtype), policy f32 [batch, 8100] (visit fractions in the frame of `view`),
         value f32 [batch] (z), q f32 [batch], mask int32 [batch, 254] of packed legal-mask words (want_mask) or None, index int64 [batch]
-        (ring slots, -1 while the ring is empty).  Slot i = (xq_rng(seed, i, counter) >> 1) % size."""
+        (ring slots, -1 while the ring is empty).  Slot i = (xq_rng(seed, i, counter) >> 1) % size.
+        compact=True: the same rows as a CompactSample -- planes, actions int32 [batch, 128] (the root's edges as policy indices in the
+        frame of `view`, list order, -1 past them), policy f32 [batch, 128] (the visit fraction of edge k), counts uint8 [batch] (edges),
+        value, q, index."""
         if dtype not in _OBS_DTYPES:
             raise ValueError(f"dtype must be one of {list(_OBS_DTYPES)}")
         v = _view(view)
         batch = int(batch)
         if batch <= 0:
             raise ValueError(f"batch must be > 0, not {batch}")
+        if compact and want_mask:
+            raise ValueError("want_mask is for the dense policy row: a compact sample lists the actions instead")
         self.tenv._enter()
         dev = self.device
         planes = torch.empty((batch, 14, 10, 9), dtype=dtype, device=dev)
+        if compact:
+            actions = torch.empty((batch, COMPACT_ACTIONS), dtype=torch.int32, device=dev)
+            policy = torch.empty((batch, COMPACT_ACTIONS), dtype=torch.float32, device=dev)
+            counts = torch.empty(batch, dtype=torch.uint8, device=dev)
+            value, q = (torch.empty(batch, dtype=torch.float32, device=dev) for _ in range(2))
+            index = torch.empty(batch, dtype=torch.int64, device=dev)
+            self.examples.sample_compact_device(batch, seed, counter, v, planes.data_ptr(), _OBS_DTYPES[dtype], actions.data_ptr(),
+                                                policy.data_ptr(), counts.data_ptr(), value.data_ptr(), q.data_ptr(), index.data_ptr())
+            return CompactSample(planes, actions, policy, counts, value, q, index)
         policy = torch.empty((batch, POLICY_ACTIONS), dtype=torch.float32, device=dev)
         value, q = (torch.empty(batch, dtype=torch.float32, device=dev) for _ in range(2))
         mask = torch.empty((batch, MASK_WORDS), dtype=torch.int32, device=dev) if want_mask else None

@@ -4,13 +4,14 @@
 Each simulation selects one leaf per tree (or, with select_leaves, several per tree with virtual loss), observes all leaves at once, calls
 the network once on them and hands its scores and values back; selection, child creation, expansion and backup run in the library's
 kernels on torch's current stream.  Actions and visit counts
-use the policy indices from * 90 + to of TorchEnv, in the frame of `view`.
+use the policy indices from * 90 + to of TorchEnv, in the frame of `view`.  With compact=True the network scores each leaf's legal actions
+only: it receives the leaves' action lists (leaf_actions) and returns scores [rows, 128] in list order, entry k = edge k.
 """
 from collections import namedtuple
 
 import torch
 
-from ._lib import POLICY_ACTIONS, SEARCH_MAX_EDGES
+from ._lib import COMPACT_ACTIONS, POLICY_ACTIONS, SEARCH_MAX_EDGES
 from .env import BatchedGumbel, BatchedSearch
 from .torch_env import _OBS_DTYPES, _SCORE_DTYPES, StepResult, _view
 
@@ -102,6 +103,24 @@ class TorchSearch:
         self.search.observe_leaves_device(planes.data_ptr(), _OBS_DTYPES[dtype], v, aux.data_ptr())
         return planes, aux
 
+    def leaf_actions(self, view="side"):
+        """(actions int32 [rows, 128], counts uint8 [rows]): each leaf record's legal actions as TorchEnv.legal_actions lists them,
+        rows as in leaves() (duplicate and terminal slots included) -- entry k is the leaf's edge k after expansion"""
+        v = _view(view)
+        self.tenv._enter()
+        actions = torch.empty((self._rows, COMPACT_ACTIONS), dtype=torch.int32, device=self.device)
+        counts = torch.empty(self._rows, dtype=torch.uint8, device=self.device)
+        self.search.leaf_actions_device(actions.data_ptr(), counts.data_ptr(), v)
+        return actions, counts
+
+    def expand_backup_compact(self, scores, values, temperature=1.0):
+        """expand_backup() with compact scores [rows, 128] (f32 / bf16): entry k is the prior logit of the leaf's edge k (leaf_actions()).
+        Root noise comes from root_noise(), not from a dense row."""
+        self.tenv._check(scores, "scores", list(_SCORE_DTYPES), (self._rows, COMPACT_ACTIONS))
+        self.tenv._check(values, "values", [torch.float32], (self._rows,))
+        self.tenv._enter()
+        self.search.expand_backup_compact_device(scores.data_ptr(), _SCORE_DTYPES[scores.dtype], temperature, values.data_ptr())
+
     def expand_backup(self, scores, values, temperature=1.0, root_noise=None, noise_eps=0.25, view="side"):
         """scores [rows, 8100] (f32 / bf16, frame of `view`) expand the leaves that need evaluation; values f32 [rows] (from each leaf's
         side to move) are backed up for every leaf but duplicates (rows as in leaves()).  root_noise f32 [n, 8100]: mixed into the
@@ -171,14 +190,18 @@ class TorchSearch:
 
     def run(self, evaluate, n_simulations, c_puct=1.5, fpu=0.0, temperature=1.0, root_noise=None, noise_eps=0.25, view="side",
             obs_dtype=torch.bfloat16, cap_value=0.0, reset=True, dirichlet_alpha=None, dirichlet_eps=0.25, noise_seed=0, leaves=1,
-            virtual_loss=1.0):
+            virtual_loss=1.0, compact=False):
         """reset + n_simulations simulations: evaluate(planes) -> (scores [rows, 8100], values [rows]) is called once per selection on
         its leaves; at terminal leaves outcome_values replaces the network's value.  reset=False continues from the current trees (after
         advance(), or to add simulations to this move's search).  dirichlet_alpha: root_noise(dirichlet_alpha, dirichlet_eps, noise_seed)
         once per root and move -- before the first simulation on the roots the last advance() kept, after it on the roots reset() or
         advance() rebuilt (expanded by the first simulation).  leaves > 1: after the first simulation (one leaf per tree, which expands
         rebuilt roots) the rest go in select_leaves(leaves, virtual_loss=virtual_loss) calls, the last one smaller, so evaluate sees
-        n * leaves planes; n_simulations counts the selected slots.  Returns root(view)."""
+        n * leaves planes; n_simulations counts the selected slots.  compact=True: evaluate(planes, actions) receives the leaves' action
+        lists (leaf_actions(view)) and returns (scores [rows, 128], values), and the move uses compact calls only; root_noise is refused
+        there (dirichlet_alpha works as above).  Returns root(view)."""
+        if compact and root_noise is not None:
+            raise ValueError("root_noise is a dense [n, 8100] row: with compact=True use dirichlet_alpha")
         if reset:
             self.reset()
         kept = None if self._kept is None else self._kept > 0
@@ -190,19 +213,22 @@ class TorchSearch:
                 self.root_noise(dirichlet_alpha, dirichlet_eps, noise_seed, mask=None if kept is None else ~kept)
             k = 1 if i == 0 else min(leaves, n_simulations - i)
             sel = self.select(c_puct, fpu) if k == 1 else self.select_leaves(k, c_puct, fpu, virtual_loss)
-            self._simulate(sel, evaluate, temperature, root_noise, noise_eps, view, obs_dtype, cap_value)
+            self._simulate(sel, evaluate, temperature, root_noise, noise_eps, view, obs_dtype, cap_value, compact)
             i += k
         return self.root(view)
 
-    def _simulate(self, sel, evaluate, temperature, root_noise, noise_eps, view, obs_dtype, cap_value):
+    def _simulate(self, sel, evaluate, temperature, root_noise, noise_eps, view, obs_dtype, cap_value, compact):
         """the rest of a simulation after the selection `sel`: its leaves observed and evaluated once, outcome_values at terminal leaves,
-        expand_backup"""
+        expand_backup (expand_backup_compact with the leaves' action lists given to evaluate when compact)"""
         status, winner = sel.status.reshape(-1), sel.winner.reshape(-1)
         planes, aux = self.observe(obs_dtype, view)
-        scores, values = evaluate(planes)
+        scores, values = evaluate(planes, self.leaf_actions(view)[0]) if compact else evaluate(planes)
         values = values.reshape(self._rows).to(torch.float32).contiguous()
         values = torch.where(status != NEEDS_EVALUATION, self.outcome_values(status, winner, aux, cap_value), values)
-        self.expand_backup(scores.contiguous(), values, temperature, root_noise, noise_eps, view)
+        if compact:
+            self.expand_backup_compact(scores.contiguous(), values, temperature)
+        else:
+            self.expand_backup(scores.contiguous(), values, temperature, root_noise, noise_eps, view)
 
 
 GumbelRootResult = namedtuple("GumbelRootResult", "policy action")
@@ -237,6 +263,15 @@ class TorchGumbel:
         self.gumbel.begin_device(scores.data_ptr(), _SCORE_DTYPES[scores.dtype], temperature, v, values.data_ptr(), n_simulations, seed,
                                  c_visit, c_scale)
 
+    def begin_compact(self, scores, values, n_simulations, seed=0, temperature=1.0, c_visit=50.0, c_scale=0.1):
+        """begin() with compact root scores [n, 128] (f32 / bf16): entry k scores the env's k-th legal action (TorchEnv.legal_actions),
+        which is root edge k"""
+        self.tenv._check(scores, "scores", list(_SCORE_DTYPES), (self.n, COMPACT_ACTIONS))
+        self.tenv._check(values, "values", [torch.float32], (self.n,))
+        self.tenv._enter()
+        self.gumbel.begin_compact_device(scores.data_ptr(), _SCORE_DTYPES[scores.dtype], temperature, values.data_ptr(), n_simulations, seed,
+                                         c_visit, c_scale)
+
     def select(self, leaves=1, c_puct=1.5, fpu=0.0, virtual_loss=1.0):
         """TorchSearch.select_leaves with the Gumbel root rule: SelectResult of tensors [n, leaves]; the search's leaves(), observe() and
         expand_backup() follow as after select_leaves"""
@@ -266,20 +301,24 @@ class TorchGumbel:
         return res
 
     def run(self, evaluate, n_simulations, seed=0, c_puct=1.5, fpu=0.0, temperature=1.0, c_visit=50.0, c_scale=0.1, view="side",
-            obs_dtype=torch.bfloat16, cap_value=0.0, leaves=1, virtual_loss=1.0, reset=True):
+            obs_dtype=torch.bfloat16, cap_value=0.0, leaves=1, virtual_loss=1.0, reset=True, compact=False):
         """one move's Gumbel search: reset() (reset=False: continue from advance()), evaluate(planes) -> (scores, values) once on the env
         boards (TorchEnv.observe) for begin(), then n_simulations selections in select(leaves) calls, the last one smaller, each
-        evaluated once with outcome_values at terminal leaves as TorchSearch.run does.  Returns root(view)."""
+        evaluated once with outcome_values at terminal leaves as TorchSearch.run does.  compact=True: evaluate(planes, actions) gets the
+        boards' action lists and returns compact scores, as in TorchSearch.run(compact=True).  Returns root(view)."""
         ts = self.tsearch
         if reset:
             ts.reset()
         planes, _ = self.tenv.observe(obs_dtype, view)
-        scores, values = evaluate(planes)
-        self.begin(scores.contiguous(), values.reshape(self.n).to(torch.float32).contiguous(), n_simulations, seed, temperature, c_visit,
-                   c_scale, view)
+        scores, values = evaluate(planes, self.tenv.legal_actions(view)[0]) if compact else evaluate(planes)
+        values = values.reshape(self.n).to(torch.float32).contiguous()
+        if compact:
+            self.begin_compact(scores.contiguous(), values, n_simulations, seed, temperature, c_visit, c_scale)
+        else:
+            self.begin(scores.contiguous(), values, n_simulations, seed, temperature, c_visit, c_scale, view)
         i = 0
         while i < n_simulations:
             k = min(leaves, n_simulations - i)
-            ts._simulate(self.select(k, c_puct, fpu, virtual_loss), evaluate, temperature, None, 0.0, view, obs_dtype, cap_value)
+            ts._simulate(self.select(k, c_puct, fpu, virtual_loss), evaluate, temperature, None, 0.0, view, obs_dtype, cap_value, compact)
             i += k
         return self.root(view)

@@ -176,6 +176,13 @@ enum { XQ_VIEW_ABSOLUTE = 0, XQ_VIEW_SIDE_TO_MOVE = 1 };
 enum { XQ_PICK_GREEDY = 0, XQ_PICK_SAMPLE = 1, XQ_PICK_GIVEN = 2 };
 #define XQ_POLICY_ACTIONS 8100            /* policy index = from*90 + to, in the frame of `view` */
 #define XQ_MASK_WORDS 254                 /* packed mask: ceil(8100/32) uint32 per env, bits >= 8100 zero */
+/* Compact rows.  Entry k of a compact row belongs to the board's k-th legal action in reference list order (xq_env_legal_moves; a
+ * search node's edge k): the first XQ_COMPACT_ACTIONS actions, which is every legal action of every board of the reference's play.
+ * Compact rows are row-major with a stride of XQ_COMPACT_ACTIONS entries; entries k >= the count are never read (any value, NaN
+ * included).  A network that scores only the listed actions gets each board's list from xq_env_legal_actions_device /
+ * xq_search_leaf_actions_device; the compact readers are bit for bit their dense counterparts given any dense row D whose entry at
+ * actions[k] equals the compact entry k. */
+#define XQ_COMPACT_ACTIONS 128
 
 /* Observation: planes_dev[n][14][10][9] of 0/1 in f32, bf16 or u8 (dtype).  Absolute view: channel code-1 holds the reference's
  * one-hot, planes[e][ch][s] == getStateRepresentation[s*14 + ch] (src/chessai.cpp:268-289).  aux_dev[n][4] int32 = player, move_count,
@@ -205,6 +212,15 @@ int xq_env_legal_mask_device(xq_env_t h, void* mask_dev, int packed, int view);
 int xq_env_policy_step_device(xq_env_t h, const void* scores_dev, int scores_dtype, int pick, float temperature, int view,
                               int auto_reset, int64_t* actions_dev, float* logp_dev, int32_t* reward_dev, uint8_t* done_dev,
                               uint8_t* winner_dev, uint8_t* captured_dev, uint8_t* valid_dev);
+/* The compact list of every env: actions_dev int32 [n][XQ_COMPACT_ACTIONS] (16-byte aligned, required), entry k = the policy index in the
+ * frame of `view` of list entry k, -1 past the count; counts_dev u8 [n] or NULL: min(count, XQ_COMPACT_ACTIONS).  Asynchronous. */
+int xq_env_legal_actions_device(xq_env_t h, int view, int32_t* actions_dev, uint8_t* counts_dev);
+/* xq_env_policy_step_device with compact scores: scores_dev [n][XQ_COMPACT_ACTIONS] f32 / bf16, 16-byte aligned, entry k = the score of
+ * list entry k.  Everything else is that call's: the arguments, the cleaning, GREEDY / SAMPLE / GIVEN, logp, the draw; actions_dev holds
+ * int64 policy indices in the frame of `view` (given and returned).  The choice is among the first XQ_COMPACT_ACTIONS actions. */
+int xq_env_policy_step_compact_device(xq_env_t h, const void* scores_dev, int scores_dtype, int pick, float temperature, int view,
+                                      int auto_reset, int64_t* actions_dev, float* logp_dev, int32_t* reward_dev, uint8_t* done_dev,
+                                      uint8_t* winner_dev, uint8_t* captured_dev, uint8_t* valid_dev);
 
 /* ---- device-resident batched tree search (PUCT / MCTS) for an external policy/value network ----
  * One tree per env of an env handle; each simulation selects one leaf per tree, the caller evaluates all leaves with ONE network call
@@ -326,6 +342,13 @@ int xq_search_observe_leaves_device(xq_search_t s, void* planes_dev, int dtype, 
  * [n * L][8100] and values [n * L], duplicate slots neither expanded nor backed up */
 int xq_search_expand_backup_device(xq_search_t s, const void* scores_dev, int scores_dtype, float temperature, int view,
                                    const float* values_dev, const float* root_noise_dev, float noise_eps);
+/* Compact rows for the search.  xq_search_leaf_actions_device: the compact list of each of the n * L leaf records of the last selection
+ * (row t * L + k, duplicate and terminal slots included), layout and view of xq_env_legal_actions_device; allowed whenever
+ * observe_leaves is.  xq_search_expand_backup_compact_device: xq_search_expand_backup_device with scores_dev [n * L][XQ_COMPACT_ACTIONS]
+ * (f32 / bf16, 16-byte aligned), entry k = the prior logit of edge k; no view is needed and no dense root noise is taken (the library's
+ * noise, xq_search_root_noise_device, applies to compact callers as to dense ones).  Call order, budget and errors are the dense call's. */
+int xq_search_leaf_actions_device(xq_search_t s, int view, int32_t* actions_dev, uint8_t* counts_dev);
+int xq_search_expand_backup_compact_device(xq_search_t s, const void* scores_dev, int scores_dtype, float temperature, const float* values_dev);
 /* per root (any output may be NULL): visits_dev int32 [n][8100] (16-byte aligned) = the root edges' N at their policy indices in the frame
  * of `view`, 0 elsewhere; q_dev f32 [n] = sum W / sum N over the root's edges (sums in list order; NaN when no edge was visited); best_dev
  * int64 [n] = policy index (frame of `view`) of the most-visited root edge, first in list order on ties, -1 when no edge was visited --
@@ -413,6 +436,10 @@ int xq_gumbel_bytes(int64_t n_trees, int max_simulations, int64_t* bytes);
  * allowed after a reset / advance when no selection is pending. */
 int xq_gumbel_begin_device(xq_gumbel_t g, const void* scores_dev, int scores_dtype, float temperature, int view, const float* root_value_dev,
                            int n_simulations, uint64_t seed, float c_visit, float c_scale);
+/* xq_gumbel_begin_device with compact root scores [n][XQ_COMPACT_ACTIONS] (f32 / bf16, 16-byte aligned; entry k = root edge k, the
+ * compact list of xq_env_legal_actions_device for the env's board); the same checks and results */
+int xq_gumbel_begin_compact_device(xq_gumbel_t g, const void* scores_dev, int scores_dtype, float temperature, const float* root_value_dev,
+                                   int n_simulations, uint64_t seed, float c_visit, float c_scale);
 /* xq_search_select_leaves_device (leaves 1 .. max_leaves, the same outputs and checks) with the Gumbel root rule; spends `leaves` of the
  * search's budget and of n_simulations */
 int xq_gumbel_select_device(xq_gumbel_t g, int leaves, float c_puct, float fpu, float virtual_loss, uint8_t* status_dev, uint8_t* winner_dev,
@@ -496,6 +523,16 @@ int xq_examples_discard_device(xq_examples_t b, const uint8_t* mask_dev);
  * slots; these four may be NULL.  An empty ring gives index -1, zero planes, policy and mask, NaN value and q. */
 int xq_examples_sample_device(xq_examples_t b, int64_t batch, uint64_t seed, uint32_t counter, int view, void* planes_dev, int dtype,
                               float* policy_dev, float* value_dev, float* q_dev, uint32_t* mask_dev, int64_t* index_dev);
+/* The same rows as xq_examples_sample_device with the same (seed, counter) -- index, planes, value and q -- with a compact policy target:
+ * actions_dev int32 [batch][XQ_COMPACT_ACTIONS] (required, 16-byte aligned) = the stored action[k] in the frame of `view`, -1 past
+ * n_edges (the root's edges: the record's compact list, so the search's scoring head scores these rows); policy_dev f32
+ * [batch][XQ_COMPACT_ACTIONS] (required, 16-byte aligned) = visits[k] / total_visits as in the dense row, 0 past n_edges and in the whole
+ * row when total_visits is 0; counts_dev u8 [batch] = n_edges.  An empty ring gives index -1, count 0, actions -1, zero planes and
+ * policy, NaN value and q.  planes_dev (dtype, view and alignment as in xq_examples_sample_device), counts, value, q and index may be
+ * NULL. */
+int xq_examples_sample_compact_device(xq_examples_t b, int64_t batch, uint64_t seed, uint32_t counter, int view, void* planes_dev,
+                                      int dtype, int32_t* actions_dev, float* policy_dev, uint8_t* counts_dev, float* value_dev,
+                                      float* q_dev, int64_t* index_dev);
 /* synchronous: size = committed examples held (<= capacity), total_committed since create, pending = staged examples, dropped / stale
  * counted since create; any pointer may be NULL */
 int xq_examples_info(xq_examples_t b, int64_t* size, int64_t* capacity, int64_t* total_committed, int64_t* pending, int64_t* dropped,
