@@ -134,6 +134,9 @@ def lib():
     L.xq_examples_sample_compact_device.argtypes = [_P, C.c_int64, C.c_uint64, C.c_uint32, C.c_int, _P, C.c_int] + [_P] * 6
     L.xq_examples_info.argtypes = [_P] + [C.POINTER(C.c_int64)] * 6
     L.xq_examples_get.argtypes = [_P, C.c_int64, C.c_int64, _P]
+    L.xq_examples_load_device.argtypes = [_P, _P, _P]
+    L.xq_examples_refresh_device.argtypes = [_P, _P, _P, _P]
+    L.xq_examples_refresh_gumbel_device.argtypes = [_P, _P, _P, _P]
     _lib = L
     return L
 

@@ -51,6 +51,11 @@ int search_roots(xq_search_t s, xq_env_t env, const char* fn, SearchRoots* out);
 // xq_examples_record_gumbel_device: the call checks of a begun Gumbel search on env `env`, its roots, and the improved-policy weights of
 // every root ([n][128], edge k at t * 128 + k) launched on the env's stream
 int gumbel_weights(xq_gumbel_t g, xq_env_t env, SearchRoots* roots, const uint32_t** w);
+// the same two for a reader of a search on any env handle of `device` (XQ_ERR_INVALID on another device), with the same call-order
+// checks; the weights are launched on `stream`, the reader's
+int search_roots_on(xq_search_t s, int device, const char* fn, SearchRoots* out);
+int gumbel_weights_on(xq_gumbel_t g, int device, cudaStream_t stream, const char* fn, SearchRoots* roots, const uint32_t** w);
+void env_boards_injected(xq_env_t h);      // boards were written from outside the env's own calls (xq_env_set_boards' after-effect)
 
 // ---- host helpers of the C ABI -----------------------------------------------------------------
 inline unsigned grid_of(int64_t n, int per_block) { return (unsigned)((n + per_block - 1) / per_block); }

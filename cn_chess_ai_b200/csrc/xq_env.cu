@@ -392,6 +392,7 @@ int env_info(xq_env_t h, EnvInfo* out) {
     return XQ_OK;
 }
 void env_advance_event_ply(xq_env_t h, uint32_t plies) { if (h) h->event_ply += plies; }
+void env_boards_injected(xq_env_t h) { h->maybe_nonstd = true; }
 void** env_scratch_slot(xq_env_t h, void (*free_fn)(void*)) { h->sp_scratch_free = free_fn; return &h->sp_scratch; }
 }  // namespace xq
 

@@ -6,8 +6,13 @@
 // example p at e * max_game_examples + p), per env the staged count, the game count and two commit scratch words, and the counters
 // (total committed, dropped, stale, and the base / count of the last commit).  The ring head is total % capacity.
 // examples_record_kernel: one warp per tree, as search_root_kernel reads a root: the lanes compare the root record with the env's, read the
-//   root's act / N / W rows coalesced, sum q in list order with s_add / s_div exactly as search_root_kernel, build the example in shared
-//   memory and store it with 16-byte stores.
+//   root's act / N / W rows coalesced, sum q in list order with s_add / s_div exactly as search_root_kernel (ex_root_targets), build the
+//   example in shared memory and store it with 16-byte stores.
+// examples_load_kernel (reanalyse): 4 threads per row, one 16-byte word of the slot's record each, onto the env.
+// examples_claim_kernel / examples_refresh_kernel (reanalyse): one thread per row takes its slot's claim word with atomicMin (the smallest
+//   row wins); then one warp per tree checks the row's status, builds the root's targets with ex_root_targets and writes only n_edges, q,
+//   total_visits, action[] and visits[] of the slot.  The claim words (one uint32 per ring slot, all-ones between calls) are allocated at
+//   the first refresh, beside the sampling scratch.
 // examples_scan_kernel: one CTA; each thread sums the counts of a contiguous segment of envs, the segment sums are scanned across the CTA
 //   (warp shuffles, then the 32 warp totals), and each thread writes the commit numbers of its envs in env order (ex_commit_offsets).
 // examples_commit_kernel: persistent warps over the commit numbers in contiguous chunks; a warp finds the env of its first number by
@@ -51,28 +56,15 @@ struct ExDev {
     ExCounters* ctr;
 };
 
-// WEIGHTS: the visits field takes the Gumbel improved-policy weights wts[t * 128 + k] instead of N (xq_examples_record_gumbel_device)
+// what ex_root_targets gives every lane: n_edges, total_visits (the sum of visits[]) and q
+struct RootTargets { int ne; uint32_t tot; float q; };
+// Step 2 of the record and refresh kernels, one warp: root g's edges read coalesced into x.action and x.visits (N, or with WEIGHTS the
+// Gumbel weights wts[t * 128 + k]), -1 / 0 past n_edges, and q = sum W / sum N in list order with s_add / s_div exactly as
+// search_root_kernel sums it.  The caller's lane 0 stores n_edges, total_visits and q (with the rest of the header in the record kernel).
 template <bool WEIGHTS>
-__global__ void __launch_bounds__(32 * kRecWarps) examples_record_kernel(ExDev b, SearchRoots r, const xq_env_rec* __restrict__ envs,
-                                                                        const uint8_t* __restrict__ mask, uint64_t env_id0,
-                                                                        const uint32_t* __restrict__ wts) {
-    __shared__ __align__(16) xq_example s_ex[kRecWarps];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t t = (int64_t)blockIdx.x * kRecWarps + warp;
-    if (t >= b.n || (mask && !mask[t])) return;
-    const int64_t g = t * r.cap, eb = g * kSearchEdges;
-    xq_example& x = s_ex[warp];
-    // 1. the root is the env's current board, all 64 bytes
-    if (root_stale_warp(r.rec + g, envs + t, lane, reinterpret_cast<uint4*>(&x.rec))) {
-        if (lane == 0) atomicAdd(&b.ctr->stale, 1ull);
-        return;
-    }
-    const uint32_t slot = b.staged[t];
-    if (slot >= (uint32_t)b.maxg) {
-        if (lane == 0) atomicAdd(&b.ctr->dropped, 1ull);
-        return;
-    }
-    // 2. the edges, coalesced; q summed in list order as search_root_kernel sums it
+__device__ __forceinline__ RootTargets ex_root_targets(const SearchRoots& r, int64_t g, const uint32_t* __restrict__ wts, int64_t t, int lane,
+                                                    xq_example& x) {
+    const int64_t eb = g * kSearchEdges;
     const int ne = r.expanded[g] ? r.nedges[g] : 0;
     float w[kSearchEdges / 32];
     uint32_t tot = 0, sn = 0;           // sum of visits[], and sum of N for q (the same sum unless WEIGHTS)
@@ -100,9 +92,35 @@ __global__ void __launch_bounds__(32 * kRecWarps) examples_record_kernel(ExDev b
             if (32 * i + j < ne) sw = s_add(sw, v);
         }
     }
+    return RootTargets{ne, tot, qn > 0 ? s_div(sw, (float)(int)qn) : NAN};
+}
+
+// WEIGHTS: the visits field takes the Gumbel improved-policy weights wts[t * 128 + k] instead of N (xq_examples_record_gumbel_device)
+template <bool WEIGHTS>
+__global__ void __launch_bounds__(32 * kRecWarps) examples_record_kernel(ExDev b, SearchRoots r, const xq_env_rec* __restrict__ envs,
+                                                                        const uint8_t* __restrict__ mask, uint64_t env_id0,
+                                                                        const uint32_t* __restrict__ wts) {
+    __shared__ __align__(16) xq_example s_ex[kRecWarps];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t t = (int64_t)blockIdx.x * kRecWarps + warp;
+    if (t >= b.n || (mask && !mask[t])) return;
+    const int64_t g = t * r.cap;
+    xq_example& x = s_ex[warp];
+    // 1. the root is the env's current board, all 64 bytes
+    if (root_stale_warp(r.rec + g, envs + t, lane, reinterpret_cast<uint4*>(&x.rec))) {
+        if (lane == 0) atomicAdd(&b.ctr->stale, 1ull);
+        return;
+    }
+    const uint32_t slot = b.staged[t];
+    if (slot >= (uint32_t)b.maxg) {
+        if (lane == 0) atomicAdd(&b.ctr->dropped, 1ull);
+        return;
+    }
+    // 2. the edges
+    const RootTargets rt = ex_root_targets<WEIGHTS>(r, g, wts, t, lane, x);
     if (lane == 0) {
-        x.env = env_id0 + (uint64_t)t; x.game = 0; x.ply = (uint16_t)slot; x.n_edges = (uint8_t)ne; x.reserved0 = 0;
-        x.z = 0.f; x.q = qn > 0 ? s_div(sw, (float)(int)qn) : NAN; x.total_visits = tot; x.reserved1 = 0;
+        x.env = env_id0 + (uint64_t)t; x.game = 0; x.ply = (uint16_t)slot; x.n_edges = (uint8_t)rt.ne; x.reserved0 = 0;
+        x.z = 0.f; x.q = rt.q; x.total_visits = rt.tot; x.reserved1 = 0;
         b.staged[t] = slot + 1;
     }
     __syncwarp();
@@ -110,6 +128,62 @@ __global__ void __launch_bounds__(32 * kRecWarps) examples_record_kernel(ExDev b
     uint4* dst = reinterpret_cast<uint4*>(b.staging + t * b.maxg + slot);
     const uint4* src = reinterpret_cast<const uint4*>(&x);
     for (int c = lane; c < kExampleVecs; c += 32) dst[c] = src[c];
+}
+
+// Reanalyse.  examples_load_kernel: 4 threads per env, each copies one 16-byte word of its slot's record onto the env.
+constexpr int kLoadThreads = 256;
+__global__ void __launch_bounds__(kLoadThreads) examples_load_kernel(ExDev b, int64_t m, const int64_t* __restrict__ index,
+                                                                      xq_env_rec* __restrict__ envs) {
+    const int64_t i = (int64_t)blockIdx.x * kLoadThreads + threadIdx.x, e = i >> 2;
+    if (e >= m) return;
+    const int64_t total = (int64_t)b.ctr->total, size = total < b.capacity ? total : b.capacity;
+    const int64_t idx = index[e];
+    if (!ex_slot_held(idx, size)) return;
+    reinterpret_cast<uint4*>(envs + e)[i & 3] = reinterpret_cast<const uint4*>(&b.ring[idx].rec)[i & 3];
+}
+
+// examples_claim_kernel: each row of a refresh claims its slot's word with its row number; the smallest row holds it afterwards
+__global__ void __launch_bounds__(256) examples_claim_kernel(ExDev b, int64_t m, const int64_t* __restrict__ index, uint32_t* __restrict__ claim) {
+    const int64_t t = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (t >= m) return;
+    const int64_t total = (int64_t)b.ctr->total, size = total < b.capacity ? total : b.capacity;
+    const int64_t idx = index[t];
+    if (ex_slot_held(idx, size)) atomicMin(claim + idx, (uint32_t)t);
+}
+
+// examples_refresh_kernel: one warp per tree, as examples_record_kernel: the status checks of ex_refresh_status (the root compared with the
+// slot's record, the edges built by ex_root_targets in shared memory), then for a REFRESHED row n_edges, q and total_visits with narrow
+// stores and action / visits (16-byte words 6 .. 53) with 16-byte stores.  The winner of a slot restores its claim word: a row that lost it
+// reads the winner's row or kNoClaim, never its own.
+template <bool WEIGHTS>
+__global__ void __launch_bounds__(32 * kRecWarps) examples_refresh_kernel(ExDev b, SearchRoots r, const int64_t* __restrict__ index,
+                                                                         uint32_t* __restrict__ claim, const uint32_t* __restrict__ wts,
+                                                                         uint8_t* __restrict__ status) {
+    __shared__ __align__(16) xq_example s_ex[kRecWarps];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t t = (int64_t)blockIdx.x * kRecWarps + warp;
+    if (t >= r.n) return;
+    const int64_t total = (int64_t)b.ctr->total, size = total < b.capacity ? total : b.capacity;
+    const int64_t idx = index[t], g = t * r.cap;
+    const bool held = ex_slot_held(idx, size);
+    const uint32_t c = __shfl_sync(0xFFFFFFFFu, lane == 0 && held ? claim[idx] : kNoClaim, 0);
+    xq_example& x = s_ex[warp];
+    bool stale = false;
+    RootTargets rt{0, 0u, 0.f};
+    if (held && c == (uint32_t)t) {
+        stale = root_stale_warp(r.rec + g, &b.ring[idx].rec, lane);
+        if (!stale) rt = ex_root_targets<WEIGHTS>(r, g, wts, t, lane, x);
+        if (lane == 0) claim[idx] = kNoClaim;
+    }
+    const uint8_t st = ex_refresh_status(idx, size, c, (uint32_t)t, stale, rt.tot);
+    if (lane == 0 && status) status[t] = st;
+    if (st != XQ_REFRESHED) return;
+    __syncwarp();
+    xq_example* dst = b.ring + idx;
+    if (lane == 0) { dst->n_edges = (uint8_t)rt.ne; dst->q = rt.q; dst->total_visits = rt.tot; }
+    constexpr int kFirst = offsetof(xq_example, action) / 16;
+    const uint4* src = reinterpret_cast<const uint4*>(&x);
+    for (int v = kFirst + lane; v < kExampleVecs; v += 32) reinterpret_cast<uint4*>(dst)[v] = src[v];
 }
 
 __global__ void __launch_bounds__(kScanThreads) examples_scan_kernel(ExDev b, const uint8_t* __restrict__ ended) {
@@ -270,6 +344,7 @@ struct xq_examples_s {
     void* slab = nullptr;
     ExDev d{};
     xq_env_rec* recs = nullptr; int64_t recs_cap = 0;     // sampling scratch, grown as needed
+    uint32_t* claim = nullptr;                            // reanalyse: one claim word per ring slot (kNoClaim between calls), made at the first refresh
 };
 
 namespace {
@@ -348,6 +423,7 @@ int xq_examples_destroy(xq_examples_t b) {
     cudaSetDevice(b->device);
     cudaFree(b->slab);             // synchronises with the work still queued on the env's stream
     cudaFree(b->recs);
+    cudaFree(b->claim);
     delete b;
     return XQ_OK;
 }
@@ -447,6 +523,64 @@ int xq_examples_sample_compact_device(xq_examples_t b, int64_t batch, uint64_t s
     XQ_LAUNCH_CHECK();
     if (planes_dev) XQ_CUDA(launch_observe(b->recs, batch, planes_dev, dtype, view, nullptr, E.stream));
     return XQ_OK;
+}
+
+int xq_examples_load_device(xq_examples_t b, xq_env_t env, const int64_t* index_dev) {
+    EnvInfo E, T;
+    if (int rc = enter(b, &E, "xq_examples_load_device")) return rc;
+    if (!env) return fail(XQ_ERR_INVALID, "xq_examples_load_device: null env");
+    if (int rc = env_info(env, &T)) return rc;
+    if (T.device != E.device) return fail(XQ_ERR_INVALID, "xq_examples_load_device: the env is on device %d, the buffer on %d", T.device, E.device);
+    if (!index_dev) return fail(XQ_ERR_INVALID, "xq_examples_load_device: index is required");
+    examples_load_kernel<<<grid_of(4 * T.n, kLoadThreads), kLoadThreads, 0, T.stream>>>(b->d, T.n, index_dev, T.d_envs);
+    XQ_LAUNCH_CHECK();
+    env_boards_injected(env);
+    return XQ_OK;
+}
+
+}  // extern "C"
+
+namespace {
+// the claim kernel and the refresh kernel of m = r.n rows on the buffer's env stream; the claim words are made at the first call
+template <bool WEIGHTS>
+int refresh(xq_examples_t b, cudaStream_t stream, const SearchRoots& r, const uint32_t* w, const int64_t* index, uint8_t* status) {
+    if (!b->claim) {
+        XQ_CUDA(cudaMalloc(&b->claim, sizeof(uint32_t) * (size_t)b->d.capacity));
+        const cudaError_t e = cudaMemsetAsync(b->claim, 0xFF, sizeof(uint32_t) * (size_t)b->d.capacity, stream);
+        if (e != cudaSuccess) {
+            cudaFree(b->claim); b->claim = nullptr;
+            return fail(XQ_ERR_CUDA, "reanalyse claim words: %s", cudaGetErrorString(e));
+        }
+    }
+    examples_claim_kernel<<<grid_of(r.n, 256), 256, 0, stream>>>(b->d, r.n, index, b->claim);
+    XQ_LAUNCH_CHECK();
+    examples_refresh_kernel<WEIGHTS><<<grid_of(r.n, kRecWarps), 32 * kRecWarps, 0, stream>>>(b->d, r, index, b->claim, w, status);
+    XQ_LAUNCH_CHECK();
+    return XQ_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int xq_examples_refresh_device(xq_examples_t b, xq_search_t s, const int64_t* index_dev, uint8_t* status_dev) {
+    EnvInfo E;
+    if (int rc = enter(b, &E, "xq_examples_refresh_device")) return rc;
+    if (!s) return fail(XQ_ERR_INVALID, "xq_examples_refresh_device: null search");
+    if (!index_dev) return fail(XQ_ERR_INVALID, "xq_examples_refresh_device: index is required");
+    SearchRoots r;
+    if (int rc = search_roots_on(s, E.device, "xq_examples_refresh_device", &r)) return rc;
+    return refresh<false>(b, E.stream, r, nullptr, index_dev, status_dev);
+}
+
+int xq_examples_refresh_gumbel_device(xq_examples_t b, xq_gumbel_t g, const int64_t* index_dev, uint8_t* status_dev) {
+    EnvInfo E;
+    if (int rc = enter(b, &E, "xq_examples_refresh_gumbel_device")) return rc;
+    if (!g) return fail(XQ_ERR_INVALID, "xq_examples_refresh_gumbel_device: null Gumbel state");
+    if (!index_dev) return fail(XQ_ERR_INVALID, "xq_examples_refresh_gumbel_device: index is required");
+    SearchRoots r;
+    const uint32_t* w = nullptr;
+    if (int rc = gumbel_weights_on(g, E.device, E.stream, "xq_examples_refresh_gumbel_device", &r, &w)) return rc;
+    return refresh<true>(b, E.stream, r, w, index_dev, status_dev);
 }
 
 int xq_examples_info(xq_examples_t b, int64_t* size, int64_t* capacity, int64_t* total_committed, int64_t* pending, int64_t* dropped,

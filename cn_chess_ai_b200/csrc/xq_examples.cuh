@@ -1,6 +1,6 @@
 // xq_examples.cuh -- host-compilable helpers of the self-play example buffer (xq_examples.cu; include/xq.h: xq_examples_*): the game
-// result and its sign per example, the policy target of one edge, the view of a stored action, the sample-index draw, and the commit
-// offsets of the ended envs' staged examples.
+// result and its sign per example, the policy target of one edge, the view of a stored action, the sample-index draw, the commit
+// offsets of the ended envs' staged examples, and the status rule of a reanalyse refresh.
 //
 // tests/hostsim/examples_shim.cpp compiles this header with -ffp-contract=off so that numpy restates every value bit for bit.
 #pragma once
@@ -60,6 +60,35 @@ XQ_HD int64_t ex_find_env(const int64_t* off, int64_t n, int64_t pos) {
         if (off[mid] <= pos) lo = mid + 1; else hi = mid;
     }
     return lo - 1;
+}
+
+// ---- reanalyse (xq_examples_refresh_device) ----
+constexpr uint32_t kNoClaim = 0xFFFFFFFFu;      // a slot's claim word outside a refresh call
+// whether ring slot idx holds a committed example (size = committed examples held)
+XQ_HD bool ex_slot_held(int64_t idx, int64_t size) { return idx >= 0 && idx < size; }
+// the status of row t, which refreshes slot idx: claim = the slot's claim word once every row of the call has claimed it (the smallest
+// row whose index is idx), stale = the slot's record differs from the root's, total = the root's visits (or weights) summed.  The checks
+// run in this order: NO_SLOT, DUPLICATE, STALE, UNSEARCHED; a row that passes all of them is REFRESHED (include/xq.h: XQ_REFRESH*).
+XQ_HD uint8_t ex_refresh_status(int64_t idx, int64_t size, uint32_t claim, uint32_t t, bool stale, uint32_t total) {
+    if (!ex_slot_held(idx, size)) return XQ_REFRESH_NO_SLOT;
+    if (claim != t) return XQ_REFRESH_DUPLICATE;
+    if (stale) return XQ_REFRESH_STALE;
+    return total ? XQ_REFRESHED : XQ_REFRESH_UNSEARCHED;
+}
+
+// host restatement of the claim and refresh kernels for the CPU suite: every row claims its slot with the smallest row (atomicMin over
+// claim[], kNoClaim on entry), each row takes its status, and the winner of a slot restores its claim word
+inline void ex_refresh_statuses(int64_t m, const int64_t* index, int64_t size, const uint8_t* stale, const uint32_t* total, uint32_t* claim,
+                                uint8_t* status) {
+    for (int64_t t = 0; t < m; ++t)
+        if (ex_slot_held(index[t], size) && (uint32_t)t < claim[index[t]]) claim[index[t]] = (uint32_t)t;
+    for (int64_t t = 0; t < m; ++t) {
+        const int64_t idx = index[t];
+        const bool held = ex_slot_held(idx, size);
+        const uint32_t c = held ? claim[idx] : kNoClaim;
+        status[t] = ex_refresh_status(idx, size, c, (uint32_t)t, stale[t] != 0, total[t]);
+        if (held && c == (uint32_t)t) claim[idx] = kNoClaim;
+    }
 }
 
 }  // namespace xq

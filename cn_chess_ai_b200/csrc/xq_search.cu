@@ -1074,6 +1074,12 @@ static int select_leaves(xq_search_t s, int leaves, float c_puct, float fpu, flo
 int xq::search_roots(xq_search_t s, xq_env_t env, const char* fn, SearchRoots* out) {
     if (!s) return fail(XQ_ERR_INVALID, "null search handle");
     if (s->env != env) return fail(XQ_ERR_INVALID, "%s: the search is on another env handle", fn);
+    return search_roots_on(s, s->device, fn, out);
+}
+
+int xq::search_roots_on(xq_search_t s, int device, const char* fn, SearchRoots* out) {
+    if (!s) return fail(XQ_ERR_INVALID, "%s: null search handle", fn);
+    if (s->device != device) return fail(XQ_ERR_INVALID, "%s: the search is on device %d, not %d", fn, s->device, device);
     if (int rc = check_phase(s, fn, kReady)) return rc;
     const SearchDev& d = s->d;
     *out = SearchRoots{d.n, d.cap, d.rec, d.nedges, d.expanded, d.N, d.W, d.act};
@@ -1393,12 +1399,19 @@ int gumbel_ready(xq_gumbel_t g, EnvInfo* E, const char* fn) {
 }  // namespace
 
 int xq::gumbel_weights(xq_gumbel_t g, xq_env_t env, SearchRoots* roots, const uint32_t** w) {
+    const char* fn = "xq_examples_record_gumbel_device";
+    if (!g) return fail(XQ_ERR_INVALID, "%s: null Gumbel state", fn);
+    if (g->s->env != env) return fail(XQ_ERR_INVALID, "%s: the search is on another env handle", fn);
     EnvInfo E;
-    if (!g) return fail(XQ_ERR_INVALID, "xq_examples_record_gumbel_device: null Gumbel state");
-    if (g->s->env != env) return fail(XQ_ERR_INVALID, "xq_examples_record_gumbel_device: the search is on another env handle");
-    if (int rc = gumbel_ready(g, &E, "xq_examples_record_gumbel_device")) return rc;
-    if (int rc = search_roots(g->s, env, "xq_examples_record_gumbel_device", roots)) return rc;
-    gumbel_weights_kernel<<<grid_of(g->s->d.n, kGumbelWarps), 32 * kGumbelWarps, 0, E.stream>>>(g->s->d, g->G);
+    if (int rc = env_info(env, &E)) return rc;
+    return gumbel_weights_on(g, E.device, E.stream, fn, roots, w);
+}
+
+int xq::gumbel_weights_on(xq_gumbel_t g, int device, cudaStream_t stream, const char* fn, SearchRoots* roots, const uint32_t** w) {
+    EnvInfo E;
+    if (int rc = gumbel_ready(g, &E, fn)) return rc;
+    if (int rc = search_roots_on(g->s, device, fn, roots)) return rc;
+    gumbel_weights_kernel<<<grid_of(g->s->d.n, kGumbelWarps), 32 * kGumbelWarps, 0, stream>>>(g->s->d, g->G);
     XQ_LAUNCH_CHECK();
     *w = g->G.w;
     return XQ_OK;

@@ -385,6 +385,20 @@ class BatchedExamples:
         check(self._L.xq_examples_sample_compact_device(self._h, int(batch), int(seed), int(counter), view, planes_ptr, dtype, actions_ptr,
                                                         policy_ptr, counts_ptr, value_ptr, q_ptr, index_ptr))
 
+    def load_device(self, env, index_ptr):
+        """xq_examples_load_device: env e of `env` (a BatchedEnv on the same device) gets the record of ring slot index[e] (int64 [env.n]);
+        rows outside the committed examples leave their board"""
+        check(self._L.xq_examples_load_device(self._h, env.handle, index_ptr))
+
+    def refresh_device(self, search, index_ptr, status_ptr=None):
+        """xq_examples_refresh_device: tree t of `search` (a BatchedSearch on any env of the device) rewrites the targets and q of ring slot
+        index[t] (int64 [search.n]); status u8 [search.n] or None"""
+        check(self._L.xq_examples_refresh_device(self._h, search._h, index_ptr, status_ptr))
+
+    def refresh_gumbel_device(self, gumbel, index_ptr, status_ptr=None):
+        """xq_examples_refresh_gumbel_device: refresh_device with the improved-policy weights of `gumbel` (a begun BatchedGumbel)"""
+        check(self._L.xq_examples_refresh_gumbel_device(self._h, gumbel._h, index_ptr, status_ptr))
+
     def info(self):
         """synchronous: dict of size, capacity, total_committed, pending, dropped, stale"""
         v = [C.c_int64() for _ in range(6)]

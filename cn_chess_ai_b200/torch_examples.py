@@ -3,7 +3,8 @@
 Each move, record(search) stores one example per env from its search tree's root: the position and the root edges' visit counts in
 sparse form.  When games end, finish(step) (or end_games) stamps each stored position of those games with the result from its side to
 move and commits them to a ring.  sample() draws a training batch -- observation planes, the visit-count policy target, the value
-target z, the root q and the packed legal mask -- with no host synchronisation.  Calls run on torch's current stream.
+target z, the root q and the packed legal mask -- with no host synchronisation.  reanalyse() searches stored positions again with the
+current network and rewrites their policy targets and q in place (load, a search, refresh).  Calls run on torch's current stream.
 """
 from collections import namedtuple
 
@@ -18,6 +19,11 @@ CompactSample = namedtuple("CompactSample", "planes actions policy counts value 
 
 # xq_env_rec piece codes of the Generals (StepResult.captured)
 RED_GENERAL, BLACK_GENERAL = 1, 8
+
+# status of a refreshed row (include/xq.h: XQ_REFRESH*), checked in this order: the slot is rewritten; the index is < 0 or >= len(); a
+# smaller row has the same index (only the smallest writes); the slot's record is no longer the root's (the ring wrapped over it); the
+# root has no edge with a visit or a weight
+REFRESHED, NO_SLOT, DUPLICATE, STALE, UNSEARCHED = 0, 1, 2, 3, 4
 
 
 class TorchExamples:
@@ -119,6 +125,43 @@ class TorchExamples:
         self.examples.sample_device(batch, seed, counter, v, planes.data_ptr(), _OBS_DTYPES[dtype], policy.data_ptr(), value.data_ptr(),
                                     q.data_ptr(), None if mask is None else mask.data_ptr(), index.data_ptr())
         return Sample(planes, policy, value, q, mask, index)
+
+    def load(self, tenv, index):
+        """env e of `tenv` (any TorchEnv on the buffer's device) gets the record of ring slot index[e] (int64 [tenv.n], e.g. sample().index
+        or a torch.arange sweep), all 64 bytes, so that a search reset on tenv has exactly the stored position as its root.  Rows with
+        an index < 0 or >= len() keep their board.  As after tenv.env.set_boards, staged examples of a buffer on tenv are stale."""
+        tenv._check(index, "index", [torch.int64], (tenv.n,))
+        self.tenv._enter()
+        tenv._enter()
+        self.examples.load_device(tenv.env, index.data_ptr())
+
+    def refresh(self, search, index):
+        """tree t of `search` (a TorchSearch on any TorchEnv of the device, after its simulations) rewrites n_edges, action, visits,
+        total_visits and q of ring slot index[t] (int64 [search.n]) as record() would store them from that tree; rec, env, game, ply and z
+        stay.  Returns the status uint8 [search.n] of each row (REFRESHED .. UNSEARCHED)."""
+        return self._refresh(search.tenv, search.n, index, lambda i, st: self.examples.refresh_device(search.search, i, st))
+
+    def refresh_gumbel(self, gumbel, index):
+        """refresh() after a Gumbel search (a begun TorchGumbel): visits are the weights of record_gumbel()"""
+        return self._refresh(gumbel.tenv, gumbel.n, index, lambda i, st: self.examples.refresh_gumbel_device(gumbel.gumbel, i, st))
+
+    def _refresh(self, tenv, n, index, call):
+        tenv._check(index, "index", [torch.int64], (n,))
+        status = torch.empty(n, dtype=torch.uint8, device=self.device)
+        self.tenv._enter()
+        tenv._enter()
+        call(index.data_ptr(), status.data_ptr())
+        return status
+
+    def reanalyse(self, runner, evaluate, index, n_simulations, **run_kwargs):
+        """Reanalyse: search the positions of ring slots index (int64 [runner.n]) again with `evaluate` and rewrite their policy targets
+        and q.  load(runner.tenv, index), then runner.run(evaluate, n_simulations, reset=True, **run_kwargs) (a TorchSearch or a
+        TorchGumbel; compact=True and leaves=L pass through; no Dirichlet noise unless run_kwargs ask for it), then refresh() (or
+        refresh_gumbel()).  Returns the statuses."""
+        from .torch_search import TorchGumbel
+        self.load(runner.tenv, index)
+        runner.run(evaluate, n_simulations, reset=True, **run_kwargs)
+        return self.refresh_gumbel(runner, index) if isinstance(runner, TorchGumbel) else self.refresh(runner, index)
 
     def info(self):
         """synchronous: dict of size, capacity, total_committed, pending (staged examples), dropped, stale"""

@@ -473,7 +473,9 @@ int xq_gumbel_get(xq_gumbel_t g, int64_t tree, float* gumbel_host, float* logit_
  * board stays): the caller ends such a game through xq_examples_end_games_device itself.  After xq_env_reset / xq_env_set_boards the
  * staged examples of the replaced games are stale: discard them (xq_examples_discard_device).
  * Memory (xq_examples_bytes): (capacity + n_envs x max_game_examples) x 864 bytes, plus 20 bytes per env of counters and commit scratch
- * and under 1.6 KB of global counters and alignment; sampling adds a scratch of 64 bytes per batch row that grows with the largest batch. */
+ * and under 1.6 KB of global counters and alignment; sampling adds a scratch of 64 bytes per batch row that grows with the largest batch,
+ * and the first xq_examples_refresh_device (or _gumbel_) adds the claim words of reanalyse: 4 bytes per ring slot, all-ones between
+ * calls.  Neither is part of xq_examples_bytes. */
 typedef struct xq_examples_s* xq_examples_t;
 typedef struct {
     xq_env_rec rec;          /* the searched position: the tree's root record when it was recorded */
@@ -533,6 +535,35 @@ int xq_examples_sample_device(xq_examples_t b, int64_t batch, uint64_t seed, uin
 int xq_examples_sample_compact_device(xq_examples_t b, int64_t batch, uint64_t seed, uint32_t counter, int view, void* planes_dev,
                                       int dtype, int32_t* actions_dev, float* policy_dev, uint8_t* counts_dev, float* value_dev,
                                       float* q_dev, int64_t* index_dev);
+/* Reanalyse (MuZero Reanalyse; EfficientZero, Gumbel MuZero): search stored positions again with the current network and overwrite their
+ * policy targets and q in place.  xq_examples_load_device puts ring slots on an env, a search of that env runs as in self-play
+ * (xq_search_reset, then the simulations), and xq_examples_refresh_device (or _gumbel_) writes each tree's root back into its slot.
+ *
+ * env: any env handle on the buffer's device (XQ_ERR_INVALID otherwise), m envs.  Env e gets the record of ring slot index_dev[e] (int64
+ * [m], required), all 64 bytes, ply counter included, so a search reset on `env` has exactly the stored position as its root.  A row whose
+ * index is < 0 or >= size (committed examples held, read on the device in stream order) leaves its env's board unchanged.  Asynchronous
+ * on env's stream (it writes env); the same after-effects as xq_env_set_boards: the boards count as injected, and staged examples of a
+ * buffer on env are stale (discard them). */
+int xq_examples_load_device(xq_examples_t b, xq_env_t env, const int64_t* index_dev);
+/* statuses of a refreshed row, checked in this order */
+enum {
+    XQ_REFRESHED = 0,            /* the slot's targets were rewritten */
+    XQ_REFRESH_NO_SLOT = 1,      /* index < 0 or >= size: nothing written */
+    XQ_REFRESH_DUPLICATE = 2,    /* a smaller row has the same index: only the smallest row writes (duplicates from a sample are deterministic) */
+    XQ_REFRESH_STALE = 3,        /* the slot's 64-byte record differs from the root's (the ring wrapped over it after the load) */
+    XQ_REFRESH_UNSEARCHED = 4    /* the root has no edge with a visit (or a weight) */
+};
+/* Tree t of search s (a search on any env handle of the buffer's device, m trees; reset and no selection pending, XQ_ERR_STATE otherwise,
+ * as xq_examples_record_device) refreshes ring slot index_dev[t] (int64 [m], required); status_dev (u8 [m], may be NULL) = the row's
+ * status.  Only a REFRESHED row writes, and only n_edges, action[], visits[], total_visits and q, each bit for bit what
+ * xq_examples_record_device would store from the same tree; rec, env, game, ply, z and the reserved words stay.  Asynchronous on the
+ * buffer's env stream (the _gumbel_ call launches its weights kernel there too): when the search's env stream is another one, the caller
+ * orders the search's work before the call and its next calls after it (TorchExamples puts both handles on torch's current stream).
+ * The duplicate rule uses one uint32 claim word per ring slot, allocated at the first refresh (see the memory note above). */
+int xq_examples_refresh_device(xq_examples_t b, xq_search_t s, const int64_t* index_dev, uint8_t* status_dev);
+/* xq_examples_refresh_device for the search of a begun Gumbel state (XQ_ERR_STATE otherwise): visits[k] and total_visits take the 2^24
+ * weights of xq_examples_record_gumbel_device, UNSEARCHED is a root without edges */
+int xq_examples_refresh_gumbel_device(xq_examples_t b, xq_gumbel_t g, const int64_t* index_dev, uint8_t* status_dev);
 /* synchronous: size = committed examples held (<= capacity), total_committed since create, pending = staged examples, dropped / stale
  * counted since create; any pointer may be NULL */
 int xq_examples_info(xq_examples_t b, int64_t* size, int64_t* capacity, int64_t* total_committed, int64_t* pending, int64_t* dropped,
