@@ -184,3 +184,67 @@ class GumbelTree(SL.LeavesTree):
         k = action(cons, nv, sc)
         return pol, (int(idx[k]) if k >= 0 else -1), p
 
+
+
+def improved_policy64(N, W, P, logit, vhat, c_visit, c_scale):
+    """(pi' in float64, a per-entry bound on |pi'_f32 - pi'_64|) of one root from its edges' N, W, P, the stored logits and the root
+    value.  The float64 restatement is completed_q / sigma / improved_policy without rounding; the bound follows their f32 operation
+    order with u = 2^-24 per rounding:
+      q_k = W_k / N_k: u |q_k|;  v_mix: the two list-order sums over the n_v visited edges, the products and the four outer operations,
+        (2 n_v + 8) u A with A = (|vhat| + sum N * sum(p |q|) / sum p) / (sum N + 1) >= |v_mix|;
+      e_q = the largest q error (it moves min and max by at most e_q); the span D = max - min by 2 e_q + 2 u D, the floor max(D, 1e-8)
+        by as much (max is 1-Lipschitz);  (q - min) / floor: (dq_k + e_q + 2 u |q - min|) / floor_lo + qh dD / floor_lo + 2 u qh;
+      sigma = ((c_visit + max N) * c_scale) * qh: C dqh + 3 u C qh;  z = logit + sigma: + 2 u |z|;
+      exp(z - max z): the argument off by dz_k + max dz + 2 u |z - max z|, expf within 2 ulp (5 u);  the list-order sum S within the
+        largest term error + (n + 2) u;  the division: u.  pi_f32 / pi_64 lies in [(1 - r)(1 - u) / (1 + r_S), (1 + r)(1 + u) / (1 - r_S)].
+    Terms below the f32 underflow are covered by an absolute 2^-126."""
+    u = 2.0 ** -24
+    N = np.asarray(N, np.int64)
+    W, P = np.asarray(W, F32).astype(np.float64), np.asarray(P, F32).astype(np.float64)
+    logit = np.asarray(logit, F32).astype(np.float64)
+    vhat = float(F32(vhat))
+    c_visit, c_scale = float(F32(c_visit)), float(F32(c_scale))
+    n = len(N)
+    vis = N > 0
+    nv, sn = int(vis.sum()), int(N.sum())
+    qv = W[vis] / N[vis]
+    p = np.maximum(P[vis], float(FLT_MIN))
+    if sn > 0:
+        vm = (vhat + sn * ((p * qv).sum() / p.sum())) / (sn + 1)
+        A = (abs(vhat) + sn * (p * np.abs(qv)).sum() / p.sum()) / (sn + 1)
+        dvm = (2 * nv + 8) * u * A
+    else:
+        vm, dvm = vhat, 0.0
+    q = np.full(n, vm)
+    q[vis] = qv
+    dq = np.full(n, dvm)
+    dq[vis] = u * np.abs(qv)
+    eq = dq.max()
+    mn, mx = q.min(), q.max()
+    floor = float(F32(1e-8))
+    den = max(mx - mn, floor)
+    dD = 2 * eq + 2 * u * (mx - mn)
+    den_lo = max(den - dD, floor)
+    a = q - mn
+    qh = a / den
+    dqh = (dq + eq + 2 * u * np.abs(a) + qh * dD) / den_lo + 2 * u * qh
+    C = (c_visit + float(N.max())) * c_scale
+    sig = C * qh
+    dsig = C * dqh + 3 * u * C * qh
+    z = logit + sig
+    fin = np.isfinite(z)
+    pi = np.zeros(n)
+    bound = np.zeros(n)
+    if not fin.any():
+        return pi, bound
+    dz = np.where(fin, dsig + 2 * u * np.abs(np.where(fin, z, 0.0)), 0.0)
+    zm = z[fin].max()
+    e = np.where(fin, np.exp(np.where(fin, z - zm, -np.inf)), 0.0)
+    pi = e / e.sum()
+    arg = dz + dz[fin].max() + 2 * u * np.abs(np.where(fin, z - zm, 0.0))
+    with np.errstate(over="ignore", invalid="ignore"):
+        r = np.expm1(arg) + 5 * u
+        rs = r[fin].max() + (n + 2) * u
+        rel = np.where(np.isfinite(r) & (rs < 1), (1 + r) * (1 + u) / (1 - min(rs, 0.5)) - 1, np.inf)
+    bound = np.where(fin, pi * rel * (1 + 1e-6) + 2.0 ** -126, 0.0)
+    return pi, bound

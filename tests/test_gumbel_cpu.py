@@ -209,3 +209,39 @@ def test_sequential_halving_counts():
                 assert nv[k] == t
                 nv[k] += 1
             assert nv.sum() == n
+
+
+def test_improved_policy64_bounds_the_f32_mirror():
+    """improved_policy64's bound holds for the f32 mirror (sigma / improved_policy) on 1 .. 128 edges: random visits and values, every
+    q equal, spans of 1e-8 (the floor), priors spread over e^-110, and a sharp float64 check: the bound is at most a few per cent of
+    pi' at ordinary roots"""
+    rng = np.random.default_rng(0)
+    F32 = np.float32
+    worst = 0.0
+    for t in range(1500):
+        n = int(rng.integers(1, 129))
+        N = rng.integers(0, 5, n) * (rng.random(n) < 0.5)
+        kind = t % 4
+        W = (N * rng.uniform(-1, 1, n)).astype(F32)
+        vh = F32(rng.uniform(-1, 1))
+        if kind == 1:
+            W, vh = (-0.5 * N).astype(F32), F32(-0.5)
+        if kind == 2:
+            W = (N * rng.integers(0, 2, n) * F32(1e-8)).astype(F32)
+        P = rng.dirichlet(np.ones(n)).astype(F32)
+        if kind == 3:
+            x = rng.uniform(-110, 0, n)
+            P = np.exp(x - x.max()).astype(F32)
+            P = (P / P.sum()).astype(F32)
+        with np.errstate(divide="ignore"):
+            lg = np.log(P).astype(F32)
+        p32, _ = G.improved_policy((lg + G.sigma(N, W, P, vh, 50.0, 0.1)).astype(F32))
+        pi, b = G.improved_policy64(N, W, P, lg, vh, 50.0, 0.1)
+        err = np.abs(p32.astype(np.float64) - pi)
+        assert (err <= b).all(), t
+        if kind == 0 and N.sum() > 0:
+            assert (b <= 0.05 * pi + 2.0 ** -126).all(), t
+        live = b > 0
+        if live.any():
+            worst = max(worst, float((err[live] / b[live]).max()))
+    assert 0 < worst < 1
